@@ -6,6 +6,9 @@ secondaries) on N B200s of one node.
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...      # CPU arm: C++ restatement of the reference algorithm
+    python bench.py ... --dump-outputs DIR    # also save what the last timed step returned, to compare two builds
+
+The inputs are made from fixed seeds, so two runs with the same arguments time the same signatures.
 
 One "step" = one verify_batch pass over this rank's shard (2^21 signatures per GPU, i.e. BASELINE
 config 4's 2^24 signatures over 8 GPUs; 10 % corrupted).  The batch shards with no exchange between
@@ -264,6 +267,20 @@ def corrupt(cols, seed, denom=10):
     return expected, cls
 
 
+DUMP_BUDGET = 64 << 20                                     # bytes over all ranks' --dump-outputs files
+
+
+def dump_outputs(out_dir, name, arr, rank, world):
+    """writes arr as float32 to out_dir/<name>[_rank<r>].npy; when the ranks' files together would exceed DUMP_BUDGET, a
+    sample of lanes drawn with a fixed seed (sorted, the same for every run with the same lane count) stands in for all"""
+    cap = (DUMP_BUDGET // world - 4096) // 4
+    if len(arr) > cap:
+        arr = arr[np.sort(np.random.default_rng(0).choice(len(arr), size=cap, replace=False))]
+    os.makedirs(out_dir, exist_ok=True)
+    fname = "%s_rank%d.npy" % (name, rank) if world > 1 else name + ".npy"
+    np.save(os.path.join(out_dir, fname), np.asarray(arr, dtype=np.float32))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -276,7 +293,14 @@ def main():
                     help="1 lane in this many is corrupted (default 10 = the 10 %% of config 4; 0 = none, for diagnosis)")
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="CPU work budget for the cpu_baseline leg")
     ap.add_argument("--log2-total", type=int, default=24, help="config 4 / 5 total batch of the single-caller and config legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the accept bits of the last timed verify_batch step to DIR/verify_ok[_rank<r>].npy (float32; a fixed "
+                         "sample of the lanes when all ranks together would exceed %d MiB)" % (DUMP_BUDGET >> 20))
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the GPU arm computed; it does not apply to --impl reference")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -512,6 +536,8 @@ def run_ours(args, rank, local_rank, world):
     clocks = sampler.finish()
     check(lib.bjj_sync(ctx), "sync")
     ok_h = ok_d.cpu().numpy()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, "verify_ok", ok_h, rank, world)
     mism = int((ok_h != expected).sum())
     dev_ms = max_over_ranks(dev_ms)
     value = world * n * args.steps / (dev_ms * 1e-3)

@@ -25,6 +25,27 @@ def test_reference_arm_json_line():
     assert d["gpu_launches"] == 0 and "workload" in d["config"]
 
 
+def test_dump_outputs_full_and_sampled(tmp_path):
+    """--dump-outputs writes float32 .npy files; an output too large for the budget is replaced by the same seeded sample
+    on every run"""
+    import importlib.util
+    import numpy as np
+    spec = importlib.util.spec_from_file_location("bench_mod", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    ok = (np.arange(1000) % 3 == 0).astype(np.uint8)
+    bench.dump_outputs(str(tmp_path / "a"), "verify_ok", ok, 0, 1)
+    got = np.load(tmp_path / "a" / "verify_ok.npy")
+    assert got.dtype == np.float32 and np.array_equal(got, ok)
+    big = np.arange(bench.DUMP_BUDGET // 16, dtype=np.uint32) % 2
+    for d in ("b", "c"):
+        bench.dump_outputs(str(tmp_path / d), "verify_ok", big, 3, 8)
+    a, b = np.load(tmp_path / "b" / "verify_ok_rank3.npy"), np.load(tmp_path / "c" / "verify_ok_rank3.npy")
+    assert 8 * a.nbytes <= bench.DUMP_BUDGET and len(a) < len(big) and np.array_equal(a, b)
+    p = _run(["--impl", "reference", "--dump-outputs", str(tmp_path / "r")], timeout=120)
+    assert p.returncode != 0 and not (tmp_path / "r").exists()
+
+
 def test_gpu_arm_refuses_to_run_without_a_device():
     p = _run(["--steps", "1", "--warmup", "1"], timeout=300)
     assert p.returncode != 0
