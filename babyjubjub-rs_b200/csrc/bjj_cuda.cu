@@ -158,11 +158,6 @@ struct PipeSlot {
     bool drain_pending;
     size_t drain_off, drain_lanes;
 };
-// what a launch runs on
-struct ComputeRef {
-    cudaStream_t stream;
-    Workspace& ws;
-};
 
 struct bjj_ctx {
     int device;
@@ -192,14 +187,18 @@ struct bjj_ctx {
         }                                  \
     } while (0)
 
-static int grid_for(bjj_ctx* ctx, const void* kernel, size_t n) {
-    int per_sm = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, BJJ_BLOCK, 0) != cudaSuccess || per_sm < 1)
-        per_sm = 1;
-    size_t want = (n + BJJ_BLOCK - 1) / BJJ_BLOCK;
-    size_t cap = (size_t)ctx->sms * per_sm;
-    if (want < 1) want = 1;
-    return (int)(want < cap ? want : cap);
+// propagates a nonzero BJJ_ERR_* code
+#define TRY(call)                \
+    do {                         \
+        int rc_ = (call);        \
+        if (rc_) return rc_;     \
+    } while (0)
+
+// counts `count` kernel launches (bjj_kernel_launches) and reports a failed launch among them
+static int launched(bjj_ctx* ctx, int count = 1) {
+    ctx->launches += count;
+    CU(ctx, cudaGetLastError());
+    return BJJ_OK;
 }
 
 static int grid_cap(bjj_ctx* ctx, int per_sm, size_t n) {
@@ -209,29 +208,53 @@ static int grid_cap(bjj_ctx* ctx, int per_sm, size_t n) {
     return (int)(want < cap ? want : cap);
 }
 
-static int ensure_table(bjj_ctx* ctx, Workspace* ws, size_t slots) {
-    if (ws->table_slots >= slots) return BJJ_OK;
-    if (ws->table) cudaFree(ws->table);
-    ws->table = nullptr;
-    ws->table_slots = 0;
-    CU(ctx, cudaMalloc(&ws->table, slots * BJJ_TABLE_U128_PER_LANE * sizeof(U128)));
-    ws->table_slots = slots;
+template <class Kernel>
+static int grid_for(bjj_ctx* ctx, Kernel* kernel, size_t n) {
+    return grid_cap(ctx, bjjk::blocks_per_sm(kernel), n);
+}
+
+// Grow-only scratch: afterwards *buf holds at least `want` units of `unit` bytes.  It is reallocated, contents lost,
+// only when it held fewer; the old buffer is freed first so that the two never coexist.  `pinned`: page-locked host
+// memory instead of device memory.
+template <class T>
+static int grow(bjj_ctx* ctx, T** buf, size_t* cap, size_t want, size_t unit, bool pinned = false) {
+    if (*cap >= want) return BJJ_OK;
+    if (*buf) pinned ? cudaFreeHost(*buf) : cudaFree(*buf);
+    *buf = nullptr;
+    *cap = 0;
+    CU(ctx, pinned ? cudaHostAlloc(buf, want * unit, cudaHostAllocDefault) : cudaMalloc(buf, want * unit));
+    *cap = want;
     return BJJ_OK;
 }
 
-// makes room for two queues of n lane indices each and zeroes both counters on `st`
-static int ensure_queue(bjj_ctx* ctx, Workspace* ws, size_t n, cudaStream_t st, ExactQueue* q, ExactQueue* q2 = nullptr) {
+// sub-batch size of the point kernels: bounds the projective scratch at 4 x 32 B x 2^21 = 256 MiB
+#define BJJ_POINT_SUBBATCH ((size_t)1 << 21)
+
+// Lanes that the lane-sized scratch of a workspace must hold for a call of n lanes: one sub-batch, and at least the
+// host flavour's largest chunk (lane_hint), so that a long host call allocates once up front.
+static size_t scratch_lanes(bjj_ctx* ctx, size_t n) {
+    const size_t lanes = n < BJJ_POINT_SUBBATCH ? n : BJJ_POINT_SUBBATCH;
+    return lanes < ctx->lane_hint ? ctx->lane_hint : lanes;
+}
+
+// f(off, m) on consecutive sub-batches [off, off + m) of at most BJJ_POINT_SUBBATCH lanes; stops at the first error
+template <class F>
+static int for_each_subbatch(size_t n, F f) {
+    for (size_t off = 0; off < n; off += BJJ_POINT_SUBBATCH)
+        TRY(f(off, n - off < BJJ_POINT_SUBBATCH ? n - off : BJJ_POINT_SUBBATCH));
+    return BJJ_OK;
+}
+
+static int ensure_table(bjj_ctx* ctx, Workspace* ws, size_t slots) {
+    return grow(ctx, &ws->table, &ws->table_slots, slots, BJJ_TABLE_U128_PER_LANE * sizeof(U128));
+}
+
+// makes room for two queues of `lanes` lane indices each and zeroes both counters on `st`
+static int ensure_queue(bjj_ctx* ctx, Workspace* ws, size_t lanes, cudaStream_t st, ExactQueue* q, ExactQueue* q2 = nullptr) {
     // 48 bytes: the two queue counters, then (at byte 16) the lane-claim counters of the verify kernels (hash, Straus)
     // and (at byte 32) the claim counter of the exact-lane kernels
     if (!ws->exact_count) CU(ctx, cudaMalloc(&ws->exact_count, 48));
-    if (n < ctx->lane_hint) n = ctx->lane_hint;
-    if (ws->exact_cap < n) {
-        if (ws->exact_list) cudaFree(ws->exact_list);
-        ws->exact_list = nullptr;
-        ws->exact_cap = 0;
-        CU(ctx, cudaMalloc(&ws->exact_list, 2 * n * sizeof(uint32_t)));
-        ws->exact_cap = n;
-    }
+    TRY(grow(ctx, &ws->exact_list, &ws->exact_cap, lanes, 2 * sizeof(uint32_t)));
     CU(ctx, cudaMemsetAsync(ws->exact_count, 0, 48, st));
     q->count = ws->exact_count;
     q->list = ws->exact_list;
@@ -255,18 +278,8 @@ static int claim_counter(bjj_ctx* ctx, Workspace* ws, cudaStream_t st, unsigned 
 
 static unsigned long long* work_counters(Workspace* ws) { return reinterpret_cast<unsigned long long*>(ws->exact_count + 4); }
 
-// sub-batch size of the point kernels: bounds the projective scratch at 4 x 32 B x 2^21 = 256 MiB
-#define BJJ_POINT_SUBBATCH ((size_t)1 << 21)
-
 static int ensure_proj(bjj_ctx* ctx, Workspace* ws, size_t lanes, ProjScratch* scr) {
-    if (lanes < ctx->lane_hint) lanes = ctx->lane_hint;
-    if (ws->proj_lanes < lanes) {
-        if (ws->proj) cudaFree(ws->proj);
-        ws->proj = nullptr;
-        ws->proj_lanes = 0;
-        CU(ctx, cudaMalloc(&ws->proj, lanes * 128));
-        ws->proj_lanes = lanes;
-    }
+    TRY(grow(ctx, &ws->proj, &ws->proj_lanes, lanes, 128));
     scr->x = ws->proj;
     scr->y = scr->x + 32 * ws->proj_lanes;
     scr->z = scr->y + 32 * ws->proj_lanes;
@@ -473,125 +486,117 @@ int bjj_sync(bjj_ctx* ctx) {
     if (n == 0) return BJJ_OK;                               \
     CU(ctx, cudaSetDevice(ctx->device));                     \
     cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
-#define DEV_EPILOGUE              \
-    ctx->launches++;              \
-    CU(ctx, cudaGetLastError()); \
-    return BJJ_OK;
 
-// `table`/`table_slots` select the per-thread window-table workspace (ctx-wide for _dev calls, per
-// pipeline slot for host calls).
+// One launch function per operation, shared by the _dev entry point and the host flavour's chunks.  `ws` is the
+// scratch of the launch: ctx-wide for _dev calls, per pipeline slot for host calls.
+static int launch_fr_op(bjj_ctx* ctx, size_t n, int op, const uint8_t* a, const uint8_t* b, uint8_t* out, cudaStream_t st) {
+    k_fr_op<<<grid_for(ctx, k_fr_op, n), BJJ_BLOCK, 0, st>>>(op, n, a, b, out, ctx->flags_dev);
+    return launched(ctx);
+}
+static int launch_split_scalars(bjj_ctx* ctx, size_t n, const uint8_t* h32, const uint8_t* s32, uint8_t* u32, uint8_t* v32,
+                                uint8_t* w32, cudaStream_t st) {
+    k_split_scalars<<<grid_for(ctx, k_split_scalars, n), BJJ_BLOCK, 0, st>>>(n, h32, s32, u32, v32, w32);
+    return launched(ctx);
+}
+static int launch_add(bjj_ctx* ctx, size_t n, const uint8_t* px, const uint8_t* py, const uint8_t* pz, const uint8_t* qx,
+                      const uint8_t* qy, const uint8_t* qz, uint8_t* rx, uint8_t* ry, uint8_t* rz, cudaStream_t st) {
+    k_add<<<grid_for(ctx, k_add, n), BJJ_BLOCK, 0, st>>>(n, px, py, pz, qx, qy, qz, rx, ry, rz, ctx->flags_dev);
+    return launched(ctx);
+}
+static int launch_affine(bjj_ctx* ctx, size_t n, const uint8_t* px, const uint8_t* py, const uint8_t* pz, uint8_t* rx,
+                         uint8_t* ry, cudaStream_t st) {
+    k_affine<<<grid_for(ctx, k_affine, n), BJJ_BLOCK, 0, st>>>(n, px, py, pz, rx, ry, ctx->flags_dev);
+    return launched(ctx);
+}
+static int launch_scalar_key(bjj_ctx* ctx, size_t n, const uint8_t* key32, uint8_t* scalar32, cudaStream_t st) {
+    k_scalar_key<<<grid_for(ctx, k_scalar_key, n), BJJ_BLOCK, 0, st>>>(n, key32, scalar32);
+    return launched(ctx);
+}
+static int launch_compress(bjj_ctx* ctx, size_t n, const uint8_t* px, const uint8_t* py, uint8_t* out32, cudaStream_t st) {
+    k_compress<<<grid_for(ctx, k_compress, n), BJJ_BLOCK, 0, st>>>(n, px, py, out32, ctx->flags_dev);
+    return launched(ctx);
+}
+
 // k_words = 8: plain 256-bit scalars.  Wider (multiples of 8 words): the on-curve lanes use the scalar reduced mod ORDER
 // (k_reduce_scalars), the off-curve lanes replay every bit of the wide scalar.
 static int launch_mul_scalar(bjj_ctx* ctx, size_t n, const uint8_t* px, const uint8_t* py, const uint8_t* k, int k_words,
                              uint8_t* rx, uint8_t* ry, cudaStream_t st, Workspace* ws) {
-    for (size_t off = 0; off < n; off += BJJ_POINT_SUBBATCH) {
-        const size_t m = (n - off) < BJJ_POINT_SUBBATCH ? (n - off) : BJJ_POINT_SUBBATCH;
+    const size_t lanes = scratch_lanes(ctx, n);
+    return for_each_subbatch(n, [&](size_t off, size_t m) -> int {
         const size_t o = 32 * off;
         const uint8_t* kw = k + (size_t)4 * k_words * off;
         int grid = grid_cap(ctx, bjjk::mul_scalar_blocks_per_sm(), m);
-        int rc = ensure_table(ctx, ws, (size_t)grid * BJJ_BLOCK);
-        if (rc) return rc;
+        TRY(ensure_table(ctx, ws, (size_t)grid * BJJ_BLOCK));
         ExactQueue q;
-        rc = ensure_queue(ctx, ws, m, st, &q);
-        if (rc) return rc;
+        TRY(ensure_queue(ctx, ws, lanes, st, &q));
         ProjScratch scr;
-        rc = ensure_proj(ctx, ws, m < BJJ_POINT_SUBBATCH && n > BJJ_POINT_SUBBATCH ? BJJ_POINT_SUBBATCH : m, &scr);
-        if (rc) return rc;
+        TRY(ensure_proj(ctx, ws, lanes, &scr));
         const uint8_t* kfast = kw;
         if (k_words > 8) {
-            const size_t want = m < ctx->lane_hint ? ctx->lane_hint : m;
-            if (ws->kred_lanes < want) {
-                if (ws->kred) cudaFree(ws->kred);
-                ws->kred = nullptr;
-                ws->kred_lanes = 0;
-                CU(ctx, cudaMalloc(&ws->kred, want * 32));
-                ws->kred_lanes = want;
-            }
+            TRY(grow(ctx, &ws->kred, &ws->kred_lanes, lanes, 32));
             bjjk::reduce_scalars(grid_cap(ctx, 8, m), st, m, kw, k_words, ws->kred);
-            ctx->launches++;
-            CU(ctx, cudaGetLastError());
+            TRY(launched(ctx));
             kfast = ws->kred;
         }
         bjjk::mul_scalar(grid, st, m, px + o, py + o, kfast, scr, ws->table, q, ctx->flags_dev);
-        ctx->launches++;
-        CU(ctx, cudaGetLastError());
+        TRY(launched(ctx));
         k_batch_affine<<<affine_grid(ctx, m), BJJ_BLOCK, 0, st>>>(m, scr, rx + o, ry + o);
-        ctx->launches++;
-        CU(ctx, cudaGetLastError());
+        TRY(launched(ctx));
         bjjk::mul_scalar_exact(ctx->sms * 4, st, px + o, py + o, kw, k_words, rx + o, ry + o, q);
-        ctx->launches++;
-        CU(ctx, cudaGetLastError());
-    }
-    return BJJ_OK;
+        return launched(ctx);
+    });
 }
 // fixed-base flavours: `from_keys` selects PrivateKey::public (BLAKE-512 + prune + >>3 first)
 static int launch_fixed_base(bjj_ctx* ctx, size_t n, const uint8_t* in, uint8_t* rx, uint8_t* ry, bool from_keys,
                              cudaStream_t st, Workspace* ws) {
-    for (size_t off = 0; off < n; off += BJJ_POINT_SUBBATCH) {
-        const size_t m = (n - off) < BJJ_POINT_SUBBATCH ? (n - off) : BJJ_POINT_SUBBATCH;
+    const size_t lanes = scratch_lanes(ctx, n);
+    return for_each_subbatch(n, [&](size_t off, size_t m) -> int {
         const size_t o = 32 * off;
         ProjScratch scr;
-        int rc = ensure_proj(ctx, ws, m < BJJ_POINT_SUBBATCH && n > BJJ_POINT_SUBBATCH ? BJJ_POINT_SUBBATCH : m, &scr);
-        if (rc) return rc;
+        TRY(ensure_proj(ctx, ws, lanes, &scr));
         unsigned long long* work = nullptr;
-        rc = claim_counter(ctx, ws, st, &work);
-        if (rc) return rc;
+        TRY(claim_counter(ctx, ws, st, &work));
         if (from_keys && ctx->public_fused) {
-            k_public<<<grid_for(ctx, (const void*)k_public, m), BJJ_BLOCK, 0, st>>>(m, in + o, scr, ctx->comb, work);
-        } else if (from_keys) {
-            // BLAKE-512 is ALU-only work with an 80 KB body: in its own kernel it neither drags the multiplier kernel's
-            // instruction supply nor makes ptxas put integer adds on the multiplier pipe.  The scalars pass through the
-            // scratch plane that only the batched inversion (afterwards) uses.
-            k_scalar_key<<<grid_for(ctx, (const void*)k_scalar_key, m), BJJ_BLOCK, 0, st>>>(m, in + o, scr.p);
-            ctx->launches++;
-            k_fixed_base<<<grid_for(ctx, (const void*)k_fixed_base, m), BJJ_BLOCK, 0, st>>>(m, scr.p, scr, ctx->comb, work);
+            k_public<<<grid_for(ctx, k_public, m), BJJ_BLOCK, 0, st>>>(m, in + o, scr, ctx->comb, work);
         } else {
-            k_fixed_base<<<grid_for(ctx, (const void*)k_fixed_base, m), BJJ_BLOCK, 0, st>>>(m, in + o, scr, ctx->comb, work);
+            const uint8_t* k = in + o;
+            if (from_keys) {
+                // BLAKE-512 is ALU-only work with an 80 KB body: in its own kernel it neither drags the multiplier
+                // kernel's instruction supply nor makes ptxas put integer adds on the multiplier pipe.  The scalars pass
+                // through the scratch plane that only the batched inversion (afterwards) uses.
+                TRY(launch_scalar_key(ctx, m, in + o, scr.p, st));
+                k = scr.p;
+            }
+            k_fixed_base<<<grid_for(ctx, k_fixed_base, m), BJJ_BLOCK, 0, st>>>(m, k, scr, ctx->comb, work);
         }
-        ctx->launches++;
-        CU(ctx, cudaGetLastError());
+        TRY(launched(ctx));
         k_batch_affine<<<affine_grid(ctx, m), BJJ_BLOCK, 0, st>>>(m, scr, rx + o, ry + o);
-        ctx->launches++;
-        CU(ctx, cudaGetLastError());
-    }
-    return BJJ_OK;
+        return launched(ctx);
+    });
 }
 static int launch_decompress(bjj_ctx* ctx, size_t n, const uint8_t* in32, uint8_t* rx, uint8_t* ry, uint8_t* status,
                              cudaStream_t st, Workspace* ws) {
-    for (size_t off = 0; off < n; off += BJJ_POINT_SUBBATCH) {
-        const size_t m = (n - off) < BJJ_POINT_SUBBATCH ? (n - off) : BJJ_POINT_SUBBATCH;
+    const size_t lanes = scratch_lanes(ctx, n);
+    return for_each_subbatch(n, [&](size_t off, size_t m) -> int {
         const size_t o = 32 * off;
         ProjScratch scr;
-        int rc = ensure_proj(ctx, ws, n > BJJ_POINT_SUBBATCH ? BJJ_POINT_SUBBATCH : m, &scr);
-        if (rc) return rc;
-        k_decompress_prepare<<<grid_for(ctx, (const void*)k_decompress_prepare, m), BJJ_BLOCK, 0, st>>>(m, in32 + o, 1, 0, scr, 0);
-        ctx->launches++;
-        CU(ctx, cudaGetLastError());
+        TRY(ensure_proj(ctx, ws, lanes, &scr));
+        k_decompress_prepare<<<grid_for(ctx, k_decompress_prepare, m), BJJ_BLOCK, 0, st>>>(m, in32 + o, 1, 0, scr, 0);
+        TRY(launched(ctx));
         k_batch_inverse<<<affine_grid(ctx, m), BJJ_BLOCK, 0, st>>>(m, scr);
-        ctx->launches++;
-        CU(ctx, cudaGetLastError());
+        TRY(launched(ctx));
         unsigned long long* work = nullptr;
-        rc = claim_counter(ctx, ws, st, &work);
-        if (rc) return rc;
-        k_decompress_finish<<<grid_for(ctx, (const void*)k_decompress_finish, m), BJJ_BLOCK, 0, st>>>(m, in32 + o, 1, 0, scr, 0, rx + o,
-                                                                                                     ry + o, status + off, 0, work);
-        ctx->launches++;
-        CU(ctx, cudaGetLastError());
-    }
-    return BJJ_OK;
+        TRY(claim_counter(ctx, ws, st, &work));
+        k_decompress_finish<<<grid_for(ctx, k_decompress_finish, m), BJJ_BLOCK, 0, st>>>(m, in32 + o, 1, 0, scr, 0, rx + o, ry + o,
+                                                                                        status + off, 0, work);
+        return launched(ctx);
+    });
 }
 
 // verify scratch: four planes hm | u | v | w (32 B / lane each; u, v, w are the Straus scalars, see split.cuh)
 // and, for the compressed pipeline, the four decompressed coordinates
 static int ensure_vscratch(bjj_ctx* ctx, Workspace* ws, size_t lanes, uint8_t** hm, uint8_t** pts) {
-    if (lanes < ctx->lane_hint) lanes = ctx->lane_hint;
-    if (ws->vs_lanes < lanes) {
-        if (ws->vs) cudaFree(ws->vs);
-        ws->vs = nullptr;
-        ws->vs_lanes = 0;
-        CU(ctx, cudaMalloc(&ws->vs, lanes * 256));
-        ws->vs_lanes = lanes;
-    }
+    TRY(grow(ctx, &ws->vs, &ws->vs_lanes, lanes, 256));
     *hm = ws->vs;
     *pts = ws->vs + 4 * 32 * ws->vs_lanes;
     return BJJ_OK;
@@ -601,24 +606,20 @@ static int ensure_vscratch(bjj_ctx* ctx, Workspace* ws, size_t lanes, uint8_t** 
 static int launch_verify(bjj_ctx* ctx, size_t n, const uint8_t* r8x, const uint8_t* r8y, const uint8_t* s,
                          const uint8_t* ax, const uint8_t* ay, const uint8_t* msg, uint8_t* ok, cudaStream_t st,
                          Workspace* ws, int mode = BJJ_MODE_EDDSA, uint8_t* msg_status = nullptr, bool defer_join = false) {
-    for (size_t off = 0; off < n; off += BJJ_POINT_SUBBATCH) {
-        const size_t m = (n - off) < BJJ_POINT_SUBBATCH ? (n - off) : BJJ_POINT_SUBBATCH;
+    const size_t lanes = scratch_lanes(ctx, n);
+    return for_each_subbatch(n, [&](size_t off, size_t m) -> int {
         const size_t o = 32 * off;
         const int grid_h = grid_cap(ctx, bjjk::verify_hash_blocks_per_sm(), m);
         const int grid_e = grid_cap(ctx, bjjk::verify_ec_blocks_per_sm(), m);
-        int rc = ensure_table(ctx, ws, 2 * (size_t)grid_e * BJJ_BLOCK);     // two per-thread tables: 8A and R8
-        if (rc) return rc;
-        rc = ensure_aux(ctx, ws);
-        if (rc) return rc;
+        TRY(ensure_table(ctx, ws, 2 * (size_t)grid_e * BJJ_BLOCK));     // two per-thread tables: 8A and R8
+        TRY(ensure_aux(ctx, ws));
         // exact lanes of an earlier batch may still be reading this workspace's queues and scratch (deferred join):
         // wait for them BEFORE the queue counters are cleared and the scratch is reused
         CU(ctx, cudaStreamWaitEvent(st, ws->ev_join, 0));
         ExactQueue qa, qr;
-        rc = ensure_queue(ctx, ws, m, st, &qa, &qr);
-        if (rc) return rc;
+        TRY(ensure_queue(ctx, ws, lanes, st, &qa, &qr));
         uint8_t *hm, *pts;
-        rc = ensure_vscratch(ctx, ws, n > BJJ_POINT_SUBBATCH ? BJJ_POINT_SUBBATCH : m, &hm, &pts);
-        if (rc) return rc;
+        TRY(ensure_vscratch(ctx, ws, lanes, &hm, &pts));
         // BJJ_PHASE_TIMING=1: synchronous per-phase CUDA-event timings on stderr (diagnosis only)
         static const bool phase_timing = getenv("BJJ_PHASE_TIMING") != nullptr;
         cudaEvent_t pe[4] = {nullptr, nullptr, nullptr, nullptr};
@@ -628,8 +629,7 @@ static int launch_verify(bjj_ctx* ctx, size_t n, const uint8_t* r8x, const uint8
         }
         bjjk::verify_hash(grid_h, st, m, r8x + o, r8y + o, ax + o, ay + o, msg + o, s + o, 1, 0, nullptr, hm, ws->vs_lanes, ok + off, true,
                           qa, qr, ctx->flags_dev, mode, ctx->verify_split, msg_status ? msg_status + off : nullptr, work_counters(ws));
-        ctx->launches++;
-        CU(ctx, cudaGetLastError());
+        TRY(launched(ctx));
         // The queues are complete after the hash kernel, and the exact lanes (rare; one long ladder each, ~4 % of the
         // step's multiplier work in the benchmark mix) need nothing else: their kernel is released HERE, on the side
         // stream, before the split and the Straus kernel.  Its CTAs are placed first; those that find the queues empty
@@ -646,28 +646,19 @@ static int launch_verify(bjj_ctx* ctx, size_t n, const uint8_t* r8x, const uint8
             CU(ctx, cudaStreamWaitEvent(ws->aux, ws->ev_fork, 0));
             bjjk::verify_exact(ctx->sms * (exact_ctas < 1 ? 1 : exact_ctas), ws->aux, r8x + o, r8y + o, s + o, ax + o, ay + o, hm, ok + off, qa, qr,
                                ctx->comb, mode, work_counters(ws) + 2);
-            ctx->launches++;
-            CU(ctx, cudaGetLastError());
+            TRY(launched(ctx));
             CU(ctx, cudaEventRecord(ws->ev_join, ws->aux));
             return BJJ_OK;
         };
-        if (exact_early) {
-            rc = launch_exact();
-            if (rc) return rc;
-        }
+        if (exact_early) TRY(launch_exact());
         if (ctx->verify_split && mode == BJJ_MODE_EDDSA) {
             bjjk::verify_split(grid_cap(ctx, bjjk::verify_split_blocks_per_sm(), m), st, m, s + o, 1, 0, hm, ws->vs_lanes, ok + off);
-            ctx->launches++;
-            CU(ctx, cudaGetLastError());
+            TRY(launched(ctx));
         }
         if (phase_timing) cudaEventRecord(pe[1], st);
         bjjk::verify_ec(grid_e, st, m, r8x + o, r8y + o, ax + o, ay + o, hm, ws->vs_lanes, ok + off, ws->table, ctx->comb, mode, work_counters(ws) + 1);
-        ctx->launches++;
-        CU(ctx, cudaGetLastError());
-        if (!exact_early) {
-            rc = launch_exact();
-            if (rc) return rc;
-        }
+        TRY(launched(ctx));
+        if (!exact_early) TRY(launch_exact());
         if (phase_timing) cudaEventRecord(pe[2], st);
         // defer_join: the caller orders whatever consumes ok[] after ws->ev_join itself, and the stream moves on
         // to the next batch while the (latency-bound) exact lanes finish beside it
@@ -683,65 +674,49 @@ static int launch_verify(bjj_ctx* ctx, size_t n, const uint8_t* r8x, const uint8
                     grid_e, t_hash, t_ec, t_join);
             for (int e = 0; e < 4; e++) cudaEventDestroy(pe[e]);
         }
-    }
-    return BJJ_OK;
+        return BJJ_OK;
+    });
 }
 static int launch_verify_compressed(bjj_ctx* ctx, size_t n, const uint8_t* sig64, const uint8_t* pk32,
                                     const uint8_t* msg, uint8_t* ok, uint8_t* status, cudaStream_t st, Workspace* ws) {
-    for (size_t off = 0; off < n; off += BJJ_POINT_SUBBATCH) {
-        const size_t m = (n - off) < BJJ_POINT_SUBBATCH ? (n - off) : BJJ_POINT_SUBBATCH;
+    const size_t lanes = scratch_lanes(ctx, n);
+    return for_each_subbatch(n, [&](size_t off, size_t m) -> int {
         const size_t o = 32 * off;
         const int grid_h = grid_cap(ctx, bjjk::verify_hash_blocks_per_sm(), m);
         const int grid_e = grid_cap(ctx, bjjk::verify_ec_blocks_per_sm(), m);
-        int rc = ensure_table(ctx, ws, 2 * (size_t)grid_e * BJJ_BLOCK);
-        if (rc) return rc;
-        rc = ensure_aux(ctx, ws);
-        if (rc) return rc;
+        TRY(ensure_table(ctx, ws, 2 * (size_t)grid_e * BJJ_BLOCK));
+        TRY(ensure_aux(ctx, ws));
         CU(ctx, cudaStreamWaitEvent(st, ws->ev_join, 0));      // a deferred exact kernel of an earlier verify on this workspace
         ExactQueue q;     // never fed here (decompressed points are on the curve) but the kernel wants a valid one
-        rc = ensure_queue(ctx, ws, 1, st, &q);
-        if (rc) return rc;
+        TRY(ensure_queue(ctx, ws, scratch_lanes(ctx, 1), st, &q));
         uint8_t *hm, *pts;
-        rc = ensure_vscratch(ctx, ws, n > BJJ_POINT_SUBBATCH ? BJJ_POINT_SUBBATCH : m, &hm, &pts);
-        if (rc) return rc;
+        TRY(ensure_vscratch(ctx, ws, lanes, &hm, &pts));
         const size_t L = 32 * ws->vs_lanes;
         uint8_t *dx = pts, *dy = pts + L, *dax = pts + 2 * L, *day = pts + 3 * L;
         // phase 0: decompress R8 (first half of each 64-byte signature) and A with one shared inversion pass
         ProjScratch scr;
-        {
-            size_t lanes = n > BJJ_POINT_SUBBATCH ? BJJ_POINT_SUBBATCH : m;
-            if (lanes < ctx->lane_hint) lanes = ctx->lane_hint;
-            rc = ensure_proj(ctx, ws, 2 * lanes, &scr);       // R8 and A share one inversion pass: two slots per lane
-        }
-        if (rc) return rc;
-        const int grid_p = grid_for(ctx, (const void*)k_decompress_prepare, m);
-        const int grid_f = grid_for(ctx, (const void*)k_decompress_finish, m);
+        TRY(ensure_proj(ctx, ws, 2 * lanes, &scr));       // R8 and A share one inversion pass: two slots per lane
+        const int grid_p = grid_for(ctx, k_decompress_prepare, m);
+        const int grid_f = grid_for(ctx, k_decompress_finish, m);
         k_decompress_prepare<<<grid_p, BJJ_BLOCK, 0, st>>>(m, sig64 + 2 * o, 2, 0, scr, 0);
         k_decompress_prepare<<<grid_p, BJJ_BLOCK, 0, st>>>(m, pk32 + o, 1, 0, scr, m);
         k_batch_inverse<<<affine_grid(ctx, 2 * m), BJJ_BLOCK, 0, st>>>(2 * m, scr);
         unsigned long long *work_r = nullptr, *work_a = nullptr;
-        rc = claim_counter(ctx, ws, st, &work_r);
-        if (rc) return rc;
-        rc = claim_counter(ctx, ws, st, &work_a);
-        if (rc) return rc;
+        TRY(claim_counter(ctx, ws, st, &work_r));
+        TRY(claim_counter(ctx, ws, st, &work_a));
         k_decompress_finish<<<grid_f, BJJ_BLOCK, 0, st>>>(m, sig64 + 2 * o, 2, 0, scr, 0, dx, dy, status + off, 0, work_r);
         k_decompress_finish<<<grid_f, BJJ_BLOCK, 0, st>>>(m, pk32 + o, 1, 0, scr, m, dax, day, status + off, 1, work_a);
-        ctx->launches += 5;
-        CU(ctx, cudaGetLastError());
+        TRY(launched(ctx, 5));
         bjjk::verify_hash(grid_h, st, m, dx, dy, dax, day, msg + o, sig64 + 2 * o, 2, 1, status + off, hm, ws->vs_lanes, ok + off, false, q,
                           q, ctx->flags_dev, BJJ_MODE_EDDSA, ctx->verify_split, nullptr, work_counters(ws));
-        ctx->launches++;
-        CU(ctx, cudaGetLastError());
+        TRY(launched(ctx));
         if (ctx->verify_split) {
             bjjk::verify_split(grid_cap(ctx, bjjk::verify_split_blocks_per_sm(), m), st, m, sig64 + 2 * o, 2, 1, hm, ws->vs_lanes, ok + off);
-            ctx->launches++;
-            CU(ctx, cudaGetLastError());
+            TRY(launched(ctx));
         }
         bjjk::verify_ec(grid_e, st, m, dx, dy, dax, day, hm, ws->vs_lanes, ok + off, ws->table, ctx->comb, BJJ_MODE_EDDSA, work_counters(ws) + 1);
-        ctx->launches++;
-        CU(ctx, cudaGetLastError());
-    }
-    return BJJ_OK;
+        return launched(ctx);
+    });
 }
 static int launch_poseidon(bjj_ctx* ctx, int n_inputs, size_t n, const uint8_t* const* in, uint8_t* out,
                            cudaStream_t st) {
@@ -749,7 +724,7 @@ static int launch_poseidon(bjj_ctx* ctx, int n_inputs, size_t n, const uint8_t* 
     for (int j = 0; j < 8; j++) pin.p[j] = j < n_inputs ? in[j] : nullptr;
     if (n_inputs < 1 || n_inputs > BJJ_POSEIDON_MAX_INPUTS) return BJJ_ERR_ARG;
     bjjk::poseidon(n_inputs + 1, grid_cap(ctx, bjjk::poseidon_blocks_per_sm(n_inputs + 1), n), st, n, pin, out, ctx->flags_dev);
-    DEV_EPILOGUE
+    return launched(ctx);
 }
 
 // PrivateKey::sign as a pipeline: k_sign_scalars (BLAKE-512 twice: sk, r) -> R8 = r * B8 and A = sk * B8 on the
@@ -760,34 +735,25 @@ static int launch_sign(bjj_ctx* ctx, size_t n, const uint8_t* key32, const uint8
                        uint8_t* status, cudaStream_t st, Workspace* ws) {
     if (ctx->sign_fused) {
         bjjk::sign(grid_cap(ctx, bjjk::sign_blocks_per_sm(), n), st, n, key32, msg32, r8x, r8y, s32, status, ctx->comb);
-        ctx->launches++;
-        CU(ctx, cudaGetLastError());
-        return BJJ_OK;
+        return launched(ctx);
     }
-    for (size_t off = 0; off < n; off += BJJ_POINT_SUBBATCH) {
-        const size_t m = (n - off) < BJJ_POINT_SUBBATCH ? (n - off) : BJJ_POINT_SUBBATCH;
+    const size_t lanes = scratch_lanes(ctx, n);
+    return for_each_subbatch(n, [&](size_t off, size_t m) -> int {
         const size_t o = 32 * off;
         uint8_t *hm, *pts;
-        int rc = ensure_vscratch(ctx, ws, n > BJJ_POINT_SUBBATCH ? BJJ_POINT_SUBBATCH : m, &hm, &pts);
-        if (rc) return rc;
+        TRY(ensure_vscratch(ctx, ws, lanes, &hm, &pts));
         const size_t L = 32 * ws->vs_lanes;
         uint8_t *sk = hm + L, *r = hm + 2 * L, *msgc = hm + 3 * L, *apx = pts, *apy = pts + L;
-        const int grid_s = grid_for(ctx, (const void*)k_scalar_key, m);      // same block size and shape of work
+        const int grid_s = grid_for(ctx, k_scalar_key, m);      // same block size and shape of work
         bjjk::sign_scalars(grid_s, st, m, key32 + o, msg32 + o, sk, r, msgc, status + off);
-        ctx->launches++;
-        CU(ctx, cudaGetLastError());
-        rc = launch_fixed_base(ctx, m, r, r8x + o, r8y + o, false, st, ws);
-        if (rc) return rc;
-        rc = launch_fixed_base(ctx, m, sk, apx, apy, false, st, ws);
-        if (rc) return rc;
+        TRY(launched(ctx));
+        TRY(launch_fixed_base(ctx, m, r, r8x + o, r8y + o, false, st, ws));
+        TRY(launch_fixed_base(ctx, m, sk, apx, apy, false, st, ws));
         const uint8_t* ins[5] = {r8x + o, r8y + o, apx, apy, msgc};
-        rc = launch_poseidon(ctx, 5, m, ins, hm, st);
-        if (rc) return rc;
+        TRY(launch_poseidon(ctx, 5, m, ins, hm, st));
         bjjk::sign_finish(grid_s, st, m, hm, sk, r, status + off, r8x + o, r8y + o, s32 + o);
-        ctx->launches++;
-        CU(ctx, cudaGetLastError());
-    }
-    return BJJ_OK;
+        return launched(ctx);
+    });
 }
 
 extern "C" {
@@ -796,16 +762,14 @@ int bjj_fr_op_batch_dev(bjj_ctx* ctx, int op, size_t n, const uint8_t* a, const 
     DEV_PROLOGUE
     if (!a || !out || op < 0 || op > BJJ_FR_SQR_LAZY) return BJJ_ERR_ARG;
     if (!b) b = a;
-    k_fr_op<<<grid_for(ctx, (const void*)k_fr_op, n), BJJ_BLOCK, 0, st>>>(op, n, a, b, out, ctx->flags_dev);
-    DEV_EPILOGUE
+    return launch_fr_op(ctx, n, op, a, b, out, st);
 }
 
 int bjj_split_scalars_batch_dev(bjj_ctx* ctx, size_t n, const uint8_t* h32, const uint8_t* s32, uint8_t* u32,
                                 uint8_t* v32, uint8_t* w32, void* stream) {
     DEV_PROLOGUE
     if (!h32 || !s32 || !u32 || !v32 || !w32) return BJJ_ERR_ARG;
-    k_split_scalars<<<grid_for(ctx, (const void*)k_split_scalars, n), BJJ_BLOCK, 0, st>>>(n, h32, s32, u32, v32, w32);
-    DEV_EPILOGUE
+    return launch_split_scalars(ctx, n, h32, s32, u32, v32, w32, st);
 }
 
 int bjj_add_batch_dev(bjj_ctx* ctx, size_t n, const uint8_t* px, const uint8_t* py, const uint8_t* pz,
@@ -813,16 +777,14 @@ int bjj_add_batch_dev(bjj_ctx* ctx, size_t n, const uint8_t* px, const uint8_t* 
                       void* stream) {
     DEV_PROLOGUE
     if (!px || !py || !pz || !qx || !qy || !qz || !rx || !ry || !rz) return BJJ_ERR_ARG;
-    k_add<<<grid_for(ctx, (const void*)k_add, n), BJJ_BLOCK, 0, st>>>(n, px, py, pz, qx, qy, qz, rx, ry, rz, ctx->flags_dev);
-    DEV_EPILOGUE
+    return launch_add(ctx, n, px, py, pz, qx, qy, qz, rx, ry, rz, st);
 }
 
 int bjj_affine_batch_dev(bjj_ctx* ctx, size_t n, const uint8_t* px, const uint8_t* py, const uint8_t* pz, uint8_t* rx,
                          uint8_t* ry, void* stream) {
     DEV_PROLOGUE
     if (!px || !py || !pz || !rx || !ry) return BJJ_ERR_ARG;
-    k_affine<<<grid_for(ctx, (const void*)k_affine, n), BJJ_BLOCK, 0, st>>>(n, px, py, pz, rx, ry, ctx->flags_dev);
-    DEV_EPILOGUE
+    return launch_affine(ctx, n, px, py, pz, rx, ry, st);
 }
 
 int bjj_mul_scalar_batch_dev(bjj_ctx* ctx, size_t n, const uint8_t* px, const uint8_t* py, const uint8_t* scalar32,
@@ -861,15 +823,13 @@ int bjj_sign_batch_dev(bjj_ctx* ctx, size_t n, const uint8_t* key32, const uint8
 int bjj_scalar_key_batch_dev(bjj_ctx* ctx, size_t n, const uint8_t* key32, uint8_t* scalar32, void* stream) {
     DEV_PROLOGUE
     if (!key32 || !scalar32) return BJJ_ERR_ARG;
-    k_scalar_key<<<grid_for(ctx, (const void*)k_scalar_key, n), BJJ_BLOCK, 0, st>>>(n, key32, scalar32);
-    DEV_EPILOGUE
+    return launch_scalar_key(ctx, n, key32, scalar32, st);
 }
 
 int bjj_compress_batch_dev(bjj_ctx* ctx, size_t n, const uint8_t* px, const uint8_t* py, uint8_t* out32, void* stream) {
     DEV_PROLOGUE
     if (!px || !py || !out32) return BJJ_ERR_ARG;
-    k_compress<<<grid_for(ctx, (const void*)k_compress, n), BJJ_BLOCK, 0, st>>>(n, px, py, out32, ctx->flags_dev);
-    DEV_EPILOGUE
+    return launch_compress(ctx, n, px, py, out32, st);
 }
 
 int bjj_decompress_batch_dev(bjj_ctx* ctx, size_t n, const uint8_t* in32, uint8_t* rx, uint8_t* ry, uint8_t* status,
@@ -1003,27 +963,16 @@ static int run_host(bjj_ctx* ctx, size_t n, HostArg* args, int nargs, Launch lau
         PipeSlot& sl = ctx->slot[which];
         m = (n - off) < cur ? (n - off) : cur;
         if (n - off - m < cur / 2 && n - off <= cap) m = n - off;      // fold a short remainder into this chunk
-        if (sl.arena_bytes < need) {
-            CU(ctx, cudaStreamSynchronize(sl.stream));
-            if (sl.arena) cudaFree(sl.arena);
-            sl.arena = nullptr;
-            sl.arena_bytes = 0;
-            CU(ctx, cudaMalloc(&sl.arena, need));
-            sl.arena_bytes = need;
-        }
+        // the slot's copies of two chunks ago may still use the arena and the mirror: let them finish before a regrowth
+        if (sl.arena_bytes < need) CU(ctx, cudaStreamSynchronize(sl.stream));
+        TRY(grow(ctx, &sl.arena, &sl.arena_bytes, need, 1));
         if (any_staged) {
             // the slot's previous chunk: its results go out to the caller, and its host-to-device copies have long
             // finished reading the mirror (they precede ev_done on the slot's stream)
             rc = drain(sl);
             if (rc) break;
-            if (sl.hstage_bytes < need) {
-                CU(ctx, cudaStreamSynchronize(sl.stream));
-                if (sl.hstage) cudaFreeHost(sl.hstage);
-                sl.hstage = nullptr;
-                sl.hstage_bytes = 0;
-                CU(ctx, cudaHostAlloc(&sl.hstage, need, cudaHostAllocDefault));
-                sl.hstage_bytes = need;
-            }
+            if (sl.hstage_bytes < need) CU(ctx, cudaStreamSynchronize(sl.stream));
+            TRY(grow(ctx, &sl.hstage, &sl.hstage_bytes, need, 1, /*pinned=*/true));
         }
         // the slot's copy stream is ordered: these copies follow the slot's previous results going out
         uint8_t* dptr[16];
@@ -1040,7 +989,7 @@ static int run_host(bjj_ctx* ctx, size_t n, HostArg* args, int nargs, Launch lau
             }
             pos += ((args[a].bytes_per_lane * cap + 255) & ~(size_t)255);
         }
-        ComputeRef comp{ctx->stream, which ? ctx->ws2 : ctx->ws};
+        Workspace* ws = which ? &ctx->ws2 : &ctx->ws;
         CU(ctx, cudaEventRecord(sl.ev_in, sl.stream));
         const bool mark = pipe_timing && nmarks < 64;
         if (mark) {
@@ -1051,13 +1000,13 @@ static int run_host(bjj_ctx* ctx, size_t n, HostArg* args, int nargs, Launch lau
             mk.lanes = m;
             cudaEventRecord(mk.in, sl.stream);
         }
-        CU(ctx, cudaStreamWaitEvent(comp.stream, sl.ev_in, 0));
-        rc = launch(m, dptr, comp);
+        CU(ctx, cudaStreamWaitEvent(ctx->stream, sl.ev_in, 0));
+        rc = launch(m, dptr, ctx->stream, ws);
         if (rc) break;
-        if (mark) cudaEventRecord(marks[nmarks].comp, comp.stream);
-        CU(ctx, cudaEventRecord(sl.ev_out, comp.stream));
+        if (mark) cudaEventRecord(marks[nmarks].comp, ctx->stream);
+        CU(ctx, cudaEventRecord(sl.ev_out, ctx->stream));
         CU(ctx, cudaStreamWaitEvent(sl.stream, sl.ev_out, 0));
-        if (comp.ws.aux) CU(ctx, cudaStreamWaitEvent(sl.stream, comp.ws.ev_join, 0));      // deferred exact lanes
+        if (ws->aux) CU(ctx, cudaStreamWaitEvent(sl.stream, ws->ev_join, 0));      // deferred exact lanes
         pos = 0;
         for (int a = 0; a < nargs; a++) {
             if (args[a].out)
@@ -1108,10 +1057,6 @@ static int run_host(bjj_ctx* ctx, size_t n, HostArg* args, int nargs, Launch lau
 
 #define H_IN(p, b) HostArg{(p), nullptr, (b)}
 #define H_OUT(p, b) HostArg{nullptr, (p), (b)}
-#define CHECK_LAUNCH(ctx)            \
-    (ctx)->launches++;               \
-    CU(ctx, cudaGetLastError());     \
-    return BJJ_OK;
 
 extern "C" {
 
@@ -1119,9 +1064,8 @@ int bjj_fr_op_batch(bjj_ctx* ctx, int op, size_t n, const uint8_t* a, const uint
     if (!ctx || !a || !out || op < 0 || op > BJJ_FR_SQR_LAZY) return BJJ_ERR_ARG;
     if (!b) b = a;
     HostArg args[] = {H_IN(a, 32), H_IN(b, 32), H_OUT(out, 32)};
-    return run_host(ctx, n, args, 3, [&](size_t m, uint8_t** d, ComputeRef sl) -> int {
-        k_fr_op<<<grid_for(ctx, (const void*)k_fr_op, m), BJJ_BLOCK, 0, sl.stream>>>(op, m, d[0], d[1], d[2], ctx->flags_dev);
-        CHECK_LAUNCH(ctx)
+    return run_host(ctx, n, args, 3, [&](size_t m, uint8_t** d, cudaStream_t st, Workspace* ws) -> int {
+        return launch_fr_op(ctx, m, op, d[0], d[1], d[2], st);
     });
 }
 
@@ -1129,9 +1073,8 @@ int bjj_split_scalars_batch(bjj_ctx* ctx, size_t n, const uint8_t* h32, const ui
                             uint8_t* w32) {
     if (!ctx) return BJJ_ERR_ARG;
     HostArg args[] = {H_IN(h32, 32), H_IN(s32, 32), H_OUT(u32, 32), H_OUT(v32, 32), H_OUT(w32, 32)};
-    return run_host(ctx, n, args, 5, [&](size_t m, uint8_t** d, ComputeRef sl) -> int {
-        k_split_scalars<<<grid_for(ctx, (const void*)k_split_scalars, m), BJJ_BLOCK, 0, sl.stream>>>(m, d[0], d[1], d[2], d[3], d[4]);
-        CHECK_LAUNCH(ctx)
+    return run_host(ctx, n, args, 5, [&](size_t m, uint8_t** d, cudaStream_t st, Workspace* ws) -> int {
+        return launch_split_scalars(ctx, m, d[0], d[1], d[2], d[3], d[4], st);
     });
 }
 
@@ -1140,10 +1083,8 @@ int bjj_add_batch(bjj_ctx* ctx, size_t n, const uint8_t* px, const uint8_t* py, 
     if (!ctx) return BJJ_ERR_ARG;
     HostArg args[] = {H_IN(px, 32), H_IN(py, 32), H_IN(pz, 32), H_IN(qx, 32), H_IN(qy, 32),
                       H_IN(qz, 32), H_OUT(rx, 32), H_OUT(ry, 32), H_OUT(rz, 32)};
-    return run_host(ctx, n, args, 9, [&](size_t m, uint8_t** d, ComputeRef sl) -> int {
-        k_add<<<grid_for(ctx, (const void*)k_add, m), BJJ_BLOCK, 0, sl.stream>>>(m, d[0], d[1], d[2], d[3], d[4], d[5], d[6],
-                                                                                d[7], d[8], ctx->flags_dev);
-        CHECK_LAUNCH(ctx)
+    return run_host(ctx, n, args, 9, [&](size_t m, uint8_t** d, cudaStream_t st, Workspace* ws) -> int {
+        return launch_add(ctx, m, d[0], d[1], d[2], d[3], d[4], d[5], d[6], d[7], d[8], st);
     });
 }
 
@@ -1151,10 +1092,8 @@ int bjj_affine_batch(bjj_ctx* ctx, size_t n, const uint8_t* px, const uint8_t* p
                      uint8_t* ry) {
     if (!ctx) return BJJ_ERR_ARG;
     HostArg args[] = {H_IN(px, 32), H_IN(py, 32), H_IN(pz, 32), H_OUT(rx, 32), H_OUT(ry, 32)};
-    return run_host(ctx, n, args, 5, [&](size_t m, uint8_t** d, ComputeRef sl) -> int {
-        k_affine<<<grid_for(ctx, (const void*)k_affine, m), BJJ_BLOCK, 0, sl.stream>>>(m, d[0], d[1], d[2], d[3], d[4],
-                                                                                      ctx->flags_dev);
-        CHECK_LAUNCH(ctx)
+    return run_host(ctx, n, args, 5, [&](size_t m, uint8_t** d, cudaStream_t st, Workspace* ws) -> int {
+        return launch_affine(ctx, m, d[0], d[1], d[2], d[3], d[4], st);
     });
 }
 
@@ -1162,8 +1101,8 @@ int bjj_mul_scalar_batch(bjj_ctx* ctx, size_t n, const uint8_t* px, const uint8_
                          uint8_t* rx, uint8_t* ry) {
     if (!ctx) return BJJ_ERR_ARG;
     HostArg args[] = {H_IN(px, 32), H_IN(py, 32), H_IN(scalar32, 32), H_OUT(rx, 32), H_OUT(ry, 32)};
-    return run_host(ctx, n, args, 5, [&](size_t m, uint8_t** d, ComputeRef sl) -> int {
-        return launch_mul_scalar(ctx, m, d[0], d[1], d[2], 8, d[3], d[4], sl.stream, &sl.ws);
+    return run_host(ctx, n, args, 5, [&](size_t m, uint8_t** d, cudaStream_t st, Workspace* ws) -> int {
+        return launch_mul_scalar(ctx, m, d[0], d[1], d[2], 8, d[3], d[4], st, ws);
     }, /*heavy=*/true);
 }
 
@@ -1171,24 +1110,24 @@ int bjj_mul_scalar_wide_batch(bjj_ctx* ctx, size_t n, const uint8_t* px, const u
                               uint8_t* rx, uint8_t* ry) {
     if (!ctx || scalar_words < 8 || scalar_words > BJJ_MAX_SCALAR_WORDS || (scalar_words & 7)) return BJJ_ERR_ARG;
     HostArg args[] = {H_IN(px, 32), H_IN(py, 32), H_IN(scalar, (size_t)4 * scalar_words), H_OUT(rx, 32), H_OUT(ry, 32)};
-    return run_host(ctx, n, args, 5, [&](size_t m, uint8_t** d, ComputeRef sl) -> int {
-        return launch_mul_scalar(ctx, m, d[0], d[1], d[2], scalar_words, d[3], d[4], sl.stream, &sl.ws);
+    return run_host(ctx, n, args, 5, [&](size_t m, uint8_t** d, cudaStream_t st, Workspace* ws) -> int {
+        return launch_mul_scalar(ctx, m, d[0], d[1], d[2], scalar_words, d[3], d[4], st, ws);
     }, /*heavy=*/true);
 }
 
 int bjj_fixed_base_batch(bjj_ctx* ctx, size_t n, const uint8_t* scalar32, uint8_t* rx, uint8_t* ry) {
     if (!ctx) return BJJ_ERR_ARG;
     HostArg args[] = {H_IN(scalar32, 32), H_OUT(rx, 32), H_OUT(ry, 32)};
-    return run_host(ctx, n, args, 3, [&](size_t m, uint8_t** d, ComputeRef sl) -> int {
-        return launch_fixed_base(ctx, m, d[0], d[1], d[2], false, sl.stream, &sl.ws);
+    return run_host(ctx, n, args, 3, [&](size_t m, uint8_t** d, cudaStream_t st, Workspace* ws) -> int {
+        return launch_fixed_base(ctx, m, d[0], d[1], d[2], false, st, ws);
     });
 }
 
 int bjj_public_batch(bjj_ctx* ctx, size_t n, const uint8_t* key32, uint8_t* rx, uint8_t* ry) {
     if (!ctx) return BJJ_ERR_ARG;
     HostArg args[] = {H_IN(key32, 32), H_OUT(rx, 32), H_OUT(ry, 32)};
-    return run_host(ctx, n, args, 3, [&](size_t m, uint8_t** d, ComputeRef sl) -> int {
-        return launch_fixed_base(ctx, m, d[0], d[1], d[2], true, sl.stream, &sl.ws);
+    return run_host(ctx, n, args, 3, [&](size_t m, uint8_t** d, cudaStream_t st, Workspace* ws) -> int {
+        return launch_fixed_base(ctx, m, d[0], d[1], d[2], true, st, ws);
     });
 }
 
@@ -1196,34 +1135,32 @@ int bjj_sign_batch(bjj_ctx* ctx, size_t n, const uint8_t* key32, const uint8_t* 
                    uint8_t* s32, uint8_t* status) {
     if (!ctx) return BJJ_ERR_ARG;
     HostArg args[] = {H_IN(key32, 32), H_IN(msg32, 32), H_OUT(r8x, 32), H_OUT(r8y, 32), H_OUT(s32, 32), H_OUT(status, 1)};
-    return run_host(ctx, n, args, 6, [&](size_t m, uint8_t** d, ComputeRef sl) -> int {
-        return launch_sign(ctx, m, d[0], d[1], d[2], d[3], d[4], d[5], sl.stream, &sl.ws);
+    return run_host(ctx, n, args, 6, [&](size_t m, uint8_t** d, cudaStream_t st, Workspace* ws) -> int {
+        return launch_sign(ctx, m, d[0], d[1], d[2], d[3], d[4], d[5], st, ws);
     });
 }
 
 int bjj_scalar_key_batch(bjj_ctx* ctx, size_t n, const uint8_t* key32, uint8_t* scalar32) {
     if (!ctx) return BJJ_ERR_ARG;
     HostArg args[] = {H_IN(key32, 32), H_OUT(scalar32, 32)};
-    return run_host(ctx, n, args, 2, [&](size_t m, uint8_t** d, ComputeRef sl) -> int {
-        k_scalar_key<<<grid_for(ctx, (const void*)k_scalar_key, m), BJJ_BLOCK, 0, sl.stream>>>(m, d[0], d[1]);
-        CHECK_LAUNCH(ctx)
+    return run_host(ctx, n, args, 2, [&](size_t m, uint8_t** d, cudaStream_t st, Workspace* ws) -> int {
+        return launch_scalar_key(ctx, m, d[0], d[1], st);
     });
 }
 
 int bjj_compress_batch(bjj_ctx* ctx, size_t n, const uint8_t* px, const uint8_t* py, uint8_t* out32) {
     if (!ctx) return BJJ_ERR_ARG;
     HostArg args[] = {H_IN(px, 32), H_IN(py, 32), H_OUT(out32, 32)};
-    return run_host(ctx, n, args, 3, [&](size_t m, uint8_t** d, ComputeRef sl) -> int {
-        k_compress<<<grid_for(ctx, (const void*)k_compress, m), BJJ_BLOCK, 0, sl.stream>>>(m, d[0], d[1], d[2], ctx->flags_dev);
-        CHECK_LAUNCH(ctx)
+    return run_host(ctx, n, args, 3, [&](size_t m, uint8_t** d, cudaStream_t st, Workspace* ws) -> int {
+        return launch_compress(ctx, m, d[0], d[1], d[2], st);
     });
 }
 
 int bjj_decompress_batch(bjj_ctx* ctx, size_t n, const uint8_t* in32, uint8_t* rx, uint8_t* ry, uint8_t* status) {
     if (!ctx) return BJJ_ERR_ARG;
     HostArg args[] = {H_IN(in32, 32), H_OUT(rx, 32), H_OUT(ry, 32), H_OUT(status, 1)};
-    return run_host(ctx, n, args, 4, [&](size_t m, uint8_t** d, ComputeRef sl) -> int {
-        return launch_decompress(ctx, m, d[0], d[1], d[2], d[3], sl.stream, &sl.ws);
+    return run_host(ctx, n, args, 4, [&](size_t m, uint8_t** d, cudaStream_t st, Workspace* ws) -> int {
+        return launch_decompress(ctx, m, d[0], d[1], d[2], d[3], st, ws);
     });
 }
 
@@ -1232,8 +1169,8 @@ int bjj_poseidon_batch(bjj_ctx* ctx, int n_inputs, size_t n, const uint8_t* cons
     HostArg args[9];
     for (int j = 0; j < n_inputs; j++) args[j] = H_IN(in[j], 32);
     args[n_inputs] = H_OUT(out, 32);
-    return run_host(ctx, n, args, n_inputs + 1, [&](size_t m, uint8_t** d, ComputeRef sl) -> int {
-        return launch_poseidon(ctx, n_inputs, m, (const uint8_t* const*)d, d[n_inputs], sl.stream);
+    return run_host(ctx, n, args, n_inputs + 1, [&](size_t m, uint8_t** d, cudaStream_t st, Workspace* ws) -> int {
+        return launch_poseidon(ctx, n_inputs, m, (const uint8_t* const*)d, d[n_inputs], st);
     });
 }
 
@@ -1241,8 +1178,8 @@ int bjj_verify_batch(bjj_ctx* ctx, size_t n, const uint8_t* r8x, const uint8_t* 
                      const uint8_t* ax, const uint8_t* ay, const uint8_t* msg32, uint8_t* ok) {
     if (!ctx) return BJJ_ERR_ARG;
     HostArg args[] = {H_IN(r8x, 32), H_IN(r8y, 32), H_IN(s32, 32), H_IN(ax, 32), H_IN(ay, 32), H_IN(msg32, 32), H_OUT(ok, 1)};
-    return run_host(ctx, n, args, 7, [&](size_t m, uint8_t** d, ComputeRef sl) -> int {
-        return launch_verify(ctx, m, d[0], d[1], d[2], d[3], d[4], d[5], d[6], sl.stream, &sl.ws, BJJ_MODE_EDDSA, nullptr, true);
+    return run_host(ctx, n, args, 7, [&](size_t m, uint8_t** d, cudaStream_t st, Workspace* ws) -> int {
+        return launch_verify(ctx, m, d[0], d[1], d[2], d[3], d[4], d[5], d[6], st, ws, BJJ_MODE_EDDSA, nullptr, true);
     }, /*heavy=*/true);
 }
 
@@ -1251,8 +1188,8 @@ int bjj_verify_schnorr_batch(bjj_ctx* ctx, size_t n, const uint8_t* pkx, const u
     if (!ctx) return BJJ_ERR_ARG;
     HostArg args[] = {H_IN(pkx, 32), H_IN(pky, 32), H_IN(msg32, 32), H_IN(rx, 32), H_IN(ry, 32), H_IN(s32, 32), H_OUT(ok, 1),
                       H_OUT(status, 1)};
-    return run_host(ctx, n, args, 8, [&](size_t m, uint8_t** d, ComputeRef sl) -> int {
-        return launch_verify(ctx, m, d[3], d[4], d[5], d[0], d[1], d[2], d[6], sl.stream, &sl.ws, BJJ_MODE_SCHNORR, d[7], true);
+    return run_host(ctx, n, args, 8, [&](size_t m, uint8_t** d, cudaStream_t st, Workspace* ws) -> int {
+        return launch_verify(ctx, m, d[3], d[4], d[5], d[0], d[1], d[2], d[6], st, ws, BJJ_MODE_SCHNORR, d[7], true);
     }, /*heavy=*/true);
 }
 
@@ -1260,8 +1197,8 @@ int bjj_verify_compressed_batch(bjj_ctx* ctx, size_t n, const uint8_t* sig64, co
                                 const uint8_t* msg32, uint8_t* ok, uint8_t* status) {
     if (!ctx) return BJJ_ERR_ARG;
     HostArg args[] = {H_IN(sig64, 64), H_IN(pk32, 32), H_IN(msg32, 32), H_OUT(ok, 1), H_OUT(status, 1)};
-    return run_host(ctx, n, args, 5, [&](size_t m, uint8_t** d, ComputeRef sl) -> int {
-        return launch_verify_compressed(ctx, m, d[0], d[1], d[2], d[3], d[4], sl.stream, &sl.ws);
+    return run_host(ctx, n, args, 5, [&](size_t m, uint8_t** d, cudaStream_t st, Workspace* ws) -> int {
+        return launch_verify_compressed(ctx, m, d[0], d[1], d[2], d[3], d[4], st, ws);
     }, /*heavy=*/true);
 }
 

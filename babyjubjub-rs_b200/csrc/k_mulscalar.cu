@@ -30,12 +30,7 @@ __global__ void __launch_bounds__(BJJ_BLOCK) k_reduce_scalars(size_t n, const ui
 
 namespace bjjk {
 
-int mul_scalar_blocks_per_sm() {
-    int per_sm = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, (const void*)k_mul_scalar, BJJ_BLOCK, 0) != cudaSuccess || per_sm < 1)
-        per_sm = 1;
-    return per_sm;
-}
+int mul_scalar_blocks_per_sm() { return blocks_per_sm(k_mul_scalar); }
 void mul_scalar(int grid, cudaStream_t st, size_t n, const uint8_t* px, const uint8_t* py, const uint8_t* k, ProjScratch scr,
                 U128* table, ExactQueue q, uint32_t* gflags) {
     k_mul_scalar<<<grid, BJJ_BLOCK, 0, st>>>(n, px, py, k, scr, table, q, gflags);

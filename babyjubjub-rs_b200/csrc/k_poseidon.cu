@@ -13,22 +13,14 @@ __global__ void __launch_bounds__(BJJ_BLOCK, 2) k_poseidon(size_t n, PoseidonIn 
 
 namespace bjjk {
 
-template <int T>
-static int occ_t() {
-    int per_sm = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, (const void*)k_poseidon<T>, BJJ_BLOCK, 0) != cudaSuccess || per_sm < 1)
-        per_sm = 1;
-    return per_sm;
-}
-
 int poseidon_blocks_per_sm(int t) {
     switch (t) {
-        case 2: return occ_t<2>();
-        case 3: return occ_t<3>();
-        case 4: return occ_t<4>();
-        case 5: return occ_t<5>();
-        case 6: return occ_t<6>();
-        default: return occ_t<7>();
+        case 2: return blocks_per_sm(k_poseidon<2>);
+        case 3: return blocks_per_sm(k_poseidon<3>);
+        case 4: return blocks_per_sm(k_poseidon<4>);
+        case 5: return blocks_per_sm(k_poseidon<5>);
+        case 6: return blocks_per_sm(k_poseidon<6>);
+        default: return blocks_per_sm(k_poseidon<7>);
     }
 }
 

@@ -21,12 +21,7 @@ __global__ void __launch_bounds__(BJJ_BLOCK) k_sign_finish(size_t n, const uint8
 
 namespace bjjk {
 
-int sign_blocks_per_sm() {
-    int per_sm = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, (const void*)k_sign, BJJ_BLOCK, 0) != cudaSuccess || per_sm < 1)
-        per_sm = 1;
-    return per_sm;
-}
+int sign_blocks_per_sm() { return blocks_per_sm(k_sign); }
 void sign(int grid, cudaStream_t st, size_t n, const uint8_t* key, const uint8_t* msg, uint8_t* r8x, uint8_t* r8y,
           uint8_t* s32, uint8_t* status, const CombEntry* comb) {
     k_sign<<<grid, BJJ_BLOCK, 0, st>>>(n, key, msg, r8x, r8y, s32, status, comb);

@@ -191,19 +191,13 @@ __global__ void __maxnreg__(BJJ_VERIFY_EXACT_REGS) k_verify_exact(const uint8_t*
 
 namespace bjjk {
 
-static int occ(const void* k, int block) {
-    int per_sm = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k, block, 0) != cudaSuccess || per_sm < 1) per_sm = 1;
-    return per_sm;
-}
-int verify_hash_blocks_per_sm() { return occ((const void*)k_verify_hash, BJJ_BLOCK); }
+int verify_hash_blocks_per_sm() { return blocks_per_sm(k_verify_hash); }
 static const size_t kEcVmSmem = vm::slot_bytes(BJJ_EC_VM_SLOTS);
 int verify_ec_blocks_per_sm() {
     static int per_sm = [] {
         cudaFuncSetAttribute((const void*)k_verify_ec_vm, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kEcVmSmem);
         cudaFuncSetAttribute((const void*)k_verify_ec_vm, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
-        int v = 0;
-        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&v, (const void*)k_verify_ec_vm, BJJ_VM_THREADS, kEcVmSmem) != cudaSuccess || v < 1) v = 1;
+        int v = blocks_per_sm(k_verify_ec_vm, BJJ_VM_THREADS, kEcVmSmem);
         // BJJ_EC_CTAS_PER_SM=n (experiments): fewer resident CTAs than fit, e.g. to leave registers for the exact-lane kernel
         if (const char* e = getenv("BJJ_EC_CTAS_PER_SM")) {
             const int cap = atoi(e);
@@ -214,7 +208,7 @@ int verify_ec_blocks_per_sm() {
     return per_sm;
 }
 
-int verify_split_blocks_per_sm() { return occ((const void*)k_verify_split, BJJ_BLOCK); }
+int verify_split_blocks_per_sm() { return blocks_per_sm(k_verify_split); }
 
 void verify_hash(int grid, cudaStream_t st, size_t n, const uint8_t* r8x, const uint8_t* r8y, const uint8_t* ax,
                  const uint8_t* ay, const uint8_t* msg, const uint8_t* s_base, size_t s_stride, size_t s_off,

@@ -47,7 +47,16 @@ struct PoseidonIn {
 
 namespace bjjk {
 
-// resident CTAs per SM of the kernel (cudaOccupancyMaxActiveBlocksPerMultiprocessor), >= 1
+// resident CTAs per SM of `kernel` launched with `block` threads and `smem` bytes of dynamic shared memory, >= 1
+template <class Kernel>
+inline int blocks_per_sm(Kernel* kernel, int block = BJJ_BLOCK, size_t smem = 0) {
+    int per_sm = 0;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, (const void*)kernel, block, smem) != cudaSuccess || per_sm < 1)
+        per_sm = 1;
+    return per_sm;
+}
+
+// blocks_per_sm of the kernels behind the launch wrappers below
 int verify_hash_blocks_per_sm();
 int verify_ec_blocks_per_sm();
 int verify_split_blocks_per_sm();
