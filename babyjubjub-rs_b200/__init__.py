@@ -13,11 +13,14 @@ follow the reference's public API (paths into the reference tree):
     verify(pk, sig, msg)                                   src/lib.rs:395-412
     + the batch entry points the north star adds: mul_scalar_batch, public_batch,
       decompress_batch, verify_batch (and add/compress/poseidon/fixed-base batches).
+    + FixedBase / mul_fixed_base_batch / mul2_fixed_base_batch: k*P and k*P + l*Q on a
+      precomputed table of a caller-chosen point P (the comb path B8 uses).
 
 Every call runs on the GPU through libbjj_cuda.so; there is no CPU fallback -- importing works
 without a GPU (so the ABI can be inspected), creating an Engine does not.
 """
 import ctypes
+import weakref
 
 import numpy as np
 
@@ -80,9 +83,12 @@ class Engine:
             raise BjjError(rc, "bjj_init", self.lib.bjj_error_string(rc).decode())
         self.ctx = ctx
         self.device = int(device)
+        self._bases = weakref.WeakSet()     # FixedBase tables of this context: freed before the context
 
     def close(self):
         if getattr(self, "ctx", None):
+            for b in list(self._bases):
+                b.close()
             self.lib.bjj_destroy(self.ctx)
             self.ctx = None
 
@@ -167,6 +173,24 @@ class Engine:
                     "bjj_fixed_base_batch")
         return tuple(outs)
 
+    def base_mul_batch(self, base, scalars):
+        """k*P for every 256-bit scalar k (raw, unreduced); base: a FixedBase of this engine, or None for B8"""
+        k = _as_u8(scalars, 32)
+        rx, ry = np.empty_like(k), np.empty_like(k)
+        self._check(self.lib.bjj_base_mul_batch(self.ctx, _handle(base), len(k), _ptr(k), _ptr(rx), _ptr(ry)),
+                    "bjj_base_mul_batch")
+        return rx, ry
+
+    def base_mul2_batch(self, p, ks, q, ls):
+        """k*P + l*Q lane by lane; p, q: FixedBase tables of this engine, or None for B8"""
+        k, l = _as_u8(ks, 32), _as_u8(ls, 32)
+        if len(k) != len(l):
+            raise ValueError("k and l differ in length")
+        rx, ry = np.empty_like(k), np.empty_like(k)
+        self._check(self.lib.bjj_base_mul2_batch(self.ctx, _handle(p), _handle(q), len(k), _ptr(k), _ptr(l), _ptr(rx),
+                                                 _ptr(ry)), "bjj_base_mul2_batch")
+        return rx, ry
+
     def public_batch(self, keys):
         k = _as_u8(keys, 32)
         outs = [np.empty_like(k) for _ in range(2)]
@@ -241,6 +265,57 @@ def default_engine():
     if _default_engine is None:
         _default_engine = Engine(0)
     return _default_engine
+
+
+class FixedBase:
+    """The comb table of one on-curve point P on one Engine (50 MB of device memory): P.mul_scalar(k) for many k at the
+    rate of B8's fixed-base path.  Raises BjjError with code 2 (BJJ_ERR_ARG) for an off-curve P -- whose reference
+    result depends on mul_scalar's exact double-and-add order, so it stays on mul_scalar_batch -- and with code 3
+    (BJJ_ERR_NONCANONICAL) for a coordinate >= Q.  Free it with close() (or let it be collected)."""
+
+    def __init__(self, point, engine=None):
+        self.engine = engine or default_engine()
+        x, y = (point.x, point.y) if isinstance(point, Point) else point
+        self.point = Point(x, y)
+        px, py = ints_to_le32([x]), ints_to_le32([y])
+        handle = ctypes.c_void_p()
+        rc = self.engine.lib.bjj_base_create(self.engine.ctx, _ptr(px), _ptr(py), ctypes.byref(handle))
+        if rc != 0:
+            self.engine._check(rc, "bjj_base_create")
+        self.handle = handle
+        self.engine._bases.add(self)
+
+    def close(self):
+        if getattr(self, "handle", None):
+            self.engine.lib.bjj_base_destroy(self.engine.ctx, self.handle)
+            self.handle = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def mul_batch(self, scalars):
+        """[P.mul_scalar(k) for k in scalars] (src/lib.rs:149-164) for Python ints of any size and sign"""
+        rx, ry = self.engine.base_mul_batch(self, ints_to_le32([_base_scalar(k) for k in scalars]))
+        return [Point(x, y) for x, y in zip(le32_to_ints(rx), le32_to_ints(ry))]
+
+
+def _handle(base):
+    if base is None:
+        return None
+    if not base.handle:
+        raise ValueError("FixedBase is closed")
+    return base.handle
+
+
+def _base_scalar(k):
+    """k as it crosses the 256-bit ABI of the fixed-base tables.  The reference multiplies by |k| (the sign is dropped,
+    src/lib.rs:156); every on-curve point has an order dividing ORDER, so a wider |k| is reduced mod ORDER -- the same
+    point.  Values below 2^256 go through unreduced."""
+    k = abs(int(k))
+    return k if k < (1 << 256) else k % ORDER
 
 
 # ---- the reference's public API, as batches of one -------------------------------------------------
@@ -426,6 +501,36 @@ def mul_scalar_batch(points, scalars, engine=None):
             raise ValueError("scalars wider than 2048 bits are not supported by the device ABI")
         buf = np.frombuffer(b"".join(k.to_bytes(4 * words, "little") for k in ks), dtype=np.uint8).reshape(-1, 4 * words)
         rx, ry = eng.mul_scalar_wide_batch(px, py, buf, words)
+    return [Point(x, y) for x, y in zip(le32_to_ints(rx), le32_to_ints(ry))]
+
+
+def mul_fixed_base_batch(point, scalars, engine=None):
+    """[point.mul_scalar(k) for k in scalars] on a table of the on-curve `point` (built for this call, then freed).
+    Keep a FixedBase to reuse the table across calls."""
+    base = FixedBase(point, engine)
+    try:
+        return base.mul_batch(scalars)
+    finally:
+        base.close()
+
+
+def mul2_fixed_base_batch(p, ks, q, ls, engine=None):
+    """[(k*p).projective().add((l*q).projective()).affine() for k, l in zip(ks, ls)] (src/lib.rs:70-131, 149-164) for
+    on-curve p, q.  Each of p, q is a Point (its table is built for this call), a FixedBase, or None for B8."""
+    eng = engine or default_engine()
+    built = []
+    try:
+        def table(b):
+            if b is None or isinstance(b, FixedBase):
+                return b
+            built.append(FixedBase(b, eng))
+            return built[-1]
+        tp, tq = table(p), table(q)
+        rx, ry = eng.base_mul2_batch(tp, ints_to_le32([_base_scalar(k) for k in ks]), tq,
+                                     ints_to_le32([_base_scalar(l) for l in ls]))
+    finally:
+        for b in built:
+            b.close()
     return [Point(x, y) for x, y in zip(le32_to_ints(rx), le32_to_ints(ry))]
 
 

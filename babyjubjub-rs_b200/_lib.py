@@ -9,6 +9,7 @@ _u8p = ctypes.c_void_p
 _sz = ctypes.c_size_t
 _ctx = ctypes.c_void_p
 _int = ctypes.c_int
+_base = ctypes.c_void_p     # bjj_base*: a fixed-base table (NULL selects B8)
 
 # symbol -> (restype, argtypes); the single source the ABI test checks against include/bjj_cuda.h
 SIGNATURES = {
@@ -43,6 +44,10 @@ SIGNATURES = {
     "bjj_verify_batch": (_int, [_ctx, _sz] + [_u8p] * 7),
     "bjj_verify_compressed_batch": (_int, [_ctx, _sz] + [_u8p] * 5),
     "bjj_verify_schnorr_batch": (_int, [_ctx, _sz] + [_u8p] * 8),
+    "bjj_base_create": (_int, [_ctx, _u8p, _u8p, ctypes.POINTER(_base)]),
+    "bjj_base_destroy": (None, [_ctx, _base]),
+    "bjj_base_mul_batch": (_int, [_ctx, _base, _sz] + [_u8p] * 3),
+    "bjj_base_mul2_batch": (_int, [_ctx, _base, _base, _sz] + [_u8p] * 4),
 }
 # every batch op also has a device-pointer flavour with a trailing `void* stream`
 for _name in [k for k in SIGNATURES if k.endswith("_batch")]:

@@ -34,6 +34,15 @@ __global__ void __launch_bounds__(BJJ_BLOCK) k_comb_build(CombEntry* comb) {
     comb_build_entry(comb, w, j);
 }
 
+// the table of the caller point (px, py) (bjj_base_create); thread 0 writes the BJJ_BASE_* outcome to *status
+__global__ void __launch_bounds__(BJJ_BLOCK) k_comb_build_point(CombEntry* comb, const uint8_t* px, const uint8_t* py,
+                                                                uint32_t* status) {
+    size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (idx >= BJJ_COMB_TOTAL) return;
+    const uint32_t st = lane_comb_build_point(comb, (int)(idx / BJJ_COMB_ENTRIES), (int)(idx % BJJ_COMB_ENTRIES), px, py);
+    if (idx == 0) *status = st;
+}
+
 __global__ void __launch_bounds__(BJJ_BLOCK) k_split_scalars(size_t n, const uint8_t* h32, const uint8_t* s32, uint8_t* u32,
                                                              uint8_t* v32, uint8_t* w32) {
     BJJ_LANE_LOOP(n) lane_split_scalars(h32, s32, u32, v32, w32, i);
@@ -80,6 +89,12 @@ __global__ void __launch_bounds__(BJJ_BLOCK) k_batch_affine(size_t n, ProjScratc
 __global__ void __launch_bounds__(BJJ_BLOCK, 2) k_fixed_base(size_t n, const uint8_t* k, ProjScratch scr,
                                                           const CombEntry* comb, unsigned long long* work) {
     BJJ_POINT_LOOP(n, work) lane_fixed_base(k, scr, i, comb);
+}
+
+__global__ void __launch_bounds__(BJJ_BLOCK, 2) k_fixed_base2(size_t n, const uint8_t* k, const uint8_t* l, ProjScratch scr,
+                                                           const CombEntry* comb_p, const CombEntry* comb_q,
+                                                           unsigned long long* work) {
+    BJJ_POINT_LOOP(n, work) lane_fixed_base2(k, l, scr, i, comb_p, comb_q);
 }
 
 #ifndef BJJ_PUBLIC_BALLAST
@@ -176,6 +191,12 @@ struct bjj_ctx {
     bool public_fused;          // BJJ_PUBLIC_FUSED=1: PrivateKey::public as ONE kernel (k_public) instead of k_scalar_key + k_fixed_base
     size_t lane_hint;           // host flavour: the largest chunk of the running call, so that lane-sized scratch is
                                 // allocated ONCE up front (a cudaFree in mid-pipeline is a device-wide synchronisation)
+};
+
+// the comb table of a caller point, on the device of the context that built it
+struct bjj_base {
+    bjj_ctx* ctx;
+    CombEntry* comb;
 };
 
 #define CU(ctx, call)                      \
@@ -478,6 +499,63 @@ int bjj_sync(bjj_ctx* ctx) {
 
 }  // extern "C"
 
+// builds the table of (px32, py32) into a new *comb and leaves the BJJ_BASE_* outcome in *status; `io` is device
+// scratch of 80 bytes (the point in, the outcome out)
+static int build_base_comb(bjj_ctx* ctx, const uint8_t* px32, const uint8_t* py32, uint8_t* io, CombEntry** comb,
+                           uint32_t* status) {
+    CU(ctx, cudaMalloc(comb, BJJ_COMB_TOTAL * sizeof(CombEntry)));
+    CU(ctx, cudaMemcpyAsync(io, px32, 32, cudaMemcpyHostToDevice, ctx->stream));
+    CU(ctx, cudaMemcpyAsync(io + 32, py32, 32, cudaMemcpyHostToDevice, ctx->stream));
+    const size_t total = BJJ_COMB_TOTAL;
+    k_comb_build_point<<<(total + BJJ_BLOCK - 1) / BJJ_BLOCK, BJJ_BLOCK, 0, ctx->stream>>>(*comb, io, io + 32, (uint32_t*)(io + 64));
+    TRY(launched(ctx));
+    CU(ctx, cudaMemcpyAsync(status, io + 64, sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+    CU(ctx, cudaStreamSynchronize(ctx->stream));
+    return BJJ_OK;
+}
+
+// the table that `base` names for a call on ctx: B8's for NULL, nullptr for a handle of another context
+static const CombEntry* base_comb(bjj_ctx* ctx, const bjj_base* base) {
+    if (!base) return ctx->comb;
+    return base->ctx == ctx ? base->comb : nullptr;
+}
+
+extern "C" {
+
+int bjj_base_create(bjj_ctx* ctx, const uint8_t* px32, const uint8_t* py32, bjj_base** out) {
+    if (!out) return BJJ_ERR_ARG;
+    *out = nullptr;
+    if (!ctx || !px32 || !py32) return BJJ_ERR_ARG;
+    CU(ctx, cudaSetDevice(ctx->device));
+    uint8_t* io = nullptr;
+    CU(ctx, cudaMalloc(&io, 80));
+    CombEntry* comb = nullptr;
+    uint32_t status = BJJ_BASE_OK;
+    int rc = build_base_comb(ctx, px32, py32, io, &comb, &status);
+    cudaFree(io);
+    if (rc == BJJ_OK && status != BJJ_BASE_OK) rc = status == BJJ_BASE_NONCANONICAL ? BJJ_ERR_NONCANONICAL : BJJ_ERR_ARG;
+    bjj_base* b = rc == BJJ_OK ? (bjj_base*)malloc(sizeof(bjj_base)) : nullptr;
+    if (rc == BJJ_OK && !b) rc = BJJ_ERR_NOMEM;
+    if (rc != BJJ_OK) {
+        if (comb) cudaFree(comb);
+        return rc;
+    }
+    b->ctx = ctx;
+    b->comb = comb;
+    *out = b;
+    return BJJ_OK;
+}
+
+void bjj_base_destroy(bjj_ctx* ctx, bjj_base* base) {
+    if (!ctx || !base || base->ctx != ctx) return;
+    cudaSetDevice(ctx->device);
+    cudaDeviceSynchronize();      // calls on any stream may still read the table
+    cudaFree(base->comb);
+    free(base);
+}
+
+}  // extern "C"
+
 // ---------------------------------------------------------------------------------------------------
 // device-pointer flavour: one launch per call
 // ---------------------------------------------------------------------------------------------------
@@ -569,6 +647,25 @@ static int launch_fixed_base(bjj_ctx* ctx, size_t n, const uint8_t* in, uint8_t*
             }
             k_fixed_base<<<grid_for(ctx, k_fixed_base, m), BJJ_BLOCK, 0, st>>>(m, k, scr, ctx->comb, work);
         }
+        TRY(launched(ctx));
+        k_batch_affine<<<affine_grid(ctx, m), BJJ_BLOCK, 0, st>>>(m, scr, rx + o, ry + o);
+        return launched(ctx);
+    });
+}
+// k * P (l == nullptr) or k * P + l * Q over the tables comb_p, comb_q (bjj_base_mul*)
+static int launch_base_mul(bjj_ctx* ctx, size_t n, const uint8_t* k, const uint8_t* l, const CombEntry* comb_p,
+                           const CombEntry* comb_q, uint8_t* rx, uint8_t* ry, cudaStream_t st, Workspace* ws) {
+    const size_t lanes = scratch_lanes(ctx, n);
+    return for_each_subbatch(n, [&](size_t off, size_t m) -> int {
+        const size_t o = 32 * off;
+        ProjScratch scr;
+        TRY(ensure_proj(ctx, ws, lanes, &scr));
+        unsigned long long* work = nullptr;
+        TRY(claim_counter(ctx, ws, st, &work));
+        if (l)
+            k_fixed_base2<<<grid_for(ctx, k_fixed_base2, m), BJJ_BLOCK, 0, st>>>(m, k + o, l + o, scr, comb_p, comb_q, work);
+        else
+            k_fixed_base<<<grid_for(ctx, k_fixed_base, m), BJJ_BLOCK, 0, st>>>(m, k + o, scr, comb_p, work);
         TRY(launched(ctx));
         k_batch_affine<<<affine_grid(ctx, m), BJJ_BLOCK, 0, st>>>(m, scr, rx + o, ry + o);
         return launched(ctx);
@@ -811,6 +908,22 @@ int bjj_public_batch_dev(bjj_ctx* ctx, size_t n, const uint8_t* key32, uint8_t* 
     DEV_PROLOGUE
     if (!key32 || !rx || !ry) return BJJ_ERR_ARG;
     return launch_fixed_base(ctx, n, key32, rx, ry, true, st, &ctx->ws);
+}
+
+int bjj_base_mul_batch_dev(bjj_ctx* ctx, const bjj_base* base, size_t n, const uint8_t* scalar32, uint8_t* rx, uint8_t* ry,
+                           void* stream) {
+    DEV_PROLOGUE
+    const CombEntry* comb = base_comb(ctx, base);
+    if (!comb || !scalar32 || !rx || !ry) return BJJ_ERR_ARG;
+    return launch_base_mul(ctx, n, scalar32, nullptr, comb, nullptr, rx, ry, st, &ctx->ws);
+}
+
+int bjj_base_mul2_batch_dev(bjj_ctx* ctx, const bjj_base* p, const bjj_base* q, size_t n, const uint8_t* k32,
+                            const uint8_t* l32, uint8_t* rx, uint8_t* ry, void* stream) {
+    DEV_PROLOGUE
+    const CombEntry *comb_p = base_comb(ctx, p), *comb_q = base_comb(ctx, q);
+    if (!comb_p || !comb_q || !k32 || !l32 || !rx || !ry) return BJJ_ERR_ARG;
+    return launch_base_mul(ctx, n, k32, l32, comb_p, comb_q, rx, ry, st, &ctx->ws);
 }
 
 int bjj_sign_batch_dev(bjj_ctx* ctx, size_t n, const uint8_t* key32, const uint8_t* msg32, uint8_t* r8x, uint8_t* r8y,
@@ -1128,6 +1241,27 @@ int bjj_public_batch(bjj_ctx* ctx, size_t n, const uint8_t* key32, uint8_t* rx, 
     HostArg args[] = {H_IN(key32, 32), H_OUT(rx, 32), H_OUT(ry, 32)};
     return run_host(ctx, n, args, 3, [&](size_t m, uint8_t** d, cudaStream_t st, Workspace* ws) -> int {
         return launch_fixed_base(ctx, m, d[0], d[1], d[2], true, st, ws);
+    });
+}
+
+int bjj_base_mul_batch(bjj_ctx* ctx, const bjj_base* base, size_t n, const uint8_t* scalar32, uint8_t* rx, uint8_t* ry) {
+    if (!ctx) return BJJ_ERR_ARG;
+    const CombEntry* comb = base_comb(ctx, base);
+    if (!comb) return BJJ_ERR_ARG;
+    HostArg args[] = {H_IN(scalar32, 32), H_OUT(rx, 32), H_OUT(ry, 32)};
+    return run_host(ctx, n, args, 3, [&](size_t m, uint8_t** d, cudaStream_t st, Workspace* ws) -> int {
+        return launch_base_mul(ctx, m, d[0], nullptr, comb, nullptr, d[1], d[2], st, ws);
+    });
+}
+
+int bjj_base_mul2_batch(bjj_ctx* ctx, const bjj_base* p, const bjj_base* q, size_t n, const uint8_t* k32, const uint8_t* l32,
+                        uint8_t* rx, uint8_t* ry) {
+    if (!ctx) return BJJ_ERR_ARG;
+    const CombEntry *comb_p = base_comb(ctx, p), *comb_q = base_comb(ctx, q);
+    if (!comb_p || !comb_q) return BJJ_ERR_ARG;
+    HostArg args[] = {H_IN(k32, 32), H_IN(l32, 32), H_OUT(rx, 32), H_OUT(ry, 32)};
+    return run_host(ctx, n, args, 4, [&](size_t m, uint8_t** d, cudaStream_t st, Workspace* ws) -> int {
+        return launch_base_mul(ctx, m, d[0], d[1], comb_p, comb_q, d[2], d[3], st, ws);
     });
 }
 

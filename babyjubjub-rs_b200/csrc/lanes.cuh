@@ -128,10 +128,11 @@ BJJ_HD void table_select(Niels& n, const LaneTable& t, int d) {
     niels_cneg(n, d < 0);
 }
 
-// ---- fixed-base comb for B8 ------------------------------------------------------------------------
+// ---- fixed-base comb for B8 (and for caller points, bjj_base_create) ------------------------------------
 // comb[w][j] = j * 65536^w * B8 as affine Niels (y+x, y-x, 2d'xy) on the a = -1 model, j = 0..32768,
 // w = 0..16 (w = 16 only holds j = 0, 1 for the recoding carry): 16 x 32,769 x 96 B = 50 MB, L2-resident,
-// gathered with ld.global.nc.  Built once per context on the device (k_comb_build, ~15 ms).  Signed 16-bit
+// gathered with ld.global.nc.  Built once per context on the device (k_comb_build, ~15 ms); a caller point's table
+// is the same with B8 replaced by that point (k_comb_build_point).  Signed 16-bit
 // digits make a fixed-base multiplication 17 mixed additions and no doubling; verify adds its B8 term (w * B8, the
 // one full-width scalar left after the split) the same way, after the Straus pass over the two per-lane points.
 #define BJJ_COMB_BITS 16
@@ -173,16 +174,18 @@ BJJ_HD void comb_select(NielsAff& n, const CombEntry* comb, int w, int d) {
     niels_aff_cneg(n, d < 0);
 }
 
-// acc = k * B8 for a 256-bit k: 17 mixed additions, no doublings.  BJJ_COMB_PREFETCH: the entry of window w - 1 is
-// requested before the addition of window w, so that its L2 latency (the 50 MB table is gathered at random) runs
+// acc += k * base (comb = the table of base) for a 256-bit k: 17 mixed additions, no doublings.  `from_identity` starts
+// acc at the identity, after the recoding as fixed_base_comb always did (so its kernels compile as before);
+// lane_fixed_base2 runs two walks over two tables into one accumulator.  BJJ_COMB_PREFETCH: the entry of window w - 1
+// is requested before the addition of window w, so that its L2 latency (the 50 MB table is gathered at random) runs
 // under ~900 multiplier instructions instead of in front of them.
 #ifndef BJJ_COMB_PREFETCH
 #define BJJ_COMB_PREFETCH 1
 #endif
-BJJ_HD void fixed_base_comb(PointExt& acc, const CombEntry* comb, const uint32_t* k) {
+BJJ_HD void fixed_base_comb_acc(PointExt& acc, const CombEntry* comb, const uint32_t* k, bool from_identity = false) {
     Recode16 rc;
     recode16(rc, k);
-    ext_identity(acc);
+    if (from_identity) ext_identity(acc);
 #if BJJ_COMB_PREFETCH
     NielsAff cur, nxt;
     int d = (int)rc.top;
@@ -209,15 +212,16 @@ BJJ_HD void fixed_base_comb(PointExt& acc, const CombEntry* comb, const uint32_t
     }
 #endif
 }
+BJJ_HD void fixed_base_comb(PointExt& acc, const CombEntry* comb, const uint32_t* k) {
+    fixed_base_comb_acc(acc, comb, k, true);
+}
 
-// one comb entry: j * 65536^w * B8   (init kernel; one thread per (w, j))
-BJJ_HD void comb_build_entry(CombEntry* comb, int w, int j) {
+// one comb entry: j * 65536^w * p for an on-curve p of the original curve   (one thread per (w, j)).  Every on-curve
+// point has an order dividing ORDER < 2^254, so the table serves every 256-bit scalar like B8's does.
+BJJ_HD void comb_build_entry(CombEntry* comb, int w, int j, const PointAff& p) {
     CombEntry* e = comb + (size_t)w * BJJ_COMB_ENTRIES + j;
-    PointAff b8;
-    b8.x = fr_const(BJJ_B8X_M);
-    b8.y = fr_const(BJJ_B8Y_M);
     PointExt base, acc;
-    ext_from_affine(base, b8);
+    ext_from_affine(base, p);
 #pragma unroll 1
     for (int i = 0; i < BJJ_COMB_BITS * w; i++) ext_dbl<true>(base, base);
     ext_identity(acc);
@@ -249,6 +253,18 @@ BJJ_HD void comb_build_entry(CombEntry* comb, int w, int j) {
         e->t2d[i] = t.v[i];
     }
 }
+// the context's B8 table (k_comb_build)
+BJJ_HD void comb_build_entry(CombEntry* comb, int w, int j) {
+    PointAff b8;
+    b8.x = fr_const(BJJ_B8X_M);
+    b8.y = fr_const(BJJ_B8Y_M);
+    comb_build_entry(comb, w, j, b8);
+}
+
+// outcome of building a caller point's table (k_comb_build_point)
+#define BJJ_BASE_OK 0
+#define BJJ_BASE_OFF_CURVE 1
+#define BJJ_BASE_NONCANONICAL 2
 
 // ---- affine output ------------------------------------------------------------------------------------
 // a = -1 extended -> canonical affine bytes on the original curve (Fermat inverse per lane)
@@ -541,6 +557,33 @@ BJJ_HD void lane_fixed_base(const uint8_t* scalar, const ProjScratch& scr, size_
     PointExt acc;
     fixed_base_comb(acc, comb, k);
     store_ext_scratch(scr, i, acc);
+}
+
+// (k * P).projective().add((l * Q).projective()).affine() (src/lib.rs:70-131, 149-164) for on-curve P, Q with tables
+// comb_p, comb_q: both products are group elements and the reference's addition is complete on the curve, so the
+// result is the group sum, accumulated in one point (34 mixed additions)
+BJJ_HD void lane_fixed_base2(const uint8_t* k, const uint8_t* l, const ProjScratch& scr, size_t i, const CombEntry* comb_p,
+                             const CombEntry* comb_q) {
+    uint32_t s[8];
+    PointExt acc;
+    ext_identity(acc);
+    load_u256(s, k, i);
+    fixed_base_comb_acc(acc, comb_p, s);
+    load_u256(s, l, i);
+    fixed_base_comb_acc(acc, comb_q, s);
+    store_ext_scratch(scr, i, acc);
+}
+
+// entry (w, j) of the table of the caller point (px, py) (bytes of element 0): every thread checks the point, builds
+// its entry only for a valid one, and returns the BJJ_BASE_* outcome
+BJJ_HD uint32_t lane_comb_build_point(CombEntry* comb, int w, int j, const uint8_t* px, const uint8_t* py) {
+    PointAff p;
+    uint32_t flags = 0;
+    load_fr(p.x, px, 0, flags);
+    load_fr(p.y, py, 0, flags);
+    const uint32_t st = flags ? BJJ_BASE_NONCANONICAL : on_curve(p) ? BJJ_BASE_OK : BJJ_BASE_OFF_CURVE;
+    if (st == BJJ_BASE_OK) comb_build_entry(comb, w, j, p);
+    return st;
 }
 
 // PrivateKey::public (src/lib.rs:304-306) = B8 * scalar_key(key)

@@ -13,6 +13,7 @@
 //   verify(pk, sig, msg)                   src/lib.rs:395-412
 //   verify_schnorr(pk, m, r, s)            src/lib.rs:375-385
 //   + batch entry points: mul_scalar_batch, public_batch, decompress_batch, verify_batch
+//   + FixedBase: the comb table of a caller-chosen point, k*P and k*P + l*Q at the fixed-base rate
 //   + MultiGpu: shards a batch over every device, one host thread + one bjj_ctx per device, no NCCL
 //
 // Header-only; link with -lbjj_cuda.  There is no CPU fallback: Engine's constructor throws when no
@@ -224,6 +225,51 @@ inline std::vector<Point> public_batch(const std::vector<PrivateKey>& keys, Engi
     }
     return out;
 }
+
+// The comb table of one on-curve point P on an Engine (50 MB of device memory, freed by the destructor): P.mul_scalar(k)
+// for many k at the rate of B8's fixed-base path.  Throws Error with BJJ_ERR_ARG for an off-curve P (use
+// mul_scalar_batch there) and BJJ_ERR_NONCANONICAL for a coordinate >= Q.  Must not outlive its Engine.
+class FixedBase {
+  public:
+    FixedBase(const Point& p, Engine& e = default_engine()) : e_(e) {
+        Engine::check(bjj_base_create(e.ctx(), p.x.data(), p.y.data(), &base_), "bjj_base_create");
+    }
+    ~FixedBase() { bjj_base_destroy(e_.ctx(), base_); }
+    FixedBase(const FixedBase&) = delete;
+    FixedBase& operator=(const FixedBase&) = delete;
+    const bjj_base* raw() const { return base_; }
+
+    // [P.mul_scalar(k) for k in scalars]; scalars are raw 256-bit values (reduce wider ones mod ORDER)
+    std::vector<Point> mul_batch(const std::vector<U256>& scalars) const {
+        const size_t n = scalars.size();
+        auto k = pack(scalars);
+        std::vector<uint8_t> rx(32 * n), ry(32 * n);
+        Engine::check(bjj_base_mul_batch(e_.ctx(), base_, n, k.data(), rx.data(), ry.data()), "bjj_base_mul_batch");
+        return points(rx, ry);
+    }
+    // k[i]*P + l[i]*q (src/lib.rs:70-131); q == nullptr selects B8
+    std::vector<Point> mul2_batch(const std::vector<U256>& k, const FixedBase* q, const std::vector<U256>& l) const {
+        if (k.size() != l.size()) throw std::invalid_argument("k and l differ in length");
+        const size_t n = k.size();
+        auto kb = pack(k), lb = pack(l);
+        std::vector<uint8_t> rx(32 * n), ry(32 * n);
+        Engine::check(bjj_base_mul2_batch(e_.ctx(), base_, q ? q->raw() : nullptr, n, kb.data(), lb.data(), rx.data(), ry.data()),
+                      "bjj_base_mul2_batch");
+        return points(rx, ry);
+    }
+
+  private:
+    static std::vector<Point> points(const std::vector<uint8_t>& rx, const std::vector<uint8_t>& ry) {
+        std::vector<Point> out(rx.size() / 32);
+        for (size_t i = 0; i < out.size(); i++) {
+            std::memcpy(out[i].x.data(), &rx[32 * i], 32);
+            std::memcpy(out[i].y.data(), &ry[32 * i], 32);
+        }
+        return out;
+    }
+    Engine& e_;
+    bjj_base* base_ = nullptr;
+};
 
 struct DecompressResult {
     Point point;

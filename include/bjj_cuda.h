@@ -133,6 +133,32 @@ int bjj_mul_scalar_wide_batch_dev(bjj_ctx* ctx, size_t n, const uint8_t* px, con
 int bjj_fixed_base_batch(bjj_ctx* ctx, size_t n, const uint8_t* scalar32, uint8_t* rx, uint8_t* ry);
 int bjj_fixed_base_batch_dev(bjj_ctx* ctx, size_t n, const uint8_t* scalar32, uint8_t* rx, uint8_t* ry, void* stream);
 
+/* ---- fixed-base tables for caller-chosen points: P.mul_scalar(k) and k*P + l*Q on the comb path ------
+ * A bjj_base is the comb table of one on-curve point P, the same 50 MB of device memory as the context's B8 table,
+ * so k*P costs what B8.mul_scalar(k) costs instead of mul_scalar's variable-base ladder.  It pays off for many
+ * scalars against one point (commitments m*G + r*H, ElGamal to one recipient, any repeated P.mul_scalar(k_i)).
+ *   - bjj_base_create builds the table on the device, synchronously on the ctx stream (one kernel).  The handle
+ *     belongs to ctx: it holds device memory of ctx's device until bjj_base_destroy, which must come before
+ *     bjj_destroy(ctx).  A call that passes it with another context returns BJJ_ERR_ARG.
+ *   - P must be on the curve: an off-curve point returns BJJ_ERR_ARG and *out = NULL.  (The reference's result for
+ *     an off-curve point depends on its exact double-and-add order, which no table reproduces; such callers keep
+ *     bjj_mul_scalar_batch, which replays it.)  A coordinate >= Q returns BJJ_ERR_NONCANONICAL and no handle.
+ *   - Scalars are raw 256-bit values, unreduced, like bjj_fixed_base_batch's: every on-curve point has an order
+ *     dividing ORDER, so every k (0, >= ORDER, points with a torsion component) gives the reference's result.
+ *   - base == NULL (p / q == NULL) selects the context's B8 table. */
+typedef struct bjj_base bjj_base;
+int bjj_base_create(bjj_ctx* ctx, const uint8_t* px32, const uint8_t* py32, bjj_base** out);
+void bjj_base_destroy(bjj_ctx* ctx, bjj_base* base);   /* waits for the device, then frees; NULL is a no-op */
+/* r = k*P  (Point::mul_scalar, src/lib.rs:149-164) */
+int bjj_base_mul_batch(bjj_ctx* ctx, const bjj_base* base, size_t n, const uint8_t* scalar32, uint8_t* rx, uint8_t* ry);
+int bjj_base_mul_batch_dev(bjj_ctx* ctx, const bjj_base* base, size_t n, const uint8_t* scalar32, uint8_t* rx,
+                           uint8_t* ry, void* stream);
+/* r = (k*P).projective().add((l*Q).projective()).affine()  (src/lib.rs:70-131, 149-164) */
+int bjj_base_mul2_batch(bjj_ctx* ctx, const bjj_base* p, const bjj_base* q, size_t n, const uint8_t* k32,
+                        const uint8_t* l32, uint8_t* rx, uint8_t* ry);
+int bjj_base_mul2_batch_dev(bjj_ctx* ctx, const bjj_base* p, const bjj_base* q, size_t n, const uint8_t* k32,
+                            const uint8_t* l32, uint8_t* rx, uint8_t* ry, void* stream);
+
 /* ---- PrivateKey::public (src/lib.rs:304-306) = B8 * scalar_key(key);  scalar_key (:284-302) ------ */
 int bjj_public_batch(bjj_ctx* ctx, size_t n, const uint8_t* key32, uint8_t* rx, uint8_t* ry);
 int bjj_public_batch_dev(bjj_ctx* ctx, size_t n, const uint8_t* key32, uint8_t* rx, uint8_t* ry, void* stream);

@@ -8,6 +8,10 @@ pub struct bjj_ctx {
     _private: [u8; 0],
 }
 #[repr(C)]
+pub struct bjj_base {
+    _private: [u8; 0],
+}
+#[repr(C)]
 pub struct bjj_multi {
     _private: [u8; 0],
 }
@@ -54,6 +58,15 @@ extern "C" {
                                      scalar_words: c_int, rx: *mut u8, ry: *mut u8) -> c_int;
     // B8.mul_scalar (src/lib.rs:305,329,405)
     pub fn bjj_fixed_base_batch(ctx: *mut bjj_ctx, n: usize, scalar32: *const u8, rx: *mut u8, ry: *mut u8) -> c_int;
+    // comb table of a caller-chosen on-curve point (50 MB of device memory, owned by ctx); NULL base = B8
+    pub fn bjj_base_create(ctx: *mut bjj_ctx, px32: *const u8, py32: *const u8, out: *mut *mut bjj_base) -> c_int;
+    pub fn bjj_base_destroy(ctx: *mut bjj_ctx, base: *mut bjj_base);
+    // P.mul_scalar(k) (src/lib.rs:149-164) on the table of P
+    pub fn bjj_base_mul_batch(ctx: *mut bjj_ctx, base: *const bjj_base, n: usize, scalar32: *const u8, rx: *mut u8,
+                              ry: *mut u8) -> c_int;
+    // (k*P).projective().add((l*Q).projective()).affine() (src/lib.rs:70-131, 149-164)
+    pub fn bjj_base_mul2_batch(ctx: *mut bjj_ctx, p: *const bjj_base, q: *const bjj_base, n: usize, k32: *const u8,
+                               l32: *const u8, rx: *mut u8, ry: *mut u8) -> c_int;
     // PrivateKey::public / scalar_key / sign (src/lib.rs:284-342)
     pub fn bjj_public_batch(ctx: *mut bjj_ctx, n: usize, key32: *const u8, rx: *mut u8, ry: *mut u8) -> c_int;
     pub fn bjj_scalar_key_batch(ctx: *mut bjj_ctx, n: usize, key32: *const u8, scalar32: *mut u8) -> c_int;

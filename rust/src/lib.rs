@@ -5,7 +5,8 @@
 //!
 //! The public names follow arnaucube/babyjubjub-rs 0.0.11: `Point`, `PointProjective`, `Signature`,
 //! `PrivateKey`, `decompress_point`, `decompress_signature`, `verify`, plus the batch entry points
-//! `mul_scalar_batch`, `public_batch`, `decompress_batch`, `verify_batch`.  `Fr` is carried as its
+//! `mul_scalar_batch`, `public_batch`, `decompress_batch`, `verify_batch`, and `FixedBase` (k*P and k*P + l*Q on
+//! the comb table of a caller-chosen point).  `Fr` is carried as its
 //! canonical 32-byte little-endian value (what ff_ce's `into_repr()` yields).  There is no CPU
 //! fallback: without a CUDA device `Engine::new` returns an error.
 pub mod ffi;
@@ -316,6 +317,62 @@ pub fn mul_scalar_batch(points: &[Point], scalars: &[BigInt]) -> Vec<Point> {
                                                       rx.as_mut_ptr(), ry.as_mut_ptr()) }, "bjj_mul_scalar_wide_batch");
     }
     (0..n).map(|i| Point { x: row(&rx, i), y: row(&ry, i) }).collect()
+}
+
+/// Reduces a scalar for the fixed-base tables: the reference multiplies by |k| (sign dropped, src/lib.rs:156); every
+/// on-curve point has an order dividing ORDER, so a |k| wider than 256 bits is reduced mod ORDER -- the same point.
+pub fn scalar_base_le32(v: &BigInt) -> [u8; 32] {
+    let m = v.magnitude();
+    if m.bits() <= 256 {
+        bigint_le32(v)
+    } else {
+        bigint_le32(&(BigInt::from(m.clone()) % (suborder() * 8)))
+    }
+}
+
+/// The comb table of one on-curve point P (50 MB of device memory on the process-wide engine's device, freed on drop):
+/// `P.mul_scalar(k)` for many `k` at the rate of B8's fixed-base path, and `k*P + l*Q` in one pass.  An off-curve P has
+/// no table (its reference result depends on mul_scalar's exact double-and-add order): `new` returns Err and the caller
+/// keeps `mul_scalar_batch`.
+pub struct FixedBase {
+    base: *mut ffi::bjj_base,
+}
+unsafe impl Send for FixedBase {}
+
+impl FixedBase {
+    pub fn new(p: &Point) -> Result<FixedBase, String> {
+        let mut base = std::ptr::null_mut();
+        let rc = unsafe { ffi::bjj_base_create(engine().raw(), p.x.as_ptr(), p.y.as_ptr(), &mut base) };
+        if rc != ffi::BJJ_OK {
+            return Err(format!("bjj_base_create failed: {}", err_str(rc)));
+        }
+        Ok(FixedBase { base })
+    }
+    /// `[P.mul_scalar(k) for k in scalars]`
+    pub fn mul_batch(&self, scalars: &[BigInt]) -> Vec<Point> {
+        let n = scalars.len();
+        let k = col(n, |i| scalar_base_le32(&scalars[i]));
+        let (mut rx, mut ry) = (vec![0u8; 32 * n], vec![0u8; 32 * n]);
+        check(unsafe { ffi::bjj_base_mul_batch(engine().raw(), self.base, n, k.as_ptr(), rx.as_mut_ptr(), ry.as_mut_ptr()) },
+              "bjj_base_mul_batch");
+        (0..n).map(|i| Point { x: row(&rx, i), y: row(&ry, i) }).collect()
+    }
+    /// `(k*P).projective().add((l*Q).projective()).affine()` lane by lane; `q == None` selects B8
+    pub fn mul2_batch(&self, ks: &[BigInt], q: Option<&FixedBase>, ls: &[BigInt]) -> Vec<Point> {
+        let n = ks.len();
+        assert_eq!(n, ls.len());
+        let (k, l) = (col(n, |i| scalar_base_le32(&ks[i])), col(n, |i| scalar_base_le32(&ls[i])));
+        let qb = q.map_or(std::ptr::null(), |b| b.base as *const ffi::bjj_base);
+        let (mut rx, mut ry) = (vec![0u8; 32 * n], vec![0u8; 32 * n]);
+        check(unsafe { ffi::bjj_base_mul2_batch(engine().raw(), self.base, qb, n, k.as_ptr(), l.as_ptr(), rx.as_mut_ptr(),
+                                                ry.as_mut_ptr()) }, "bjj_base_mul2_batch");
+        (0..n).map(|i| Point { x: row(&rx, i), y: row(&ry, i) }).collect()
+    }
+}
+impl Drop for FixedBase {
+    fn drop(&mut self) {
+        unsafe { ffi::bjj_base_destroy(engine().raw(), self.base) }
+    }
 }
 
 pub fn public_batch(keys: &[PrivateKey]) -> Vec<Point> {
