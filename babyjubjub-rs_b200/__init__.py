@@ -15,6 +15,8 @@ follow the reference's public API (paths into the reference tree):
       decompress_batch, verify_batch (and add/compress/poseidon/fixed-base batches).
     + FixedBase / mul_fixed_base_batch / mul2_fixed_base_batch: k*P and k*P + l*Q on a
       precomputed table of a caller-chosen point P (the comb path B8 uses).
+    + public_compressed_batch / sign_compressed_batch: PrivateKey::public().compress() and
+      PrivateKey::sign(msg).compress() with the compression done on the device.
 
 Every call runs on the GPU through libbjj_cuda.so; there is no CPU fallback -- importing works
 without a GPU (so the ABI can be inspected), creating an Engine does not.
@@ -197,6 +199,13 @@ class Engine:
         self._check(self.lib.bjj_public_batch(self.ctx, len(k), _ptr(k), _ptr(outs[0]), _ptr(outs[1])), "bjj_public_batch")
         return tuple(outs)
 
+    def public_compressed_batch(self, keys):
+        """compress(PrivateKey::public(key)) for every key -> (n, 32) uint8"""
+        k = _as_u8(keys, 32)
+        out = np.empty_like(k)
+        self._check(self.lib.bjj_public_compressed_batch(self.ctx, len(k), _ptr(k), _ptr(out)), "bjj_public_compressed_batch")
+        return out
+
     def scalar_key_batch(self, keys):
         k = _as_u8(keys, 32)
         out = np.empty_like(k)
@@ -210,6 +219,16 @@ class Engine:
         self._check(self.lib.bjj_sign_batch(self.ctx, len(k), _ptr(k), _ptr(m), _ptr(rx), _ptr(ry), _ptr(s), _ptr(status)),
                     "bjj_sign_batch")
         return rx, ry, s, status
+
+    def sign_compressed_batch(self, keys, msgs):
+        """PrivateKey::sign(msg).compress() for every lane -> (sig (n, 64) uint8, status (n,) uint8); a lane with
+        status 4 (msg > Q) has 64 zero bytes"""
+        k, m = _as_u8(keys, 32), _as_u8(msgs, 32)
+        sig = np.empty((len(k), 64), dtype=np.uint8)
+        status = np.empty(len(k), dtype=np.uint8)
+        self._check(self.lib.bjj_sign_compressed_batch(self.ctx, len(k), _ptr(k), _ptr(m), _ptr(sig), _ptr(status)),
+                    "bjj_sign_compressed_batch")
+        return sig, status
 
     def compress_batch(self, px, py):
         x, y = _as_u8(px, 32), _as_u8(py, 32)
@@ -541,6 +560,34 @@ def public_batch(keys, engine=None):
     return [Point(x, y) for x, y in zip(le32_to_ints(rx), le32_to_ints(ry))]
 
 
+def _keys_u8(keys):
+    return np.frombuffer(b"".join(bytes(k.key if isinstance(k, PrivateKey) else k) for k in keys),
+                         dtype=np.uint8).reshape(-1, 32)
+
+
+def public_compressed_batch(keys, engine=None):
+    """[k.public().compress() for k in keys] (src/lib.rs:304-306, 166-178) as 32-byte strings"""
+    out = (engine or default_engine()).public_compressed_batch(_keys_u8(keys))
+    return [bytes(r) for r in out]
+
+
+def _sign_msgs(msgs):
+    """messages of sign_compressed_batch as 32-byte words: a negative msg raises like verify; msg > Q, whose lane
+    fails with the reference's Err, is clamped to an all-ones word (still > Q) so that it fits, as in verify_batch"""
+    mm = [int(m) for m in msgs]
+    if any(m < 0 for m in mm):
+        raise ValueError("negative msg (the reference panics in Fr::from_str)")
+    return ints_to_le32([m if m <= Q else (1 << 256) - 1 for m in mm])
+
+
+def sign_compressed_batch(keys, msgs, engine=None):
+    """[k.sign(m).compress() for k, m in zip(keys, msgs)] (src/lib.rs:308-342, 245-257) -> list of 64-byte strings, or
+    ValueError("msg outside the Finite Field") instances for msg > Q (the reference returns Result)"""
+    m = _sign_msgs(msgs)
+    sig, st = (engine or default_engine()).sign_compressed_batch(_keys_u8(keys), m)
+    return [bytes(r) if s == 0 else ValueError(STATUS_STRINGS[int(s)]) for r, s in zip(sig, st)]
+
+
 def decompress_batch(blobs, engine=None):
     """-> list of Point or ValueError instances (the reference returns Result<Point, String>)."""
     eng = engine or default_engine()
@@ -656,6 +703,21 @@ class MultiEngine:
         self._check(self.lib.bjj_multi_public_batch(self.handle, len(keys), _ptr(keys), _ptr(rx), _ptr(ry)),
                     "bjj_multi_public_batch")
         return rx, ry
+
+    def public_compressed_batch(self, keys, out=None):
+        keys = _as_u8(keys, 32)
+        out = np.empty_like(keys) if out is None else out
+        self._check(self.lib.bjj_multi_public_compressed_batch(self.handle, len(keys), _ptr(keys), _ptr(out)),
+                    "bjj_multi_public_compressed_batch")
+        return out
+
+    def sign_compressed_batch(self, keys, msgs, out=None):
+        keys, msgs = _as_u8(keys, 32), _as_u8(msgs, 32)
+        n = len(keys)
+        sig, st = (np.empty((n, 64), dtype=np.uint8), np.empty(n, dtype=np.uint8)) if out is None else out
+        self._check(self.lib.bjj_multi_sign_compressed_batch(self.handle, n, _ptr(keys), _ptr(msgs), _ptr(sig), _ptr(st)),
+                    "bjj_multi_sign_compressed_batch")
+        return sig, st
 
     def fixed_base_batch(self, scalars, out=None):
         k = _as_u8(scalars, 32)

@@ -36,8 +36,10 @@ SIGNATURES = {
     "bjj_mul_scalar_batch": (_int, [_ctx, _sz] + [_u8p] * 5),
     "bjj_fixed_base_batch": (_int, [_ctx, _sz] + [_u8p] * 3),
     "bjj_public_batch": (_int, [_ctx, _sz] + [_u8p] * 3),
+    "bjj_public_compressed_batch": (_int, [_ctx, _sz] + [_u8p] * 2),
     "bjj_scalar_key_batch": (_int, [_ctx, _sz] + [_u8p] * 2),
     "bjj_sign_batch": (_int, [_ctx, _sz] + [_u8p] * 6),
+    "bjj_sign_compressed_batch": (_int, [_ctx, _sz] + [_u8p] * 4),
     "bjj_compress_batch": (_int, [_ctx, _sz] + [_u8p] * 3),
     "bjj_decompress_batch": (_int, [_ctx, _sz] + [_u8p] * 4),
     "bjj_poseidon_batch": (_int, [_ctx, _int, _sz, ctypes.POINTER(_u8p), _u8p]),
@@ -70,6 +72,8 @@ SIGNATURES.update({
     "bjj_multi_verify_compressed_batch": (_int, [_multi, _sz] + [_u8p] * 5),
     "bjj_multi_mul_scalar_batch": (_int, [_multi, _sz] + [_u8p] * 5),
     "bjj_multi_public_batch": (_int, [_multi, _sz] + [_u8p] * 3),
+    "bjj_multi_public_compressed_batch": (_int, [_multi, _sz] + [_u8p] * 2),
+    "bjj_multi_sign_compressed_batch": (_int, [_multi, _sz] + [_u8p] * 4),
     "bjj_multi_fixed_base_batch": (_int, [_multi, _sz] + [_u8p] * 3),
     "bjj_multi_decompress_batch": (_int, [_multi, _sz] + [_u8p] * 4),
 })

@@ -74,6 +74,10 @@ __global__ void __launch_bounds__(BJJ_BLOCK) k_affine(size_t n, const uint8_t* p
 __global__ void __launch_bounds__(BJJ_BLOCK) k_batch_affine(size_t n, ProjScratch scr, uint8_t* rx, uint8_t* ry) {
     batch_affine_strided(scr, rx, ry, n, (size_t)blockIdx.x * blockDim.x + threadIdx.x, (size_t)gridDim.x * blockDim.x);
 }
+// the same pass writing Point::compress of each affine result: one 32-byte plane instead of two
+__global__ void __launch_bounds__(BJJ_BLOCK) k_batch_affine_compressed(size_t n, ProjScratch scr, uint8_t* out32) {
+    batch_affine_strided(scr, CompressedOut{out32}, n, (size_t)blockIdx.x * blockDim.x + threadIdx.x, (size_t)gridDim.x * blockDim.x);
+}
 
 // The point kernels claim their lanes dynamically (BJJ_CLAIM_LOOP), like the verify kernels: with a static grid-stride
 // split the kernel lasts as long as its slowest CTA and ncu showed 80 % (k_fixed_base, k_public) and 68 %
@@ -624,9 +628,13 @@ static int launch_mul_scalar(bjj_ctx* ctx, size_t n, const uint8_t* px, const ui
         return launched(ctx);
     });
 }
+// what the batched affine pass that closes a point sub-batch writes: the (x, y) planes rx, ry (k_batch_affine), or
+// Point::compress into the one 32-byte plane rx (k_batch_affine_compressed; ry unused)
+enum class PointOut { affine, compressed };
+
 // fixed-base flavours: `from_keys` selects PrivateKey::public (BLAKE-512 + prune + >>3 first)
 static int launch_fixed_base(bjj_ctx* ctx, size_t n, const uint8_t* in, uint8_t* rx, uint8_t* ry, bool from_keys,
-                             cudaStream_t st, Workspace* ws) {
+                             cudaStream_t st, Workspace* ws, PointOut form = PointOut::affine) {
     const size_t lanes = scratch_lanes(ctx, n);
     return for_each_subbatch(n, [&](size_t off, size_t m) -> int {
         const size_t o = 32 * off;
@@ -648,7 +656,10 @@ static int launch_fixed_base(bjj_ctx* ctx, size_t n, const uint8_t* in, uint8_t*
             k_fixed_base<<<grid_for(ctx, k_fixed_base, m), BJJ_BLOCK, 0, st>>>(m, k, scr, ctx->comb, work);
         }
         TRY(launched(ctx));
-        k_batch_affine<<<affine_grid(ctx, m), BJJ_BLOCK, 0, st>>>(m, scr, rx + o, ry + o);
+        if (form == PointOut::compressed)
+            k_batch_affine_compressed<<<affine_grid(ctx, m), BJJ_BLOCK, 0, st>>>(m, scr, rx + o);
+        else
+            k_batch_affine<<<affine_grid(ctx, m), BJJ_BLOCK, 0, st>>>(m, scr, rx + o, ry + o);
         return launched(ctx);
     });
 }
@@ -828,9 +839,13 @@ static int launch_poseidon(bjj_ctx* ctx, int n_inputs, size_t n, const uint8_t* 
 // fixed-base kernels with batched inversions -> hm = Poseidon(R8, A, msg) on k_poseidon<6> -> k_sign_finish (S).  The
 // fused k_sign (one lane start to finish in one thread: 244 registers with spills, a Fermat inversion per lane, 67 % of
 // the multiplier pipe) stays available as BJJ_SIGN_FUSED=1; the pipeline reuses kernels that run at 84-92 %.
+// form == PointOut::compressed writes Signature::compress into the 64-byte-stride array r8x (r8y and s32 unused) and
+// always runs the pipeline: R8's affine coordinates then go to the two verify-scratch planes that signing leaves free,
+// and k_sign_finish_compressed packs compress(R8) || S.
 static int launch_sign(bjj_ctx* ctx, size_t n, const uint8_t* key32, const uint8_t* msg32, uint8_t* r8x, uint8_t* r8y, uint8_t* s32,
-                       uint8_t* status, cudaStream_t st, Workspace* ws) {
-    if (ctx->sign_fused) {
+                       uint8_t* status, cudaStream_t st, Workspace* ws, PointOut form = PointOut::affine) {
+    const bool packed = form == PointOut::compressed;
+    if (ctx->sign_fused && !packed) {
         bjjk::sign(grid_cap(ctx, bjjk::sign_blocks_per_sm(), n), st, n, key32, msg32, r8x, r8y, s32, status, ctx->comb);
         return launched(ctx);
     }
@@ -841,14 +856,18 @@ static int launch_sign(bjj_ctx* ctx, size_t n, const uint8_t* key32, const uint8
         TRY(ensure_vscratch(ctx, ws, lanes, &hm, &pts));
         const size_t L = 32 * ws->vs_lanes;
         uint8_t *sk = hm + L, *r = hm + 2 * L, *msgc = hm + 3 * L, *apx = pts, *apy = pts + L;
+        uint8_t *rx = packed ? pts + 2 * L : r8x + o, *ry = packed ? pts + 3 * L : r8y + o;
         const int grid_s = grid_for(ctx, k_scalar_key, m);      // same block size and shape of work
         bjjk::sign_scalars(grid_s, st, m, key32 + o, msg32 + o, sk, r, msgc, status + off);
         TRY(launched(ctx));
-        TRY(launch_fixed_base(ctx, m, r, r8x + o, r8y + o, false, st, ws));
+        TRY(launch_fixed_base(ctx, m, r, rx, ry, false, st, ws));
         TRY(launch_fixed_base(ctx, m, sk, apx, apy, false, st, ws));
-        const uint8_t* ins[5] = {r8x + o, r8y + o, apx, apy, msgc};
+        const uint8_t* ins[5] = {rx, ry, apx, apy, msgc};
         TRY(launch_poseidon(ctx, 5, m, ins, hm, st));
-        bjjk::sign_finish(grid_s, st, m, hm, sk, r, status + off, r8x + o, r8y + o, s32 + o);
+        if (packed)
+            bjjk::sign_finish_compressed(grid_s, st, m, hm, sk, r, status + off, rx, ry, r8x + 2 * o);
+        else
+            bjjk::sign_finish(grid_s, st, m, hm, sk, r, status + off, rx, ry, s32 + o);
         return launched(ctx);
     });
 }
@@ -910,6 +929,12 @@ int bjj_public_batch_dev(bjj_ctx* ctx, size_t n, const uint8_t* key32, uint8_t* 
     return launch_fixed_base(ctx, n, key32, rx, ry, true, st, &ctx->ws);
 }
 
+int bjj_public_compressed_batch_dev(bjj_ctx* ctx, size_t n, const uint8_t* key32, uint8_t* out32, void* stream) {
+    DEV_PROLOGUE
+    if (!key32 || !out32) return BJJ_ERR_ARG;
+    return launch_fixed_base(ctx, n, key32, out32, nullptr, true, st, &ctx->ws, PointOut::compressed);
+}
+
 int bjj_base_mul_batch_dev(bjj_ctx* ctx, const bjj_base* base, size_t n, const uint8_t* scalar32, uint8_t* rx, uint8_t* ry,
                            void* stream) {
     DEV_PROLOGUE
@@ -931,6 +956,13 @@ int bjj_sign_batch_dev(bjj_ctx* ctx, size_t n, const uint8_t* key32, const uint8
     DEV_PROLOGUE
     if (!key32 || !msg32 || !r8x || !r8y || !s32 || !status) return BJJ_ERR_ARG;
     return launch_sign(ctx, n, key32, msg32, r8x, r8y, s32, status, st, &ctx->ws);
+}
+
+int bjj_sign_compressed_batch_dev(bjj_ctx* ctx, size_t n, const uint8_t* key32, const uint8_t* msg32, uint8_t* sig64,
+                                  uint8_t* status, void* stream) {
+    DEV_PROLOGUE
+    if (!key32 || !msg32 || !sig64 || !status) return BJJ_ERR_ARG;
+    return launch_sign(ctx, n, key32, msg32, sig64, nullptr, nullptr, status, st, &ctx->ws, PointOut::compressed);
 }
 
 int bjj_scalar_key_batch_dev(bjj_ctx* ctx, size_t n, const uint8_t* key32, uint8_t* scalar32, void* stream) {
@@ -1244,6 +1276,14 @@ int bjj_public_batch(bjj_ctx* ctx, size_t n, const uint8_t* key32, uint8_t* rx, 
     });
 }
 
+int bjj_public_compressed_batch(bjj_ctx* ctx, size_t n, const uint8_t* key32, uint8_t* out32) {
+    if (!ctx) return BJJ_ERR_ARG;
+    HostArg args[] = {H_IN(key32, 32), H_OUT(out32, 32)};
+    return run_host(ctx, n, args, 2, [&](size_t m, uint8_t** d, cudaStream_t st, Workspace* ws) -> int {
+        return launch_fixed_base(ctx, m, d[0], d[1], nullptr, true, st, ws, PointOut::compressed);
+    });
+}
+
 int bjj_base_mul_batch(bjj_ctx* ctx, const bjj_base* base, size_t n, const uint8_t* scalar32, uint8_t* rx, uint8_t* ry) {
     if (!ctx) return BJJ_ERR_ARG;
     const CombEntry* comb = base_comb(ctx, base);
@@ -1271,6 +1311,15 @@ int bjj_sign_batch(bjj_ctx* ctx, size_t n, const uint8_t* key32, const uint8_t* 
     HostArg args[] = {H_IN(key32, 32), H_IN(msg32, 32), H_OUT(r8x, 32), H_OUT(r8y, 32), H_OUT(s32, 32), H_OUT(status, 1)};
     return run_host(ctx, n, args, 6, [&](size_t m, uint8_t** d, cudaStream_t st, Workspace* ws) -> int {
         return launch_sign(ctx, m, d[0], d[1], d[2], d[3], d[4], d[5], st, ws);
+    });
+}
+
+int bjj_sign_compressed_batch(bjj_ctx* ctx, size_t n, const uint8_t* key32, const uint8_t* msg32, uint8_t* sig64,
+                              uint8_t* status) {
+    if (!ctx) return BJJ_ERR_ARG;
+    HostArg args[] = {H_IN(key32, 32), H_IN(msg32, 32), H_OUT(sig64, 64), H_OUT(status, 1)};
+    return run_host(ctx, n, args, 4, [&](size_t m, uint8_t** d, cudaStream_t st, Workspace* ws) -> int {
+        return launch_sign(ctx, m, d[0], d[1], d[2], nullptr, nullptr, d[3], st, ws, PointOut::compressed);
     });
 }
 

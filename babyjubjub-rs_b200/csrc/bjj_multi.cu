@@ -8,7 +8,8 @@
 // value of another lane, so there is no collective and no peer access on the data path.
 //
 // Reference items batched: verify (src/lib.rs:395-412), Point::mul_scalar (:149-164), PrivateKey::public (:304-306),
-// decompress_point (:192-224), decompress_signature + verify (:260-268).
+// decompress_point (:192-224), decompress_signature + verify (:260-268), and the compressed outputs of
+// PrivateKey::public and PrivateKey::sign (:304-306 / :308-342 with :166-178 / :245-257).
 #include <cuda_runtime.h>
 
 #include <condition_variable>
@@ -176,6 +177,23 @@ int bjj_multi_public_batch(bjj_multi* m, size_t n, const uint8_t* key32, uint8_t
     return run_sharded(m, n, {{key32, 32 * n}, {rx, 32 * n}, {ry, 32 * n}}, [&](int d, size_t off, size_t k) {
         const size_t o = 32 * off;
         return bjj_public_batch(m->ctx[d], k, key32 + o, rx + o, ry + o);
+    });
+}
+
+int bjj_multi_public_compressed_batch(bjj_multi* m, size_t n, const uint8_t* key32, uint8_t* out32) {
+    if (!m || !key32 || !out32) return BJJ_ERR_ARG;
+    return run_sharded(m, n, {{key32, 32 * n}, {out32, 32 * n}}, [&](int d, size_t off, size_t k) {
+        const size_t o = 32 * off;
+        return bjj_public_compressed_batch(m->ctx[d], k, key32 + o, out32 + o);
+    });
+}
+
+int bjj_multi_sign_compressed_batch(bjj_multi* m, size_t n, const uint8_t* key32, const uint8_t* msg32, uint8_t* sig64,
+                                    uint8_t* status) {
+    if (!m || !key32 || !msg32 || !sig64 || !status) return BJJ_ERR_ARG;
+    return run_sharded(m, n, {{key32, 32 * n}, {msg32, 32 * n}, {sig64, 64 * n}, {status, n}}, [&](int d, size_t off, size_t k) {
+        const size_t o = 32 * off;
+        return bjj_sign_compressed_batch(m->ctx[d], k, key32 + o, msg32 + o, sig64 + 2 * o, status + off);
     });
 }
 

@@ -18,6 +18,12 @@ __global__ void __launch_bounds__(BJJ_BLOCK) k_sign_finish(size_t n, const uint8
                                                          const uint8_t* status, uint8_t* r8x, uint8_t* r8y, uint8_t* s32) {
     BJJ_LANE_LOOP(n) lane_sign_finish(hm, sk, r, status, r8x, r8y, s32, i);
 }
+// the same last phase writing Signature::compress: compress(R8) || S into lane i of sig64 (64-byte stride)
+__global__ void __launch_bounds__(BJJ_BLOCK) k_sign_finish_compressed(size_t n, const uint8_t* hm, const uint8_t* sk, const uint8_t* r,
+                                                                    const uint8_t* status, const uint8_t* r8x, const uint8_t* r8y,
+                                                                    uint8_t* sig64) {
+    BJJ_LANE_LOOP(n) lane_sign_finish(hm, sk, r, status, SignCompressedOut{r8x, r8y, sig64}, i);
+}
 
 namespace bjjk {
 
@@ -34,6 +40,10 @@ void sign_scalars(int grid, cudaStream_t st, size_t n, const uint8_t* key, const
 void sign_finish(int grid, cudaStream_t st, size_t n, const uint8_t* hm, const uint8_t* sk, const uint8_t* r, const uint8_t* status,
                  uint8_t* r8x, uint8_t* r8y, uint8_t* s32) {
     k_sign_finish<<<grid, BJJ_BLOCK, 0, st>>>(n, hm, sk, r, status, r8x, r8y, s32);
+}
+void sign_finish_compressed(int grid, cudaStream_t st, size_t n, const uint8_t* hm, const uint8_t* sk, const uint8_t* r,
+                            const uint8_t* status, const uint8_t* r8x, const uint8_t* r8y, uint8_t* sig64) {
+    k_sign_finish_compressed<<<grid, BJJ_BLOCK, 0, st>>>(n, hm, sk, r, status, r8x, r8y, sig64);
 }
 
 }  // namespace bjjk

@@ -87,6 +87,8 @@ void sign_scalars(int grid, cudaStream_t st, size_t n, const uint8_t* key, const
                   uint8_t* status);
 void sign_finish(int grid, cudaStream_t st, size_t n, const uint8_t* hm, const uint8_t* sk, const uint8_t* r, const uint8_t* status,
                  uint8_t* r8x, uint8_t* r8y, uint8_t* s32);
+void sign_finish_compressed(int grid, cudaStream_t st, size_t n, const uint8_t* hm, const uint8_t* sk, const uint8_t* r,
+                            const uint8_t* status, const uint8_t* r8x, const uint8_t* r8y, uint8_t* sig64);
 void poseidon(int t, int grid, cudaStream_t st, size_t n, PoseidonIn in, uint8_t* out, uint32_t* gflags);
 
 }  // namespace bjjk

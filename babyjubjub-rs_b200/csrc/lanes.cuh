@@ -314,7 +314,11 @@ BJJ_HD void store_zero_scratch(const ProjScratch& s, size_t i) {
 // merged before the one inversion, were measured as well: 2.570 against 2.564 ms per 2^20 keys at 32 lanes per thread,
 // 2.61 / 2.88 ms at 64 / 128 lanes per thread -- the kernel lives on the number of resident warps, and lanes per thread
 // take them away.  profiles/r2_ab_exact_early_chunks.txt.)
-BJJ_HD void batch_affine_strided(const ProjScratch& s, uint8_t* rx, uint8_t* ry, size_t n, size_t t, size_t T) {
+//
+// `Out` is the output form, fixed at compile time: out(i, x, y) receives lane i's affine (x, y) in Montgomery form
+// ((0, 0) for Z == 0).  AffineOut stores the two coordinates, CompressedOut stores Point::compress of them.
+template <class Out>
+BJJ_HD void batch_affine_strided(const ProjScratch& s, Out out, size_t n, size_t t, size_t T) {
     const Fr one = fr_const(BJJ_ONE_M);
     Fr acc = one, z;
     size_t last = t;
@@ -344,10 +348,36 @@ BJJ_HD void batch_affine_strided(const ProjScratch& s, uint8_t* rx, uint8_t* ry,
             fr_zero(x);
             fr_zero(y);
         }
-        store_fr(rx, i, x);
-        store_fr(ry, i, y);
+        out(i, x, y);
         if (i < t + T) break;
     }
+}
+
+// Point::compress's sign rule (src/lib.rs:166-178): bit 255 of the compressed y is set when x > Q/2 (x, y canonical)
+BJJ_HD void compress_sign(uint32_t* y, const uint32_t* x) {
+    if (u256_lt(BJJ_QHALF, x)) y[7] |= 0x80000000u;
+}
+
+struct AffineOut {
+    uint8_t *rx, *ry;
+    BJJ_HD void operator()(size_t i, const Fr& x, const Fr& y) const {
+        store_fr(rx, i, x);
+        store_fr(ry, i, y);
+    }
+};
+struct CompressedOut {
+    uint8_t* out32;
+    BJJ_HD void operator()(size_t i, const Fr& x, const Fr& y) const {
+        Fr cx, cy;
+        fr_from_mont(cx, x);
+        fr_from_mont(cy, y);
+        compress_sign(cy.v, cx.v);
+        store_u256(out32, i, cy.v);
+    }
+};
+
+BJJ_HD void batch_affine_strided(const ProjScratch& s, uint8_t* rx, uint8_t* ry, size_t n, size_t t, size_t T) {
+    batch_affine_strided(s, AffineOut{rx, ry}, n, t, T);
 }
 
 // ---- lane bodies --------------------------------------------------------------------------------------
@@ -611,7 +641,7 @@ BJJ_HD void lane_compress(const uint8_t* px, const uint8_t* py, uint8_t* out, si
     load_u256(y, py, i);
     const uint32_t q[8] = BJJ_LIMBS8(BJJ_Q);
     if (!u256_lt(x, q) || !u256_lt(y, q)) flags |= BJJ_FLAG_NONCANONICAL;
-    if (u256_lt(BJJ_QHALF, x)) y[7] |= 0x80000000u;
+    compress_sign(y, x);
     store_u256(out, i, y);
 }
 
@@ -954,23 +984,55 @@ BJJ_HD void lane_sign_scalars(const uint8_t* key32, const uint8_t* msg32, uint8_
     store_u256(msg_out, i, msg);
     status[i] = bad ? (uint8_t)BJJ_ST_MSG_RANGE : (uint8_t)BJJ_ST_OK;
 }
-// last phase: S from the hash; rejected lanes return zeros like the fused lane
-BJJ_HD void lane_sign_finish(const uint8_t* hm32, const uint8_t* sk32, const uint8_t* r32, const uint8_t* status, uint8_t* r8x,
-                             uint8_t* r8y, uint8_t* s32, size_t i) {
+// last phase: S from the hash; rejected lanes return zeros like the fused lane.  `Out` is the output form, fixed at
+// compile time: out.reject(i, zero) for a lane whose status is not OK, out.accept(i, S) otherwise.
+template <class Out>
+BJJ_HD void lane_sign_finish(const uint8_t* hm32, const uint8_t* sk32, const uint8_t* r32, const uint8_t* status, Out out,
+                             size_t i) {
     uint32_t hm[8], sk[8], r[8], s[8];
     if (status[i] != BJJ_ST_OK) {
 #pragma unroll
         for (int k = 0; k < 8; k++) s[k] = 0;
-        store_u256(r8x, i, s);
-        store_u256(r8y, i, s);
-        store_u256(s32, i, s);
+        out.reject(i, s);
         return;
     }
     load_u256(hm, hm32, i);
     load_u256(sk, sk32, i);
     load_u256(r, r32, i);
     sign_finish(s, hm, sk, r);
-    store_u256(s32, i, s);
+    out.accept(i, s);
+}
+// R8 is already in r8x, r8y (the fixed-base pass wrote it there); S goes to s32
+struct SignOut {
+    uint8_t *r8x, *r8y, *s32;
+    BJJ_HD void reject(size_t i, const uint32_t* zero) const {
+        store_u256(r8x, i, zero);
+        store_u256(r8y, i, zero);
+        store_u256(s32, i, zero);
+    }
+    BJJ_HD void accept(size_t i, const uint32_t* s) const { store_u256(s32, i, s); }
+};
+// Signature::compress (src/lib.rs:245-257): compress(R8) || S into lane i of the 64-byte-stride sig64; R8 is read from
+// the canonical affine planes r8x, r8y
+struct SignCompressedOut {
+    const uint8_t *r8x, *r8y;
+    uint8_t* sig64;
+    BJJ_HD void reject(size_t i, const uint32_t* zero) const {
+        store_u256(sig64, 2 * i, zero);
+        store_u256(sig64, 2 * i + 1, zero);
+    }
+    BJJ_HD void accept(size_t i, const uint32_t* s) const {
+        uint32_t x[8], y[8];
+        load_u256(x, r8x, i);
+        load_u256(y, r8y, i);
+        compress_sign(y, x);
+        store_u256(sig64, 2 * i, y);
+        store_u256(sig64, 2 * i + 1, s);
+    }
+};
+BJJ_HD void lane_sign_finish(const uint8_t* hm32, const uint8_t* sk32, const uint8_t* r32, const uint8_t* status, uint8_t* r8x,
+                             uint8_t* r8y, uint8_t* s32, size_t i) {
+    lane_sign_finish(hm32, sk32, r32, status, SignOut{r8x, r8y, s32}, i);
 }
 
 BJJ_HD void lane_sign(const uint8_t* key32, const uint8_t* msg32, uint8_t* r8x, uint8_t* r8y, uint8_t* s32,

@@ -12,7 +12,8 @@
 //   PrivateKey{key}::scalar_key/public/sign src/lib.rs:270-342
 //   verify(pk, sig, msg)                   src/lib.rs:395-412
 //   verify_schnorr(pk, m, r, s)            src/lib.rs:375-385
-//   + batch entry points: mul_scalar_batch, public_batch, decompress_batch, verify_batch
+//   + batch entry points: mul_scalar_batch, public_batch, decompress_batch, verify_batch,
+//     public_compressed_batch, sign_compressed_batch
 //   + FixedBase: the comb table of a caller-chosen point, k*P and k*P + l*Q at the fixed-base rate
 //   + MultiGpu: shards a batch over every device, one host thread + one bjj_ctx per device, no NCCL
 //
@@ -222,6 +223,38 @@ inline std::vector<Point> public_batch(const std::vector<PrivateKey>& keys, Engi
     for (size_t i = 0; i < n; i++) {
         std::memcpy(out[i].x.data(), &rx[32 * i], 32);
         std::memcpy(out[i].y.data(), &ry[32 * i], 32);
+    }
+    return out;
+}
+
+// [k.public_key().compress() for k in keys] (src/lib.rs:304-306, 166-178), compressed on the device
+inline std::vector<std::array<uint8_t, 32>> public_compressed_batch(const std::vector<PrivateKey>& keys,
+                                                                    Engine& e = default_engine()) {
+    const size_t n = keys.size();
+    std::vector<uint8_t> k(32 * n), out(32 * n);
+    for (size_t i = 0; i < n; i++) std::memcpy(&k[32 * i], keys[i].key.data(), 32);
+    Engine::check(bjj_public_compressed_batch(e.ctx(), n, k.data(), out.data()), "bjj_public_compressed_batch");
+    return unpack(out);
+}
+
+struct SignCompressedResult {
+    std::array<uint8_t, 64> sig;          // compress(R8) || S; 64 zero bytes when status != 0
+    uint8_t status;                       // 0 ok; otherwise bjj_status_string(status) is the reference's Err text
+};
+// [k.sign(m).compress() for k, m in zip(keys, msgs)] (src/lib.rs:308-342, 245-257); msg > Q gives status
+// BJJ_STATUS_MSG_RANGE ("msg outside the Finite Field")
+inline std::vector<SignCompressedResult> sign_compressed_batch(const std::vector<PrivateKey>& keys, const std::vector<U256>& msgs,
+                                                               Engine& e = default_engine()) {
+    if (keys.size() != msgs.size()) throw std::invalid_argument("keys and msgs differ in length");
+    const size_t n = keys.size();
+    std::vector<uint8_t> k(32 * n), sig(64 * n), st(n);
+    for (size_t i = 0; i < n; i++) std::memcpy(&k[32 * i], keys[i].key.data(), 32);
+    auto m = pack(msgs);
+    Engine::check(bjj_sign_compressed_batch(e.ctx(), n, k.data(), m.data(), sig.data(), st.data()), "bjj_sign_compressed_batch");
+    std::vector<SignCompressedResult> out(n);
+    for (size_t i = 0; i < n; i++) {
+        std::memcpy(out[i].sig.data(), &sig[64 * i], 64);
+        out[i].status = st[i];
     }
     return out;
 }

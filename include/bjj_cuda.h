@@ -162,6 +162,11 @@ int bjj_base_mul2_batch_dev(bjj_ctx* ctx, const bjj_base* p, const bjj_base* q, 
 /* ---- PrivateKey::public (src/lib.rs:304-306) = B8 * scalar_key(key);  scalar_key (:284-302) ------ */
 int bjj_public_batch(bjj_ctx* ctx, size_t n, const uint8_t* key32, uint8_t* rx, uint8_t* ry);
 int bjj_public_batch_dev(bjj_ctx* ctx, size_t n, const uint8_t* key32, uint8_t* rx, uint8_t* ry, void* stream);
+/* compress(PrivateKey::public(key)) (src/lib.rs:304-306, 166-178): 32 B per lane, the same bytes as bjj_public_batch
+ * followed by bjj_compress_batch, without the affine coordinates crossing PCIe.  Runs the kernels of bjj_public_batch
+ * (BJJ_PUBLIC_FUSED selects the same path) with a compressing last pass. */
+int bjj_public_compressed_batch(bjj_ctx* ctx, size_t n, const uint8_t* key32, uint8_t* out32);
+int bjj_public_compressed_batch_dev(bjj_ctx* ctx, size_t n, const uint8_t* key32, uint8_t* out32, void* stream);
 int bjj_scalar_key_batch(bjj_ctx* ctx, size_t n, const uint8_t* key32, uint8_t* scalar32);
 int bjj_scalar_key_batch_dev(bjj_ctx* ctx, size_t n, const uint8_t* key32, uint8_t* scalar32, void* stream);
 
@@ -172,6 +177,13 @@ int bjj_sign_batch(bjj_ctx* ctx, size_t n, const uint8_t* key32, const uint8_t* 
                    uint8_t* s32, uint8_t* status);
 int bjj_sign_batch_dev(bjj_ctx* ctx, size_t n, const uint8_t* key32, const uint8_t* msg32, uint8_t* r8x,
                        uint8_t* r8y, uint8_t* s32, uint8_t* status, void* stream);
+/* PrivateKey::sign(msg).compress() (src/lib.rs:308-342, 245-257): sig64[i] = compress(R8) || S;
+ * status[i] = BJJ_STATUS_MSG_RANGE when msg > Q, and then sig64[i] is 64 zero bytes.  Always the kernel pipeline:
+ * BJJ_SIGN_FUSED selects the fused kernel for bjj_sign_batch only. */
+int bjj_sign_compressed_batch(bjj_ctx* ctx, size_t n, const uint8_t* key32, const uint8_t* msg32, uint8_t* sig64,
+                              uint8_t* status);
+int bjj_sign_compressed_batch_dev(bjj_ctx* ctx, size_t n, const uint8_t* key32, const uint8_t* msg32, uint8_t* sig64,
+                                  uint8_t* status, void* stream);
 
 /* ---- Point::compress (src/lib.rs:166-178) / decompress_point (src/lib.rs:192-224) ---------------- */
 int bjj_compress_batch(bjj_ctx* ctx, size_t n, const uint8_t* px, const uint8_t* py, uint8_t* out32);
@@ -235,6 +247,9 @@ int bjj_multi_verify_compressed_batch(bjj_multi* m, size_t n, const uint8_t* sig
 int bjj_multi_mul_scalar_batch(bjj_multi* m, size_t n, const uint8_t* px, const uint8_t* py, const uint8_t* scalar32,
                                uint8_t* rx, uint8_t* ry);
 int bjj_multi_public_batch(bjj_multi* m, size_t n, const uint8_t* key32, uint8_t* rx, uint8_t* ry);
+int bjj_multi_public_compressed_batch(bjj_multi* m, size_t n, const uint8_t* key32, uint8_t* out32);
+int bjj_multi_sign_compressed_batch(bjj_multi* m, size_t n, const uint8_t* key32, const uint8_t* msg32, uint8_t* sig64,
+                                    uint8_t* status);
 int bjj_multi_fixed_base_batch(bjj_multi* m, size_t n, const uint8_t* scalar32, uint8_t* rx, uint8_t* ry);
 int bjj_multi_decompress_batch(bjj_multi* m, size_t n, const uint8_t* in32, uint8_t* rx, uint8_t* ry, uint8_t* status);
 

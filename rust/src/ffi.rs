@@ -72,6 +72,10 @@ extern "C" {
     pub fn bjj_scalar_key_batch(ctx: *mut bjj_ctx, n: usize, key32: *const u8, scalar32: *mut u8) -> c_int;
     pub fn bjj_sign_batch(ctx: *mut bjj_ctx, n: usize, key32: *const u8, msg32: *const u8, r8x: *mut u8, r8y: *mut u8,
                           s32: *mut u8, status: *mut u8) -> c_int;
+    // compress(PrivateKey::public) / PrivateKey::sign(msg).compress() (src/lib.rs:166-178, 245-257, 304-342)
+    pub fn bjj_public_compressed_batch(ctx: *mut bjj_ctx, n: usize, key32: *const u8, out32: *mut u8) -> c_int;
+    pub fn bjj_sign_compressed_batch(ctx: *mut bjj_ctx, n: usize, key32: *const u8, msg32: *const u8, sig64: *mut u8,
+                                     status: *mut u8) -> c_int;
     // Point::compress / decompress_point (src/lib.rs:166-178, 192-224)
     pub fn bjj_compress_batch(ctx: *mut bjj_ctx, n: usize, px: *const u8, py: *const u8, out32: *mut u8) -> c_int;
     pub fn bjj_decompress_batch(ctx: *mut bjj_ctx, n: usize, in32: *const u8, rx: *mut u8, ry: *mut u8,
@@ -102,6 +106,9 @@ extern "C" {
     pub fn bjj_multi_mul_scalar_batch(m: *mut bjj_multi, n: usize, px: *const u8, py: *const u8, scalar32: *const u8,
                                       rx: *mut u8, ry: *mut u8) -> c_int;
     pub fn bjj_multi_public_batch(m: *mut bjj_multi, n: usize, key32: *const u8, rx: *mut u8, ry: *mut u8) -> c_int;
+    pub fn bjj_multi_public_compressed_batch(m: *mut bjj_multi, n: usize, key32: *const u8, out32: *mut u8) -> c_int;
+    pub fn bjj_multi_sign_compressed_batch(m: *mut bjj_multi, n: usize, key32: *const u8, msg32: *const u8, sig64: *mut u8,
+                                           status: *mut u8) -> c_int;
     pub fn bjj_multi_fixed_base_batch(m: *mut bjj_multi, n: usize, scalar32: *const u8, rx: *mut u8, ry: *mut u8) -> c_int;
     pub fn bjj_multi_decompress_batch(m: *mut bjj_multi, n: usize, in32: *const u8, rx: *mut u8, ry: *mut u8,
                                       status: *mut u8) -> c_int;

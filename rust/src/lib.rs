@@ -384,6 +384,39 @@ pub fn public_batch(keys: &[PrivateKey]) -> Vec<Point> {
     (0..n).map(|i| Point { x: row(&rx, i), y: row(&ry, i) }).collect()
 }
 
+/// `keys[i].public().compress()` (src/lib.rs:304-306, 166-178) without the affine coordinates crossing PCIe
+pub fn public_compressed_batch(keys: &[PrivateKey]) -> Vec<[u8; 32]> {
+    let n = keys.len();
+    let k = col(n, |i| keys[i].key);
+    let mut out = vec![0u8; 32 * n];
+    check(unsafe { ffi::bjj_public_compressed_batch(engine().raw(), n, k.as_ptr(), out.as_mut_ptr()) },
+          "bjj_public_compressed_batch");
+    (0..n).map(|i| row(&out, i)).collect()
+}
+
+/// `keys[i].sign(msgs[i]).map(|s| s.compress())` (src/lib.rs:308-342, 245-257); msg > Q gives the reference's Err.
+/// Panics on a negative msg, which the reference cannot convert to Fr.
+pub fn sign_compressed_batch(keys: &[PrivateKey], msgs: &[BigInt]) -> Vec<Result<[u8; 64], String>> {
+    let n = keys.len();
+    assert_eq!(n, msgs.len());
+    assert!(msgs.iter().all(|m| m.sign() != Sign::Minus), "negative msg");
+    let k = col(n, |i| keys[i].key);
+    let m = col(n, |i| msg_le32(&msgs[i]));
+    let (mut sig, mut st) = (vec![0u8; 64 * n], vec![0u8; n]);
+    check(unsafe { ffi::bjj_sign_compressed_batch(engine().raw(), n, k.as_ptr(), m.as_ptr(), sig.as_mut_ptr(),
+                                                  st.as_mut_ptr()) }, "bjj_sign_compressed_batch");
+    (0..n)
+        .map(|i| {
+            if st[i] != 0 {
+                return Err(status_str(st[i]));
+            }
+            let mut r = [0u8; 64];
+            r.copy_from_slice(&sig[64 * i..64 * i + 64]);
+            Ok(r)
+        })
+        .collect()
+}
+
 pub fn decompress_batch(blobs: &[[u8; 32]]) -> Vec<Result<Point, String>> {
     let n = blobs.len();
     let inp = col(n, |i| blobs[i]);
@@ -450,6 +483,14 @@ impl MultiEngine {
         let (mut rx, mut ry) = (vec![0u8; 32 * n], vec![0u8; 32 * n]);
         check(unsafe { ffi::bjj_multi_public_batch(self.m, n, k.as_ptr(), rx.as_mut_ptr(), ry.as_mut_ptr()) }, "bjj_multi_public_batch");
         (0..n).map(|i| Point { x: row(&rx, i), y: row(&ry, i) }).collect()
+    }
+    pub fn public_compressed_batch(&mut self, keys: &[PrivateKey]) -> Vec<[u8; 32]> {
+        let n = keys.len();
+        let k = col(n, |i| keys[i].key);
+        let mut out = vec![0u8; 32 * n];
+        check(unsafe { ffi::bjj_multi_public_compressed_batch(self.m, n, k.as_ptr(), out.as_mut_ptr()) },
+              "bjj_multi_public_compressed_batch");
+        (0..n).map(|i| row(&out, i)).collect()
     }
 }
 impl Drop for MultiEngine {
