@@ -17,6 +17,8 @@ follow the reference's public API (paths into the reference tree):
       precomputed table of a caller-chosen point P (the comb path B8 uses).
     + public_compressed_batch / sign_compressed_batch: PrivateKey::public().compress() and
       PrivateKey::sign(msg).compress() with the compression done on the device.
+    + verify_base_batch: verify for many signatures of ONE key, with the key's FixedBase table
+      (two comb walks per signature instead of verify_batch's per-lane ladder).
 
 Every call runs on the GPU through libbjj_cuda.so; there is no CPU fallback -- importing works
 without a GPU (so the ABI can be inspected), creating an Engine does not.
@@ -275,6 +277,25 @@ class Engine:
                     "bjj_verify_compressed_batch")
         return ok, status
 
+    def verify_base_batch(self, base, r8x, r8y, s, msg):
+        """verify for every lane against the one key of `base` (a FixedBase of this engine) -> ok (n,) uint8"""
+        ins = [_as_u8(v, 32) for v in (r8x, r8y, s, msg)]
+        ok = np.empty(len(ins[0]), dtype=np.uint8)
+        self._check(self.lib.bjj_verify_base_batch(self.ctx, _key_handle(base), len(ins[0]), *[_ptr(v) for v in ins], _ptr(ok)),
+                    "bjj_verify_base_batch")
+        return ok
+
+    def verify_base_compressed_batch(self, base, sig64, msg):
+        """verify of 64-byte compressed signatures against the one key of `base` -> (ok, status), both (n,) uint8;
+        status is R8's decompression error"""
+        sg, m = _as_u8(sig64, 64), _as_u8(msg, 32)
+        ok = np.empty(len(sg), dtype=np.uint8)
+        status = np.empty(len(sg), dtype=np.uint8)
+        self._check(self.lib.bjj_verify_base_compressed_batch(self.ctx, _key_handle(base), len(sg), _ptr(sg), _ptr(m), _ptr(ok),
+                                                              _ptr(status)), "bjj_verify_base_compressed_batch")
+        return ok, status
+
+
 
 _default_engine = None
 
@@ -327,6 +348,13 @@ def _handle(base):
     if not base.handle:
         raise ValueError("FixedBase is closed")
     return base.handle
+
+
+def _key_handle(base):
+    """the handle of a verify_base call, which must name its key (None does not select B8 there)"""
+    if base is None:
+        raise ValueError("verify_base_batch needs a FixedBase of the public key")
+    return _handle(base)
 
 
 def _base_scalar(k):
@@ -598,11 +626,24 @@ def decompress_batch(blobs, engine=None):
 
 def verify_batch(pks, sigs, msgs, engine=None):
     eng = engine or default_engine()
-    # msg > Q is `false` in the reference; clamp such messages to an all-ones word (still > Q) so they fit 32 bytes
-    mm = [int(m) if int(m) <= Q else (1 << 256) - 1 for m in msgs]
     ok = eng.verify_batch(ints_to_le32([s.r_b8.x for s in sigs]), ints_to_le32([s.r_b8.y for s in sigs]),
                           ints_to_le32([_verify_scalar(s.s) for s in sigs]), ints_to_le32([p.x for p in pks]),
-                          ints_to_le32([p.y for p in pks]), ints_to_le32(mm))
+                          ints_to_le32([p.y for p in pks]), _verify_msgs(msgs))
+    return [bool(v) for v in ok]
+
+
+def _verify_msgs(msgs):
+    """messages of verify_batch / verify_base_batch as 32-byte words: msg > Q is `false` in the reference, so such
+    messages are clamped to an all-ones word (still > Q) to fit"""
+    return ints_to_le32([int(m) if int(m) <= Q else (1 << 256) - 1 for m in msgs])
+
+
+def verify_base_batch(base, sigs, msgs, engine=None):
+    """[verify(base.point, sig, msg) for sig, msg in zip(sigs, msgs)] (src/lib.rs:395-412) for signatures of ONE key,
+    whose FixedBase table `base` serves every lane; the same results as verify_batch with the key in every lane"""
+    eng = engine or base.engine
+    ok = eng.verify_base_batch(base, ints_to_le32([s.r_b8.x for s in sigs]), ints_to_le32([s.r_b8.y for s in sigs]),
+                               ints_to_le32([_verify_scalar(s.s) for s in sigs]), _verify_msgs(msgs))
     return [bool(v) for v in ok]
 
 

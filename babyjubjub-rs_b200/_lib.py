@@ -50,6 +50,8 @@ SIGNATURES = {
     "bjj_base_destroy": (None, [_ctx, _base]),
     "bjj_base_mul_batch": (_int, [_ctx, _base, _sz] + [_u8p] * 3),
     "bjj_base_mul2_batch": (_int, [_ctx, _base, _base, _sz] + [_u8p] * 4),
+    "bjj_verify_base_batch": (_int, [_ctx, _base, _sz] + [_u8p] * 5),
+    "bjj_verify_base_compressed_batch": (_int, [_ctx, _base, _sz] + [_u8p] * 4),
 }
 # every batch op also has a device-pointer flavour with a trailing `void* stream`
 for _name in [k for k in SIGNATURES if k.endswith("_batch")]:

@@ -15,7 +15,7 @@ OBJ = os.path.join(HERE, "build")
 BIN = os.path.join(HERE, "bin")
 GEN = os.path.join(CSRC, "generated", "bjj_consts.inc")
 LIB = os.path.join(HERE, "libbjj_cuda.so")
-LIB_UNITS = ["bjj_cuda.cu", "bjj_multi.cu", "k_verify.cu", "k_mulscalar.cu", "k_sign.cu", "k_poseidon.cu"]
+LIB_UNITS = ["bjj_cuda.cu", "bjj_multi.cu", "k_verify.cu", "k_verify_base.cu", "k_mulscalar.cu", "k_sign.cu", "k_poseidon.cu"]
 MB = os.path.join(HERE, "tools", "microbench")
 TOOLS = ["imad_bench.cu", "pipe_probe.cu", "fr_layouts.cu"]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]

@@ -197,10 +197,12 @@ struct bjj_ctx {
                                 // allocated ONCE up front (a cudaFree in mid-pipeline is a device-wide synchronisation)
 };
 
-// the comb table of a caller point, on the device of the context that built it
+// the comb table of a caller point, on the device of the context that built it, and the point's canonical affine
+// coordinates (little-endian bytes; verify_base hashes them)
 struct bjj_base {
     bjj_ctx* ctx;
     CombEntry* comb;
+    uint8_t x[32], y[32];
 };
 
 #define CU(ctx, call)                      \
@@ -546,6 +548,8 @@ int bjj_base_create(bjj_ctx* ctx, const uint8_t* px32, const uint8_t* py32, bjj_
     }
     b->ctx = ctx;
     b->comb = comb;
+    memcpy(b->x, px32, 32);
+    memcpy(b->y, py32, 32);
     *out = b;
     return BJJ_OK;
 }
@@ -826,6 +830,59 @@ static int launch_verify_compressed(bjj_ctx* ctx, size_t n, const uint8_t* sig64
         return launched(ctx);
     });
 }
+// verify against the one key of `base` (bjj_verify_base*): k_verify_base_hash -> k_verify_base_ec, no window tables
+// and no exact-lane queue (off-curve R8 lanes take a branch of the EC kernel).  sig64 != nullptr is the compressed
+// form: R8 (the first half of each 64-byte signature) is decompressed first into two verify-scratch planes, by phase
+// 0 of launch_verify_compressed for R8 alone; `status` receives its decompression status and failed lanes are
+// rejected.  The key's coordinates are kernel arguments: base_create checked them.
+static int launch_verify_base(bjj_ctx* ctx, const bjj_base* base, size_t n, const uint8_t* r8x, const uint8_t* r8y,
+                              const uint8_t* s32, const uint8_t* sig64, const uint8_t* msg, uint8_t* ok, uint8_t* status,
+                              cudaStream_t st, Workspace* ws) {
+    const size_t lanes = scratch_lanes(ctx, n);
+    return for_each_subbatch(n, [&](size_t off, size_t m) -> int {
+        const size_t o = 32 * off;
+        // the deferred exact kernel of an earlier verify on this workspace may still read its scratch
+        if (ws->aux) CU(ctx, cudaStreamWaitEvent(st, ws->ev_join, 0));
+        uint8_t *hm, *pts;
+        TRY(ensure_vscratch(ctx, ws, lanes, &hm, &pts));
+        const uint8_t *rx, *ry, *sb, *skip = nullptr;
+        size_t s_stride = 1, s_off = 0;
+        if (!sig64) {
+            rx = r8x + o;
+            ry = r8y + o;
+            sb = s32 + o;
+        } else {
+            uint8_t *dx = pts, *dy = pts + 32 * ws->vs_lanes;
+            ProjScratch scr;
+            TRY(ensure_proj(ctx, ws, lanes, &scr));
+            k_decompress_prepare<<<grid_for(ctx, k_decompress_prepare, m), BJJ_BLOCK, 0, st>>>(m, sig64 + 2 * o, 2, 0, scr, 0);
+            k_batch_inverse<<<affine_grid(ctx, m), BJJ_BLOCK, 0, st>>>(m, scr);
+            unsigned long long* work = nullptr;
+            TRY(claim_counter(ctx, ws, st, &work));
+            k_decompress_finish<<<grid_for(ctx, k_decompress_finish, m), BJJ_BLOCK, 0, st>>>(m, sig64 + 2 * o, 2, 0, scr, 0, dx, dy,
+                                                                                            status + off, 0, work);
+            TRY(launched(ctx, 3));
+            rx = dx;
+            ry = dy;
+            sb = sig64 + 2 * o;
+            s_stride = 2;
+            s_off = 1;
+            skip = status + off;
+        }
+        unsigned long long *work_h = nullptr, *work_e = nullptr;
+        TRY(claim_counter(ctx, ws, st, &work_h));
+        TRY(claim_counter(ctx, ws, st, &work_e));
+        bjjk::verify_base_hash(grid_cap(ctx, bjjk::verify_base_hash_blocks_per_sm(), m), st, m, rx, ry, base->x, base->y, msg + o, skip,
+                               hm, ok + off, ctx->flags_dev, work_h);
+        TRY(launched(ctx));
+        bjjk::verify_base_ec(grid_cap(ctx, bjjk::verify_base_ec_blocks_per_sm(), m), st, m, rx, ry, sb, s_stride, s_off, hm, ok + off,
+                             ctx->comb, base->comb, work_e);
+        return launched(ctx);
+    });
+}
+// a verify_base call names its key: NULL or a handle of another context is an argument error
+static bool base_of(bjj_ctx* ctx, const bjj_base* base) { return base && base->ctx == ctx; }
+
 static int launch_poseidon(bjj_ctx* ctx, int n_inputs, size_t n, const uint8_t* const* in, uint8_t* out,
                            cudaStream_t st) {
     PoseidonIn pin;
@@ -1012,6 +1069,22 @@ int bjj_verify_compressed_batch_dev(bjj_ctx* ctx, size_t n, const uint8_t* sig64
     DEV_PROLOGUE
     if (!sig64 || !pk32 || !msg32 || !ok || !status) return BJJ_ERR_ARG;
     return launch_verify_compressed(ctx, n, sig64, pk32, msg32, ok, status, st, &ctx->ws);
+}
+
+int bjj_verify_base_batch_dev(bjj_ctx* ctx, const bjj_base* pk, size_t n, const uint8_t* r8x, const uint8_t* r8y,
+                              const uint8_t* s32, const uint8_t* msg32, uint8_t* ok, void* stream) {
+    if (!base_of(ctx, pk)) return BJJ_ERR_ARG;
+    DEV_PROLOGUE
+    if (!r8x || !r8y || !s32 || !msg32 || !ok) return BJJ_ERR_ARG;
+    return launch_verify_base(ctx, pk, n, r8x, r8y, s32, nullptr, msg32, ok, nullptr, st, &ctx->ws);
+}
+
+int bjj_verify_base_compressed_batch_dev(bjj_ctx* ctx, const bjj_base* pk, size_t n, const uint8_t* sig64, const uint8_t* msg32,
+                                         uint8_t* ok, uint8_t* status, void* stream) {
+    if (!base_of(ctx, pk)) return BJJ_ERR_ARG;
+    DEV_PROLOGUE
+    if (!sig64 || !msg32 || !ok || !status) return BJJ_ERR_ARG;
+    return launch_verify_base(ctx, pk, n, nullptr, nullptr, nullptr, sig64, msg32, ok, status, st, &ctx->ws);
 }
 
 }  // extern "C"
@@ -1382,6 +1455,24 @@ int bjj_verify_compressed_batch(bjj_ctx* ctx, size_t n, const uint8_t* sig64, co
     HostArg args[] = {H_IN(sig64, 64), H_IN(pk32, 32), H_IN(msg32, 32), H_OUT(ok, 1), H_OUT(status, 1)};
     return run_host(ctx, n, args, 5, [&](size_t m, uint8_t** d, cudaStream_t st, Workspace* ws) -> int {
         return launch_verify_compressed(ctx, m, d[0], d[1], d[2], d[3], d[4], st, ws);
+    }, /*heavy=*/true);
+}
+
+int bjj_verify_base_batch(bjj_ctx* ctx, const bjj_base* pk, size_t n, const uint8_t* r8x, const uint8_t* r8y, const uint8_t* s32,
+                          const uint8_t* msg32, uint8_t* ok) {
+    if (!base_of(ctx, pk)) return BJJ_ERR_ARG;
+    HostArg args[] = {H_IN(r8x, 32), H_IN(r8y, 32), H_IN(s32, 32), H_IN(msg32, 32), H_OUT(ok, 1)};
+    return run_host(ctx, n, args, 5, [&](size_t m, uint8_t** d, cudaStream_t st, Workspace* ws) -> int {
+        return launch_verify_base(ctx, pk, m, d[0], d[1], d[2], nullptr, d[3], d[4], nullptr, st, ws);
+    }, /*heavy=*/true);
+}
+
+int bjj_verify_base_compressed_batch(bjj_ctx* ctx, const bjj_base* pk, size_t n, const uint8_t* sig64, const uint8_t* msg32,
+                                     uint8_t* ok, uint8_t* status) {
+    if (!base_of(ctx, pk)) return BJJ_ERR_ARG;
+    HostArg args[] = {H_IN(sig64, 64), H_IN(msg32, 32), H_OUT(ok, 1), H_OUT(status, 1)};
+    return run_host(ctx, n, args, 4, [&](size_t m, uint8_t** d, cudaStream_t st, Workspace* ws) -> int {
+        return launch_verify_base(ctx, pk, m, nullptr, nullptr, nullptr, d[0], d[1], d[2], d[3], st, ws);
     }, /*heavy=*/true);
 }
 

@@ -90,5 +90,14 @@ void sign_finish(int grid, cudaStream_t st, size_t n, const uint8_t* hm, const u
 void sign_finish_compressed(int grid, cudaStream_t st, size_t n, const uint8_t* hm, const uint8_t* sk, const uint8_t* r,
                             const uint8_t* status, const uint8_t* r8x, const uint8_t* r8y, uint8_t* sig64);
 void poseidon(int t, int grid, cudaStream_t st, size_t n, PoseidonIn in, uint8_t* out, uint32_t* gflags);
+// verify against one key with a comb table (k_verify_base.cu); ax32, ay32: the key's canonical coordinates (host bytes)
+void verify_base_hash(int grid, cudaStream_t st, size_t n, const uint8_t* r8x, const uint8_t* r8y, const uint8_t* ax32,
+                      const uint8_t* ay32, const uint8_t* msg, const uint8_t* skip, uint8_t* hm, uint8_t* ok, uint32_t* gflags,
+                      unsigned long long* work);
+int verify_base_hash_blocks_per_sm();
+void verify_base_ec(int grid, cudaStream_t st, size_t n, const uint8_t* r8x, const uint8_t* r8y, const uint8_t* s_base,
+                    size_t s_stride, size_t s_off, const uint8_t* hm, uint8_t* ok, const bjj::CombEntry* comb,
+                    const bjj::CombEntry* comb_a, unsigned long long* work);
+int verify_base_ec_blocks_per_sm();
 
 }  // namespace bjjk

@@ -538,8 +538,25 @@ BJJ_HD void lane_mul_scalar(const uint8_t* px, const uint8_t* py, const uint8_t*
 // 32-bit little-endian words, nwords a multiple of 8 up to BJJ_MAX_SCALAR_WORDS.
 #define BJJ_MAX_SCALAR_WORDS 64
 
-// out = x mod ORDER for a wide x: on-curve points have order dividing ORDER = 8 * SUBORDER, so the fast ladder may use
-// the reduced scalar (exact).  Shift-and-subtract, MSB first; ORDER < 2^254, so 2 * acc + 1 fits 256 bits.
+// acc = (acc * 2^256 + w) mod ORDER for acc < ORDER: shift-and-subtract, MSB first; ORDER < 2^254, so 2 * acc + 1
+// fits 256 bits.  On-curve points have order dividing ORDER = 8 * SUBORDER, so a ladder may use the reduced scalar.
+BJJ_HD void reduce_order_block(uint32_t* acc, uint32_t* t, const uint32_t* w) {     // t: 8 words of scratch
+#pragma unroll 1
+    for (int bit = 255; bit >= 0; bit--) {
+        uint32_t b = 0;
+#pragma unroll
+        for (int j = 0; j < 8; j++) b = ((bit >> 5) == j) ? w[j] : b;
+        b = (b >> (bit & 31)) & 1u;
+#pragma unroll
+        for (int k = 7; k > 0; k--) acc[k] = (acc[k] << 1) | (acc[k - 1] >> 31);
+        acc[0] = (acc[0] << 1) | b;
+        const uint32_t borrow = sub256(t, acc, BJJ_ORDER);
+#pragma unroll
+        for (int k = 0; k < 8; k++) acc[k] = borrow ? acc[k] : t[k];
+    }
+}
+
+// out = x mod ORDER for a wide x (the fast ladder of mul_scalar uses the reduced scalar: exact, see above)
 BJJ_HD void lane_reduce_scalar_order(const uint8_t* wide, int nwords, uint8_t* out32, size_t i) {
     uint32_t acc[8], t[8];
 #pragma unroll
@@ -548,19 +565,7 @@ BJJ_HD void lane_reduce_scalar_order(const uint8_t* wide, int nwords, uint8_t* o
     for (int blk = (nwords >> 3) - 1; blk >= 0; blk--) {
         uint32_t w[8];
         load_u256(w, wide, i * (size_t)(nwords >> 3) + (size_t)blk);
-#pragma unroll 1
-        for (int bit = 255; bit >= 0; bit--) {
-            uint32_t b = 0;
-#pragma unroll
-            for (int j = 0; j < 8; j++) b = ((bit >> 5) == j) ? w[j] : b;
-            b = (b >> (bit & 31)) & 1u;
-#pragma unroll
-            for (int k = 7; k > 0; k--) acc[k] = (acc[k] << 1) | (acc[k - 1] >> 31);
-            acc[0] = (acc[0] << 1) | b;
-            const uint32_t borrow = sub256(t, acc, BJJ_ORDER);
-#pragma unroll
-            for (int k = 0; k < 8; k++) acc[k] = borrow ? acc[k] : t[k];
-        }
+        reduce_order_block(acc, t, w);
     }
     store_u256(out32, i, acc);
 }
@@ -1408,6 +1413,117 @@ BJJ_HD void lane_verify_exact(const uint8_t* r8x, const uint8_t* r8y, const uint
     load_fr(a.x, ax, i, flags);
     load_fr(a.y, ay, i, flags);
     ok[i] = (uint8_t)verify_exact<A_OFF>(r8, s, a, hm, comb, mode);
+}
+
+// ---- verify against one key with a comb table (bjj_verify_base_batch) -------------------------------------------
+// Every lane has the same A, an on-curve point whose table comb_a was built by bjj_base_create, so
+//   A.mul_scalar(8*hm) = k * A  with  k = 8*hm mod ORDER   (the order of A divides ORDER)
+// comes from 17 mixed additions like S*B8 does, and a lane needs no doubling.  Two kernels:
+//   phase 1 (lane_verify_base_hash): msg range check, R8's on-curve flag, hm = Poseidon(R8.x, R8.y, A.x, A.y, msg)
+//   phase 2 (lane_verify_base_ec):   the two combs, then the group test (R8 on the curve) or the reference's literal
+//                                    sum and affine comparison (R8 off the curve), in the same kernel.
+// ok[i] between the phases: 0 (rejected), BJJ_OK_PENDING (R8 on the curve) or BJJ_OK_PENDING_EXACT (off the curve).
+#define BJJ_OK_PENDING_EXACT 3
+
+// a: A in Montgomery form (the same for every lane).  `skip` (may be null): lanes whose R8 did not decompress.
+BJJ_HD void lane_verify_base_hash(const uint8_t* r8x, const uint8_t* r8y, const PointAff& a, const uint8_t* msg32,
+                                  const uint8_t* skip, uint8_t* hm_out, uint8_t* ok, size_t i, uint32_t& flags) {
+    if (skip && skip[i]) {
+        ok[i] = 0;
+        return;
+    }
+    uint32_t msg[8];
+    load_u256(msg, msg32, i);
+    const uint32_t qq[8] = BJJ_LIMBS8(BJJ_Q);
+    if (u256_lt(qq, msg)) {     // msg > Q -> false; msg == Q is accepted and hashed as 0 (src/lib.rs:396-399)
+        ok[i] = 0;
+        return;
+    }
+    PointAff r8;
+    load_fr(r8.x, r8x, i, flags);
+    load_fr(r8.y, r8y, i, flags);
+    Fr mraw, mm, hm;
+    fr_set(mraw, msg);
+    fr_to_mont(mm, mraw);
+    verify_hm(hm, r8, a, mm, BJJ_MODE_EDDSA);
+    store_u256(hm_out, i, hm.v);
+    ok[i] = on_curve(r8) ? (uint8_t)BJJ_OK_PENDING : (uint8_t)BJJ_OK_PENDING_EXACT;
+}
+
+// k = 8*hm mod ORDER for a canonical hm < Q < 2^254 (8*hm has 257 bits: its top word is below ORDER already)
+BJJ_HD void verify_base_scalar(uint32_t* k, const uint32_t* hm) {
+    uint32_t lo[8], t[8];
+    lo[0] = hm[0] << 3;
+#pragma unroll
+    for (int j = 1; j < 8; j++) lo[j] = (hm[j] << 3) | (hm[j - 1] >> 29);
+#pragma unroll
+    for (int j = 0; j < 8; j++) k[j] = j == 0 ? hm[7] >> 29 : 0u;
+    reduce_order_block(k, t, lo);
+}
+
+// R8 on the curve: accept iff  S*B8 + (ORDER - k)*A - R8 == O,  checked projectively (the addition law is complete on
+// the curve, so this is the reference's affine comparison).  R8 off the curve: verify_exact<false>'s replay, with both
+// products from the combs: l = S*B8 and kA in affine form (one shared inversion), literal add-2008-bbjlp of R8 and kA
+// with Z = 1, PointProjective::affine (Z == 0 -> (0, 0)), compare with l (src/lib.rs:405-411).  The two comb walks run
+// for every lane, so a warp that holds both kinds of lanes diverges only in the short tails.
+BJJ_HD void lane_verify_base_ec(const uint8_t* r8x, const uint8_t* r8y, const uint8_t* s_base, size_t s_stride, size_t s_off,
+                                const uint8_t* hm_in, uint8_t* ok, size_t i, const CombEntry* comb, const CombEntry* comb_a) {
+    const uint32_t state = ok[i];
+    if (state != BJJ_OK_PENDING && state != BJJ_OK_PENDING_EXACT) return;
+    const bool exact = state == BJJ_OK_PENDING_EXACT;
+    uint32_t s[8], hm[8], k[8];
+    load_u256(s, s_base, i * s_stride + s_off);
+    load_u256(hm, hm_in, i);
+    verify_base_scalar(k, hm);
+    PointExt acc, l;
+    ext_identity(acc);
+    fixed_base_comb_acc(acc, comb, s);
+    if (exact) {      // keep S*B8 apart and walk k*A from the identity
+        l = acc;
+        ext_identity(acc);
+    } else {          // -k*A = (ORDER - k)*A  (k = 0 gives ORDER*A = O as well)
+        sub256(k, BJJ_ORDER, k);
+    }
+    fixed_base_comb_acc(acc, comb_a, k);
+    uint32_t flags = 0;
+    PointAff r8;
+    load_fr(r8.x, r8x, i, flags);
+    load_fr(r8.y, r8y, i, flags);
+    if (!exact) {
+        PointExt p;
+        ext_from_affine(p, r8);
+        fr_neg(p.X, p.X);     // -R8: (-X, Y, Z, -T)
+        fr_neg(p.T, p.T);
+        Niels n;
+        niels_from_ext(n, p);
+        ext_add_niels<false>(acc, acc, n);
+        ok[i] = (fr_is_zero(acc.X) && fr_eq(acc.Y, acc.Z)) ? 1 : 0;     // acc == O = (0 : 1 : 1) ?  (Z != 0)
+        return;
+    }
+    PointProj pl, pk, pr, sum;
+    ext_to_proj(pl, l);
+    ext_to_proj(pk, acc);
+    PointAff la, ka, ra;
+    {     // both Z are non-zero (complete formulas on curve points): one shared inversion
+        Fr t, ti, zl, zk;
+        fr_mul(t, pl.z, pk.z);
+        fr_inv(ti, t);
+        fr_mul(zl, ti, pk.z);
+        fr_mul(zk, ti, pl.z);
+        fr_mul(la.x, pl.x, zl);
+        fr_mul(la.y, pl.y, zl);
+        fr_mul(ka.x, pk.x, zk);
+        fr_mul(ka.y, pk.y, zk);
+    }
+    pr.x = r8.x;
+    pr.y = r8.y;
+    pr.z = fr_const(BJJ_ONE_M);
+    pk.x = ka.x;
+    pk.y = ka.y;
+    pk.z = fr_const(BJJ_ONE_M);
+    proj_add_bbjlp(sum, pr, pk);
+    proj_affine(ra, sum);
+    ok[i] = (fr_eq(la.x, ra.x) && fr_eq(la.y, ra.y)) ? 1 : 0;
 }
 
 }  // namespace bjj

@@ -14,7 +14,8 @@
 //   verify_schnorr(pk, m, r, s)            src/lib.rs:375-385
 //   + batch entry points: mul_scalar_batch, public_batch, decompress_batch, verify_batch,
 //     public_compressed_batch, sign_compressed_batch
-//   + FixedBase: the comb table of a caller-chosen point, k*P and k*P + l*Q at the fixed-base rate
+//   + FixedBase: the comb table of a caller-chosen point, k*P and k*P + l*Q at the fixed-base rate, and verify for
+//     many signatures of that one key
 //   + MultiGpu: shards a batch over every device, one host thread + one bjj_ctx per device, no NCCL
 //
 // Header-only; link with -lbjj_cuda.  There is no CPU fallback: Engine's constructor throws when no
@@ -289,6 +290,35 @@ class FixedBase {
         Engine::check(bjj_base_mul2_batch(e_.ctx(), base_, q ? q->raw() : nullptr, n, kb.data(), lb.data(), rx.data(), ry.data()),
                       "bjj_base_mul2_batch");
         return points(rx, ry);
+    }
+    // [verify(P, sig, msg) for sig, msg in zip(sigs, msgs)] (src/lib.rs:395-412) for signatures of the one key P: the
+    // same bytes as verify_batch with P in every lane; msg > Q gives 0
+    std::vector<uint8_t> verify_batch(const std::vector<Signature>& sigs, const std::vector<U256>& msgs) const {
+        if (sigs.size() != msgs.size()) throw std::invalid_argument("sigs and msgs differ in length");
+        const size_t n = sigs.size();
+        std::vector<uint8_t> r8x(32 * n), r8y(32 * n), s(32 * n), ok(n);
+        for (size_t i = 0; i < n; i++) {
+            std::memcpy(&r8x[32 * i], sigs[i].r_b8.x.data(), 32);
+            std::memcpy(&r8y[32 * i], sigs[i].r_b8.y.data(), 32);
+            std::memcpy(&s[32 * i], sigs[i].s.data(), 32);
+        }
+        auto m = pack(msgs);
+        Engine::check(bjj_verify_base_batch(e_.ctx(), base_, n, r8x.data(), r8y.data(), s.data(), m.data(), ok.data()),
+                      "bjj_verify_base_batch");
+        return ok;
+    }
+    // the same from 64-byte compressed signatures: ok and R8's decompression status per lane
+    std::vector<uint8_t> verify_compressed_batch(const std::vector<std::array<uint8_t, 64>>& sigs, const std::vector<U256>& msgs,
+                                                 std::vector<uint8_t>* status = nullptr) const {
+        if (sigs.size() != msgs.size()) throw std::invalid_argument("sigs and msgs differ in length");
+        const size_t n = sigs.size();
+        std::vector<uint8_t> sg(64 * n), ok(n), st(n);
+        for (size_t i = 0; i < n; i++) std::memcpy(&sg[64 * i], sigs[i].data(), 64);
+        auto m = pack(msgs);
+        Engine::check(bjj_verify_base_compressed_batch(e_.ctx(), base_, n, sg.data(), m.data(), ok.data(), st.data()),
+                      "bjj_verify_base_compressed_batch");
+        if (status) *status = st;
+        return ok;
     }
 
   private:

@@ -158,6 +158,24 @@ int bjj_base_mul2_batch(bjj_ctx* ctx, const bjj_base* p, const bjj_base* q, size
                         const uint8_t* l32, uint8_t* rx, uint8_t* ry);
 int bjj_base_mul2_batch_dev(bjj_ctx* ctx, const bjj_base* p, const bjj_base* q, size_t n, const uint8_t* k32,
                             const uint8_t* l32, uint8_t* rx, uint8_t* ry, void* stream);
+/* verify (src/lib.rs:395-412) of n signatures made by ONE key A, the point of pk: ok[i] = 1 iff
+ * S*B8 == R8 + (8*hm)*A, hm = Poseidon(R8.x, R8.y, A.x, A.y, msg); msg > Q -> 0 (msg == Q hashes as 0).  The same
+ * results as bjj_verify_batch with A in every lane, from two comb walks per lane (S against B8's table, 8*hm mod ORDER
+ * against pk's) instead of the per-lane window tables and 4 doublings per window.  S is raw 256-bit, unreduced.
+ * R8 off the curve replays the reference's sum literally.  A coordinate of R8 >= Q returns BJJ_ERR_NONCANONICAL
+ * (the batch is computed mod Q).  pk == NULL or a handle of another context returns BJJ_ERR_ARG: unlike
+ * bjj_base_mul, NULL does not select B8 here. */
+int bjj_verify_base_batch(bjj_ctx* ctx, const bjj_base* pk, size_t n, const uint8_t* r8x, const uint8_t* r8y,
+                          const uint8_t* s32, const uint8_t* msg32, uint8_t* ok);
+int bjj_verify_base_batch_dev(bjj_ctx* ctx, const bjj_base* pk, size_t n, const uint8_t* r8x, const uint8_t* r8y,
+                              const uint8_t* s32, const uint8_t* msg32, uint8_t* ok, void* stream);
+/* the same from 64-byte compressed signatures (decompress_signature, src/lib.rs:260-268): status[i] = R8's
+ * decompression error (the codes of bjj_verify_compressed_batch), and ok[i] = 0 whenever status[i] != 0.  There is
+ * no status for A: bjj_base_create checked it. */
+int bjj_verify_base_compressed_batch(bjj_ctx* ctx, const bjj_base* pk, size_t n, const uint8_t* sig64,
+                                     const uint8_t* msg32, uint8_t* ok, uint8_t* status);
+int bjj_verify_base_compressed_batch_dev(bjj_ctx* ctx, const bjj_base* pk, size_t n, const uint8_t* sig64,
+                                         const uint8_t* msg32, uint8_t* ok, uint8_t* status, void* stream);
 
 /* ---- PrivateKey::public (src/lib.rs:304-306) = B8 * scalar_key(key);  scalar_key (:284-302) ------ */
 int bjj_public_batch(bjj_ctx* ctx, size_t n, const uint8_t* key32, uint8_t* rx, uint8_t* ry);

@@ -67,6 +67,11 @@ extern "C" {
     // (k*P).projective().add((l*Q).projective()).affine() (src/lib.rs:70-131, 149-164)
     pub fn bjj_base_mul2_batch(ctx: *mut bjj_ctx, p: *const bjj_base, q: *const bjj_base, n: usize, k32: *const u8,
                                l32: *const u8, rx: *mut u8, ry: *mut u8) -> c_int;
+    // verify (src/lib.rs:395-412) of signatures made by the one key of `pk` (NULL is an argument error here)
+    pub fn bjj_verify_base_batch(ctx: *mut bjj_ctx, pk: *const bjj_base, n: usize, r8x: *const u8, r8y: *const u8,
+                                 s32: *const u8, msg32: *const u8, ok: *mut u8) -> c_int;
+    pub fn bjj_verify_base_compressed_batch(ctx: *mut bjj_ctx, pk: *const bjj_base, n: usize, sig64: *const u8,
+                                            msg32: *const u8, ok: *mut u8, status: *mut u8) -> c_int;
     // PrivateKey::public / scalar_key / sign (src/lib.rs:284-342)
     pub fn bjj_public_batch(ctx: *mut bjj_ctx, n: usize, key32: *const u8, rx: *mut u8, ry: *mut u8) -> c_int;
     pub fn bjj_scalar_key_batch(ctx: *mut bjj_ctx, n: usize, key32: *const u8, scalar32: *mut u8) -> c_int;

@@ -368,6 +368,31 @@ impl FixedBase {
                                                 ry.as_mut_ptr()) }, "bjj_base_mul2_batch");
         (0..n).map(|i| Point { x: row(&rx, i), y: row(&ry, i) }).collect()
     }
+    /// `verify(P, sig, msg)` (src/lib.rs:395-412) lane by lane for signatures of the one key P: the results of
+    /// `verify_batch` with P in every lane, from the two comb tables
+    pub fn verify_batch(&self, sigs: &[Signature], msgs: &[BigInt]) -> Vec<bool> {
+        let n = sigs.len();
+        assert_eq!(n, msgs.len());
+        let (r8x, r8y) = (col(n, |i| sigs[i].r_b8.x), col(n, |i| sigs[i].r_b8.y));
+        let s = col(n, |i| scalar_b8_le32(&sigs[i].s));
+        let m = col(n, |i| msg_le32(&msgs[i]));
+        let mut ok = vec![0u8; n];
+        check(unsafe { ffi::bjj_verify_base_batch(engine().raw(), self.base, n, r8x.as_ptr(), r8y.as_ptr(), s.as_ptr(),
+                                                  m.as_ptr(), ok.as_mut_ptr()) }, "bjj_verify_base_batch");
+        ok.into_iter().map(|b| b == 1).collect()
+    }
+    /// the same from 64-byte compressed signatures: `Err` carries R8's decompression error
+    pub fn verify_compressed_batch(&self, sigs: &[[u8; 64]], msgs: &[BigInt]) -> Vec<Result<bool, String>> {
+        let n = sigs.len();
+        assert_eq!(n, msgs.len());
+        let sg: Vec<u8> = sigs.iter().flat_map(|s| s.iter().copied()).collect();
+        let m = col(n, |i| msg_le32(&msgs[i]));
+        let (mut ok, mut st) = (vec![0u8; n], vec![0u8; n]);
+        check(unsafe { ffi::bjj_verify_base_compressed_batch(engine().raw(), self.base, n, sg.as_ptr(), m.as_ptr(),
+                                                             ok.as_mut_ptr(), st.as_mut_ptr()) },
+              "bjj_verify_base_compressed_batch");
+        (0..n).map(|i| if st[i] == 0 { Ok(ok[i] == 1) } else { Err(status_str(st[i])) }).collect()
+    }
 }
 impl Drop for FixedBase {
     fn drop(&mut self) {
