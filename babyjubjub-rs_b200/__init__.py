@@ -19,6 +19,8 @@ follow the reference's public API (paths into the reference tree):
       PrivateKey::sign(msg).compress() with the compression done on the device.
     + verify_base_batch: verify for many signatures of ONE key, with the key's FixedBase table
       (two comb walks per signature instead of verify_batch's per-lane ladder).
+    + sign_schnorr_batch: PrivateKey::sign_schnorr over a batch, with caller-supplied (or random 1024-bit)
+      nonces and the unreduced s of the reference.
 
 Every call runs on the GPU through libbjj_cuda.so; there is no CPU fallback -- importing works
 without a GPU (so the ABI can be inspected), creating an Engine does not.
@@ -231,6 +233,21 @@ class Engine:
         self._check(self.lib.bjj_sign_compressed_batch(self.ctx, len(k), _ptr(k), _ptr(m), _ptr(sig), _ptr(status)),
                     "bjj_sign_compressed_batch")
         return sig, status
+
+    def sign_schnorr_batch(self, keys, msgs, nonces, words):
+        """PrivateKey::sign_schnorr with caller nonces: nonces is a uint8 array (n, 4 * words), little-endian, words a
+        multiple of 8 in [8, 64] -> (rx, ry, s (n, 4 * (words + 8)) unreduced, status (n,)); a lane with status 4
+        (msg > Q) has zero r and s"""
+        k, m = _as_u8(keys, 32), _as_u8(msgs, 32)
+        kn = _as_u8(nonces, 4 * int(words))
+        if not len(k) == len(m) == len(kn):
+            raise ValueError("keys, msgs and nonces differ in length")
+        rx, ry = np.empty_like(k), np.empty_like(k)
+        s = np.empty((len(k), 4 * (int(words) + 8)), dtype=np.uint8)
+        status = np.empty(len(k), dtype=np.uint8)
+        self._check(self.lib.bjj_sign_schnorr_batch(self.ctx, len(k), _ptr(k), _ptr(m), _ptr(kn), int(words), _ptr(rx), _ptr(ry),
+                                                    _ptr(s), _ptr(status)), "bjj_sign_schnorr_batch")
+        return rx, ry, s, status
 
     def compress_batch(self, px, py):
         x, y = _as_u8(px, 32), _as_u8(py, 32)
@@ -616,6 +633,40 @@ def sign_compressed_batch(keys, msgs, engine=None):
     return [bytes(r) if s == 0 else ValueError(STATUS_STRINGS[int(s)]) for r, s in zip(sig, st)]
 
 
+def _schnorr_nonces(nonces):
+    """nonces of sign_schnorr_batch as one uint8 array (n, 4 * words) and its word count: the smallest multiple of 8 words
+    (256 bits) that holds the widest nonce, up to 64 words (2048 bits)"""
+    ks = [int(k) for k in nonces]
+    if any(k < 0 for k in ks):
+        raise ValueError("negative nonce")
+    bits = max([k.bit_length() for k in ks] + [1])
+    if bits > 2048:
+        raise ValueError("nonces wider than 2048 bits are not supported by the device ABI")
+    words = 8 * ((bits + 255) // 256)
+    buf = b"".join(k.to_bytes(4 * words, "little") for k in ks)
+    return np.frombuffer(buf, dtype=np.uint8).reshape(-1, 4 * words).copy(), words
+
+
+def sign_schnorr_batch(keys, msgs, nonces=None, engine=None):
+    """[k.sign_schnorr(m) for k, m in zip(keys, msgs)] (src/lib.rs:344-362) -> list of (r: Point, s: int), s = k + x*h
+    unreduced.  nonces: one non-negative int per lane (at most 2048 bits); None draws 1024 random bits per lane, as the
+    reference does.  Raises ValueError("msg outside the Finite Field") if any msg > Q, and ValueError for a negative msg
+    or nonce."""
+    mm = [int(m) for m in msgs]
+    if any(m > Q for m in mm):
+        raise ValueError(STATUS_STRINGS[4])
+    m = _sign_msgs(mm)
+    if nonces is None:
+        import secrets
+        nonces = [secrets.randbits(1024) for _ in mm]
+    kn, words = _schnorr_nonces(nonces)
+    rx, ry, s, st = (engine or default_engine()).sign_schnorr_batch(_keys_u8(keys), m, kn, words)
+    sw = 4 * (words + 8)
+    raw = s.tobytes()
+    return [(Point(x, y), int.from_bytes(raw[sw * i:sw * (i + 1)], "little"))
+            for i, (x, y) in enumerate(zip(le32_to_ints(rx), le32_to_ints(ry)))]
+
+
 def decompress_batch(blobs, engine=None):
     """-> list of Point or ValueError instances (the reference returns Result<Point, String>)."""
     eng = engine or default_engine()
@@ -759,6 +810,18 @@ class MultiEngine:
         self._check(self.lib.bjj_multi_sign_compressed_batch(self.handle, n, _ptr(keys), _ptr(msgs), _ptr(sig), _ptr(st)),
                     "bjj_multi_sign_compressed_batch")
         return sig, st
+
+    def sign_schnorr_batch(self, keys, msgs, nonces, words, out=None):
+        keys, msgs = _as_u8(keys, 32), _as_u8(msgs, 32)
+        kn = _as_u8(nonces, 4 * int(words))
+        n = len(keys)
+        if not n == len(msgs) == len(kn):
+            raise ValueError("keys, msgs and nonces differ in length")
+        rx, ry, s, st = ((np.empty_like(keys), np.empty_like(keys), np.empty((n, 4 * (int(words) + 8)), dtype=np.uint8),
+                          np.empty(n, dtype=np.uint8)) if out is None else out)
+        self._check(self.lib.bjj_multi_sign_schnorr_batch(self.handle, n, _ptr(keys), _ptr(msgs), _ptr(kn), int(words), _ptr(rx),
+                                                          _ptr(ry), _ptr(s), _ptr(st)), "bjj_multi_sign_schnorr_batch")
+        return rx, ry, s, st
 
     def fixed_base_batch(self, scalars, out=None):
         k = _as_u8(scalars, 32)

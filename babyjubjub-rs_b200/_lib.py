@@ -60,6 +60,8 @@ for _name in [k for k in SIGNATURES if k.endswith("_batch")]:
 
 SIGNATURES["bjj_mul_scalar_wide_batch"] = (_int, [_ctx, _sz, _u8p, _u8p, _u8p, _int, _u8p, _u8p])
 SIGNATURES["bjj_mul_scalar_wide_batch_dev"] = (_int, [_ctx, _sz, _u8p, _u8p, _u8p, _int, _u8p, _u8p, ctypes.c_void_p])
+SIGNATURES["bjj_sign_schnorr_batch"] = (_int, [_ctx, _sz, _u8p, _u8p, _u8p, _int] + [_u8p] * 4)
+SIGNATURES["bjj_sign_schnorr_batch_dev"] = (_int, [_ctx, _sz, _u8p, _u8p, _u8p, _int] + [_u8p] * 4 + [ctypes.c_void_p])
 
 # multi-device layer (one caller, one host batch, N devices); host pointers only
 _multi = ctypes.c_void_p
@@ -76,6 +78,7 @@ SIGNATURES.update({
     "bjj_multi_public_batch": (_int, [_multi, _sz] + [_u8p] * 3),
     "bjj_multi_public_compressed_batch": (_int, [_multi, _sz] + [_u8p] * 2),
     "bjj_multi_sign_compressed_batch": (_int, [_multi, _sz] + [_u8p] * 4),
+    "bjj_multi_sign_schnorr_batch": (_int, [_multi, _sz, _u8p, _u8p, _u8p, _int] + [_u8p] * 4),
     "bjj_multi_fixed_base_batch": (_int, [_multi, _sz] + [_u8p] * 3),
     "bjj_multi_decompress_batch": (_int, [_multi, _sz] + [_u8p] * 4),
 })

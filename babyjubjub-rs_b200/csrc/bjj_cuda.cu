@@ -929,6 +929,39 @@ static int launch_sign(bjj_ctx* ctx, size_t n, const uint8_t* key32, const uint8
     });
 }
 
+// PrivateKey::sign_schnorr with caller nonces, shaped like launch_sign: k_sign_schnorr_scalars (BLAKE-512 once: sk; the
+// nonce mod SUBORDER: kr) -> r = kr * B8 straight into the caller's planes and pk = sk * B8 on the fixed-base kernels ->
+// h = Poseidon(pk, r, msg) on k_poseidon<6> -> k_sign_schnorr_finish (s = k + sk * h, exact).  sk, kr, msgc, h, pk.x and
+// pk.y take six of the eight verify-scratch planes.  The nonce and s advance by their own strides (4 * nonce_words and
+// 4 * (nonce_words + 8) bytes per lane).
+static int launch_sign_schnorr(bjj_ctx* ctx, size_t n, const uint8_t* key32, const uint8_t* msg32, const uint8_t* nonce,
+                               int nonce_words, uint8_t* rx, uint8_t* ry, uint8_t* s, uint8_t* status, cudaStream_t st,
+                               Workspace* ws) {
+    const size_t lanes = scratch_lanes(ctx, n);
+    return for_each_subbatch(n, [&](size_t off, size_t m) -> int {
+        const size_t o = 32 * off;
+        const uint8_t* k = nonce + (size_t)4 * nonce_words * off;
+        uint8_t* so = s + (size_t)4 * (nonce_words + 8) * off;
+        // the deferred exact kernel of an earlier verify on this workspace may still read its scratch
+        if (ws->aux) CU(ctx, cudaStreamWaitEvent(st, ws->ev_join, 0));
+        uint8_t *h, *pts;
+        TRY(ensure_vscratch(ctx, ws, lanes, &h, &pts));
+        const size_t L = 32 * ws->vs_lanes;
+        uint8_t *sk = h + L, *kr = h + 2 * L, *msgc = h + 3 * L, *pkx = pts, *pky = pts + L;
+        const int grid_s = grid_for(ctx, k_scalar_key, m);      // same block size and shape of work
+        bjjk::sign_schnorr_scalars(grid_s, st, m, key32 + o, msg32 + o, k, nonce_words, sk, kr, msgc, status + off);
+        TRY(launched(ctx));
+        TRY(launch_fixed_base(ctx, m, kr, rx + o, ry + o, false, st, ws));
+        TRY(launch_fixed_base(ctx, m, sk, pkx, pky, false, st, ws));
+        const uint8_t* ins[5] = {pkx, pky, rx + o, ry + o, msgc};
+        TRY(launch_poseidon(ctx, 5, m, ins, h, st));
+        bjjk::sign_schnorr_finish(grid_s, st, m, h, sk, k, nonce_words, status + off, rx + o, ry + o, so);
+        return launched(ctx);
+    });
+}
+// the nonce widths of bjj_sign_schnorr_batch: those of bjj_mul_scalar_wide_batch
+static bool nonce_words_ok(int w) { return w >= 8 && w <= BJJ_MAX_SCALAR_WORDS && !(w & 7); }
+
 extern "C" {
 
 int bjj_fr_op_batch_dev(bjj_ctx* ctx, int op, size_t n, const uint8_t* a, const uint8_t* b, uint8_t* out, void* stream) {
@@ -1020,6 +1053,13 @@ int bjj_sign_compressed_batch_dev(bjj_ctx* ctx, size_t n, const uint8_t* key32, 
     DEV_PROLOGUE
     if (!key32 || !msg32 || !sig64 || !status) return BJJ_ERR_ARG;
     return launch_sign(ctx, n, key32, msg32, sig64, nullptr, nullptr, status, st, &ctx->ws, PointOut::compressed);
+}
+
+int bjj_sign_schnorr_batch_dev(bjj_ctx* ctx, size_t n, const uint8_t* key32, const uint8_t* msg32, const uint8_t* nonce,
+                               int nonce_words, uint8_t* rx, uint8_t* ry, uint8_t* s, uint8_t* status, void* stream) {
+    DEV_PROLOGUE
+    if (!key32 || !msg32 || !nonce || !nonce_words_ok(nonce_words) || !rx || !ry || !s || !status) return BJJ_ERR_ARG;
+    return launch_sign_schnorr(ctx, n, key32, msg32, nonce, nonce_words, rx, ry, s, status, st, &ctx->ws);
 }
 
 int bjj_scalar_key_batch_dev(bjj_ctx* ctx, size_t n, const uint8_t* key32, uint8_t* scalar32, void* stream) {
@@ -1393,6 +1433,16 @@ int bjj_sign_compressed_batch(bjj_ctx* ctx, size_t n, const uint8_t* key32, cons
     HostArg args[] = {H_IN(key32, 32), H_IN(msg32, 32), H_OUT(sig64, 64), H_OUT(status, 1)};
     return run_host(ctx, n, args, 4, [&](size_t m, uint8_t** d, cudaStream_t st, Workspace* ws) -> int {
         return launch_sign(ctx, m, d[0], d[1], d[2], nullptr, nullptr, d[3], st, ws, PointOut::compressed);
+    });
+}
+
+int bjj_sign_schnorr_batch(bjj_ctx* ctx, size_t n, const uint8_t* key32, const uint8_t* msg32, const uint8_t* nonce, int nonce_words,
+                           uint8_t* rx, uint8_t* ry, uint8_t* s, uint8_t* status) {
+    if (!ctx || !nonce_words_ok(nonce_words)) return BJJ_ERR_ARG;
+    HostArg args[] = {H_IN(key32, 32), H_IN(msg32, 32), H_IN(nonce, (size_t)4 * nonce_words), H_OUT(rx, 32), H_OUT(ry, 32),
+                      H_OUT(s, (size_t)4 * (nonce_words + 8)), H_OUT(status, 1)};
+    return run_host(ctx, n, args, 7, [&](size_t m, uint8_t** d, cudaStream_t st, Workspace* ws) -> int {
+        return launch_sign_schnorr(ctx, m, d[0], d[1], d[2], nonce_words, d[3], d[4], d[5], d[6], st, ws);
     });
 }
 

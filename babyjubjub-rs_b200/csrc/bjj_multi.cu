@@ -8,8 +8,9 @@
 // value of another lane, so there is no collective and no peer access on the data path.
 //
 // Reference items batched: verify (src/lib.rs:395-412), Point::mul_scalar (:149-164), PrivateKey::public (:304-306),
-// decompress_point (:192-224), decompress_signature + verify (:260-268), and the compressed outputs of
-// PrivateKey::public and PrivateKey::sign (:304-306 / :308-342 with :166-178 / :245-257).
+// decompress_point (:192-224), decompress_signature + verify (:260-268), the compressed outputs of
+// PrivateKey::public and PrivateKey::sign (:304-306 / :308-342 with :166-178 / :245-257), and PrivateKey::sign_schnorr
+// with caller nonces (:344-362).
 #include <cuda_runtime.h>
 
 #include <condition_variable>
@@ -195,6 +196,19 @@ int bjj_multi_sign_compressed_batch(bjj_multi* m, size_t n, const uint8_t* key32
         const size_t o = 32 * off;
         return bjj_sign_compressed_batch(m->ctx[d], k, key32 + o, msg32 + o, sig64 + 2 * o, status + off);
     });
+}
+
+int bjj_multi_sign_schnorr_batch(bjj_multi* m, size_t n, const uint8_t* key32, const uint8_t* msg32, const uint8_t* nonce,
+                                 int nonce_words, uint8_t* rx, uint8_t* ry, uint8_t* s, uint8_t* status) {
+    if (!m || !key32 || !msg32 || !nonce || !rx || !ry || !s || !status) return BJJ_ERR_ARG;
+    if (nonce_words < 8 || nonce_words > 64 || (nonce_words & 7)) return BJJ_ERR_ARG;
+    const size_t kw = (size_t)4 * nonce_words, sw = (size_t)4 * (nonce_words + 8);     // bytes per lane of nonce and s
+    return run_sharded(m, n, {{key32, 32 * n}, {msg32, 32 * n}, {nonce, kw * n}, {rx, 32 * n}, {ry, 32 * n}, {s, sw * n}, {status, n}},
+                       [&](int d, size_t off, size_t k) {
+                           const size_t o = 32 * off;
+                           return bjj_sign_schnorr_batch(m->ctx[d], k, key32 + o, msg32 + o, nonce + kw * off, nonce_words, rx + o,
+                                                         ry + o, s + sw * off, status + off);
+                       });
 }
 
 int bjj_multi_fixed_base_batch(bjj_multi* m, size_t n, const uint8_t* scalar32, uint8_t* rx, uint8_t* ry) {

@@ -25,7 +25,30 @@ __global__ void __launch_bounds__(BJJ_BLOCK) k_sign_finish_compressed(size_t n, 
     BJJ_LANE_LOOP(n) lane_sign_finish(hm, sk, r, status, SignCompressedOut{r8x, r8y, sig64}, i);
 }
 
+// sign_schnorr pipeline (reference: PrivateKey::sign_schnorr, src/lib.rs:344-362, with caller nonces): the scalars
+// (BLAKE-512 once, the nonce mod SUBORDER) and the exact s = k + sk * h; r, pk and h run on k_fixed_base /
+// k_batch_affine / k_poseidon<6> in between
+__global__ void __launch_bounds__(BJJ_BLOCK) k_sign_schnorr_scalars(size_t n, const uint8_t* key, const uint8_t* msg,
+                                                                  const uint8_t* nonce, int nonce_words, uint8_t* sk, uint8_t* kr,
+                                                                  uint8_t* msgc, uint8_t* status) {
+    BJJ_LANE_LOOP(n) lane_sign_schnorr_scalars(key, msg, nonce, nonce_words, sk, kr, msgc, status, i);
+}
+__global__ void __launch_bounds__(BJJ_BLOCK) k_sign_schnorr_finish(size_t n, const uint8_t* h, const uint8_t* sk, const uint8_t* nonce,
+                                                                 int nonce_words, const uint8_t* status, uint8_t* rx, uint8_t* ry,
+                                                                 uint8_t* s) {
+    BJJ_LANE_LOOP(n) lane_sign_schnorr_finish(h, sk, nonce, nonce_words, status, rx, ry, s, i);
+}
+
 namespace bjjk {
+
+void sign_schnorr_scalars(int grid, cudaStream_t st, size_t n, const uint8_t* key, const uint8_t* msg, const uint8_t* nonce,
+                          int nonce_words, uint8_t* sk, uint8_t* kr, uint8_t* msgc, uint8_t* status) {
+    k_sign_schnorr_scalars<<<grid, BJJ_BLOCK, 0, st>>>(n, key, msg, nonce, nonce_words, sk, kr, msgc, status);
+}
+void sign_schnorr_finish(int grid, cudaStream_t st, size_t n, const uint8_t* h, const uint8_t* sk, const uint8_t* nonce, int nonce_words,
+                         const uint8_t* status, uint8_t* rx, uint8_t* ry, uint8_t* s) {
+    k_sign_schnorr_finish<<<grid, BJJ_BLOCK, 0, st>>>(n, h, sk, nonce, nonce_words, status, rx, ry, s);
+}
 
 int sign_blocks_per_sm() { return blocks_per_sm(k_sign); }
 void sign(int grid, cudaStream_t st, size_t n, const uint8_t* key, const uint8_t* msg, uint8_t* r8x, uint8_t* r8y,

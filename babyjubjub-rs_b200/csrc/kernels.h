@@ -89,6 +89,10 @@ void sign_finish(int grid, cudaStream_t st, size_t n, const uint8_t* hm, const u
                  uint8_t* r8x, uint8_t* r8y, uint8_t* s32);
 void sign_finish_compressed(int grid, cudaStream_t st, size_t n, const uint8_t* hm, const uint8_t* sk, const uint8_t* r,
                             const uint8_t* status, const uint8_t* r8x, const uint8_t* r8y, uint8_t* sig64);
+void sign_schnorr_scalars(int grid, cudaStream_t st, size_t n, const uint8_t* key, const uint8_t* msg, const uint8_t* nonce,
+                          int nonce_words, uint8_t* sk, uint8_t* kr, uint8_t* msgc, uint8_t* status);
+void sign_schnorr_finish(int grid, cudaStream_t st, size_t n, const uint8_t* h, const uint8_t* sk, const uint8_t* nonce, int nonce_words,
+                         const uint8_t* status, uint8_t* rx, uint8_t* ry, uint8_t* s);
 void poseidon(int t, int grid, cudaStream_t st, size_t n, PoseidonIn in, uint8_t* out, uint32_t* gflags);
 // verify against one key with a comb table (k_verify_base.cu); ax32, ay32: the key's canonical coordinates (host bytes)
 void verify_base_hash(int grid, cudaStream_t st, size_t n, const uint8_t* r8x, const uint8_t* r8y, const uint8_t* ax32,

@@ -1058,6 +1058,107 @@ BJJ_HD void lane_sign(const uint8_t* key32, const uint8_t* msg32, uint8_t* r8x, 
     status[i] = (uint8_t)st;
 }
 
+// acc = x mod SUBORDER, canonical, for lane i of a wide array (nwords a multiple of 8 up to BJJ_MAX_SCALAR_WORDS).
+// Horner over the 256-bit blocks from the top, acc <- acc * R + block (mod l), R = 2^256: montmul_suborder(acc, R^2 mod l)
+// = acc * R and montmul_suborder(block, R mod l) = block (mod l), each below 2l (acc * R^2 < l^2 and block * R < R l),
+// so the sum is below 4l and two conditional subtractions (2l, l) finish.  Two products per block where
+// reduce_order_block would take 256 shift-and-subtract steps.
+BJJ_HD void lane_mod_suborder_wide(uint32_t* acc, const uint8_t* wide, int nwords, size_t i) {
+#pragma unroll
+    for (int k = 0; k < 8; k++) acc[k] = 0;
+#pragma unroll 1
+    for (int blk = (nwords >> 3) - 1; blk >= 0; blk--) {
+        uint32_t w[8], t[8], u[8];
+        load_u256(w, wide, i * (size_t)(nwords >> 3) + (size_t)blk);
+        montmul_suborder(t, acc, BJJ_L_R2);
+        montmul_suborder(u, w, BJJ_L_R1);
+        add256(acc, t, u);
+#pragma unroll 1
+        for (int k = 1; k >= 0; k--) {
+            uint32_t lk[8];
+            u256_shl(lk, BJJ_SUBORDER, k);
+            const uint32_t borrow = sub256(t, acc, lk);
+#pragma unroll
+            for (int j = 0; j < 8; j++) acc[j] = borrow ? acc[j] : t[j];
+        }
+    }
+}
+
+// ---- PrivateKey::sign_schnorr (src/lib.rs:344-362) with the caller's nonce k, as a pipeline
+// (bjj_cuda.cu::launch_sign_schnorr): r = B8 * k; pk = public(); h = Poseidon(pk.x, pk.y, r.x, r.y, msg); s = k + sk * h,
+// unreduced.  The nonce of lane i is nwords words at word offset nwords * i; s is nwords + 8 words.
+// phase 1: status, sk = scalar_key(key), kr = k mod SUBORDER (B8 has order SUBORDER, so kr * B8 = k * B8 for every k), and
+// the msg to hash (0 where msg > Q, and msg == Q hashes as 0).  Rejected lanes get sk = kr = 0, as in lane_sign_scalars.
+BJJ_HD void lane_sign_schnorr_scalars(const uint8_t* key32, const uint8_t* msg32, const uint8_t* nonce, int nwords, uint8_t* sk_out,
+                                      uint8_t* kr_out, uint8_t* msg_out, uint8_t* status, size_t i) {
+    uint32_t key[8], msg[8], sk[8], kr[8];
+    load_u256(key, key32, i);
+    load_u256(msg, msg32, i);
+    const uint32_t q[8] = BJJ_LIMBS8(BJJ_Q);
+    const bool bad = u256_lt(q, msg), eq_q = u256_eq(q, msg);
+    scalar_key_from_key(sk, key);
+    lane_mod_suborder_wide(kr, nonce, nwords, i);
+#pragma unroll
+    for (int k = 0; k < 8; k++) {
+        sk[k] = bad ? 0u : sk[k];
+        kr[k] = bad ? 0u : kr[k];
+        msg[k] = (bad || eq_q) ? 0u : msg[k];
+    }
+    store_u256(sk_out, i, sk);
+    store_u256(kr_out, i, kr);
+    store_u256(msg_out, i, msg);
+    status[i] = bad ? (uint8_t)BJJ_ST_MSG_RANGE : (uint8_t)BJJ_ST_OK;
+}
+// last phase: s = k + sk * h exactly, carried through nwords + 8 words (sk < 2^252 and h < Q < 2^254, so s < k + 2^506).
+// A lane whose status is not OK gets zero r and s: the affine pass wrote (0, 1) there for kr = 0.
+BJJ_HD void lane_sign_schnorr_finish(const uint8_t* h32, const uint8_t* sk32, const uint8_t* nonce, int nwords, const uint8_t* status,
+                                     uint8_t* rx, uint8_t* ry, uint8_t* s, size_t i) {
+    const size_t kb = (size_t)(nwords >> 3), sb = kb + 1;     // 256-bit blocks of k and of s
+    uint32_t w[8];
+    if (status[i] != BJJ_ST_OK) {
+#pragma unroll
+        for (int k = 0; k < 8; k++) w[k] = 0;
+        store_u256(rx, i, w);
+        store_u256(ry, i, w);
+#pragma unroll 1
+        for (size_t b = 0; b < sb; b++) store_u256(s, i * sb + b, w);
+        return;
+    }
+    uint32_t h[8], sk[8], p[16];
+    load_u256(h, h32, i);
+    load_u256(sk, sk32, i);
+#pragma unroll
+    for (int k = 0; k < 16; k++) p[k] = 0;
+#pragma unroll
+    for (int a = 0; a < 8; a++) {
+        uint64_t c = 0;
+#pragma unroll
+        for (int b = 0; b < 8; b++) {
+            c += (uint64_t)sk[a] * h[b] + p[a + b];
+            p[a + b] = (uint32_t)c;
+            c >>= 32;
+        }
+        p[a + 8] = (uint32_t)c;
+    }
+    uint64_t c = 0;
+#pragma unroll 1
+    for (size_t b = 0; b < sb; b++) {
+        if (b < kb) {
+            load_u256(w, nonce, i * kb + b);
+        } else {
+#pragma unroll
+            for (int k = 0; k < 8; k++) w[k] = 0;
+        }
+#pragma unroll
+        for (int k = 0; k < 8; k++) {
+            c += (uint64_t)w[k] + (b == 0 ? p[k] : (b == 1 ? p[8 + k] : 0u));
+            w[k] = (uint32_t)c;
+            c >>= 32;
+        }
+        store_u256(s, i * sb + b, w);
+    }
+}
+
 // verify (src/lib.rs:395-412).  Returns 0/1 like the reference's bool.
 //   msg > Q -> false; hm = Poseidon(R8.x, R8.y, A.x, A.y, msg mod Q);
 //   accept iff  S*B8 == R8 + (8*hm)*A   compared in affine coordinates.

@@ -13,7 +13,7 @@
 //   verify(pk, sig, msg)                   src/lib.rs:395-412
 //   verify_schnorr(pk, m, r, s)            src/lib.rs:375-385
 //   + batch entry points: mul_scalar_batch, public_batch, decompress_batch, verify_batch,
-//     public_compressed_batch, sign_compressed_batch
+//     public_compressed_batch, sign_compressed_batch, sign_schnorr_batch (caller nonces)
 //   + FixedBase: the comb table of a caller-chosen point, k*P and k*P + l*Q at the fixed-base rate, and verify for
 //     many signatures of that one key
 //   + MultiGpu: shards a batch over every device, one host thread + one bjj_ctx per device, no NCCL
@@ -255,6 +255,38 @@ inline std::vector<SignCompressedResult> sign_compressed_batch(const std::vector
     std::vector<SignCompressedResult> out(n);
     for (size_t i = 0; i < n; i++) {
         std::memcpy(out[i].sig.data(), &sig[64 * i], 64);
+        out[i].status = st[i];
+    }
+    return out;
+}
+
+struct SignSchnorrResult {
+    Point r;                              // B8 * k; zero when status != 0
+    std::vector<uint8_t> s;               // k + scalar_key * h, unreduced: 4 * (nonce_words + 8) bytes little-endian
+    uint8_t status;                       // 0 ok; otherwise bjj_status_string(status) is the reference's Err text
+};
+// [k.sign_schnorr(m) for k, m in zip(keys, msgs)] (src/lib.rs:344-362) with the caller's nonces instead of the
+// reference's random ones: nonce i is nonces[nonce_words * i ..] (little-endian 32-bit words), nonce_words a multiple
+// of 8 in 8..64 (the reference's 1024-bit nonce is 32 words).  msg > Q gives status BJJ_STATUS_MSG_RANGE.
+inline std::vector<SignSchnorrResult> sign_schnorr_batch(const std::vector<PrivateKey>& keys, const std::vector<U256>& msgs,
+                                                         const std::vector<uint32_t>& nonces, int nonce_words,
+                                                         Engine& e = default_engine()) {
+    const size_t n = keys.size();
+    if (msgs.size() != n || nonce_words <= 0 || nonces.size() != (size_t)nonce_words * n)
+        throw std::invalid_argument("keys, msgs and nonces differ in length");
+    const size_t sw = 4 * ((size_t)nonce_words + 8);
+    std::vector<uint8_t> k(32 * n), kn(4 * nonces.size()), rx(32 * n), ry(32 * n), s(sw * n), st(n);
+    for (size_t i = 0; i < n; i++) std::memcpy(&k[32 * i], keys[i].key.data(), 32);
+    for (size_t j = 0; j < nonces.size(); j++)
+        for (int b = 0; b < 4; b++) kn[4 * j + b] = (uint8_t)(nonces[j] >> (8 * b));
+    auto m = pack(msgs);
+    Engine::check(bjj_sign_schnorr_batch(e.ctx(), n, k.data(), m.data(), kn.data(), nonce_words, rx.data(), ry.data(), s.data(),
+                                         st.data()), "bjj_sign_schnorr_batch");
+    std::vector<SignSchnorrResult> out(n);
+    for (size_t i = 0; i < n; i++) {
+        std::memcpy(out[i].r.x.data(), &rx[32 * i], 32);
+        std::memcpy(out[i].r.y.data(), &ry[32 * i], 32);
+        out[i].s.assign(s.begin() + sw * i, s.begin() + sw * (i + 1));
         out[i].status = st[i];
     }
     return out;

@@ -203,6 +203,20 @@ int bjj_sign_compressed_batch(bjj_ctx* ctx, size_t n, const uint8_t* key32, cons
 int bjj_sign_compressed_batch_dev(bjj_ctx* ctx, size_t n, const uint8_t* key32, const uint8_t* msg32, uint8_t* sig64,
                                   uint8_t* status, void* stream);
 
+/* ---- PrivateKey::sign_schnorr (src/lib.rs:344-362) with the nonce k supplied by the caller (the reference draws
+ *      gen_biguint(1024)): r = B8*k, h = schnorr_hash(pk, msg, r) = Poseidon(pk.x, pk.y, r.x, r.y, msg) (src/lib.rs:364-373),
+ *      s = k + scalar_key(key)*h, NOT reduced, exactly the reference's BigInt.
+ *      Nonce i is `nonce_words` little-endian 32-bit words at byte offset 4*nonce_words*i, nonce_words a multiple of 8 in
+ *      8..64 (as bjj_mul_scalar_wide_batch; the reference's 1024-bit nonce is nonce_words = 32); other widths return
+ *      BJJ_ERR_ARG.  s[i] is nonce_words + 8 words at byte offset 4*(nonce_words + 8)*i, which always holds it
+ *      (scalar_key < 2^252, h < Q < 2^254).  r is (0, 1) for k = 0 and every multiple of SUBORDER, as in the reference.
+ *      status[i] = BJJ_STATUS_MSG_RANGE when msg > Q (Err("msg outside the Finite Field")), and then rx, ry and s of the
+ *      lane are zero; msg == Q hashes as 0. */
+int bjj_sign_schnorr_batch(bjj_ctx* ctx, size_t n, const uint8_t* key32, const uint8_t* msg32, const uint8_t* nonce,
+                           int nonce_words, uint8_t* rx, uint8_t* ry, uint8_t* s, uint8_t* status);
+int bjj_sign_schnorr_batch_dev(bjj_ctx* ctx, size_t n, const uint8_t* key32, const uint8_t* msg32, const uint8_t* nonce,
+                               int nonce_words, uint8_t* rx, uint8_t* ry, uint8_t* s, uint8_t* status, void* stream);
+
 /* ---- Point::compress (src/lib.rs:166-178) / decompress_point (src/lib.rs:192-224) ---------------- */
 int bjj_compress_batch(bjj_ctx* ctx, size_t n, const uint8_t* px, const uint8_t* py, uint8_t* out32);
 int bjj_compress_batch_dev(bjj_ctx* ctx, size_t n, const uint8_t* px, const uint8_t* py, uint8_t* out32, void* stream);
@@ -268,6 +282,8 @@ int bjj_multi_public_batch(bjj_multi* m, size_t n, const uint8_t* key32, uint8_t
 int bjj_multi_public_compressed_batch(bjj_multi* m, size_t n, const uint8_t* key32, uint8_t* out32);
 int bjj_multi_sign_compressed_batch(bjj_multi* m, size_t n, const uint8_t* key32, const uint8_t* msg32, uint8_t* sig64,
                                     uint8_t* status);
+int bjj_multi_sign_schnorr_batch(bjj_multi* m, size_t n, const uint8_t* key32, const uint8_t* msg32, const uint8_t* nonce,
+                                 int nonce_words, uint8_t* rx, uint8_t* ry, uint8_t* s, uint8_t* status);
 int bjj_multi_fixed_base_batch(bjj_multi* m, size_t n, const uint8_t* scalar32, uint8_t* rx, uint8_t* ry);
 int bjj_multi_decompress_batch(bjj_multi* m, size_t n, const uint8_t* in32, uint8_t* rx, uint8_t* ry, uint8_t* status);
 

@@ -81,6 +81,9 @@ extern "C" {
     pub fn bjj_public_compressed_batch(ctx: *mut bjj_ctx, n: usize, key32: *const u8, out32: *mut u8) -> c_int;
     pub fn bjj_sign_compressed_batch(ctx: *mut bjj_ctx, n: usize, key32: *const u8, msg32: *const u8, sig64: *mut u8,
                                      status: *mut u8) -> c_int;
+    // PrivateKey::sign_schnorr with caller nonces (src/lib.rs:344-362): nonce_words-word nonces, (nonce_words + 8)-word s
+    pub fn bjj_sign_schnorr_batch(ctx: *mut bjj_ctx, n: usize, key32: *const u8, msg32: *const u8, nonce: *const u8,
+                                  nonce_words: c_int, rx: *mut u8, ry: *mut u8, s: *mut u8, status: *mut u8) -> c_int;
     // Point::compress / decompress_point (src/lib.rs:166-178, 192-224)
     pub fn bjj_compress_batch(ctx: *mut bjj_ctx, n: usize, px: *const u8, py: *const u8, out32: *mut u8) -> c_int;
     pub fn bjj_decompress_batch(ctx: *mut bjj_ctx, n: usize, in32: *const u8, rx: *mut u8, ry: *mut u8,
@@ -114,6 +117,8 @@ extern "C" {
     pub fn bjj_multi_public_compressed_batch(m: *mut bjj_multi, n: usize, key32: *const u8, out32: *mut u8) -> c_int;
     pub fn bjj_multi_sign_compressed_batch(m: *mut bjj_multi, n: usize, key32: *const u8, msg32: *const u8, sig64: *mut u8,
                                            status: *mut u8) -> c_int;
+    pub fn bjj_multi_sign_schnorr_batch(m: *mut bjj_multi, n: usize, key32: *const u8, msg32: *const u8, nonce: *const u8,
+                                        nonce_words: c_int, rx: *mut u8, ry: *mut u8, s: *mut u8, status: *mut u8) -> c_int;
     pub fn bjj_multi_fixed_base_batch(m: *mut bjj_multi, n: usize, scalar32: *const u8, rx: *mut u8, ry: *mut u8) -> c_int;
     pub fn bjj_multi_decompress_batch(m: *mut bjj_multi, n: usize, in32: *const u8, rx: *mut u8, ry: *mut u8,
                                       status: *mut u8) -> c_int;

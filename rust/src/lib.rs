@@ -442,6 +442,39 @@ pub fn sign_compressed_batch(keys: &[PrivateKey], msgs: &[BigInt]) -> Vec<Result
         .collect()
 }
 
+/// `keys[i].sign_schnorr(msgs[i])` (src/lib.rs:344-362) with the nonce `nonces[i]` instead of the reference's random
+/// 1024-bit one: `(r, s)` with `s = k + scalar_key * h` unreduced; msg > Q gives the reference's Err.  The nonces cross
+/// the ABI in the smallest multiple of 256 bits that holds the widest.  Panics on a negative msg or nonce, or on a nonce
+/// wider than 2048 bits.
+pub fn sign_schnorr_batch_with_nonces(keys: &[PrivateKey], msgs: &[BigInt], nonces: &[BigInt]) -> Vec<Result<(Point, BigInt), String>> {
+    let n = keys.len();
+    assert!(n == msgs.len() && n == nonces.len());
+    assert!(msgs.iter().all(|m| m.sign() != Sign::Minus), "negative msg");
+    assert!(nonces.iter().all(|k| k.sign() != Sign::Minus), "negative nonce");
+    let bits = nonces.iter().map(|k| k.bits()).max().unwrap_or(0).max(1);
+    assert!(bits <= 2048, "nonce wider than 2048 bits");
+    let words = (8 * ((bits + 255) / 256)) as usize;
+    let mut kb = vec![0u8; 4 * words * n];
+    for (i, k) in nonces.iter().enumerate() {
+        let (_, bytes) = k.to_bytes_le();
+        kb[4 * words * i..4 * words * i + bytes.len()].copy_from_slice(&bytes);
+    }
+    let k = col(n, |i| keys[i].key);
+    let m = col(n, |i| msg_le32(&msgs[i]));
+    let sw = 4 * (words + 8);
+    let (mut rx, mut ry, mut s, mut st) = (vec![0u8; 32 * n], vec![0u8; 32 * n], vec![0u8; sw * n], vec![0u8; n]);
+    check(unsafe { ffi::bjj_sign_schnorr_batch(engine().raw(), n, k.as_ptr(), m.as_ptr(), kb.as_ptr(), words as i32, rx.as_mut_ptr(),
+                                               ry.as_mut_ptr(), s.as_mut_ptr(), st.as_mut_ptr()) }, "bjj_sign_schnorr_batch");
+    (0..n)
+        .map(|i| {
+            if st[i] != 0 {
+                return Err(status_str(st[i]));
+            }
+            Ok((Point { x: row(&rx, i), y: row(&ry, i) }, BigInt::from_bytes_le(Sign::Plus, &s[sw * i..sw * (i + 1)])))
+        })
+        .collect()
+}
+
 pub fn decompress_batch(blobs: &[[u8; 32]]) -> Vec<Result<Point, String>> {
     let n = blobs.len();
     let inp = col(n, |i| blobs[i]);
