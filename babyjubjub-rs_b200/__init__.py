@@ -19,6 +19,8 @@ follow the reference's public API (paths into the reference tree):
       PrivateKey::sign(msg).compress() with the compression done on the device.
     + verify_base_batch: verify for many signatures of ONE key, with the key's FixedBase table
       (two comb walks per signature instead of verify_batch's per-lane ladder).
+    + KeySet / verify_keyset_batch: verify for batches that mix many known keys, each key with a compact
+      comb table (4,130 entries, 396 KB) and a key index per signature.
     + sign_schnorr_batch: PrivateKey::sign_schnorr over a batch, with caller-supplied (or random 1024-bit)
       nonces and the unreduced s of the reference.
 
@@ -89,7 +91,7 @@ class Engine:
             raise BjjError(rc, "bjj_init", self.lib.bjj_error_string(rc).decode())
         self.ctx = ctx
         self.device = int(device)
-        self._bases = weakref.WeakSet()     # FixedBase tables of this context: freed before the context
+        self._bases = weakref.WeakSet()     # FixedBase tables and KeySets of this context: freed before the context
 
     def close(self):
         if getattr(self, "ctx", None):
@@ -312,6 +314,35 @@ class Engine:
                                                               _ptr(status)), "bjj_verify_base_compressed_batch")
         return ok, status
 
+    def verify_keyset_batch(self, keyset, key_index, r8x, r8y, s, msg):
+        """verify for every lane against key key_index[i] of `keyset` (a KeySet of this engine) -> ok (n,) uint8"""
+        ins = [_as_u8(v, 32) for v in (r8x, r8y, s, msg)]
+        ki = _key_index(key_index, len(ins[0]))
+        ok = np.empty(len(ins[0]), dtype=np.uint8)
+        self._check(self.lib.bjj_verify_keyset_batch(self.ctx, _keyset_handle(keyset), len(ki), _ptr(ki), *[_ptr(v) for v in ins],
+                                                     _ptr(ok)), "bjj_verify_keyset_batch")
+        return ok
+
+    def verify_keyset_compressed_batch(self, keyset, key_index, sig64, msg):
+        """verify of 64-byte compressed signatures against key key_index[i] of `keyset` -> (ok, status), both (n,) uint8;
+        status is R8's decompression error"""
+        sg, m = _as_u8(sig64, 64), _as_u8(msg, 32)
+        ki = _key_index(key_index, len(sg))
+        ok = np.empty(len(sg), dtype=np.uint8)
+        status = np.empty(len(sg), dtype=np.uint8)
+        self._check(self.lib.bjj_verify_keyset_compressed_batch(self.ctx, _keyset_handle(keyset), len(ki), _ptr(ki), _ptr(sg), _ptr(m),
+                                                                _ptr(ok), _ptr(status)), "bjj_verify_keyset_compressed_batch")
+        return ok, status
+
+    def keyset_mul_batch(self, keyset, key_index, scalars):
+        """P_{key_index[i]} * k_i for every 256-bit scalar k_i (raw, unreduced) -> (rx, ry), (n, 32) uint8 each"""
+        k = _as_u8(scalars, 32)
+        ki = _key_index(key_index, len(k))
+        rx, ry = np.empty_like(k), np.empty_like(k)
+        self._check(self.lib.bjj_keyset_mul_batch(self.ctx, _keyset_handle(keyset), len(ki), _ptr(ki), _ptr(k), _ptr(rx), _ptr(ry)),
+                    "bjj_keyset_mul_batch")
+        return rx, ry
+
 
 
 _default_engine = None
@@ -357,6 +388,67 @@ class FixedBase:
         """[P.mul_scalar(k) for k in scalars] (src/lib.rs:149-164) for Python ints of any size and sign"""
         rx, ry = self.engine.base_mul_batch(self, ints_to_le32([_base_scalar(k) for k in scalars]))
         return [Point(x, y) for x, y in zip(le32_to_ints(rx), le32_to_ints(ry))]
+
+
+class KeySet:
+    """N on-curve public keys on one Engine, each with a compact comb table (396,480 B of device memory per key):
+    verify and k*P for batches that name a key per lane.  Raises BjjError with code 3 (BJJ_ERR_NONCANONICAL) when a
+    coordinate is >= Q and with code 2 (BJJ_ERR_ARG) when a key is off the curve (or the list is empty); `status` then
+    holds one code per key (0 ok, 1 off the curve, 2 non-canonical).  Free it with close() (or let it be collected)."""
+
+    def __init__(self, points, engine=None):
+        self.engine = engine or default_engine()
+        pts = [(p.x, p.y) if isinstance(p, Point) else tuple(p) for p in points]
+        self.points = [Point(x, y) for x, y in pts]
+        self.handle = None
+        ax, ay = ints_to_le32([p[0] for p in pts]), ints_to_le32([p[1] for p in pts])
+        self.status = np.zeros(len(pts), dtype=np.uint8)
+        handle = ctypes.c_void_p()
+        rc = self.engine.lib.bjj_keyset_create(self.engine.ctx, len(pts), _ptr(ax), _ptr(ay), _ptr(self.status), ctypes.byref(handle))
+        if rc != 0:
+            self.engine._check(rc, "bjj_keyset_create")
+        self.handle = handle
+        self.engine._bases.add(self)
+
+    def __len__(self):
+        return len(self.points)
+
+    def close(self):
+        if getattr(self, "handle", None):
+            self.engine.lib.bjj_keyset_destroy(self.engine.ctx, self.handle)
+            self.handle = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def mul_batch(self, key_index, scalars):
+        """[points[j].mul_scalar(k) for j, k in zip(key_index, scalars)] (src/lib.rs:149-164), Python ints of any size
+        and sign"""
+        rx, ry = self.engine.keyset_mul_batch(self, key_index, ints_to_le32([_base_scalar(k) for k in scalars]))
+        return [Point(x, y) for x, y in zip(le32_to_ints(rx), le32_to_ints(ry))]
+
+
+def _keyset_handle(keyset):
+    if keyset is None:
+        raise ValueError("a keyset call needs a KeySet")
+    if not keyset.handle:
+        raise ValueError("KeySet is closed")
+    return keyset.handle
+
+
+def _key_index(key_index, n):
+    """key indices as the ABI's little-endian uint32 per lane; an index outside [0, 2^32) cannot name a key"""
+    ki = np.asarray(key_index)
+    if ki.ndim != 1 or len(ki) != n:
+        raise ValueError("expected %d key indices, got shape %r" % (n, ki.shape))
+    if ki.dtype != np.uint32:
+        if len(ki) and (ki.min() < 0 or ki.max() > 0xFFFFFFFF):
+            raise ValueError("key index outside [0, 2^32)")
+        ki = ki.astype(np.uint32)
+    return np.ascontiguousarray(ki, dtype="<u4")
 
 
 def _handle(base):
@@ -695,6 +787,17 @@ def verify_base_batch(base, sigs, msgs, engine=None):
     eng = engine or base.engine
     ok = eng.verify_base_batch(base, ints_to_le32([s.r_b8.x for s in sigs]), ints_to_le32([s.r_b8.y for s in sigs]),
                                ints_to_le32([_verify_scalar(s.s) for s in sigs]), _verify_msgs(msgs))
+    return [bool(v) for v in ok]
+
+
+def verify_keyset_batch(keyset, key_index, sigs, msgs, engine=None):
+    """[verify(keyset.points[j], sig, msg) for j, sig, msg in zip(key_index, sigs, msgs)] (src/lib.rs:395-412) for
+    signatures of many known keys; the same results as verify_batch with those keys.  An index outside the set raises
+    BjjError (BJJ_ERR_ARG)."""
+    eng = engine or keyset.engine
+    ok = eng.verify_keyset_batch(keyset, np.asarray(key_index, dtype=np.int64).reshape(-1), ints_to_le32([s.r_b8.x for s in sigs]),
+                                 ints_to_le32([s.r_b8.y for s in sigs]), ints_to_le32([_verify_scalar(s.s) for s in sigs]),
+                                 _verify_msgs(msgs))
     return [bool(v) for v in ok]
 
 

@@ -10,6 +10,7 @@ _sz = ctypes.c_size_t
 _ctx = ctypes.c_void_p
 _int = ctypes.c_int
 _base = ctypes.c_void_p     # bjj_base*: a fixed-base table (NULL selects B8)
+_keyset = ctypes.c_void_p   # bjj_keyset*: keys with compact comb tables
 
 # symbol -> (restype, argtypes); the single source the ABI test checks against include/bjj_cuda.h
 SIGNATURES = {
@@ -52,6 +53,11 @@ SIGNATURES = {
     "bjj_base_mul2_batch": (_int, [_ctx, _base, _base, _sz] + [_u8p] * 4),
     "bjj_verify_base_batch": (_int, [_ctx, _base, _sz] + [_u8p] * 5),
     "bjj_verify_base_compressed_batch": (_int, [_ctx, _base, _sz] + [_u8p] * 4),
+    "bjj_keyset_create": (_int, [_ctx, _sz, _u8p, _u8p, _u8p, ctypes.POINTER(_keyset)]),
+    "bjj_keyset_destroy": (None, [_ctx, _keyset]),
+    "bjj_verify_keyset_batch": (_int, [_ctx, _keyset, _sz] + [_u8p] * 6),
+    "bjj_verify_keyset_compressed_batch": (_int, [_ctx, _keyset, _sz] + [_u8p] * 5),
+    "bjj_keyset_mul_batch": (_int, [_ctx, _keyset, _sz] + [_u8p] * 4),
 }
 # every batch op also has a device-pointer flavour with a trailing `void* stream`
 for _name in [k for k in SIGNATURES if k.endswith("_batch")]:

@@ -43,6 +43,22 @@ __global__ void __launch_bounds__(BJJ_BLOCK) k_comb_build_point(CombEntry* comb,
     if (idx == 0) *status = st;
 }
 
+// key sets (bjj_keyset_create): check the keys and rewrite them in Montgomery form, then per sub-batch of keys the
+// window chains (one thread per (key, window)) and the batched affine pass that writes the table entries
+__global__ void __launch_bounds__(BJJ_BLOCK) k_keyset_check(size_t n, uint8_t* kx, uint8_t* ky, uint8_t* status) {
+    BJJ_LANE_LOOP(n) status[i] = (uint8_t)lane_keyset_check(kx, ky, i);
+}
+__global__ void __launch_bounds__(BJJ_BLOCK) k_keyset_build(size_t keys, const uint8_t* kx, const uint8_t* ky, ProjScratch scr,
+                                                            CombEntry* tables) {
+    BJJ_LANE_LOOP(keys * Comb8::WINDOWS) {
+        const size_t k = i / Comb8::WINDOWS;
+        lane_keyset_build(kx, ky, k, (int)(i % Comb8::WINDOWS), scr, k * BJJ_KEY_BUILD_POINTS, tables + k * BJJ_KEY_COMB_TOTAL);
+    }
+}
+__global__ void __launch_bounds__(BJJ_BLOCK) k_keyset_affine(size_t n, ProjScratch scr, CombEntry* tables) {
+    batch_affine_strided(scr, KeysetCombOut{tables}, n, (size_t)blockIdx.x * blockDim.x + threadIdx.x, (size_t)gridDim.x * blockDim.x);
+}
+
 __global__ void __launch_bounds__(BJJ_BLOCK) k_split_scalars(size_t n, const uint8_t* h32, const uint8_t* s32, uint8_t* u32,
                                                              uint8_t* v32, uint8_t* w32) {
     BJJ_LANE_LOOP(n) lane_split_scalars(h32, s32, u32, v32, w32, i);
@@ -99,6 +115,15 @@ __global__ void __launch_bounds__(BJJ_BLOCK, 2) k_fixed_base2(size_t n, const ui
                                                            const CombEntry* comb_p, const CombEntry* comb_q,
                                                            unsigned long long* work) {
     BJJ_POINT_LOOP(n, work) lane_fixed_base2(k, l, scr, i, comb_p, comb_q);
+}
+
+// P_{key_index[i]}.mul_scalar(k) over a key set's compact tables (bjj_keyset_mul)
+__global__ void __launch_bounds__(BJJ_BLOCK, 2) k_keyset_mul(size_t n, const uint8_t* k, const uint8_t* key_index, uint32_t n_keys,
+                                                          const CombEntry* tables, ProjScratch scr, uint32_t* gflags,
+                                                          unsigned long long* work) {
+    BJJ_FLAGS_BEGIN
+    BJJ_POINT_LOOP(n, work) lane_keyset_mul(k, key_index, n_keys, tables, scr, i, flags);
+    BJJ_FLAGS_END(gflags)
 }
 
 #ifndef BJJ_PUBLIC_BALLAST
@@ -203,6 +228,15 @@ struct bjj_base {
     bjj_ctx* ctx;
     CombEntry* comb;
     uint8_t x[32], y[32];
+};
+
+// N keys with their compact combs (bjj_keyset_create), on the device of the context that built them: `keys` holds the
+// x plane then the y plane (Montgomery form, 32 B per key each), `tables` the N Comb8 tables
+struct bjj_keyset {
+    bjj_ctx* ctx;
+    size_t n_keys;
+    uint8_t* keys;
+    CombEntry* tables;
 };
 
 #define CU(ctx, call)                      \
@@ -499,6 +533,7 @@ int bjj_sync(bjj_ctx* ctx) {
     CU(ctx, cudaMemsetAsync(ctx->flags_dev, 0, sizeof(uint32_t), ctx->stream));
     CU(ctx, cudaStreamSynchronize(ctx->stream));
     uint32_t f = *ctx->flags_host;
+    if (f & BJJ_FLAG_KEY_INDEX) return BJJ_ERR_ARG;
     if (f & BJJ_FLAG_NONCANONICAL) return BJJ_ERR_NONCANONICAL;
     return BJJ_OK;
 }
@@ -560,6 +595,88 @@ void bjj_base_destroy(bjj_ctx* ctx, bjj_base* base) {
     cudaDeviceSynchronize();      // calls on any stream may still read the table
     cudaFree(base->comb);
     free(base);
+}
+
+// keys per build sub-batch of bjj_keyset_create: their build lanes fit the point kernels' sub-batch of scratch
+#define BJJ_KEYSET_SUBBATCH (BJJ_POINT_SUBBATCH / BJJ_KEY_BUILD_POINTS)
+
+// cudaMalloc that reports a failure as BJJ_ERR_NOMEM with the CUDA error cleared: the tables of a large key set may
+// simply not fit
+static int dev_alloc(void** p, size_t bytes) {
+    if (cudaMalloc(p, bytes) == cudaSuccess) return BJJ_OK;
+    cudaGetLastError();
+    *p = nullptr;
+    return BJJ_ERR_NOMEM;
+}
+
+static void keyset_free(bjj_keyset* ks) {
+    if (ks->keys) cudaFree(ks->keys);
+    if (ks->tables) cudaFree(ks->tables);
+    free(ks);
+}
+
+int bjj_keyset_create(bjj_ctx* ctx, size_t n_keys, const uint8_t* ax, const uint8_t* ay, uint8_t* key_status, bjj_keyset** out) {
+    if (!out) return BJJ_ERR_ARG;
+    *out = nullptr;
+    if (!ctx || !ax || !ay || n_keys == 0 || n_keys > 0xFFFFFFFFull) return BJJ_ERR_ARG;
+    CU(ctx, cudaSetDevice(ctx->device));
+    bjj_keyset* ks = (bjj_keyset*)calloc(1, sizeof(bjj_keyset));
+    uint8_t* status = (uint8_t*)malloc(n_keys);
+    int rc = ks && status ? BJJ_OK : BJJ_ERR_NOMEM;
+    // the key planes, then one status byte per key
+    if (rc == BJJ_OK) rc = dev_alloc((void**)&ks->keys, 65 * n_keys);
+    auto body = [&]() -> int {
+        uint8_t *kx = ks->keys, *ky = kx + 32 * n_keys, *st_dev = ky + 32 * n_keys;
+        cudaStream_t st = ctx->stream;
+        CU(ctx, cudaMemcpyAsync(kx, ax, 32 * n_keys, cudaMemcpyHostToDevice, st));
+        CU(ctx, cudaMemcpyAsync(ky, ay, 32 * n_keys, cudaMemcpyHostToDevice, st));
+        k_keyset_check<<<grid_for(ctx, k_keyset_check, n_keys), BJJ_BLOCK, 0, st>>>(n_keys, kx, ky, st_dev);
+        TRY(launched(ctx));
+        CU(ctx, cudaMemcpyAsync(status, st_dev, n_keys, cudaMemcpyDeviceToHost, st));
+        CU(ctx, cudaStreamSynchronize(st));
+        if (key_status) memcpy(key_status, status, n_keys);
+        // a coordinate >= Q outranks a key off the curve; the reference's product with an off-curve key depends on its
+        // double-and-add order, which a comb does not follow, so such keys are refused as by bjj_base_create
+        bool off = false;
+        for (size_t j = 0; j < n_keys; j++) {
+            if (status[j] == BJJ_BASE_NONCANONICAL) return BJJ_ERR_NONCANONICAL;
+            off = off || status[j] != BJJ_BASE_OK;
+        }
+        if (off) return BJJ_ERR_ARG;
+        TRY(dev_alloc((void**)&ks->tables, n_keys * BJJ_KEY_COMB_TOTAL * sizeof(CombEntry)));
+        // the build borrows the context's projective scratch, which a _dev call on another stream may still use
+        CU(ctx, cudaDeviceSynchronize());
+        for (size_t k0 = 0; k0 < n_keys; k0 += BJJ_KEYSET_SUBBATCH) {
+            const size_t keys = n_keys - k0 < BJJ_KEYSET_SUBBATCH ? n_keys - k0 : BJJ_KEYSET_SUBBATCH;
+            const size_t lanes = keys * BJJ_KEY_BUILD_POINTS;
+            ProjScratch scr;
+            TRY(ensure_proj(ctx, &ctx->ws, lanes, &scr));
+            CombEntry* tbl = ks->tables + k0 * BJJ_KEY_COMB_TOTAL;
+            k_keyset_build<<<grid_for(ctx, k_keyset_build, keys * Comb8::WINDOWS), BJJ_BLOCK, 0, st>>>(keys, kx + 32 * k0, ky + 32 * k0,
+                                                                                                     scr, tbl);
+            k_keyset_affine<<<affine_grid(ctx, lanes), BJJ_BLOCK, 0, st>>>(lanes, scr, tbl);
+            TRY(launched(ctx, 2));
+        }
+        CU(ctx, cudaStreamSynchronize(st));
+        return BJJ_OK;
+    };
+    if (rc == BJJ_OK) rc = body();
+    free(status);
+    if (rc != BJJ_OK) {
+        if (ks) keyset_free(ks);
+        return rc;
+    }
+    ks->ctx = ctx;
+    ks->n_keys = n_keys;
+    *out = ks;
+    return BJJ_OK;
+}
+
+void bjj_keyset_destroy(bjj_ctx* ctx, bjj_keyset* ks) {
+    if (!ctx || !ks || ks->ctx != ctx) return;
+    cudaSetDevice(ctx->device);
+    cudaDeviceSynchronize();      // calls on any stream may still read the tables
+    keyset_free(ks);
 }
 
 }  // extern "C"
@@ -681,6 +798,23 @@ static int launch_base_mul(bjj_ctx* ctx, size_t n, const uint8_t* k, const uint8
             k_fixed_base2<<<grid_for(ctx, k_fixed_base2, m), BJJ_BLOCK, 0, st>>>(m, k + o, l + o, scr, comb_p, comb_q, work);
         else
             k_fixed_base<<<grid_for(ctx, k_fixed_base, m), BJJ_BLOCK, 0, st>>>(m, k + o, scr, comb_p, work);
+        TRY(launched(ctx));
+        k_batch_affine<<<affine_grid(ctx, m), BJJ_BLOCK, 0, st>>>(m, scr, rx + o, ry + o);
+        return launched(ctx);
+    });
+}
+// P_{key_index[i]} * k_i over the compact tables of a key set (bjj_keyset_mul*)
+static int launch_keyset_mul(bjj_ctx* ctx, const bjj_keyset* ks, size_t n, const uint8_t* key_index, const uint8_t* k, uint8_t* rx,
+                             uint8_t* ry, cudaStream_t st, Workspace* ws) {
+    const size_t lanes = scratch_lanes(ctx, n);
+    return for_each_subbatch(n, [&](size_t off, size_t m) -> int {
+        const size_t o = 32 * off;
+        ProjScratch scr;
+        TRY(ensure_proj(ctx, ws, lanes, &scr));
+        unsigned long long* work = nullptr;
+        TRY(claim_counter(ctx, ws, st, &work));
+        k_keyset_mul<<<grid_for(ctx, k_keyset_mul, m), BJJ_BLOCK, 0, st>>>(m, k + o, key_index + 4 * off, (uint32_t)ks->n_keys, ks->tables,
+                                                                          scr, ctx->flags_dev, work);
         TRY(launched(ctx));
         k_batch_affine<<<affine_grid(ctx, m), BJJ_BLOCK, 0, st>>>(m, scr, rx + o, ry + o);
         return launched(ctx);
@@ -834,10 +968,12 @@ static int launch_verify_compressed(bjj_ctx* ctx, size_t n, const uint8_t* sig64
 // and no exact-lane queue (off-curve R8 lanes take a branch of the EC kernel).  sig64 != nullptr is the compressed
 // form: R8 (the first half of each 64-byte signature) is decompressed first into two verify-scratch planes, by phase
 // 0 of launch_verify_compressed for R8 alone; `status` receives its decompression status and failed lanes are
-// rejected.  The key's coordinates are kernel arguments: base_create checked them.
-static int launch_verify_base(bjj_ctx* ctx, const bjj_base* base, size_t n, const uint8_t* r8x, const uint8_t* r8y,
-                              const uint8_t* s32, const uint8_t* sig64, const uint8_t* msg, uint8_t* ok, uint8_t* status,
-                              cudaStream_t st, Workspace* ws) {
+// rejected.  The key's coordinates are kernel arguments: base_create checked them.  With a key set `ks` instead of
+// `base` (bjj_verify_keyset*), lane i takes key key_index[i] of the set and its compact table: the kernels
+// k_verify_keyset_hash -> k_verify_keyset_ec, with the same launches.
+static int launch_verify_base(bjj_ctx* ctx, const bjj_base* base, const bjj_keyset* ks, const uint8_t* key_index, size_t n,
+                              const uint8_t* r8x, const uint8_t* r8y, const uint8_t* s32, const uint8_t* sig64, const uint8_t* msg,
+                              uint8_t* ok, uint8_t* status, cudaStream_t st, Workspace* ws) {
     const size_t lanes = scratch_lanes(ctx, n);
     return for_each_subbatch(n, [&](size_t off, size_t m) -> int {
         const size_t o = 32 * off;
@@ -872,6 +1008,16 @@ static int launch_verify_base(bjj_ctx* ctx, const bjj_base* base, size_t n, cons
         unsigned long long *work_h = nullptr, *work_e = nullptr;
         TRY(claim_counter(ctx, ws, st, &work_h));
         TRY(claim_counter(ctx, ws, st, &work_e));
+        if (ks) {
+            const uint8_t *ki = key_index + 4 * off, *kx = ks->keys, *ky = kx + 32 * ks->n_keys;
+            const uint32_t nk = (uint32_t)ks->n_keys;
+            bjjk::verify_keyset_hash(grid_cap(ctx, bjjk::verify_keyset_hash_blocks_per_sm(), m), st, m, rx, ry, ki, kx, ky, nk, msg + o,
+                                     skip, hm, ok + off, ctx->flags_dev, work_h);
+            TRY(launched(ctx));
+            bjjk::verify_keyset_ec(grid_cap(ctx, bjjk::verify_keyset_ec_blocks_per_sm(), m), st, m, rx, ry, sb, s_stride, s_off, hm,
+                                   ok + off, ctx->comb, ki, nk, ks->tables, work_e);
+            return launched(ctx);
+        }
         bjjk::verify_base_hash(grid_cap(ctx, bjjk::verify_base_hash_blocks_per_sm(), m), st, m, rx, ry, base->x, base->y, msg + o, skip,
                                hm, ok + off, ctx->flags_dev, work_h);
         TRY(launched(ctx));
@@ -882,6 +1028,8 @@ static int launch_verify_base(bjj_ctx* ctx, const bjj_base* base, size_t n, cons
 }
 // a verify_base call names its key: NULL or a handle of another context is an argument error
 static bool base_of(bjj_ctx* ctx, const bjj_base* base) { return base && base->ctx == ctx; }
+// the same for a key set
+static bool keyset_of(bjj_ctx* ctx, const bjj_keyset* ks) { return ks && ks->ctx == ctx; }
 
 static int launch_poseidon(bjj_ctx* ctx, int n_inputs, size_t n, const uint8_t* const* in, uint8_t* out,
                            cudaStream_t st) {
@@ -1116,7 +1264,7 @@ int bjj_verify_base_batch_dev(bjj_ctx* ctx, const bjj_base* pk, size_t n, const 
     if (!base_of(ctx, pk)) return BJJ_ERR_ARG;
     DEV_PROLOGUE
     if (!r8x || !r8y || !s32 || !msg32 || !ok) return BJJ_ERR_ARG;
-    return launch_verify_base(ctx, pk, n, r8x, r8y, s32, nullptr, msg32, ok, nullptr, st, &ctx->ws);
+    return launch_verify_base(ctx, pk, nullptr, nullptr, n, r8x, r8y, s32, nullptr, msg32, ok, nullptr, st, &ctx->ws);
 }
 
 int bjj_verify_base_compressed_batch_dev(bjj_ctx* ctx, const bjj_base* pk, size_t n, const uint8_t* sig64, const uint8_t* msg32,
@@ -1124,7 +1272,32 @@ int bjj_verify_base_compressed_batch_dev(bjj_ctx* ctx, const bjj_base* pk, size_
     if (!base_of(ctx, pk)) return BJJ_ERR_ARG;
     DEV_PROLOGUE
     if (!sig64 || !msg32 || !ok || !status) return BJJ_ERR_ARG;
-    return launch_verify_base(ctx, pk, n, nullptr, nullptr, nullptr, sig64, msg32, ok, status, st, &ctx->ws);
+    return launch_verify_base(ctx, pk, nullptr, nullptr, n, nullptr, nullptr, nullptr, sig64, msg32, ok, status, st, &ctx->ws);
+}
+
+int bjj_verify_keyset_batch_dev(bjj_ctx* ctx, const bjj_keyset* ks, size_t n, const uint32_t* key_index, const uint8_t* r8x,
+                                const uint8_t* r8y, const uint8_t* s32, const uint8_t* msg32, uint8_t* ok, void* stream) {
+    if (!keyset_of(ctx, ks)) return BJJ_ERR_ARG;
+    DEV_PROLOGUE
+    if (!key_index || !r8x || !r8y || !s32 || !msg32 || !ok) return BJJ_ERR_ARG;
+    return launch_verify_base(ctx, nullptr, ks, (const uint8_t*)key_index, n, r8x, r8y, s32, nullptr, msg32, ok, nullptr, st, &ctx->ws);
+}
+
+int bjj_verify_keyset_compressed_batch_dev(bjj_ctx* ctx, const bjj_keyset* ks, size_t n, const uint32_t* key_index,
+                                           const uint8_t* sig64, const uint8_t* msg32, uint8_t* ok, uint8_t* status, void* stream) {
+    if (!keyset_of(ctx, ks)) return BJJ_ERR_ARG;
+    DEV_PROLOGUE
+    if (!key_index || !sig64 || !msg32 || !ok || !status) return BJJ_ERR_ARG;
+    return launch_verify_base(ctx, nullptr, ks, (const uint8_t*)key_index, n, nullptr, nullptr, nullptr, sig64, msg32, ok, status, st,
+                              &ctx->ws);
+}
+
+int bjj_keyset_mul_batch_dev(bjj_ctx* ctx, const bjj_keyset* ks, size_t n, const uint32_t* key_index, const uint8_t* scalar32,
+                             uint8_t* rx, uint8_t* ry, void* stream) {
+    if (!keyset_of(ctx, ks)) return BJJ_ERR_ARG;
+    DEV_PROLOGUE
+    if (!key_index || !scalar32 || !rx || !ry) return BJJ_ERR_ARG;
+    return launch_keyset_mul(ctx, ks, n, (const uint8_t*)key_index, scalar32, rx, ry, st, &ctx->ws);
 }
 
 }  // extern "C"
@@ -1513,7 +1686,7 @@ int bjj_verify_base_batch(bjj_ctx* ctx, const bjj_base* pk, size_t n, const uint
     if (!base_of(ctx, pk)) return BJJ_ERR_ARG;
     HostArg args[] = {H_IN(r8x, 32), H_IN(r8y, 32), H_IN(s32, 32), H_IN(msg32, 32), H_OUT(ok, 1)};
     return run_host(ctx, n, args, 5, [&](size_t m, uint8_t** d, cudaStream_t st, Workspace* ws) -> int {
-        return launch_verify_base(ctx, pk, m, d[0], d[1], d[2], nullptr, d[3], d[4], nullptr, st, ws);
+        return launch_verify_base(ctx, pk, nullptr, nullptr, m, d[0], d[1], d[2], nullptr, d[3], d[4], nullptr, st, ws);
     }, /*heavy=*/true);
 }
 
@@ -1522,7 +1695,34 @@ int bjj_verify_base_compressed_batch(bjj_ctx* ctx, const bjj_base* pk, size_t n,
     if (!base_of(ctx, pk)) return BJJ_ERR_ARG;
     HostArg args[] = {H_IN(sig64, 64), H_IN(msg32, 32), H_OUT(ok, 1), H_OUT(status, 1)};
     return run_host(ctx, n, args, 4, [&](size_t m, uint8_t** d, cudaStream_t st, Workspace* ws) -> int {
-        return launch_verify_base(ctx, pk, m, nullptr, nullptr, nullptr, d[0], d[1], d[2], d[3], st, ws);
+        return launch_verify_base(ctx, pk, nullptr, nullptr, m, nullptr, nullptr, nullptr, d[0], d[1], d[2], d[3], st, ws);
+    }, /*heavy=*/true);
+}
+
+int bjj_verify_keyset_batch(bjj_ctx* ctx, const bjj_keyset* ks, size_t n, const uint32_t* key_index, const uint8_t* r8x,
+                            const uint8_t* r8y, const uint8_t* s32, const uint8_t* msg32, uint8_t* ok) {
+    if (!keyset_of(ctx, ks)) return BJJ_ERR_ARG;
+    HostArg args[] = {H_IN((const uint8_t*)key_index, 4), H_IN(r8x, 32), H_IN(r8y, 32), H_IN(s32, 32), H_IN(msg32, 32), H_OUT(ok, 1)};
+    return run_host(ctx, n, args, 6, [&](size_t m, uint8_t** d, cudaStream_t st, Workspace* ws) -> int {
+        return launch_verify_base(ctx, nullptr, ks, d[0], m, d[1], d[2], d[3], nullptr, d[4], d[5], nullptr, st, ws);
+    }, /*heavy=*/true);
+}
+
+int bjj_verify_keyset_compressed_batch(bjj_ctx* ctx, const bjj_keyset* ks, size_t n, const uint32_t* key_index, const uint8_t* sig64,
+                                       const uint8_t* msg32, uint8_t* ok, uint8_t* status) {
+    if (!keyset_of(ctx, ks)) return BJJ_ERR_ARG;
+    HostArg args[] = {H_IN((const uint8_t*)key_index, 4), H_IN(sig64, 64), H_IN(msg32, 32), H_OUT(ok, 1), H_OUT(status, 1)};
+    return run_host(ctx, n, args, 5, [&](size_t m, uint8_t** d, cudaStream_t st, Workspace* ws) -> int {
+        return launch_verify_base(ctx, nullptr, ks, d[0], m, nullptr, nullptr, nullptr, d[1], d[2], d[3], d[4], st, ws);
+    }, /*heavy=*/true);
+}
+
+int bjj_keyset_mul_batch(bjj_ctx* ctx, const bjj_keyset* ks, size_t n, const uint32_t* key_index, const uint8_t* scalar32, uint8_t* rx,
+                         uint8_t* ry) {
+    if (!keyset_of(ctx, ks)) return BJJ_ERR_ARG;
+    HostArg args[] = {H_IN((const uint8_t*)key_index, 4), H_IN(scalar32, 32), H_OUT(rx, 32), H_OUT(ry, 32)};
+    return run_host(ctx, n, args, 4, [&](size_t m, uint8_t** d, cudaStream_t st, Workspace* ws) -> int {
+        return launch_keyset_mul(ctx, ks, m, d[0], d[1], d[2], d[3], st, ws);
     }, /*heavy=*/true);
 }
 

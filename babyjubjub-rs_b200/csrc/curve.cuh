@@ -300,4 +300,19 @@ BJJ_HD int recode16_digit(const Recode16& rc, int i) {   // i in [0, 16)
     return (int)((rc.w[i >> 1] >> ((i & 1) * 16)) & 65535u) - 32768;
 }
 
+// Signed radix-2^8: n = sum_{i<32} d_i 256^i + c 256^32, d_i in [-128, 127], c in {0, 1}.
+struct Recode8 {
+    uint32_t w[8];
+    uint32_t top;
+};
+BJJ_HD void recode8(Recode8& rc, const uint32_t* n) {
+    uint32_t off[8];
+#pragma unroll
+    for (int i = 0; i < 8; i++) off[i] = 0x80808080u;
+    rc.top = add256(rc.w, n, off);
+}
+BJJ_HD int recode8_digit(const Recode8& rc, int i) {   // i in [0, 32)
+    return (int)((rc.w[i >> 2] >> ((i & 3) * 8)) & 255u) - 128;
+}
+
 }  // namespace bjj

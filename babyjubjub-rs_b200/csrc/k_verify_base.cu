@@ -3,7 +3,8 @@
 // (lane_verify_base_hash, lane_verify_base_ec).
 //
 //   (bjj_cuda.cu: k_decompress_prepare / k_batch_inverse / k_decompress_finish for compressed R8) ->
-//   k_verify_base_hash -> k_verify_base_ec
+//   k_verify_base_hash -> k_verify_base_ec       (one key, bjj_verify_base*)
+//   k_verify_keyset_hash -> k_verify_keyset_ec   (a key per lane from a key set, bjj_verify_keyset*)
 #include "kernels.h"
 
 using namespace bjj;
@@ -38,6 +39,27 @@ __global__ void __launch_bounds__(BJJ_BLOCK, 2) k_verify_base_ec(size_t n, const
     if (i < n) lane_verify_base_ec(r8x, r8y, s_base, s_stride, s_off, hm, ok, i, comb, comb_a);
 }
 
+// the same two phases against a key set: key key_index[i] of the set serves lane i (lanes.cuh: lane_verify_keyset_*)
+__global__ void __launch_bounds__(BJJ_BLOCK, 2) k_verify_keyset_hash(size_t n, const uint8_t* r8x, const uint8_t* r8y,
+                                                                     const uint8_t* key_index, const uint8_t* kx, const uint8_t* ky,
+                                                                     uint32_t n_keys, const uint8_t* msg, const uint8_t* skip,
+                                                                     uint8_t* hm, uint8_t* ok, uint32_t* gflags,
+                                                                     unsigned long long* work) {
+    BJJ_FLAGS_BEGIN
+    BJJ_CLAIM_LOOP(n, work)
+    if (i < n) lane_verify_keyset_hash(r8x, r8y, key_index, kx, ky, n_keys, msg, skip, hm, ok, i, flags);
+    BJJ_FLAGS_END(gflags)
+}
+
+__global__ void __launch_bounds__(BJJ_BLOCK, 2) k_verify_keyset_ec(size_t n, const uint8_t* r8x, const uint8_t* r8y,
+                                                                   const uint8_t* s_base, size_t s_stride, size_t s_off,
+                                                                   const uint8_t* hm, uint8_t* ok, const CombEntry* comb,
+                                                                   const uint8_t* key_index, uint32_t n_keys,
+                                                                   const CombEntry* tables, unsigned long long* work) {
+    BJJ_CLAIM_LOOP(n, work)
+    if (i < n) lane_verify_keyset_ec(r8x, r8y, s_base, s_stride, s_off, hm, ok, i, comb, key_index, n_keys, tables);
+}
+
 namespace bjjk {
 
 void verify_base_hash(int grid, cudaStream_t st, size_t n, const uint8_t* r8x, const uint8_t* r8y, const uint8_t* ax32,
@@ -56,5 +78,19 @@ void verify_base_ec(int grid, cudaStream_t st, size_t n, const uint8_t* r8x, con
     k_verify_base_ec<<<grid, BJJ_BLOCK, 0, st>>>(n, r8x, r8y, s_base, s_stride, s_off, hm, ok, comb, comb_a, work);
 }
 int verify_base_ec_blocks_per_sm() { return blocks_per_sm(k_verify_base_ec); }
+
+void verify_keyset_hash(int grid, cudaStream_t st, size_t n, const uint8_t* r8x, const uint8_t* r8y, const uint8_t* key_index,
+                        const uint8_t* kx, const uint8_t* ky, uint32_t n_keys, const uint8_t* msg, const uint8_t* skip, uint8_t* hm,
+                        uint8_t* ok, uint32_t* gflags, unsigned long long* work) {
+    k_verify_keyset_hash<<<grid, BJJ_BLOCK, 0, st>>>(n, r8x, r8y, key_index, kx, ky, n_keys, msg, skip, hm, ok, gflags, work);
+}
+int verify_keyset_hash_blocks_per_sm() { return blocks_per_sm(k_verify_keyset_hash); }
+
+void verify_keyset_ec(int grid, cudaStream_t st, size_t n, const uint8_t* r8x, const uint8_t* r8y, const uint8_t* s_base,
+                      size_t s_stride, size_t s_off, const uint8_t* hm, uint8_t* ok, const bjj::CombEntry* comb,
+                      const uint8_t* key_index, uint32_t n_keys, const bjj::CombEntry* tables, unsigned long long* work) {
+    k_verify_keyset_ec<<<grid, BJJ_BLOCK, 0, st>>>(n, r8x, r8y, s_base, s_stride, s_off, hm, ok, comb, key_index, n_keys, tables, work);
+}
+int verify_keyset_ec_blocks_per_sm() { return blocks_per_sm(k_verify_keyset_ec); }
 
 }  // namespace bjjk

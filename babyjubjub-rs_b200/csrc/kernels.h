@@ -103,5 +103,15 @@ void verify_base_ec(int grid, cudaStream_t st, size_t n, const uint8_t* r8x, con
                     size_t s_stride, size_t s_off, const uint8_t* hm, uint8_t* ok, const bjj::CombEntry* comb,
                     const bjj::CombEntry* comb_a, unsigned long long* work);
 int verify_base_ec_blocks_per_sm();
+// the same against a key set: key_index (uint32 per lane) selects the key; kx, ky: the set's Montgomery key planes,
+// tables: its compact combs
+void verify_keyset_hash(int grid, cudaStream_t st, size_t n, const uint8_t* r8x, const uint8_t* r8y, const uint8_t* key_index,
+                        const uint8_t* kx, const uint8_t* ky, uint32_t n_keys, const uint8_t* msg, const uint8_t* skip, uint8_t* hm,
+                        uint8_t* ok, uint32_t* gflags, unsigned long long* work);
+int verify_keyset_hash_blocks_per_sm();
+void verify_keyset_ec(int grid, cudaStream_t st, size_t n, const uint8_t* r8x, const uint8_t* r8y, const uint8_t* s_base,
+                      size_t s_stride, size_t s_off, const uint8_t* hm, uint8_t* ok, const bjj::CombEntry* comb,
+                      const uint8_t* key_index, uint32_t n_keys, const bjj::CombEntry* tables, unsigned long long* work);
+int verify_keyset_ec_blocks_per_sm();
 
 }  // namespace bjjk

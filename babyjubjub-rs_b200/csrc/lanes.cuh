@@ -135,10 +135,27 @@ BJJ_HD void table_select(Niels& n, const LaneTable& t, int d) {
 // is the same with B8 replaced by that point (k_comb_build_point).  Signed 16-bit
 // digits make a fixed-base multiplication 17 mixed additions and no doubling; verify adds its B8 term (w * B8, the
 // one full-width scalar left after the split) the same way, after the Straus pass over the two per-lane points.
+// The keys of a key set (bjj_keyset_create) have a compact table of the same form with 8-bit windows (Comb8 below).
 #define BJJ_COMB_BITS 16
 #define BJJ_COMB_WINDOWS 17
 #define BJJ_COMB_ENTRIES 32769
 #define BJJ_COMB_TOTAL ((size_t)(BJJ_COMB_WINDOWS - 1) * BJJ_COMB_ENTRIES + 2)
+
+// Comb geometries: BITS per window, ENTRIES = 2^(BITS-1) + 1 per window (j = 0..2^(BITS-1)), WINDOWS = 256 / BITS + 1
+// (the last holds only j = 0, 1 for the recoding carry), and the signed recoding that yields the digits.
+struct Comb16 {
+    static constexpr int BITS = BJJ_COMB_BITS, WINDOWS = BJJ_COMB_WINDOWS, ENTRIES = BJJ_COMB_ENTRIES;
+    typedef Recode16 Recode;
+    static BJJ_HD void recode(Recode& rc, const uint32_t* k) { recode16(rc, k); }
+    static BJJ_HD int digit(const Recode& rc, int w) { return recode16_digit(rc, w); }
+};
+struct Comb8 {      // 33 windows x 129 entries: 4,130 x 96 B = 396,480 B per point
+    static constexpr int BITS = 8, WINDOWS = 33, ENTRIES = 129;
+    typedef Recode8 Recode;
+    static BJJ_HD void recode(Recode& rc, const uint32_t* k) { recode8(rc, k); }
+    static BJJ_HD int digit(const Recode& rc, int w) { return recode8_digit(rc, w); }
+};
+#define BJJ_KEY_COMB_TOTAL ((size_t)(Comb8::WINDOWS - 1) * Comb8::ENTRIES + 2)
 #if !BJJ_DEVICE_CODE && defined(BJJ_HOST_EMU)
 // the host test harness fills table entries on demand instead of building all 524,290 of them
 void bjj_emu_need_comb_entry(const struct CombEntry* comb, int w, int j);
@@ -148,11 +165,12 @@ struct CombEntry {   // 96 bytes
 };
 
 // the raw entry |d| of window w (no sign applied yet)
+template <class G = Comb16>
 BJJ_HD void comb_fetch(NielsAff& n, const CombEntry* comb, int w, int d) {
     int ad = d < 0 ? -d : d;
-    const CombEntry* e = comb + (size_t)w * BJJ_COMB_ENTRIES + ad;
+    const CombEntry* e = comb + (size_t)w * G::ENTRIES + ad;
 #if !BJJ_DEVICE_CODE && defined(BJJ_HOST_EMU)
-    bjj_emu_need_comb_entry(comb, w, ad);
+    if (G::BITS == BJJ_COMB_BITS) bjj_emu_need_comb_entry(comb, w, ad);     // the host harnesses build compact tables whole
 #endif
 #if BJJ_DEVICE_CODE
     const uint4* p = reinterpret_cast<const uint4*>(e);
@@ -169,31 +187,34 @@ BJJ_HD void comb_fetch(NielsAff& n, const CombEntry* comb, int w, int d) {
     fr_set(n.t2d, e->t2d);
 #endif
 }
+template <class G = Comb16>
 BJJ_HD void comb_select(NielsAff& n, const CombEntry* comb, int w, int d) {
-    comb_fetch(n, comb, w, d);
+    comb_fetch<G>(n, comb, w, d);
     niels_aff_cneg(n, d < 0);
 }
 
-// acc += k * base (comb = the table of base) for a 256-bit k: 17 mixed additions, no doublings.  `from_identity` starts
-// acc at the identity, after the recoding as fixed_base_comb always did (so its kernels compile as before);
-// lane_fixed_base2 runs two walks over two tables into one accumulator.  BJJ_COMB_PREFETCH: the entry of window w - 1
-// is requested before the addition of window w, so that its L2 latency (the 50 MB table is gathered at random) runs
-// under ~900 multiplier instructions instead of in front of them.
+// acc += k * base (comb = the table of base, geometry G) for a 256-bit k: G::WINDOWS mixed additions (17 on the 16-bit
+// comb, 33 on the 8-bit one), no doublings.  `from_identity` starts acc at the identity, after the recoding as
+// fixed_base_comb always did (so its kernels compile as before); lane_fixed_base2 runs two walks over two tables into
+// one accumulator.  BJJ_COMB_PREFETCH: the entry of window w - 1 is requested before the addition of window w, so that
+// its L2 / HBM latency (the tables are gathered at random) runs under ~900 multiplier instructions instead of in
+// front of them.
 #ifndef BJJ_COMB_PREFETCH
 #define BJJ_COMB_PREFETCH 1
 #endif
+template <class G = Comb16>
 BJJ_HD void fixed_base_comb_acc(PointExt& acc, const CombEntry* comb, const uint32_t* k, bool from_identity = false) {
-    Recode16 rc;
-    recode16(rc, k);
+    typename G::Recode rc;
+    G::recode(rc, k);
     if (from_identity) ext_identity(acc);
 #if BJJ_COMB_PREFETCH
     NielsAff cur, nxt;
     int d = (int)rc.top;
-    comb_fetch(cur, comb, BJJ_COMB_WINDOWS - 1, d);
+    comb_fetch<G>(cur, comb, G::WINDOWS - 1, d);
 #pragma unroll 1
-    for (int w = BJJ_COMB_WINDOWS - 2; w >= 0; w--) {
-        const int dn = recode16_digit(rc, w);
-        comb_fetch(nxt, comb, w, dn);
+    for (int w = G::WINDOWS - 2; w >= 0; w--) {
+        const int dn = G::digit(rc, w);
+        comb_fetch<G>(nxt, comb, w, dn);
         niels_aff_cneg(cur, d < 0);
         ext_add_niels_aff<true>(acc, acc, cur);
         cur = nxt;
@@ -203,17 +224,37 @@ BJJ_HD void fixed_base_comb_acc(PointExt& acc, const CombEntry* comb, const uint
     ext_add_niels_aff<true>(acc, acc, cur);
 #else
     NielsAff n;
-    comb_select(n, comb, BJJ_COMB_WINDOWS - 1, (int)rc.top);
+    comb_select<G>(n, comb, G::WINDOWS - 1, (int)rc.top);
     ext_add_niels_aff<true>(acc, acc, n);
 #pragma unroll 1
-    for (int w = BJJ_COMB_WINDOWS - 2; w >= 0; w--) {
-        comb_select(n, comb, w, recode16_digit(rc, w));
+    for (int w = G::WINDOWS - 2; w >= 0; w--) {
+        comb_select<G>(n, comb, w, G::digit(rc, w));
         ext_add_niels_aff<true>(acc, acc, n);
     }
 #endif
 }
 BJJ_HD void fixed_base_comb(PointExt& acc, const CombEntry* comb, const uint32_t* k) {
     fixed_base_comb_acc(acc, comb, k, true);
+}
+
+// a comb entry from the affine point (x, y) of the a = -1 model: (y + x, y - x, 2d'xy), fully reduced
+BJJ_HD void comb_store_niels(CombEntry* e, const Fr& x, const Fr& y) {
+    Fr t;
+    fr_mul(t, x, y);
+    const Fr d2 = fr_const(BJJ_TWO_DP_M);
+    fr_mul(t, t, d2);
+    Fr ypx, ymx;
+    fr_add(ypx, y, x);
+    fr_sub(ymx, y, x);
+    fr_reduce(ypx);
+    fr_reduce(ymx);
+    fr_reduce(t);
+#pragma unroll
+    for (int i = 0; i < 8; i++) {
+        e->ypx[i] = ypx.v[i];
+        e->ymx[i] = ymx.v[i];
+        e->t2d[i] = t.v[i];
+    }
 }
 
 // one comb entry: j * 65536^w * p for an on-curve p of the original curve   (one thread per (w, j)).  Every on-curve
@@ -232,7 +273,8 @@ BJJ_HD void comb_build_entry(CombEntry* comb, int w, int j, const PointAff& p) {
         ext_dbl<true>(acc, acc);
         if ((j >> bit) & 1) ext_add_niels<true>(acc, acc, nb);
     }
-    // affine on the a = -1 model, then Niels form
+    // affine on the a = -1 model, then Niels form (comb_store_niels's steps, written out: through the helper nvcc
+    // schedules k_comb_build differently)
     Fr zi, x, y, t;
     fr_inv(zi, acc.Z);
     fr_mul(x, acc.X, zi);
@@ -1566,7 +1608,9 @@ BJJ_HD void verify_base_scalar(uint32_t* k, const uint32_t* hm) {
 // the curve, so this is the reference's affine comparison).  R8 off the curve: verify_exact<false>'s replay, with both
 // products from the combs: l = S*B8 and kA in affine form (one shared inversion), literal add-2008-bbjlp of R8 and kA
 // with Z = 1, PointProjective::affine (Z == 0 -> (0, 0)), compare with l (src/lib.rs:405-411).  The two comb walks run
-// for every lane, so a warp that holds both kinds of lanes diverges only in the short tails.
+// for every lane, so a warp that holds both kinds of lanes diverges only in the short tails.  GA: the geometry of comb_a
+// (Comb16 for a bjj_base, Comb8 for a key of a key set).
+template <class GA = Comb16>
 BJJ_HD void lane_verify_base_ec(const uint8_t* r8x, const uint8_t* r8y, const uint8_t* s_base, size_t s_stride, size_t s_off,
                                 const uint8_t* hm_in, uint8_t* ok, size_t i, const CombEntry* comb, const CombEntry* comb_a) {
     const uint32_t state = ok[i];
@@ -1585,7 +1629,7 @@ BJJ_HD void lane_verify_base_ec(const uint8_t* r8x, const uint8_t* r8y, const ui
     } else {          // -k*A = (ORDER - k)*A  (k = 0 gives ORDER*A = O as well)
         sub256(k, BJJ_ORDER, k);
     }
-    fixed_base_comb_acc(acc, comb_a, k);
+    fixed_base_comb_acc<GA>(acc, comb_a, k);
     uint32_t flags = 0;
     PointAff r8;
     load_fr(r8.x, r8x, i, flags);
@@ -1625,6 +1669,131 @@ BJJ_HD void lane_verify_base_ec(const uint8_t* r8x, const uint8_t* r8y, const ui
     proj_add_bbjlp(sum, pr, pk);
     proj_affine(ra, sum);
     ok[i] = (fr_eq(la.x, ra.x) && fr_eq(la.y, ra.y)) ? 1 : 0;
+}
+
+// ---- key sets: many keys, each with a compact comb (bjj_keyset_create, bjj_verify_keyset*, bjj_keyset_mul) -----------
+// A key set holds N on-curve keys P_0..P_{N-1}: their coordinates in Montgomery form (two planes of 32 B per key) and one
+// Comb8 table per key, tbl[w][j] = j * 256^w * P, 4,130 entries of 96 B, key after key.  A lane names its key by a
+// uint32 index; an index >= N rejects the lane (ok = 0, or the point (0, 0)) and sets BJJ_FLAG_KEY_INDEX, which
+// bjj_sync turns into BJJ_ERR_ARG.  Every on-curve point has an order dividing ORDER < 2^254, so a table serves every
+// raw 256-bit scalar (the argument of comb_build_entry).
+#define BJJ_FLAG_KEY_INDEX 2u
+
+// build scratch of one key: the points j * 256^w * P with j >= 1 that need an inversion, 128 per window w < 32 and
+// j = 1 of the carry window; build lane m holds (w, j) = (m / 128, m % 128 + 1), and m = 4096 holds (32, 1)
+#define BJJ_KEY_BUILD_POINTS ((Comb8::WINDOWS - 1) * (Comb8::ENTRIES - 1) + 1)
+BJJ_HD size_t keyset_entry_of(size_t m) {
+    return m < (size_t)BJJ_KEY_BUILD_POINTS - 1 ? (m >> 7) * Comb8::ENTRIES + (m & 127) + 1 : (size_t)(Comb8::WINDOWS - 1) * Comb8::ENTRIES + 1;
+}
+
+// key i of the set: checks the canonical bytes (BJJ_BASE_* outcome) and rewrites them in place in Montgomery form
+BJJ_HD uint32_t lane_keyset_check(uint8_t* kx, uint8_t* ky, size_t i) {
+    PointAff p;
+    uint32_t flags = 0;
+    load_fr(p.x, kx, i, flags);
+    load_fr(p.y, ky, i, flags);
+    store_u256(kx, i, p.x.v);
+    store_u256(ky, i, p.y.v);
+    return flags ? BJJ_BASE_NONCANONICAL : on_curve(p) ? BJJ_BASE_OK : BJJ_BASE_OFF_CURVE;
+}
+
+// key `key` of the set (Montgomery planes kx, ky)
+BJJ_HD void keyset_point(PointAff& a, const uint8_t* kx, const uint8_t* ky, size_t key) {
+    load_u256(a.x.v, kx, key);
+    load_u256(a.y.v, ky, key);
+}
+
+// window w of key `key` (one thread per (key, w)): 8w doublings reach B = 256^w * P, then j * B for j = 1..128 (1 in
+// the carry window) by successive additions, parked as (X : Y : Z) of the a = -1 model in scratch lanes lane0 + m (m
+// as keyset_entry_of reads it) for one batched inversion; entry (w, 0), the identity, is written directly.
+BJJ_HD void lane_keyset_build(const uint8_t* kx, const uint8_t* ky, size_t key, int w, const ProjScratch& scr, size_t lane0,
+                              CombEntry* tbl) {
+    PointAff p;
+    keyset_point(p, kx, ky, key);
+    PointExt b, acc;
+    ext_from_affine(b, p);
+#pragma unroll 1
+    for (int i = 0; i < Comb8::BITS * w; i++) ext_dbl<true>(b, b);
+    Niels nb;
+    niels_from_ext(nb, b);
+    {
+        Fr zero, one = fr_const(BJJ_ONE_M);
+        fr_zero(zero);
+        comb_store_niels(tbl + (size_t)w * Comb8::ENTRIES, zero, one);
+    }
+    const int nj = w == Comb8::WINDOWS - 1 ? 1 : Comb8::ENTRIES - 1;
+    acc = b;
+#pragma unroll 1
+    for (int j = 1; j <= nj; j++) {
+        if (j > 1) ext_add_niels<true>(acc, acc, nb);
+        const size_t at = lane0 + (size_t)w * (Comb8::ENTRIES - 1) + (size_t)(j - 1);
+        store_u256(scr.x, at, acc.X.v);
+        store_u256(scr.y, at, acc.Y.v);
+        store_u256(scr.z, at, acc.Z.v);
+    }
+}
+
+// batch_affine_strided output of the build: scratch lane i = key k (counted from tbl's key) and build lane m -> the
+// key's table entry, from the a = -1 affine point
+struct KeysetCombOut {
+    CombEntry* tbl;
+    BJJ_HD void operator()(size_t i, const Fr& x, const Fr& y) const {
+        const size_t k = i / BJJ_KEY_BUILD_POINTS, m = i % BJJ_KEY_BUILD_POINTS;
+        comb_store_niels(tbl + k * BJJ_KEY_COMB_TOTAL + keyset_entry_of(m), x, y);
+    }
+};
+
+// the key of lane i, or false (and BJJ_FLAG_KEY_INDEX) for an index outside the set
+BJJ_HD bool keyset_index(uint32_t& key, const uint8_t* key_index, uint32_t n_keys, size_t i, uint32_t& flags) {
+    uint32_t k;
+#if BJJ_DEVICE_CODE
+    k = __ldg(reinterpret_cast<const uint32_t*>(key_index) + i);
+#else
+    memcpy(&k, key_index + 4 * i, 4);
+#endif
+    key = k;
+    if (k < n_keys) return true;
+    flags |= BJJ_FLAG_KEY_INDEX;
+    return false;
+}
+
+// verify phase 1 against key key_index[i] of the set: lane_verify_base_hash with that key
+BJJ_HD void lane_verify_keyset_hash(const uint8_t* r8x, const uint8_t* r8y, const uint8_t* key_index, const uint8_t* kx,
+                                    const uint8_t* ky, uint32_t n_keys, const uint8_t* msg32, const uint8_t* skip, uint8_t* hm_out,
+                                    uint8_t* ok, size_t i, uint32_t& flags) {
+    uint32_t key;
+    if (!keyset_index(key, key_index, n_keys, i, flags)) {
+        ok[i] = 0;
+        return;
+    }
+    PointAff a;
+    keyset_point(a, kx, ky, key);
+    lane_verify_base_hash(r8x, r8y, a, msg32, skip, hm_out, ok, i, flags);
+}
+
+// verify phase 2: lane_verify_base_ec with the key's compact table (lanes rejected in phase 1 return at once)
+BJJ_HD void lane_verify_keyset_ec(const uint8_t* r8x, const uint8_t* r8y, const uint8_t* s_base, size_t s_stride, size_t s_off,
+                                  const uint8_t* hm_in, uint8_t* ok, size_t i, const CombEntry* comb, const uint8_t* key_index,
+                                  uint32_t n_keys, const CombEntry* tables) {
+    uint32_t key, flags = 0;
+    if (!keyset_index(key, key_index, n_keys, i, flags)) return;
+    lane_verify_base_ec<Comb8>(r8x, r8y, s_base, s_stride, s_off, hm_in, ok, i, comb, tables + (size_t)key * BJJ_KEY_COMB_TOTAL);
+}
+
+// P_{key_index[i]}.mul_scalar(k) for a raw 256-bit k (src/lib.rs:149-164), 33 mixed additions; a lane with an index
+// outside the set parks Z = 0, which the batched affine pass turns into (0, 0)
+BJJ_HD void lane_keyset_mul(const uint8_t* scalar, const uint8_t* key_index, uint32_t n_keys, const CombEntry* tables,
+                            const ProjScratch& scr, size_t i, uint32_t& flags) {
+    uint32_t key;
+    if (!keyset_index(key, key_index, n_keys, i, flags)) {
+        store_zero_scratch(scr, i);
+        return;
+    }
+    uint32_t k[8];
+    load_u256(k, scalar, i);
+    PointExt acc;
+    fixed_base_comb_acc<Comb8>(acc, tables + (size_t)key * BJJ_KEY_COMB_TOTAL, k, true);
+    store_ext_scratch(scr, i, acc);
 }
 
 }  // namespace bjj

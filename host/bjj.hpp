@@ -16,6 +16,7 @@
 //     public_compressed_batch, sign_compressed_batch, sign_schnorr_batch (caller nonces)
 //   + FixedBase: the comb table of a caller-chosen point, k*P and k*P + l*Q at the fixed-base rate, and verify for
 //     many signatures of that one key
+//   + KeySet: many known keys with compact comb tables, verify and k*P with a key index per lane
 //   + MultiGpu: shards a batch over every device, one host thread + one bjj_ctx per device, no NCCL
 //
 // Header-only; link with -lbjj_cuda.  There is no CPU fallback: Engine's constructor throws when no
@@ -364,6 +365,82 @@ class FixedBase {
     }
     Engine& e_;
     bjj_base* base_ = nullptr;
+};
+
+// N on-curve public keys on an Engine, each with a compact comb table (396,480 B of device memory per key, freed by the
+// destructor): verify and k*P for batches that name a key per lane.  Throws Error with BJJ_ERR_NONCANONICAL for a
+// coordinate >= Q and BJJ_ERR_ARG for an off-curve key or an empty list (key_status(), when given, receives one BJJ_KEY_*
+// code per key).  A lane whose index is outside the set throws BJJ_ERR_ARG.  Must not outlive its Engine.
+class KeySet {
+  public:
+    KeySet(const std::vector<Point>& keys, Engine& e = default_engine(), std::vector<uint8_t>* key_status = nullptr) : e_(e) {
+        const size_t n = keys.size();
+        std::vector<uint8_t> ax(32 * n), ay(32 * n), st(n);
+        for (size_t i = 0; i < n; i++) {
+            std::memcpy(&ax[32 * i], keys[i].x.data(), 32);
+            std::memcpy(&ay[32 * i], keys[i].y.data(), 32);
+        }
+        const int rc = bjj_keyset_create(e.ctx(), n, ax.data(), ay.data(), st.data(), &ks_);
+        if (key_status) *key_status = st;
+        Engine::check(rc, "bjj_keyset_create");
+        n_ = n;
+    }
+    ~KeySet() { bjj_keyset_destroy(e_.ctx(), ks_); }
+    KeySet(const KeySet&) = delete;
+    KeySet& operator=(const KeySet&) = delete;
+    const bjj_keyset* raw() const { return ks_; }
+    size_t size() const { return n_; }
+
+    // [verify(keys[key_index[i]], sigs[i], msgs[i])] (src/lib.rs:395-412): the bytes of verify_batch with those keys
+    std::vector<uint8_t> verify_batch(const std::vector<uint32_t>& key_index, const std::vector<Signature>& sigs,
+                                      const std::vector<U256>& msgs) const {
+        if (sigs.size() != msgs.size() || sigs.size() != key_index.size())
+            throw std::invalid_argument("key_index, sigs and msgs differ in length");
+        const size_t n = sigs.size();
+        std::vector<uint8_t> r8x(32 * n), r8y(32 * n), s(32 * n), ok(n);
+        for (size_t i = 0; i < n; i++) {
+            std::memcpy(&r8x[32 * i], sigs[i].r_b8.x.data(), 32);
+            std::memcpy(&r8y[32 * i], sigs[i].r_b8.y.data(), 32);
+            std::memcpy(&s[32 * i], sigs[i].s.data(), 32);
+        }
+        auto m = pack(msgs);
+        Engine::check(bjj_verify_keyset_batch(e_.ctx(), ks_, n, key_index.data(), r8x.data(), r8y.data(), s.data(), m.data(), ok.data()),
+                      "bjj_verify_keyset_batch");
+        return ok;
+    }
+    // the same from 64-byte compressed signatures: ok and R8's decompression status per lane
+    std::vector<uint8_t> verify_compressed_batch(const std::vector<uint32_t>& key_index, const std::vector<std::array<uint8_t, 64>>& sigs,
+                                                 const std::vector<U256>& msgs, std::vector<uint8_t>* status = nullptr) const {
+        if (sigs.size() != msgs.size() || sigs.size() != key_index.size())
+            throw std::invalid_argument("key_index, sigs and msgs differ in length");
+        const size_t n = sigs.size();
+        std::vector<uint8_t> sg(64 * n), ok(n), st(n);
+        for (size_t i = 0; i < n; i++) std::memcpy(&sg[64 * i], sigs[i].data(), 64);
+        auto m = pack(msgs);
+        Engine::check(bjj_verify_keyset_compressed_batch(e_.ctx(), ks_, n, key_index.data(), sg.data(), m.data(), ok.data(), st.data()),
+                      "bjj_verify_keyset_compressed_batch");
+        if (status) *status = st;
+        return ok;
+    }
+    // [keys[key_index[i]].mul_scalar(k[i])]; scalars are raw 256-bit values (reduce wider ones mod ORDER)
+    std::vector<Point> mul_batch(const std::vector<uint32_t>& key_index, const std::vector<U256>& scalars) const {
+        if (scalars.size() != key_index.size()) throw std::invalid_argument("key_index and scalars differ in length");
+        const size_t n = scalars.size();
+        auto k = pack(scalars);
+        std::vector<uint8_t> rx(32 * n), ry(32 * n);
+        Engine::check(bjj_keyset_mul_batch(e_.ctx(), ks_, n, key_index.data(), k.data(), rx.data(), ry.data()), "bjj_keyset_mul_batch");
+        std::vector<Point> out(n);
+        for (size_t i = 0; i < n; i++) {
+            std::memcpy(out[i].x.data(), &rx[32 * i], 32);
+            std::memcpy(out[i].y.data(), &ry[32 * i], 32);
+        }
+        return out;
+    }
+
+  private:
+    Engine& e_;
+    bjj_keyset* ks_ = nullptr;
+    size_t n_ = 0;
 };
 
 struct DecompressResult {

@@ -177,6 +177,46 @@ int bjj_verify_base_compressed_batch(bjj_ctx* ctx, const bjj_base* pk, size_t n,
 int bjj_verify_base_compressed_batch_dev(bjj_ctx* ctx, const bjj_base* pk, size_t n, const uint8_t* sig64,
                                          const uint8_t* msg32, uint8_t* ok, uint8_t* status, void* stream);
 
+/* ---- key sets: many known keys, each with a compact comb; a key per lane ------------------------------------
+ * A bjj_keyset holds n_keys on-curve public keys, each with a table of 8-bit windows (4,130 entries, 396,480 B per
+ * key: 65,536 keys take 26 GB) instead of bjj_base's 50 MB, so a batch may mix many keys.  Calls name the key of lane i
+ * by key_index[i] (little-endian uint32).  k*P costs 33 mixed additions and no doubling.
+ *   - bjj_keyset_create copies the SoA coordinates ax, ay (32 B per key) and builds the tables on the device,
+ *     synchronously on the ctx stream.  No handle comes back when: a coordinate is >= Q (BJJ_ERR_NONCANONICAL, which
+ *     outranks the next), a key is off the curve (BJJ_ERR_ARG, for the reason given for bjj_base_create), n_keys is 0
+ *     or above 2^32 - 1 or a pointer is NULL (BJJ_ERR_ARG), or the tables do not fit in device memory (BJJ_ERR_NOMEM,
+ *     with the CUDA error cleared).  key_status (may be NULL) receives one BJJ_KEY_* code per key.
+ *   - The handle belongs to ctx like a bjj_base: bjj_keyset_destroy must come before bjj_destroy(ctx), and a call that
+ *     passes it with another context returns BJJ_ERR_ARG.
+ *   - key_index[i] >= n_keys: that lane gets ok = 0 (status 0 in the compressed form; the point (0, 0) in
+ *     bjj_keyset_mul), the other lanes are computed, and the call returns BJJ_ERR_ARG (a _dev call: the next bjj_sync,
+ *     where BJJ_ERR_ARG outranks BJJ_ERR_NONCANONICAL). */
+typedef struct bjj_keyset bjj_keyset;
+#define BJJ_KEY_OK 0            /* key_status codes; the same values as BJJ_BASE_* */
+#define BJJ_KEY_OFF_CURVE 1
+#define BJJ_KEY_NONCANONICAL 2
+int bjj_keyset_create(bjj_ctx* ctx, size_t n_keys, const uint8_t* ax, const uint8_t* ay, uint8_t* key_status,
+                      bjj_keyset** out);
+void bjj_keyset_destroy(bjj_ctx* ctx, bjj_keyset* ks);   /* waits for the device, then frees; NULL is a no-op */
+/* verify (src/lib.rs:395-412) with A = key key_index[i] of ks: byte for byte bjj_verify_batch with those keys in ax, ay
+ * (msg > Q -> 0, msg == Q hashes as 0, S raw and unreduced, torsion components accepted, R8 off the curve replayed
+ * literally, an R8 coordinate >= Q -> BJJ_ERR_NONCANONICAL), from two comb walks per lane like bjj_verify_base_batch */
+int bjj_verify_keyset_batch(bjj_ctx* ctx, const bjj_keyset* ks, size_t n, const uint32_t* key_index, const uint8_t* r8x,
+                            const uint8_t* r8y, const uint8_t* s32, const uint8_t* msg32, uint8_t* ok);
+int bjj_verify_keyset_batch_dev(bjj_ctx* ctx, const bjj_keyset* ks, size_t n, const uint32_t* key_index, const uint8_t* r8x,
+                                const uint8_t* r8y, const uint8_t* s32, const uint8_t* msg32, uint8_t* ok, void* stream);
+/* the same from 64-byte signatures (decompress_signature, src/lib.rs:260-268): status[i] = R8's decompression error */
+int bjj_verify_keyset_compressed_batch(bjj_ctx* ctx, const bjj_keyset* ks, size_t n, const uint32_t* key_index,
+                                       const uint8_t* sig64, const uint8_t* msg32, uint8_t* ok, uint8_t* status);
+int bjj_verify_keyset_compressed_batch_dev(bjj_ctx* ctx, const bjj_keyset* ks, size_t n, const uint32_t* key_index,
+                                           const uint8_t* sig64, const uint8_t* msg32, uint8_t* ok, uint8_t* status,
+                                           void* stream);
+/* r_i = P_{key_index[i]}.mul_scalar(k_i) (src/lib.rs:149-164), k raw 256-bit and unreduced, as bjj_base_mul_batch */
+int bjj_keyset_mul_batch(bjj_ctx* ctx, const bjj_keyset* ks, size_t n, const uint32_t* key_index, const uint8_t* scalar32,
+                         uint8_t* rx, uint8_t* ry);
+int bjj_keyset_mul_batch_dev(bjj_ctx* ctx, const bjj_keyset* ks, size_t n, const uint32_t* key_index, const uint8_t* scalar32,
+                             uint8_t* rx, uint8_t* ry, void* stream);
+
 /* ---- PrivateKey::public (src/lib.rs:304-306) = B8 * scalar_key(key);  scalar_key (:284-302) ------ */
 int bjj_public_batch(bjj_ctx* ctx, size_t n, const uint8_t* key32, uint8_t* rx, uint8_t* ry);
 int bjj_public_batch_dev(bjj_ctx* ctx, size_t n, const uint8_t* key32, uint8_t* rx, uint8_t* ry, void* stream);

@@ -12,6 +12,10 @@ pub struct bjj_base {
     _private: [u8; 0],
 }
 #[repr(C)]
+pub struct bjj_keyset {
+    _private: [u8; 0],
+}
+#[repr(C)]
 pub struct bjj_multi {
     _private: [u8; 0],
 }
@@ -72,6 +76,16 @@ extern "C" {
                                  s32: *const u8, msg32: *const u8, ok: *mut u8) -> c_int;
     pub fn bjj_verify_base_compressed_batch(ctx: *mut bjj_ctx, pk: *const bjj_base, n: usize, sig64: *const u8,
                                             msg32: *const u8, ok: *mut u8, status: *mut u8) -> c_int;
+    // key sets: many keys with compact comb tables, a key index per lane (an index outside the set is BJJ_ERR_ARG)
+    pub fn bjj_keyset_create(ctx: *mut bjj_ctx, n_keys: usize, ax: *const u8, ay: *const u8, key_status: *mut u8,
+                             out: *mut *mut bjj_keyset) -> c_int;
+    pub fn bjj_keyset_destroy(ctx: *mut bjj_ctx, ks: *mut bjj_keyset);
+    pub fn bjj_verify_keyset_batch(ctx: *mut bjj_ctx, ks: *const bjj_keyset, n: usize, key_index: *const u32, r8x: *const u8,
+                                   r8y: *const u8, s32: *const u8, msg32: *const u8, ok: *mut u8) -> c_int;
+    pub fn bjj_verify_keyset_compressed_batch(ctx: *mut bjj_ctx, ks: *const bjj_keyset, n: usize, key_index: *const u32,
+                                              sig64: *const u8, msg32: *const u8, ok: *mut u8, status: *mut u8) -> c_int;
+    pub fn bjj_keyset_mul_batch(ctx: *mut bjj_ctx, ks: *const bjj_keyset, n: usize, key_index: *const u32, scalar32: *const u8,
+                                rx: *mut u8, ry: *mut u8) -> c_int;
     // PrivateKey::public / scalar_key / sign (src/lib.rs:284-342)
     pub fn bjj_public_batch(ctx: *mut bjj_ctx, n: usize, key32: *const u8, rx: *mut u8, ry: *mut u8) -> c_int;
     pub fn bjj_scalar_key_batch(ctx: *mut bjj_ctx, n: usize, key32: *const u8, scalar32: *mut u8) -> c_int;

@@ -400,6 +400,70 @@ impl Drop for FixedBase {
     }
 }
 
+/// N on-curve public keys with compact comb tables (396,480 B of device memory per key): verify and k*P for batches
+/// that name a key per lane.  Freed on drop.
+pub struct KeySet {
+    ks: *mut ffi::bjj_keyset,
+}
+unsafe impl Send for KeySet {}
+
+impl KeySet {
+    /// `Err` for an empty list, a coordinate >= Q or an off-curve key; `key_status` says which keys and why
+    pub fn new(keys: &[Point]) -> Result<KeySet, (String, Vec<u8>)> {
+        let n = keys.len();
+        let (ax, ay) = (col(n, |i| keys[i].x), col(n, |i| keys[i].y));
+        let mut st = vec![0u8; n];
+        let mut ks = std::ptr::null_mut();
+        let rc = unsafe { ffi::bjj_keyset_create(engine().raw(), n, ax.as_ptr(), ay.as_ptr(), st.as_mut_ptr(), &mut ks) };
+        if rc != ffi::BJJ_OK {
+            return Err((format!("bjj_keyset_create failed: {}", err_str(rc)), st));
+        }
+        Ok(KeySet { ks })
+    }
+    /// `verify(keys[key_index[i]], sigs[i], msgs[i])` (src/lib.rs:395-412) lane by lane: the results of `verify_batch`
+    /// with those keys
+    pub fn verify_batch(&self, key_index: &[u32], sigs: &[Signature], msgs: &[BigInt]) -> Vec<bool> {
+        let n = sigs.len();
+        assert_eq!(n, msgs.len());
+        assert_eq!(n, key_index.len());
+        let (r8x, r8y) = (col(n, |i| sigs[i].r_b8.x), col(n, |i| sigs[i].r_b8.y));
+        let s = col(n, |i| scalar_b8_le32(&sigs[i].s));
+        let m = col(n, |i| msg_le32(&msgs[i]));
+        let mut ok = vec![0u8; n];
+        check(unsafe { ffi::bjj_verify_keyset_batch(engine().raw(), self.ks, n, key_index.as_ptr(), r8x.as_ptr(), r8y.as_ptr(),
+                                                    s.as_ptr(), m.as_ptr(), ok.as_mut_ptr()) }, "bjj_verify_keyset_batch");
+        ok.into_iter().map(|b| b == 1).collect()
+    }
+    /// the same from 64-byte compressed signatures: `Err` carries R8's decompression error
+    pub fn verify_compressed_batch(&self, key_index: &[u32], sigs: &[[u8; 64]], msgs: &[BigInt]) -> Vec<Result<bool, String>> {
+        let n = sigs.len();
+        assert_eq!(n, msgs.len());
+        assert_eq!(n, key_index.len());
+        let sg: Vec<u8> = sigs.iter().flat_map(|s| s.iter().copied()).collect();
+        let m = col(n, |i| msg_le32(&msgs[i]));
+        let (mut ok, mut st) = (vec![0u8; n], vec![0u8; n]);
+        check(unsafe { ffi::bjj_verify_keyset_compressed_batch(engine().raw(), self.ks, n, key_index.as_ptr(), sg.as_ptr(),
+                                                               m.as_ptr(), ok.as_mut_ptr(), st.as_mut_ptr()) },
+              "bjj_verify_keyset_compressed_batch");
+        (0..n).map(|i| if st[i] == 0 { Ok(ok[i] == 1) } else { Err(status_str(st[i])) }).collect()
+    }
+    /// `[keys[key_index[i]].mul_scalar(k[i])]`
+    pub fn mul_batch(&self, key_index: &[u32], scalars: &[BigInt]) -> Vec<Point> {
+        let n = scalars.len();
+        assert_eq!(n, key_index.len());
+        let k = col(n, |i| scalar_base_le32(&scalars[i]));
+        let (mut rx, mut ry) = (vec![0u8; 32 * n], vec![0u8; 32 * n]);
+        check(unsafe { ffi::bjj_keyset_mul_batch(engine().raw(), self.ks, n, key_index.as_ptr(), k.as_ptr(), rx.as_mut_ptr(),
+                                                 ry.as_mut_ptr()) }, "bjj_keyset_mul_batch");
+        (0..n).map(|i| Point { x: row(&rx, i), y: row(&ry, i) }).collect()
+    }
+}
+impl Drop for KeySet {
+    fn drop(&mut self) {
+        unsafe { ffi::bjj_keyset_destroy(engine().raw(), self.ks) }
+    }
+}
+
 pub fn public_batch(keys: &[PrivateKey]) -> Vec<Point> {
     let n = keys.len();
     let k = col(n, |i| keys[i].key);
