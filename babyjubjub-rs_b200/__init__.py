@@ -23,6 +23,8 @@ follow the reference's public API (paths into the reference tree):
       comb table (4,130 entries, 396 KB) and a key index per signature.
     + sign_schnorr_batch: PrivateKey::sign_schnorr over a batch, with caller-supplied (or random 1024-bit)
       nonces and the unreduced s of the reference.
+    + verify_schnorr_batch / verify_schnorr_base_batch / verify_schnorr_keyset_batch: verify_schnorr over a batch,
+      taking sign_schnorr_batch's unreduced s as it is (any key; one key's FixedBase; a KeySet and a key per lane).
 
 Every call runs on the GPU through libbjj_cuda.so; there is no CPU fallback -- importing works
 without a GPU (so the ABI can be inspected), creating an Engine does not.
@@ -342,6 +344,35 @@ class Engine:
         self._check(self.lib.bjj_keyset_mul_batch(self.ctx, _keyset_handle(keyset), len(ki), _ptr(ki), _ptr(k), _ptr(rx), _ptr(ry)),
                     "bjj_keyset_mul_batch")
         return rx, ry
+
+    # verify_schnorr with s as sign_schnorr_batch writes it: a uint8 array (n, 4 * words), little-endian and unreduced,
+    # words a multiple of 8 in [8, 72]; each returns (ok, status), both (n,) uint8, status 4 where msg > Q
+    def _schnorr_call(self, name, head, msg, rx, ry, s, words):
+        ins = [_as_u8(v, 32) for v in (msg, rx, ry)] + [_as_u8(s, 4 * int(words))]
+        n = len(ins[0])
+        if any(len(v) != n for v in ins):
+            raise ValueError("msg, r and s differ in length")
+        ok = np.empty(n, dtype=np.uint8)
+        status = np.empty(n, dtype=np.uint8)
+        self._check(getattr(self.lib, name)(self.ctx, *head(n), *[_ptr(v) for v in ins], int(words), _ptr(ok), _ptr(status)), name)
+        return ok, status
+
+    def verify_schnorr_base_batch(self, base, msg, rx, ry, s, words):
+        """verify_schnorr for every lane against the one key of `base` (a FixedBase of this engine)"""
+        return self._schnorr_call("bjj_verify_schnorr_base_batch", lambda n: (_key_handle(base), n), msg, rx, ry, s, words)
+
+    def verify_schnorr_keyset_batch(self, keyset, key_index, msg, rx, ry, s, words):
+        """verify_schnorr for every lane against key key_index[i] of `keyset` (a KeySet of this engine)"""
+        ki = _key_index(key_index, len(_as_u8(msg, 32)))
+        return self._schnorr_call("bjj_verify_schnorr_keyset_batch", lambda n: (_keyset_handle(keyset), n, _ptr(ki)), msg, rx, ry, s,
+                                  words)
+
+    def verify_schnorr_wide_batch(self, pkx, pky, msg, rx, ry, s, words):
+        """verify_schnorr for every lane against its own key (pkx, pky)"""
+        pk = [_as_u8(v, 32) for v in (pkx, pky)]
+        if len(pk[0]) != len(pk[1]) or len(pk[0]) != len(_as_u8(msg, 32)):
+            raise ValueError("pk, msg, r and s differ in length")
+        return self._schnorr_call("bjj_verify_schnorr_wide_batch", lambda n: (n, _ptr(pk[0]), _ptr(pk[1])), msg, rx, ry, s, words)
 
 
 
@@ -799,6 +830,50 @@ def verify_keyset_batch(keyset, key_index, sigs, msgs, engine=None):
                                  ints_to_le32([s.r_b8.y for s in sigs]), ints_to_le32([_verify_scalar(s.s) for s in sigs]),
                                  _verify_msgs(msgs))
     return [bool(v) for v in ok]
+
+
+def _schnorr_sigs(msgs, sigs):
+    """messages and (r, s) pairs of the verify_schnorr batches -> (msg, rx, ry, s, words): s (sign dropped, as
+    B8.mul_scalar does) in the smallest multiple of 8 words (256 bits) that holds the widest, up to 72 words (2304 bits,
+    sign_schnorr_batch's widest s).  A negative msg raises; msg > Q is clamped to an all-ones word (still > Q)."""
+    if len(msgs) != len(sigs):
+        raise ValueError("msgs and sigs differ in length")
+    ss = [abs(int(s)) for _, s in sigs]
+    bits = max([s.bit_length() for s in ss] + [1])
+    if bits > 72 * 32:
+        raise ValueError("s wider than 2304 bits is not supported by the device ABI")
+    words = 8 * ((bits + 255) // 256)
+    rs = [(r.x, r.y) if isinstance(r, Point) else tuple(r) for r, _ in sigs]
+    sb = np.frombuffer(b"".join(s.to_bytes(4 * words, "little") for s in ss), dtype=np.uint8).reshape(-1, 4 * words)
+    return _sign_msgs(msgs), ints_to_le32([r[0] for r in rs]), ints_to_le32([r[1] for r in rs]), sb, words
+
+
+def _schnorr_results(ok, st):
+    return [bool(o) if s == 0 else ValueError(STATUS_STRINGS[int(s)]) for o, s in zip(ok, st)]
+
+
+def verify_schnorr_batch(pks, msgs, sigs, engine=None):
+    """[verify_schnorr(pk, m, r, s) for pk, m, (r, s) in zip(pks, msgs, sigs)] (src/lib.rs:364-385), sigs as
+    sign_schnorr_batch returns them, s unreduced and reduced mod SUBORDER on the device -> list of bool, or
+    ValueError("msg outside the Finite Field") instances for msg > Q (the reference returns Result)"""
+    eng = engine or default_engine()
+    ok, st = eng.verify_schnorr_wide_batch(ints_to_le32([p.x for p in pks]), ints_to_le32([p.y for p in pks]), *_schnorr_sigs(msgs, sigs))
+    return _schnorr_results(ok, st)
+
+
+def verify_schnorr_base_batch(base, msgs, sigs, engine=None):
+    """verify_schnorr_batch for signatures of ONE key, whose FixedBase table `base` serves every lane (two comb walks
+    per signature)"""
+    eng = engine or base.engine
+    return _schnorr_results(*eng.verify_schnorr_base_batch(base, *_schnorr_sigs(msgs, sigs)))
+
+
+def verify_schnorr_keyset_batch(keyset, key_index, msgs, sigs, engine=None):
+    """verify_schnorr_batch with pk = keyset.points[key_index[i]] (two comb walks per signature).  An index outside the
+    set raises BjjError (BJJ_ERR_ARG)."""
+    eng = engine or keyset.engine
+    ki = np.asarray(key_index, dtype=np.int64).reshape(-1)
+    return _schnorr_results(*eng.verify_schnorr_keyset_batch(keyset, ki, *_schnorr_sigs(msgs, sigs)))
 
 
 def multi_gpu(devices=None):

@@ -68,6 +68,12 @@ SIGNATURES["bjj_mul_scalar_wide_batch"] = (_int, [_ctx, _sz, _u8p, _u8p, _u8p, _
 SIGNATURES["bjj_mul_scalar_wide_batch_dev"] = (_int, [_ctx, _sz, _u8p, _u8p, _u8p, _int, _u8p, _u8p, ctypes.c_void_p])
 SIGNATURES["bjj_sign_schnorr_batch"] = (_int, [_ctx, _sz, _u8p, _u8p, _u8p, _int] + [_u8p] * 4)
 SIGNATURES["bjj_sign_schnorr_batch_dev"] = (_int, [_ctx, _sz, _u8p, _u8p, _u8p, _int] + [_u8p] * 4 + [ctypes.c_void_p])
+# verify_schnorr with s at the signer's width (s_words words per lane)
+for _name, _head in (("bjj_verify_schnorr_base_batch", [_ctx, _base, _sz] + [_u8p] * 4),
+                     ("bjj_verify_schnorr_keyset_batch", [_ctx, _keyset, _sz] + [_u8p] * 5),
+                     ("bjj_verify_schnorr_wide_batch", [_ctx, _sz] + [_u8p] * 6)):
+    SIGNATURES[_name] = (_int, _head + [_int, _u8p, _u8p])
+    SIGNATURES[_name + "_dev"] = (_int, _head + [_int, _u8p, _u8p, ctypes.c_void_p])
 
 # multi-device layer (one caller, one host batch, N devices); host pointers only
 _multi = ctypes.c_void_p

@@ -59,6 +59,15 @@ __global__ void __launch_bounds__(BJJ_BLOCK) k_keyset_affine(size_t n, ProjScrat
     batch_affine_strided(scr, KeysetCombOut{tables}, n, (size_t)blockIdx.x * blockDim.x + threadIdx.x, (size_t)gridDim.x * blockDim.x);
 }
 
+// s mod SUBORDER of the signer's wide s (nwords words per lane) into 32 B per lane (bjj_verify_schnorr_wide)
+__global__ void __launch_bounds__(BJJ_BLOCK) k_mod_suborder_wide(size_t n, const uint8_t* wide, int nwords, uint8_t* out32) {
+    BJJ_LANE_LOOP(n) {
+        uint32_t acc[8];
+        lane_mod_suborder_wide(acc, wide, nwords, i);
+        store_u256(out32, i, acc);
+    }
+}
+
 __global__ void __launch_bounds__(BJJ_BLOCK) k_split_scalars(size_t n, const uint8_t* h32, const uint8_t* s32, uint8_t* u32,
                                                              uint8_t* v32, uint8_t* w32) {
     BJJ_LANE_LOOP(n) lane_split_scalars(h32, s32, u32, v32, w32, i);
@@ -970,10 +979,12 @@ static int launch_verify_compressed(bjj_ctx* ctx, size_t n, const uint8_t* sig64
 // 0 of launch_verify_compressed for R8 alone; `status` receives its decompression status and failed lanes are
 // rejected.  The key's coordinates are kernel arguments: base_create checked them.  With a key set `ks` instead of
 // `base` (bjj_verify_keyset*), lane i takes key key_index[i] of the set and its compact table: the kernels
-// k_verify_keyset_hash -> k_verify_keyset_ec, with the same launches.
+// k_verify_keyset_hash -> k_verify_keyset_ec, with the same launches.  s_words != 0 is verify_schnorr
+// (bjj_verify_schnorr_base* / _keyset*): r8x, r8y hold r, s32 the signer's s of s_words words per lane, `status` receives
+// the msg status, and phase 1 reduces s into the u plane of the verify scratch, which phase 2 reads.
 static int launch_verify_base(bjj_ctx* ctx, const bjj_base* base, const bjj_keyset* ks, const uint8_t* key_index, size_t n,
                               const uint8_t* r8x, const uint8_t* r8y, const uint8_t* s32, const uint8_t* sig64, const uint8_t* msg,
-                              uint8_t* ok, uint8_t* status, cudaStream_t st, Workspace* ws) {
+                              uint8_t* ok, uint8_t* status, cudaStream_t st, Workspace* ws, int s_words = 0) {
     const size_t lanes = scratch_lanes(ctx, n);
     return for_each_subbatch(n, [&](size_t off, size_t m) -> int {
         const size_t o = 32 * off;
@@ -1008,6 +1019,26 @@ static int launch_verify_base(bjj_ctx* ctx, const bjj_base* base, const bjj_keys
         unsigned long long *work_h = nullptr, *work_e = nullptr;
         TRY(claim_counter(ctx, ws, st, &work_h));
         TRY(claim_counter(ctx, ws, st, &work_e));
+        if (s_words) {
+            uint8_t* sred = hm + 32 * ws->vs_lanes;
+            const SchnorrWide sw{s32 + (size_t)4 * s_words * off, s_words, sred, status + off};
+            if (ks) {
+                const uint8_t *ki = key_index + 4 * off, *kx = ks->keys, *ky = kx + 32 * ks->n_keys;
+                const uint32_t nk = (uint32_t)ks->n_keys;
+                bjjk::verify_schnorr_keyset_hash(grid_cap(ctx, bjjk::verify_schnorr_keyset_hash_blocks_per_sm(), m), st, m, rx, ry, ki, kx, ky,
+                                                 nk, msg + o, sw, hm, ok + off, ctx->flags_dev, work_h);
+                TRY(launched(ctx));
+                bjjk::verify_schnorr_keyset_ec(grid_cap(ctx, bjjk::verify_schnorr_keyset_ec_blocks_per_sm(), m), st, m, rx, ry, sred, hm,
+                                               ok + off, ctx->comb, ki, nk, ks->tables, work_e);
+                return launched(ctx);
+            }
+            bjjk::verify_schnorr_base_hash(grid_cap(ctx, bjjk::verify_schnorr_base_hash_blocks_per_sm(), m), st, m, rx, ry, base->x, base->y,
+                                           msg + o, sw, hm, ok + off, ctx->flags_dev, work_h);
+            TRY(launched(ctx));
+            bjjk::verify_schnorr_base_ec(grid_cap(ctx, bjjk::verify_schnorr_base_ec_blocks_per_sm(), m), st, m, rx, ry, sred, hm, ok + off,
+                                         ctx->comb, base->comb, work_e);
+            return launched(ctx);
+        }
         if (ks) {
             const uint8_t *ki = key_index + 4 * off, *kx = ks->keys, *ky = kx + 32 * ks->n_keys;
             const uint32_t nk = (uint32_t)ks->n_keys;
@@ -1026,6 +1057,28 @@ static int launch_verify_base(bjj_ctx* ctx, const bjj_base* base, const bjj_keys
         return launched(ctx);
     });
 }
+// verify_schnorr with s at the signer's width on the Straus path (bjj_verify_schnorr_wide*): per sub-batch,
+// k_mod_suborder_wide reduces s into the first decompressed-point plane of the verify scratch (launch_verify's plain
+// form does not use it), then launch_verify runs unchanged with that plane as s.
+static int launch_verify_schnorr_wide(bjj_ctx* ctx, size_t n, const uint8_t* pkx, const uint8_t* pky, const uint8_t* msg,
+                                      const uint8_t* rx, const uint8_t* ry, const uint8_t* s, int s_words, uint8_t* ok, uint8_t* status,
+                                      cudaStream_t st, Workspace* ws, bool defer_join = false) {
+    const size_t lanes = scratch_lanes(ctx, n);
+    return for_each_subbatch(n, [&](size_t off, size_t m) -> int {
+        const size_t o = 32 * off;
+        // the deferred exact kernel of an earlier verify on this workspace may still read the plane
+        if (ws->aux) CU(ctx, cudaStreamWaitEvent(st, ws->ev_join, 0));
+        uint8_t *hm, *sred;
+        TRY(ensure_vscratch(ctx, ws, lanes, &hm, &sred));
+        k_mod_suborder_wide<<<grid_for(ctx, k_mod_suborder_wide, m), BJJ_BLOCK, 0, st>>>(m, s + (size_t)4 * s_words * off, s_words, sred);
+        TRY(launched(ctx));
+        return launch_verify(ctx, m, rx + o, ry + o, sred, pkx + o, pky + o, msg + o, ok + off, st, ws, BJJ_MODE_SCHNORR, status + off,
+                             defer_join);
+    });
+}
+// the widths of s that bjj_verify_schnorr_{base,keyset,wide}* take: those bjj_sign_schnorr_batch writes (nonce_words + 8)
+static bool s_words_ok(int w) { return w >= 8 && w <= BJJ_MAX_SCALAR_WORDS + 8 && !(w & 7); }
+
 // a verify_base call names its key: NULL or a handle of another context is an argument error
 static bool base_of(bjj_ctx* ctx, const bjj_base* base) { return base && base->ctx == ctx; }
 // the same for a key set
@@ -1298,6 +1351,33 @@ int bjj_keyset_mul_batch_dev(bjj_ctx* ctx, const bjj_keyset* ks, size_t n, const
     DEV_PROLOGUE
     if (!key_index || !scalar32 || !rx || !ry) return BJJ_ERR_ARG;
     return launch_keyset_mul(ctx, ks, n, (const uint8_t*)key_index, scalar32, rx, ry, st, &ctx->ws);
+}
+
+int bjj_verify_schnorr_base_batch_dev(bjj_ctx* ctx, const bjj_base* pk, size_t n, const uint8_t* msg32, const uint8_t* rx,
+                                      const uint8_t* ry, const uint8_t* s, int s_words, uint8_t* ok, uint8_t* status, void* stream) {
+    if (!base_of(ctx, pk) || !s_words_ok(s_words)) return BJJ_ERR_ARG;
+    DEV_PROLOGUE
+    if (!msg32 || !rx || !ry || !s || !ok || !status) return BJJ_ERR_ARG;
+    return launch_verify_base(ctx, pk, nullptr, nullptr, n, rx, ry, s, nullptr, msg32, ok, status, st, &ctx->ws, s_words);
+}
+
+int bjj_verify_schnorr_keyset_batch_dev(bjj_ctx* ctx, const bjj_keyset* ks, size_t n, const uint32_t* key_index, const uint8_t* msg32,
+                                        const uint8_t* rx, const uint8_t* ry, const uint8_t* s, int s_words, uint8_t* ok, uint8_t* status,
+                                        void* stream) {
+    if (!keyset_of(ctx, ks) || !s_words_ok(s_words)) return BJJ_ERR_ARG;
+    DEV_PROLOGUE
+    if (!key_index || !msg32 || !rx || !ry || !s || !ok || !status) return BJJ_ERR_ARG;
+    return launch_verify_base(ctx, nullptr, ks, (const uint8_t*)key_index, n, rx, ry, s, nullptr, msg32, ok, status, st, &ctx->ws,
+                              s_words);
+}
+
+int bjj_verify_schnorr_wide_batch_dev(bjj_ctx* ctx, size_t n, const uint8_t* pkx, const uint8_t* pky, const uint8_t* msg32,
+                                      const uint8_t* rx, const uint8_t* ry, const uint8_t* s, int s_words, uint8_t* ok, uint8_t* status,
+                                      void* stream) {
+    if (!s_words_ok(s_words)) return BJJ_ERR_ARG;
+    DEV_PROLOGUE
+    if (!pkx || !pky || !msg32 || !rx || !ry || !s || !ok || !status) return BJJ_ERR_ARG;
+    return launch_verify_schnorr_wide(ctx, n, pkx, pky, msg32, rx, ry, s, s_words, ok, status, st, &ctx->ws);
 }
 
 }  // extern "C"
@@ -1723,6 +1803,35 @@ int bjj_keyset_mul_batch(bjj_ctx* ctx, const bjj_keyset* ks, size_t n, const uin
     HostArg args[] = {H_IN((const uint8_t*)key_index, 4), H_IN(scalar32, 32), H_OUT(rx, 32), H_OUT(ry, 32)};
     return run_host(ctx, n, args, 4, [&](size_t m, uint8_t** d, cudaStream_t st, Workspace* ws) -> int {
         return launch_keyset_mul(ctx, ks, m, d[0], d[1], d[2], d[3], st, ws);
+    }, /*heavy=*/true);
+}
+
+int bjj_verify_schnorr_base_batch(bjj_ctx* ctx, const bjj_base* pk, size_t n, const uint8_t* msg32, const uint8_t* rx, const uint8_t* ry,
+                                  const uint8_t* s, int s_words, uint8_t* ok, uint8_t* status) {
+    if (!base_of(ctx, pk) || !s_words_ok(s_words)) return BJJ_ERR_ARG;
+    HostArg args[] = {H_IN(msg32, 32), H_IN(rx, 32), H_IN(ry, 32), H_IN(s, (size_t)4 * s_words), H_OUT(ok, 1), H_OUT(status, 1)};
+    return run_host(ctx, n, args, 6, [&](size_t m, uint8_t** d, cudaStream_t st, Workspace* ws) -> int {
+        return launch_verify_base(ctx, pk, nullptr, nullptr, m, d[1], d[2], d[3], nullptr, d[0], d[4], d[5], st, ws, s_words);
+    }, /*heavy=*/true);
+}
+
+int bjj_verify_schnorr_keyset_batch(bjj_ctx* ctx, const bjj_keyset* ks, size_t n, const uint32_t* key_index, const uint8_t* msg32,
+                                    const uint8_t* rx, const uint8_t* ry, const uint8_t* s, int s_words, uint8_t* ok, uint8_t* status) {
+    if (!keyset_of(ctx, ks) || !s_words_ok(s_words)) return BJJ_ERR_ARG;
+    HostArg args[] = {H_IN((const uint8_t*)key_index, 4), H_IN(msg32, 32), H_IN(rx, 32),    H_IN(ry, 32),
+                      H_IN(s, (size_t)4 * s_words),       H_OUT(ok, 1),      H_OUT(status, 1)};
+    return run_host(ctx, n, args, 7, [&](size_t m, uint8_t** d, cudaStream_t st, Workspace* ws) -> int {
+        return launch_verify_base(ctx, nullptr, ks, d[0], m, d[2], d[3], d[4], nullptr, d[1], d[5], d[6], st, ws, s_words);
+    }, /*heavy=*/true);
+}
+
+int bjj_verify_schnorr_wide_batch(bjj_ctx* ctx, size_t n, const uint8_t* pkx, const uint8_t* pky, const uint8_t* msg32, const uint8_t* rx,
+                                  const uint8_t* ry, const uint8_t* s, int s_words, uint8_t* ok, uint8_t* status) {
+    if (!ctx || !s_words_ok(s_words)) return BJJ_ERR_ARG;
+    HostArg args[] = {H_IN(pkx, 32), H_IN(pky, 32), H_IN(msg32, 32), H_IN(rx, 32), H_IN(ry, 32), H_IN(s, (size_t)4 * s_words), H_OUT(ok, 1),
+                      H_OUT(status, 1)};
+    return run_host(ctx, n, args, 8, [&](size_t m, uint8_t** d, cudaStream_t st, Workspace* ws) -> int {
+        return launch_verify_schnorr_wide(ctx, m, d[0], d[1], d[2], d[3], d[4], d[5], s_words, d[6], d[7], st, ws, true);
     }, /*heavy=*/true);
 }
 

@@ -113,5 +113,23 @@ void verify_keyset_ec(int grid, cudaStream_t st, size_t n, const uint8_t* r8x, c
                       size_t s_stride, size_t s_off, const uint8_t* hm, uint8_t* ok, const bjj::CombEntry* comb,
                       const uint8_t* key_index, uint32_t n_keys, const bjj::CombEntry* tables, unsigned long long* work);
 int verify_keyset_ec_blocks_per_sm();
+// verify_schnorr on the same two phases (one key / a key set): sw carries the signer's wide s, its reduced plane s_red
+// (read by phase 2) and the msg status array
+void verify_schnorr_base_hash(int grid, cudaStream_t st, size_t n, const uint8_t* rx, const uint8_t* ry, const uint8_t* pkx32,
+                              const uint8_t* pky32, const uint8_t* msg, const bjj::SchnorrWide& sw, uint8_t* hm, uint8_t* ok,
+                              uint32_t* gflags, unsigned long long* work);
+int verify_schnorr_base_hash_blocks_per_sm();
+void verify_schnorr_base_ec(int grid, cudaStream_t st, size_t n, const uint8_t* rx, const uint8_t* ry, const uint8_t* s_red,
+                            const uint8_t* hm, uint8_t* ok, const bjj::CombEntry* comb, const bjj::CombEntry* comb_a,
+                            unsigned long long* work);
+int verify_schnorr_base_ec_blocks_per_sm();
+void verify_schnorr_keyset_hash(int grid, cudaStream_t st, size_t n, const uint8_t* rx, const uint8_t* ry, const uint8_t* key_index,
+                                const uint8_t* kx, const uint8_t* ky, uint32_t n_keys, const uint8_t* msg, const bjj::SchnorrWide& sw,
+                                uint8_t* hm, uint8_t* ok, uint32_t* gflags, unsigned long long* work);
+int verify_schnorr_keyset_hash_blocks_per_sm();
+void verify_schnorr_keyset_ec(int grid, cudaStream_t st, size_t n, const uint8_t* rx, const uint8_t* ry, const uint8_t* s_red,
+                              const uint8_t* hm, uint8_t* ok, const bjj::CombEntry* comb, const uint8_t* key_index, uint32_t n_keys,
+                              const bjj::CombEntry* tables, unsigned long long* work);
+int verify_schnorr_keyset_ec_blocks_per_sm();
 
 }  // namespace bjjk

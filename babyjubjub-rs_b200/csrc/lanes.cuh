@@ -1100,7 +1100,8 @@ BJJ_HD void lane_sign(const uint8_t* key32, const uint8_t* msg32, uint8_t* r8x, 
     status[i] = (uint8_t)st;
 }
 
-// acc = x mod SUBORDER, canonical, for lane i of a wide array (nwords a multiple of 8 up to BJJ_MAX_SCALAR_WORDS).
+// acc = x mod SUBORDER, canonical, for lane i of a wide array (nwords a multiple of 8: up to BJJ_MAX_SCALAR_WORDS for a
+// nonce, up to BJJ_MAX_SCALAR_WORDS + 8 for the s that bjj_sign_schnorr_batch writes).
 // Horner over the 256-bit blocks from the top, acc <- acc * R + block (mod l), R = 2^256: montmul_suborder(acc, R^2 mod l)
 // = acc * R and montmul_suborder(block, R mod l) = block (mod l), each below 2l (acc * R^2 < l^2 and block * R < R l),
 // so the sum is below 4l and two conditional subtractions (2l, l) finish.  Two products per block where
@@ -1568,9 +1569,26 @@ BJJ_HD void lane_verify_exact(const uint8_t* r8x, const uint8_t* r8y, const uint
 // ok[i] between the phases: 0 (rejected), BJJ_OK_PENDING (R8 on the curve) or BJJ_OK_PENDING_EXACT (off the curve).
 #define BJJ_OK_PENDING_EXACT 3
 
+// verify_schnorr (src/lib.rs:364-385) on the same two phases (bjj_verify_schnorr_base*, bjj_verify_schnorr_keyset*):
+// MODE = BJJ_MODE_SCHNORR, `a` is pk and R8 is r.  Phase 1 hashes h = Poseidon(pk.x, pk.y, r.x, r.y, msg), writes the
+// msg range status of every lane, and reduces the signer's wide s (nwords words at word offset nwords * i) mod SUBORDER
+// into s_out; phase 2 reads s there.  Exactness: B8 has order SUBORDER, so B8.mul_scalar(s) = (s mod SUBORDER) * B8 for
+// s of any width; pk is on the curve (checked when its table was built), so its order divides ORDER and
+// pk.mul_scalar(h) = h * pk with h < Q < ORDER used raw -- never reduced mod SUBORDER, which would be wrong for a pk with
+// a torsion component.  r on the curve: accept iff (s mod SUBORDER)*B8 + (ORDER - h)*pk - r == O; r off the curve: the
+// reference's literal sum and affine comparison, as for EdDSA.
+struct SchnorrWide {
+    const uint8_t* s;       // the signer's s, nwords words per lane
+    int nwords;
+    uint8_t* s_out;         // s mod SUBORDER, 32 B per lane
+    uint8_t* status;        // BJJ_ST_MSG_RANGE where msg > Q, else BJJ_ST_OK
+};
+
 // a: A in Montgomery form (the same for every lane).  `skip` (may be null): lanes whose R8 did not decompress.
+template <int MODE = BJJ_MODE_EDDSA>
 BJJ_HD void lane_verify_base_hash(const uint8_t* r8x, const uint8_t* r8y, const PointAff& a, const uint8_t* msg32,
-                                  const uint8_t* skip, uint8_t* hm_out, uint8_t* ok, size_t i, uint32_t& flags) {
+                                  const uint8_t* skip, uint8_t* hm_out, uint8_t* ok, size_t i, uint32_t& flags,
+                                  const SchnorrWide& sw = SchnorrWide{}) {
     if (skip && skip[i]) {
         ok[i] = 0;
         return;
@@ -1578,7 +1596,10 @@ BJJ_HD void lane_verify_base_hash(const uint8_t* r8x, const uint8_t* r8y, const 
     uint32_t msg[8];
     load_u256(msg, msg32, i);
     const uint32_t qq[8] = BJJ_LIMBS8(BJJ_Q);
-    if (u256_lt(qq, msg)) {     // msg > Q -> false; msg == Q is accepted and hashed as 0 (src/lib.rs:396-399)
+    const bool msg_bad = u256_lt(qq, msg);
+    // verify_schnorr: Err("msg outside the Finite Field") (src/lib.rs:365-367)
+    if constexpr (MODE == BJJ_MODE_SCHNORR) sw.status[i] = msg_bad ? (uint8_t)BJJ_ST_MSG_RANGE : (uint8_t)BJJ_ST_OK;
+    if (msg_bad) {     // msg > Q -> false; msg == Q is accepted and hashed as 0 (src/lib.rs:396-399)
         ok[i] = 0;
         return;
     }
@@ -1588,8 +1609,13 @@ BJJ_HD void lane_verify_base_hash(const uint8_t* r8x, const uint8_t* r8y, const 
     Fr mraw, mm, hm;
     fr_set(mraw, msg);
     fr_to_mont(mm, mraw);
-    verify_hm(hm, r8, a, mm, BJJ_MODE_EDDSA);
+    verify_hm(hm, r8, a, mm, MODE);
     store_u256(hm_out, i, hm.v);
+    if constexpr (MODE == BJJ_MODE_SCHNORR) {
+        uint32_t sr[8];
+        lane_mod_suborder_wide(sr, sw.s, sw.nwords, i);
+        store_u256(sw.s_out, i, sr);
+    }
     ok[i] = on_curve(r8) ? (uint8_t)BJJ_OK_PENDING : (uint8_t)BJJ_OK_PENDING_EXACT;
 }
 
@@ -1609,8 +1635,8 @@ BJJ_HD void verify_base_scalar(uint32_t* k, const uint32_t* hm) {
 // products from the combs: l = S*B8 and kA in affine form (one shared inversion), literal add-2008-bbjlp of R8 and kA
 // with Z = 1, PointProjective::affine (Z == 0 -> (0, 0)), compare with l (src/lib.rs:405-411).  The two comb walks run
 // for every lane, so a warp that holds both kinds of lanes diverges only in the short tails.  GA: the geometry of comb_a
-// (Comb16 for a bjj_base, Comb8 for a key of a key set).
-template <class GA = Comb16>
+// (Comb16 for a bjj_base, Comb8 for a key of a key set).  MODE = BJJ_MODE_SCHNORR: k = h as it is (see SchnorrWide).
+template <class GA = Comb16, int MODE = BJJ_MODE_EDDSA>
 BJJ_HD void lane_verify_base_ec(const uint8_t* r8x, const uint8_t* r8y, const uint8_t* s_base, size_t s_stride, size_t s_off,
                                 const uint8_t* hm_in, uint8_t* ok, size_t i, const CombEntry* comb, const CombEntry* comb_a) {
     const uint32_t state = ok[i];
@@ -1619,7 +1645,12 @@ BJJ_HD void lane_verify_base_ec(const uint8_t* r8x, const uint8_t* r8y, const ui
     uint32_t s[8], hm[8], k[8];
     load_u256(s, s_base, i * s_stride + s_off);
     load_u256(hm, hm_in, i);
-    verify_base_scalar(k, hm);
+    if constexpr (MODE == BJJ_MODE_SCHNORR) {
+#pragma unroll
+        for (int j = 0; j < 8; j++) k[j] = hm[j];
+    } else {
+        verify_base_scalar(k, hm);
+    }
     PointExt acc, l;
     ext_identity(acc);
     fixed_base_comb_acc(acc, comb, s);
@@ -1757,27 +1788,36 @@ BJJ_HD bool keyset_index(uint32_t& key, const uint8_t* key_index, uint32_t n_key
     return false;
 }
 
-// verify phase 1 against key key_index[i] of the set: lane_verify_base_hash with that key
+// verify phase 1 against key key_index[i] of the set: lane_verify_base_hash with that key (MODE and sw as there; a
+// Schnorr lane with an index outside the set still gets its msg status)
+template <int MODE = BJJ_MODE_EDDSA>
 BJJ_HD void lane_verify_keyset_hash(const uint8_t* r8x, const uint8_t* r8y, const uint8_t* key_index, const uint8_t* kx,
                                     const uint8_t* ky, uint32_t n_keys, const uint8_t* msg32, const uint8_t* skip, uint8_t* hm_out,
-                                    uint8_t* ok, size_t i, uint32_t& flags) {
+                                    uint8_t* ok, size_t i, uint32_t& flags, const SchnorrWide& sw = SchnorrWide{}) {
     uint32_t key;
     if (!keyset_index(key, key_index, n_keys, i, flags)) {
+        if constexpr (MODE == BJJ_MODE_SCHNORR) {
+            uint32_t msg[8];
+            load_u256(msg, msg32, i);
+            const uint32_t qq[8] = BJJ_LIMBS8(BJJ_Q);
+            sw.status[i] = u256_lt(qq, msg) ? (uint8_t)BJJ_ST_MSG_RANGE : (uint8_t)BJJ_ST_OK;
+        }
         ok[i] = 0;
         return;
     }
     PointAff a;
     keyset_point(a, kx, ky, key);
-    lane_verify_base_hash(r8x, r8y, a, msg32, skip, hm_out, ok, i, flags);
+    lane_verify_base_hash<MODE>(r8x, r8y, a, msg32, skip, hm_out, ok, i, flags, sw);
 }
 
 // verify phase 2: lane_verify_base_ec with the key's compact table (lanes rejected in phase 1 return at once)
+template <int MODE = BJJ_MODE_EDDSA>
 BJJ_HD void lane_verify_keyset_ec(const uint8_t* r8x, const uint8_t* r8y, const uint8_t* s_base, size_t s_stride, size_t s_off,
                                   const uint8_t* hm_in, uint8_t* ok, size_t i, const CombEntry* comb, const uint8_t* key_index,
                                   uint32_t n_keys, const CombEntry* tables) {
     uint32_t key, flags = 0;
     if (!keyset_index(key, key_index, n_keys, i, flags)) return;
-    lane_verify_base_ec<Comb8>(r8x, r8y, s_base, s_stride, s_off, hm_in, ok, i, comb, tables + (size_t)key * BJJ_KEY_COMB_TOTAL);
+    lane_verify_base_ec<Comb8, MODE>(r8x, r8y, s_base, s_stride, s_off, hm_in, ok, i, comb, tables + (size_t)key * BJJ_KEY_COMB_TOTAL);
 }
 
 // P_{key_index[i]}.mul_scalar(k) for a raw 256-bit k (src/lib.rs:149-164), 33 mixed additions; a lane with an index

@@ -13,7 +13,8 @@
 //   verify(pk, sig, msg)                   src/lib.rs:395-412
 //   verify_schnorr(pk, m, r, s)            src/lib.rs:375-385
 //   + batch entry points: mul_scalar_batch, public_batch, decompress_batch, verify_batch,
-//     public_compressed_batch, sign_compressed_batch, sign_schnorr_batch (caller nonces)
+//     public_compressed_batch, sign_compressed_batch, sign_schnorr_batch (caller nonces), verify_schnorr_batch (the
+//     signer's unreduced s, reduced on the device; FixedBase / KeySet members on the comb path)
 //   + FixedBase: the comb table of a caller-chosen point, k*P and k*P + l*Q at the fixed-base rate, and verify for
 //     many signatures of that one key
 //   + KeySet: many known keys with compact comb tables, verify and k*P with a key index per lane
@@ -293,6 +294,54 @@ inline std::vector<SignSchnorrResult> sign_schnorr_batch(const std::vector<Priva
     return out;
 }
 
+// Inputs of the verify_schnorr batches: messages and the (r, s) of sign_schnorr_batch as they come, every s of one width
+// (4 * s_words bytes, s_words a multiple of 8 in 8..72)
+struct SchnorrLanes {
+    size_t n;
+    int s_words;
+    std::vector<uint8_t> m, rx, ry, s;
+    std::vector<uint8_t> ok, status;
+};
+inline SchnorrLanes schnorr_lanes(const std::vector<U256>& msgs, const std::vector<SignSchnorrResult>& sigs) {
+    if (sigs.size() != msgs.size()) throw std::invalid_argument("sigs and msgs differ in length");
+    SchnorrLanes l;
+    l.n = sigs.size();
+    const size_t sw = l.n ? sigs[0].s.size() : 32;
+    l.s_words = (int)(sw / 4);
+    l.m = pack(msgs);
+    l.rx.resize(32 * l.n);
+    l.ry.resize(32 * l.n);
+    l.s.resize(sw * l.n);
+    l.ok.resize(l.n);
+    l.status.resize(l.n);
+    for (size_t i = 0; i < l.n; i++) {
+        if (sigs[i].s.size() != sw) throw std::invalid_argument("s of different widths in one batch");
+        std::memcpy(&l.rx[32 * i], sigs[i].r.x.data(), 32);
+        std::memcpy(&l.ry[32 * i], sigs[i].r.y.data(), 32);
+        std::memcpy(&l.s[sw * i], sigs[i].s.data(), sw);
+    }
+    return l;
+}
+
+// [verify_schnorr(pks[i], msgs[i], r, s)] (src/lib.rs:364-385) for the (r, s) of sign_schnorr_batch, s reduced on the
+// device: ok per lane, and status (when given) BJJ_STATUS_MSG_RANGE where msg > Q (the reference's Err)
+inline std::vector<uint8_t> verify_schnorr_batch(const std::vector<Point>& pks, const std::vector<U256>& msgs,
+                                                 const std::vector<SignSchnorrResult>& sigs, std::vector<uint8_t>* status = nullptr,
+                                                 Engine& e = default_engine()) {
+    if (pks.size() != msgs.size()) throw std::invalid_argument("pks and msgs differ in length");
+    SchnorrLanes l = schnorr_lanes(msgs, sigs);
+    std::vector<U256> px(l.n), py(l.n);
+    for (size_t i = 0; i < l.n; i++) {
+        px[i] = pks[i].x;
+        py[i] = pks[i].y;
+    }
+    auto ax = pack(px), ay = pack(py);
+    Engine::check(bjj_verify_schnorr_wide_batch(e.ctx(), l.n, ax.data(), ay.data(), l.m.data(), l.rx.data(), l.ry.data(), l.s.data(),
+                                                l.s_words, l.ok.data(), l.status.data()), "bjj_verify_schnorr_wide_batch");
+    if (status) *status = l.status;
+    return l.ok;
+}
+
 // The comb table of one on-curve point P on an Engine (50 MB of device memory, freed by the destructor): P.mul_scalar(k)
 // for many k at the rate of B8's fixed-base path.  Throws Error with BJJ_ERR_ARG for an off-curve P (use
 // mul_scalar_batch there) and BJJ_ERR_NONCANONICAL for a coordinate >= Q.  Must not outlive its Engine.
@@ -352,6 +401,15 @@ class FixedBase {
                       "bjj_verify_base_compressed_batch");
         if (status) *status = st;
         return ok;
+    }
+    // verify_schnorr_batch with P in every lane, on the comb path
+    std::vector<uint8_t> verify_schnorr_batch(const std::vector<U256>& msgs, const std::vector<SignSchnorrResult>& sigs,
+                                              std::vector<uint8_t>* status = nullptr) const {
+        SchnorrLanes l = schnorr_lanes(msgs, sigs);
+        Engine::check(bjj_verify_schnorr_base_batch(e_.ctx(), base_, l.n, l.m.data(), l.rx.data(), l.ry.data(), l.s.data(), l.s_words,
+                                                    l.ok.data(), l.status.data()), "bjj_verify_schnorr_base_batch");
+        if (status) *status = l.status;
+        return l.ok;
     }
 
   private:
@@ -421,6 +479,17 @@ class KeySet {
                       "bjj_verify_keyset_compressed_batch");
         if (status) *status = st;
         return ok;
+    }
+    // verify_schnorr_batch with pk = keys[key_index[i]], on the comb path
+    std::vector<uint8_t> verify_schnorr_batch(const std::vector<uint32_t>& key_index, const std::vector<U256>& msgs,
+                                              const std::vector<SignSchnorrResult>& sigs, std::vector<uint8_t>* status = nullptr) const {
+        if (key_index.size() != msgs.size()) throw std::invalid_argument("key_index and msgs differ in length");
+        SchnorrLanes l = schnorr_lanes(msgs, sigs);
+        Engine::check(bjj_verify_schnorr_keyset_batch(e_.ctx(), ks_, l.n, key_index.data(), l.m.data(), l.rx.data(), l.ry.data(),
+                                                      l.s.data(), l.s_words, l.ok.data(), l.status.data()),
+                      "bjj_verify_schnorr_keyset_batch");
+        if (status) *status = l.status;
+        return l.ok;
     }
     // [keys[key_index[i]].mul_scalar(k[i])]; scalars are raw 256-bit values (reduce wider ones mod ORDER)
     std::vector<Point> mul_batch(const std::vector<uint32_t>& key_index, const std::vector<U256>& scalars) const {

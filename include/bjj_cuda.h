@@ -290,6 +290,38 @@ int bjj_verify_schnorr_batch_dev(bjj_ctx* ctx, size_t n, const uint8_t* pkx, con
                                  const uint8_t* rx, const uint8_t* ry, const uint8_t* s32, uint8_t* ok, uint8_t* status,
                                  void* stream);
 
+/* ---- verify_schnorr (src/lib.rs:364-385) on the signer's own output: s at the width bjj_sign_schnorr_batch writes it.
+ *      s[i] is s_words little-endian 32-bit words at byte offset 4*s_words*i: exactly bjj_sign_schnorr_batch's s with
+ *      s_words = nonce_words + 8.  s_words a multiple of 8 in 8..72, else BJJ_ERR_ARG.  s is reduced mod SUBORDER on the
+ *      device (B8 has that order, so B8.mul_scalar(s) is unchanged).  status[i] = BJJ_STATUS_MSG_RANGE iff msg > Q (then
+ *      ok[i] = 0), for every lane; msg == Q hashes as 0.  An r coordinate >= Q returns BJJ_ERR_NONCANONICAL (the batch
+ *      is computed mod Q).
+ *   - _base: every lane's pk is the key of `pk` (bjj_base_create), on the comb path of bjj_verify_base_batch: one
+ *     Poseidon and two comb walks per lane.  pk == NULL or a handle of another context returns BJJ_ERR_ARG.
+ *   - _keyset: pk = key key_index[i] of ks, on the comb path of bjj_verify_keyset_batch.  key_index[i] >= n_keys: that
+ *     lane gets ok = 0, the other lanes are computed, and the call returns BJJ_ERR_ARG (a _dev call: the next bjj_sync).
+ *   - _wide: any pk per lane, on bjj_verify_schnorr_batch's path after the reduction of s (off-curve pk or r replayed
+ *     like there).
+ *   The comb forms use h < Q raw against the key's table (never reduced mod SUBORDER), so keys with a torsion component
+ *   give the reference's answer. */
+int bjj_verify_schnorr_base_batch(bjj_ctx* ctx, const bjj_base* pk, size_t n, const uint8_t* msg32, const uint8_t* rx,
+                                  const uint8_t* ry, const uint8_t* s, int s_words, uint8_t* ok, uint8_t* status);
+int bjj_verify_schnorr_base_batch_dev(bjj_ctx* ctx, const bjj_base* pk, size_t n, const uint8_t* msg32, const uint8_t* rx,
+                                      const uint8_t* ry, const uint8_t* s, int s_words, uint8_t* ok, uint8_t* status,
+                                      void* stream);
+int bjj_verify_schnorr_keyset_batch(bjj_ctx* ctx, const bjj_keyset* ks, size_t n, const uint32_t* key_index,
+                                    const uint8_t* msg32, const uint8_t* rx, const uint8_t* ry, const uint8_t* s, int s_words,
+                                    uint8_t* ok, uint8_t* status);
+int bjj_verify_schnorr_keyset_batch_dev(bjj_ctx* ctx, const bjj_keyset* ks, size_t n, const uint32_t* key_index,
+                                        const uint8_t* msg32, const uint8_t* rx, const uint8_t* ry, const uint8_t* s,
+                                        int s_words, uint8_t* ok, uint8_t* status, void* stream);
+int bjj_verify_schnorr_wide_batch(bjj_ctx* ctx, size_t n, const uint8_t* pkx, const uint8_t* pky, const uint8_t* msg32,
+                                  const uint8_t* rx, const uint8_t* ry, const uint8_t* s, int s_words, uint8_t* ok,
+                                  uint8_t* status);
+int bjj_verify_schnorr_wide_batch_dev(bjj_ctx* ctx, size_t n, const uint8_t* pkx, const uint8_t* pky, const uint8_t* msg32,
+                                      const uint8_t* rx, const uint8_t* ry, const uint8_t* s, int s_words, uint8_t* ok,
+                                      uint8_t* status, void* stream);
+
 /* ---- decompress_signature + decompress_point(pk) + verify (src/lib.rs:260-268, 192-224, 395-412):
  *      status[i] = first decompression error (R8 first, then A); ok[i] = 0 whenever status[i] != 0. -- */
 int bjj_verify_compressed_batch(bjj_ctx* ctx, size_t n, const uint8_t* sig64, const uint8_t* pk32,

@@ -110,6 +110,16 @@ extern "C" {
     // verify_schnorr + schnorr_hash (src/lib.rs:364-385)
     pub fn bjj_verify_schnorr_batch(ctx: *mut bjj_ctx, n: usize, pkx: *const u8, pky: *const u8, msg32: *const u8,
                                     rx: *const u8, ry: *const u8, s32: *const u8, ok: *mut u8, status: *mut u8) -> c_int;
+    // the same on the signer's unreduced s (s_words words per lane, reduced on the device): one key's table, a key set,
+    // or any key per lane
+    pub fn bjj_verify_schnorr_base_batch(ctx: *mut bjj_ctx, pk: *const bjj_base, n: usize, msg32: *const u8, rx: *const u8,
+                                         ry: *const u8, s: *const u8, s_words: c_int, ok: *mut u8, status: *mut u8) -> c_int;
+    pub fn bjj_verify_schnorr_keyset_batch(ctx: *mut bjj_ctx, ks: *const bjj_keyset, n: usize, key_index: *const u32,
+                                           msg32: *const u8, rx: *const u8, ry: *const u8, s: *const u8, s_words: c_int,
+                                           ok: *mut u8, status: *mut u8) -> c_int;
+    pub fn bjj_verify_schnorr_wide_batch(ctx: *mut bjj_ctx, n: usize, pkx: *const u8, pky: *const u8, msg32: *const u8,
+                                         rx: *const u8, ry: *const u8, s: *const u8, s_words: c_int, ok: *mut u8,
+                                         status: *mut u8) -> c_int;
     // decompress_signature + decompress_point + verify (src/lib.rs:260-268)
     pub fn bjj_verify_compressed_batch(ctx: *mut bjj_ctx, n: usize, sig64: *const u8, pk32: *const u8,
                                        msg32: *const u8, ok: *mut u8, status: *mut u8) -> c_int;

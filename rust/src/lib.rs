@@ -279,6 +279,48 @@ pub fn verify_schnorr(pk: Point, m: BigInt, r: Point, s: BigInt) -> Result<bool,
     Ok(ok == 1)
 }
 
+/// Inputs of the verify_schnorr batches: messages and `(r, s)` pairs as `sign_schnorr_batch_with_nonces` returns them,
+/// s (sign dropped) in the smallest multiple of 256 bits that holds the widest.  Panics on a negative msg, on s wider than
+/// 2304 bits, or on lengths that differ.
+struct SchnorrLanes {
+    n: usize,
+    words: usize,
+    m: Vec<u8>,
+    rx: Vec<u8>,
+    ry: Vec<u8>,
+    s: Vec<u8>,
+}
+fn schnorr_lanes(msgs: &[BigInt], sigs: &[(Point, BigInt)]) -> SchnorrLanes {
+    let n = sigs.len();
+    assert_eq!(n, msgs.len());
+    assert!(msgs.iter().all(|m| m.sign() != Sign::Minus), "negative msg");
+    let bits = sigs.iter().map(|(_, s)| s.bits()).max().unwrap_or(0).max(1);
+    assert!(bits <= 2304, "s wider than 2304 bits");
+    let words = (8 * ((bits + 255) / 256)) as usize;
+    let mut s = vec![0u8; 4 * words * n];
+    for (i, (_, v)) in sigs.iter().enumerate() {
+        let (_, bytes) = v.to_bytes_le();
+        s[4 * words * i..4 * words * i + bytes.len()].copy_from_slice(&bytes);
+    }
+    SchnorrLanes { n, words, m: col(n, |i| msg_le32(&msgs[i])), rx: col(n, |i| sigs[i].0.x), ry: col(n, |i| sigs[i].0.y), s }
+}
+fn schnorr_results(ok: &[u8], st: &[u8]) -> Vec<Result<bool, String>> {
+    (0..ok.len()).map(|i| if st[i] == 0 { Ok(ok[i] == 1) } else { Err(status_str(st[i])) }).collect()
+}
+
+/// `verify_schnorr(pks[i], msgs[i], r, s)` (src/lib.rs:364-385) lane by lane on the signer's unreduced `(r, s)`, reduced
+/// mod SUBORDER on the device
+pub fn verify_schnorr_batch(pks: &[Point], msgs: &[BigInt], sigs: &[(Point, BigInt)]) -> Vec<Result<bool, String>> {
+    let l = schnorr_lanes(msgs, sigs);
+    assert_eq!(l.n, pks.len());
+    let (ax, ay) = (col(l.n, |i| pks[i].x), col(l.n, |i| pks[i].y));
+    let (mut ok, mut st) = (vec![0u8; l.n], vec![0u8; l.n]);
+    check(unsafe { ffi::bjj_verify_schnorr_wide_batch(engine().raw(), l.n, ax.as_ptr(), ay.as_ptr(), l.m.as_ptr(), l.rx.as_ptr(),
+                                                      l.ry.as_ptr(), l.s.as_ptr(), l.words as i32, ok.as_mut_ptr(),
+                                                      st.as_mut_ptr()) }, "bjj_verify_schnorr_wide_batch");
+    schnorr_results(&ok, &st)
+}
+
 /// src/lib.rs:387-393 draws 1024 random bits and keeps the first 32 big-endian bytes; here the caller supplies the
 /// 32 random bytes (no RNG dependency in this crate).
 pub fn new_key_from_bytes(random32: [u8; 32]) -> PrivateKey {
@@ -393,6 +435,15 @@ impl FixedBase {
               "bjj_verify_base_compressed_batch");
         (0..n).map(|i| if st[i] == 0 { Ok(ok[i] == 1) } else { Err(status_str(st[i])) }).collect()
     }
+    /// `verify_schnorr_batch` with P in every lane, on the comb tables
+    pub fn verify_schnorr_batch(&self, msgs: &[BigInt], sigs: &[(Point, BigInt)]) -> Vec<Result<bool, String>> {
+        let l = schnorr_lanes(msgs, sigs);
+        let (mut ok, mut st) = (vec![0u8; l.n], vec![0u8; l.n]);
+        check(unsafe { ffi::bjj_verify_schnorr_base_batch(engine().raw(), self.base, l.n, l.m.as_ptr(), l.rx.as_ptr(), l.ry.as_ptr(),
+                                                          l.s.as_ptr(), l.words as i32, ok.as_mut_ptr(), st.as_mut_ptr()) },
+              "bjj_verify_schnorr_base_batch");
+        schnorr_results(&ok, &st)
+    }
 }
 impl Drop for FixedBase {
     fn drop(&mut self) {
@@ -446,6 +497,16 @@ impl KeySet {
                                                                m.as_ptr(), ok.as_mut_ptr(), st.as_mut_ptr()) },
               "bjj_verify_keyset_compressed_batch");
         (0..n).map(|i| if st[i] == 0 { Ok(ok[i] == 1) } else { Err(status_str(st[i])) }).collect()
+    }
+    /// `verify_schnorr_batch` with pk = keys[key_index[i]], on the compact tables
+    pub fn verify_schnorr_batch(&self, key_index: &[u32], msgs: &[BigInt], sigs: &[(Point, BigInt)]) -> Vec<Result<bool, String>> {
+        let l = schnorr_lanes(msgs, sigs);
+        assert_eq!(l.n, key_index.len());
+        let (mut ok, mut st) = (vec![0u8; l.n], vec![0u8; l.n]);
+        check(unsafe { ffi::bjj_verify_schnorr_keyset_batch(engine().raw(), self.ks, l.n, key_index.as_ptr(), l.m.as_ptr(),
+                                                            l.rx.as_ptr(), l.ry.as_ptr(), l.s.as_ptr(), l.words as i32,
+                                                            ok.as_mut_ptr(), st.as_mut_ptr()) }, "bjj_verify_schnorr_keyset_batch");
+        schnorr_results(&ok, &st)
     }
     /// `[keys[key_index[i]].mul_scalar(k[i])]`
     pub fn mul_batch(&self, key_index: &[u32], scalars: &[BigInt]) -> Vec<Point> {
