@@ -21,6 +21,8 @@ follow the reference's public API (paths into the reference tree):
       (two comb walks per signature instead of verify_batch's per-lane ladder).
     + KeySet / verify_keyset_batch: verify for batches that mix many known keys, each key with a compact
       comb table (4,130 entries, 396 KB) and a key index per signature.
+    + KeySet.lookup / verify_keyset_lookup_batch: the same keys found by their 32-byte compressed form on the device,
+      so that a key-set verify takes verify_compressed's arrays; a key outside the set is a per-lane None.
     + sign_schnorr_batch: PrivateKey::sign_schnorr over a batch, with caller-supplied (or random 1024-bit)
       nonces and the unreduced s of the reference.
     + verify_schnorr_batch / verify_schnorr_base_batch / verify_schnorr_keyset_batch: verify_schnorr over a batch,
@@ -53,6 +55,7 @@ STATUS_STRINGS = {
     4: "msg outside the Finite Field",
 }
 ERR_NONCANONICAL = 3
+KEY_NONE = 0xFFFFFFFF       # key index of the lookup calls for a key outside the set
 
 
 # ---- conversions ---------------------------------------------------------------------------------
@@ -345,6 +348,28 @@ class Engine:
                     "bjj_keyset_mul_batch")
         return rx, ry
 
+    def keyset_lookup_batch(self, keyset, pk32):
+        """the index of the key of `keyset` whose compressed bytes are pk32[i], or KEY_NONE -> (n,) uint32"""
+        pk = _as_u8(pk32, 32)
+        ki = np.empty(len(pk), dtype="<u4")
+        self._check(self.lib.bjj_keyset_lookup_batch(self.ctx, _keyset_handle(keyset), len(pk), _ptr(pk), _ptr(ki)),
+                    "bjj_keyset_lookup_batch")
+        return ki
+
+    def verify_keyset_lookup_compressed_batch(self, keyset, sig64, pk32, msg):
+        """verify_compressed_batch's arrays, for keys of `keyset` found by their compressed bytes -> (ok, status,
+        key_index): (n,) uint8, uint8 and uint32.  A key outside the set gives ok 0, R8's status and KEY_NONE."""
+        sg, pk, m = _as_u8(sig64, 64), _as_u8(pk32, 32), _as_u8(msg, 32)
+        if len(pk) != len(sg) or len(m) != len(sg):
+            raise ValueError("sig64, pk32 and msg differ in length")
+        ok = np.empty(len(sg), dtype=np.uint8)
+        status = np.empty(len(sg), dtype=np.uint8)
+        ki = np.empty(len(sg), dtype="<u4")
+        self._check(self.lib.bjj_verify_keyset_lookup_compressed_batch(self.ctx, _keyset_handle(keyset), len(sg), _ptr(sg), _ptr(pk),
+                                                                       _ptr(m), _ptr(ok), _ptr(status), _ptr(ki)),
+                    "bjj_verify_keyset_lookup_compressed_batch")
+        return ok, status, ki
+
     # verify_schnorr with s as sign_schnorr_batch writes it: a uint8 array (n, 4 * words), little-endian and unreduced,
     # words a multiple of 8 in [8, 72]; each returns (ok, status), both (n,) uint8, status 4 where msg > Q
     def _schnorr_call(self, name, head, msg, rx, ry, s, words):
@@ -460,6 +485,29 @@ class KeySet:
         and sign"""
         rx, ry = self.engine.keyset_mul_batch(self, key_index, ints_to_le32([_base_scalar(k) for k in scalars]))
         return [Point(x, y) for x, y in zip(le32_to_ints(rx), le32_to_ints(ry))]
+
+    def lookup(self, pks):
+        """the index of each key (a Point or its 32 compressed bytes) in the set, the smallest if the set holds it twice,
+        or None.  Keys with x = 0 are never found: decompress_point rejects their compressed forms."""
+        ki = self.engine.keyset_lookup_batch(self, _pk32s(pks))
+        return [None if k == KEY_NONE else int(k) for k in ki]
+
+
+def _pk32s(pks):
+    """Points or 32-byte compressed keys -> uint8 array (n, 32); a Point is compressed on the host (Point::compress)"""
+    out = []
+    for p in pks:
+        if isinstance(p, Point):
+            b = bytearray(p.y.to_bytes(32, "little"))
+            if p.x > Q >> 1:
+                b[31] |= 0x80
+            out.append(bytes(b))
+        else:
+            b = bytes(p)
+            if len(b) != 32:
+                raise ValueError("a compressed key is 32 bytes, got %d" % len(b))
+            out.append(b)
+    return np.frombuffer(b"".join(out), dtype=np.uint8).reshape(-1, 32).copy()
 
 
 def _keyset_handle(keyset):
@@ -830,6 +878,20 @@ def verify_keyset_batch(keyset, key_index, sigs, msgs, engine=None):
                                  ints_to_le32([s.r_b8.y for s in sigs]), ints_to_le32([_verify_scalar(s.s) for s in sigs]),
                                  _verify_msgs(msgs))
     return [bool(v) for v in ok]
+
+
+def verify_keyset_lookup_batch(keyset, pk32s, sig64s, msgs, engine=None):
+    """decompress_signature + decompress_point + verify (src/lib.rs:260-268, 192-224, 395-412) for 32-byte compressed
+    keys of `keyset`, found by their bytes on the device -> per lane True / False, ValueError(<the reference's Err
+    string>) when R8 does not decompress, else None when the key is not in the set"""
+    if not (len(pk32s) == len(sig64s) == len(msgs)):
+        raise ValueError("pk32s, sig64s and msgs differ in length")
+    if any(len(bytes(s)) != 64 for s in sig64s):
+        raise ValueError("a compressed signature is 64 bytes")
+    eng = engine or keyset.engine
+    sg = np.frombuffer(b"".join(bytes(s) for s in sig64s), dtype=np.uint8).reshape(-1, 64)
+    ok, st, ki = eng.verify_keyset_lookup_compressed_batch(keyset, sg, _pk32s(pk32s), _verify_msgs(msgs))
+    return [ValueError(STATUS_STRINGS[int(s)]) if s else None if k == KEY_NONE else bool(o) for o, s, k in zip(ok, st, ki)]
 
 
 def _schnorr_sigs(msgs, sigs):

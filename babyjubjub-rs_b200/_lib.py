@@ -58,6 +58,8 @@ SIGNATURES = {
     "bjj_verify_keyset_batch": (_int, [_ctx, _keyset, _sz] + [_u8p] * 6),
     "bjj_verify_keyset_compressed_batch": (_int, [_ctx, _keyset, _sz] + [_u8p] * 5),
     "bjj_keyset_mul_batch": (_int, [_ctx, _keyset, _sz] + [_u8p] * 4),
+    "bjj_keyset_lookup_batch": (_int, [_ctx, _keyset, _sz] + [_u8p] * 2),
+    "bjj_verify_keyset_lookup_compressed_batch": (_int, [_ctx, _keyset, _sz] + [_u8p] * 6),
 }
 # every batch op also has a device-pointer flavour with a trailing `void* stream`
 for _name in [k for k in SIGNATURES if k.endswith("_batch")]:

@@ -9,6 +9,9 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <random>
+#include <vector>
+
 #include "../../include/bjj_cuda.h"
 #include "kernels.h"
 
@@ -135,6 +138,13 @@ __global__ void __launch_bounds__(BJJ_BLOCK, 2) k_keyset_mul(size_t n, const uin
     BJJ_FLAGS_END(gflags)
 }
 
+// the key of a key set whose compressed bytes are pk32[i], or BJJ_KEY_NONE (bjj_keyset_lookup)
+__global__ void __launch_bounds__(BJJ_BLOCK) k_keyset_lookup(size_t n, const uint8_t* pk32, const uint8_t* comp, const uint32_t* slots,
+                                                             uint64_t mask, uint64_t seed, uint32_t* key_index,
+                                                             unsigned long long* work) {
+    BJJ_POINT_LOOP(n, work) lane_keyset_lookup(pk32, comp, slots, mask, seed, key_index, i);
+}
+
 #ifndef BJJ_PUBLIC_BALLAST
 #define BJJ_PUBLIC_BALLAST 1
 #endif
@@ -240,13 +250,22 @@ struct bjj_base {
 };
 
 // N keys with their compact combs (bjj_keyset_create), on the device of the context that built them: `keys` holds the
-// x plane then the y plane (Montgomery form, 32 B per key each), `tables` the N Comb8 tables
+// x plane then the y plane (Montgomery form, 32 B per key each), `tables` the N Comb8 tables.  `index` is the lookup by
+// compressed bytes (lanes.cuh: keyset_index_build): compress(P_j) (32 B per key), then `slot_mask` + 1 uint32 slots,
+// then one flags word that the lookup verify passes to its kernels instead of the context's (nobody reads it).
 struct bjj_keyset {
     bjj_ctx* ctx;
     size_t n_keys;
     uint8_t* keys;
     CombEntry* tables;
+    uint8_t* index;
+    uint64_t slot_mask;
+    uint64_t seed;
 };
+
+static const uint8_t* keyset_comp(const bjj_keyset* ks) { return ks->index; }
+static const uint32_t* keyset_slots(const bjj_keyset* ks) { return (const uint32_t*)(ks->index + 32 * ks->n_keys); }
+static uint32_t* keyset_quiet_flags(const bjj_keyset* ks) { return (uint32_t*)(ks->index + 32 * ks->n_keys) + ks->slot_mask + 1; }
 
 #define CU(ctx, call)                      \
     do {                                   \
@@ -621,6 +640,7 @@ static int dev_alloc(void** p, size_t bytes) {
 static void keyset_free(bjj_keyset* ks) {
     if (ks->keys) cudaFree(ks->keys);
     if (ks->tables) cudaFree(ks->tables);
+    if (ks->index) cudaFree(ks->index);
     free(ks);
 }
 
@@ -653,6 +673,15 @@ int bjj_keyset_create(bjj_ctx* ctx, size_t n_keys, const uint8_t* ax, const uint
         }
         if (off) return BJJ_ERR_ARG;
         TRY(dev_alloc((void**)&ks->tables, n_keys * BJJ_KEY_COMB_TOTAL * sizeof(CombEntry)));
+        // the index by compressed bytes, built here from the caller's coordinates and uploaded before the final
+        // synchronise; its flags word starts at 0
+        const size_t slots = keyset_index_slots(n_keys), index_bytes = 32 * n_keys + 4 * slots + 4;
+        std::vector<uint8_t> index(index_bytes, 0);
+        ks->slot_mask = slots - 1;
+        ks->seed = (uint64_t)std::random_device{}() << 32 ^ std::random_device{}();
+        keyset_index_build(n_keys, ax, ay, ks->seed, index.data(), (uint32_t*)(index.data() + 32 * n_keys));
+        TRY(dev_alloc((void**)&ks->index, index_bytes));
+        CU(ctx, cudaMemcpyAsync(ks->index, index.data(), index_bytes, cudaMemcpyHostToDevice, st));
         // the build borrows the context's projective scratch, which a _dev call on another stream may still use
         CU(ctx, cudaDeviceSynchronize());
         for (size_t k0 = 0; k0 < n_keys; k0 += BJJ_KEYSET_SUBBATCH) {
@@ -848,6 +877,22 @@ static int launch_decompress(bjj_ctx* ctx, size_t n, const uint8_t* in32, uint8_
     });
 }
 
+// key_index[i] of the key of ks whose compressed bytes are pk32[i], or BJJ_KEY_NONE, for m <= BJJ_POINT_SUBBATCH lanes
+static int lookup_subbatch(bjj_ctx* ctx, const bjj_keyset* ks, size_t m, const uint8_t* pk32, uint32_t* key_index, cudaStream_t st,
+                           Workspace* ws) {
+    unsigned long long* work = nullptr;
+    TRY(claim_counter(ctx, ws, st, &work));
+    k_keyset_lookup<<<grid_for(ctx, k_keyset_lookup, m), BJJ_BLOCK, 0, st>>>(m, pk32, keyset_comp(ks), keyset_slots(ks), ks->slot_mask,
+                                                                            ks->seed, key_index, work);
+    return launched(ctx);
+}
+static int launch_keyset_lookup(bjj_ctx* ctx, const bjj_keyset* ks, size_t n, const uint8_t* pk32, uint32_t* key_index, cudaStream_t st,
+                                Workspace* ws) {
+    return for_each_subbatch(n, [&](size_t off, size_t m) -> int {
+        return lookup_subbatch(ctx, ks, m, pk32 + 32 * off, key_index + off, st, ws);
+    });
+}
+
 // verify scratch: four planes hm | u | v | w (32 B / lane each; u, v, w are the Straus scalars, see split.cuh)
 // and, for the compressed pipeline, the four decompressed coordinates
 static int ensure_vscratch(bjj_ctx* ctx, Workspace* ws, size_t lanes, uint8_t** hm, uint8_t** pts) {
@@ -981,10 +1026,15 @@ static int launch_verify_compressed(bjj_ctx* ctx, size_t n, const uint8_t* sig64
 // `base` (bjj_verify_keyset*), lane i takes key key_index[i] of the set and its compact table: the kernels
 // k_verify_keyset_hash -> k_verify_keyset_ec, with the same launches.  s_words != 0 is verify_schnorr
 // (bjj_verify_schnorr_base* / _keyset*): r8x, r8y hold r, s32 the signer's s of s_words words per lane, `status` receives
-// the msg status, and phase 1 reduces s into the u plane of the verify scratch, which phase 2 reads.
+// the msg status, and phase 1 reduces s into the u plane of the verify scratch, which phase 2 reads.  pk32 != nullptr
+// (bjj_verify_keyset_lookup_compressed*, with sig64 and ks): after R8's decompression k_keyset_lookup writes the key of
+// each lane's compressed key into `found`, which the caller also passes as key_index.  The key-set kernels then raise
+// BJJ_FLAG_KEY_INDEX for BJJ_KEY_NONE lanes into the set's own flags word, which nobody reports, instead of the
+// context's: an unknown key is data there.  (R8 comes out of decompression canonical, so no other bit can go there.)
 static int launch_verify_base(bjj_ctx* ctx, const bjj_base* base, const bjj_keyset* ks, const uint8_t* key_index, size_t n,
                               const uint8_t* r8x, const uint8_t* r8y, const uint8_t* s32, const uint8_t* sig64, const uint8_t* msg,
-                              uint8_t* ok, uint8_t* status, cudaStream_t st, Workspace* ws, int s_words = 0) {
+                              uint8_t* ok, uint8_t* status, cudaStream_t st, Workspace* ws, int s_words = 0,
+                              const uint8_t* pk32 = nullptr, uint32_t* found = nullptr) {
     const size_t lanes = scratch_lanes(ctx, n);
     return for_each_subbatch(n, [&](size_t off, size_t m) -> int {
         const size_t o = 32 * off;
@@ -1016,6 +1066,7 @@ static int launch_verify_base(bjj_ctx* ctx, const bjj_base* base, const bjj_keys
             s_off = 1;
             skip = status + off;
         }
+        if (pk32) TRY(lookup_subbatch(ctx, ks, m, pk32 + o, found + off, st, ws));
         unsigned long long *work_h = nullptr, *work_e = nullptr;
         TRY(claim_counter(ctx, ws, st, &work_h));
         TRY(claim_counter(ctx, ws, st, &work_e));
@@ -1043,7 +1094,7 @@ static int launch_verify_base(bjj_ctx* ctx, const bjj_base* base, const bjj_keys
             const uint8_t *ki = key_index + 4 * off, *kx = ks->keys, *ky = kx + 32 * ks->n_keys;
             const uint32_t nk = (uint32_t)ks->n_keys;
             bjjk::verify_keyset_hash(grid_cap(ctx, bjjk::verify_keyset_hash_blocks_per_sm(), m), st, m, rx, ry, ki, kx, ky, nk, msg + o,
-                                     skip, hm, ok + off, ctx->flags_dev, work_h);
+                                     skip, hm, ok + off, pk32 ? keyset_quiet_flags(ks) : ctx->flags_dev, work_h);
             TRY(launched(ctx));
             bjjk::verify_keyset_ec(grid_cap(ctx, bjjk::verify_keyset_ec_blocks_per_sm(), m), st, m, rx, ry, sb, s_stride, s_off, hm,
                                    ok + off, ctx->comb, ki, nk, ks->tables, work_e);
@@ -1351,6 +1402,22 @@ int bjj_keyset_mul_batch_dev(bjj_ctx* ctx, const bjj_keyset* ks, size_t n, const
     DEV_PROLOGUE
     if (!key_index || !scalar32 || !rx || !ry) return BJJ_ERR_ARG;
     return launch_keyset_mul(ctx, ks, n, (const uint8_t*)key_index, scalar32, rx, ry, st, &ctx->ws);
+}
+
+int bjj_keyset_lookup_batch_dev(bjj_ctx* ctx, const bjj_keyset* ks, size_t n, const uint8_t* pk32, uint32_t* key_index, void* stream) {
+    if (!keyset_of(ctx, ks)) return BJJ_ERR_ARG;
+    DEV_PROLOGUE
+    if (!pk32 || !key_index) return BJJ_ERR_ARG;
+    return launch_keyset_lookup(ctx, ks, n, pk32, key_index, st, &ctx->ws);
+}
+
+int bjj_verify_keyset_lookup_compressed_batch_dev(bjj_ctx* ctx, const bjj_keyset* ks, size_t n, const uint8_t* sig64, const uint8_t* pk32,
+                                                  const uint8_t* msg32, uint8_t* ok, uint8_t* status, uint32_t* key_index, void* stream) {
+    if (!keyset_of(ctx, ks)) return BJJ_ERR_ARG;
+    DEV_PROLOGUE
+    if (!sig64 || !pk32 || !msg32 || !ok || !status || !key_index) return BJJ_ERR_ARG;
+    return launch_verify_base(ctx, nullptr, ks, (const uint8_t*)key_index, n, nullptr, nullptr, nullptr, sig64, msg32, ok, status, st,
+                              &ctx->ws, 0, pk32, key_index);
 }
 
 int bjj_verify_schnorr_base_batch_dev(bjj_ctx* ctx, const bjj_base* pk, size_t n, const uint8_t* msg32, const uint8_t* rx,
@@ -1803,6 +1870,24 @@ int bjj_keyset_mul_batch(bjj_ctx* ctx, const bjj_keyset* ks, size_t n, const uin
     HostArg args[] = {H_IN((const uint8_t*)key_index, 4), H_IN(scalar32, 32), H_OUT(rx, 32), H_OUT(ry, 32)};
     return run_host(ctx, n, args, 4, [&](size_t m, uint8_t** d, cudaStream_t st, Workspace* ws) -> int {
         return launch_keyset_mul(ctx, ks, m, d[0], d[1], d[2], d[3], st, ws);
+    }, /*heavy=*/true);
+}
+
+int bjj_keyset_lookup_batch(bjj_ctx* ctx, const bjj_keyset* ks, size_t n, const uint8_t* pk32, uint32_t* key_index) {
+    if (!keyset_of(ctx, ks)) return BJJ_ERR_ARG;
+    HostArg args[] = {H_IN(pk32, 32), H_OUT((uint8_t*)key_index, 4)};
+    return run_host(ctx, n, args, 2, [&](size_t m, uint8_t** d, cudaStream_t st, Workspace* ws) -> int {
+        return launch_keyset_lookup(ctx, ks, m, d[0], (uint32_t*)d[1], st, ws);
+    });
+}
+
+int bjj_verify_keyset_lookup_compressed_batch(bjj_ctx* ctx, const bjj_keyset* ks, size_t n, const uint8_t* sig64, const uint8_t* pk32,
+                                              const uint8_t* msg32, uint8_t* ok, uint8_t* status, uint32_t* key_index) {
+    if (!keyset_of(ctx, ks)) return BJJ_ERR_ARG;
+    HostArg args[] = {H_IN(sig64, 64), H_IN(pk32, 32), H_IN(msg32, 32), H_OUT(ok, 1), H_OUT(status, 1), H_OUT((uint8_t*)key_index, 4)};
+    return run_host(ctx, n, args, 6, [&](size_t m, uint8_t** d, cudaStream_t st, Workspace* ws) -> int {
+        return launch_verify_base(ctx, nullptr, ks, d[5], m, nullptr, nullptr, nullptr, d[0], d[2], d[3], d[4], st, ws, 0, d[1],
+                                  (uint32_t*)d[5]);
     }, /*heavy=*/true);
 }
 

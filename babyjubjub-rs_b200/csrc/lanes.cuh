@@ -1836,4 +1836,84 @@ BJJ_HD void lane_keyset_mul(const uint8_t* scalar, const uint8_t* key_index, uin
     store_ext_scratch(scr, i, acc);
 }
 
+// ---- key lookup by compressed bytes (bjj_keyset_lookup, bjj_verify_keyset_lookup_compressed) ----------------------------
+// bjj_keyset_create indexes the keys of a set by compress(P) (src/lib.rs:166-178: y little-endian, bit 255 = x > (Q-1)/2)
+// in an open-addressing table of uint32 key indices: a power of two of slots >= 2 N, BJJ_KEY_NONE in an empty slot,
+// linear probing.  The load factor stays <= 1/2, so every probe ends at an empty slot.  Keys go in in index order, so a
+// point held twice is found under its smallest index.  Keys with x = 0, (0, 1) and (0, Q-1), stay out: decompress_point
+// rejects their compressed forms (modsqrt of 0, src/utils.rs:118), so no compressed key of a verify can name them.
+// The hash is keyed with a 64-bit seed drawn per set: key owners choose their keys, and with a public hash they could
+// grind keys into one probe chain.  The seed moves keys between slots; it never changes a result.
+#define BJJ_KEY_NONE 0xFFFFFFFFu
+
+// the slot hash of 32 compressed bytes (8 little-endian words): each 64-bit word through splitmix64's finaliser, chained
+BJJ_HD uint64_t keyset_hash(const uint32_t* w, uint64_t seed) {
+    uint64_t h = seed;
+#pragma unroll
+    for (int k = 0; k < 4; k++) {
+        h ^= (uint64_t)w[2 * k] | (uint64_t)w[2 * k + 1] << 32;
+        h = (h ^ (h >> 30)) * 0xBF58476D1CE4E5B9ull;
+        h = (h ^ (h >> 27)) * 0x94D049BB133111EBull;
+        h ^= h >> 31;
+    }
+    return h;
+}
+
+// slots of the index of n keys: the smallest power of two >= 2 n
+inline size_t keyset_index_slots(size_t n) {
+    size_t c = 2;
+    while (c < 2 * n) c <<= 1;
+    return c;
+}
+
+// The index of n keys with canonical affine coordinates ax, ay (32 B per key, on the host): comp receives compress(P_j)
+// (32 B per key), slots the keyset_index_slots(n) table.
+inline void keyset_index_build(size_t n, const uint8_t* ax, const uint8_t* ay, uint64_t seed, uint8_t* comp, uint32_t* slots) {
+    const size_t mask = keyset_index_slots(n) - 1;
+    for (size_t s = 0; s <= mask; s++) slots[s] = BJJ_KEY_NONE;
+    const uint32_t q[8] = BJJ_LIMBS8(BJJ_Q);
+    for (size_t j = 0; j < n; j++) {
+        uint32_t x[8], y[8], x2[8];
+        memcpy(x, ax + 32 * j, 32);
+        memcpy(y, ay + 32 * j, 32);
+        // x > (Q-1)/2 <=> 2x >= Q (x < Q < 2^254, so 2x fits)
+        uint32_t any = 0;
+        for (int k = 0; k < 8; k++) {
+            x2[k] = x[k] << 1 | (k ? x[k - 1] >> 31 : 0);
+            any |= x[k];
+        }
+        if (!u256_lt(x2, q)) y[7] |= 0x80000000u;
+        memcpy(comp + 32 * j, y, 32);
+        if (!any) continue;
+        size_t s = keyset_hash(y, seed) & mask;
+        while (slots[s] != BJJ_KEY_NONE && memcmp(comp + 32 * (size_t)slots[s], y, 32) != 0) s = (s + 1) & mask;
+        if (slots[s] == BJJ_KEY_NONE) slots[s] = (uint32_t)j;
+    }
+}
+
+// key_index[i] = the key whose compressed bytes equal pk32[i], or BJJ_KEY_NONE: hash, then probe linearly to an empty
+// slot, comparing all 32 bytes with the stored compressed key (mask = slots - 1)
+BJJ_HD void lane_keyset_lookup(const uint8_t* pk32, const uint8_t* comp, const uint32_t* slots, uint64_t mask, uint64_t seed,
+                               uint32_t* key_index, size_t i) {
+    uint32_t b[8];
+    load_u256(b, pk32, i);
+    uint64_t s = keyset_hash(b, seed) & mask;
+    uint32_t k;
+#pragma unroll 1
+    for (;; s = (s + 1) & mask) {
+#if BJJ_DEVICE_CODE
+        k = __ldg(slots + s);
+#else
+        k = slots[s];
+#endif
+        if (k == BJJ_KEY_NONE) break;
+        uint32_t c[8], diff = 0;
+        load_u256(c, comp, k);
+#pragma unroll
+        for (int w = 0; w < 8; w++) diff |= c[w] ^ b[w];
+        if (!diff) break;
+    }
+    key_index[i] = k;
+}
+
 }  // namespace bjj

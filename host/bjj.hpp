@@ -17,7 +17,8 @@
 //     signer's unreduced s, reduced on the device; FixedBase / KeySet members on the comb path)
 //   + FixedBase: the comb table of a caller-chosen point, k*P and k*P + l*Q at the fixed-base rate, and verify for
 //     many signatures of that one key
-//   + KeySet: many known keys with compact comb tables, verify and k*P with a key index per lane
+//   + KeySet: many known keys with compact comb tables, verify and k*P with a key index per lane, and the lookup of
+//     keys by their compressed bytes (verify_compressed_by_key)
 //   + MultiGpu: shards a batch over every device, one host thread + one bjj_ctx per device, no NCCL
 //
 // Header-only; link with -lbjj_cuda.  There is no CPU fallback: Engine's constructor throws when no
@@ -490,6 +491,37 @@ class KeySet {
                       "bjj_verify_schnorr_keyset_batch");
         if (status) *status = l.status;
         return l.ok;
+    }
+    // the index of each 32-byte compressed key in the set (the smallest if the set holds the point twice), or BJJ_KEY_NONE
+    std::vector<uint32_t> lookup(const std::vector<std::array<uint8_t, 32>>& pks) const {
+        const size_t n = pks.size();
+        std::vector<uint8_t> pk(32 * n);
+        for (size_t i = 0; i < n; i++) std::memcpy(&pk[32 * i], pks[i].data(), 32);
+        std::vector<uint32_t> ki(n);
+        Engine::check(bjj_keyset_lookup_batch(e_.ctx(), ks_, n, pk.data(), ki.data()), "bjj_keyset_lookup_batch");
+        return ki;
+    }
+    // verify_compressed_batch's arrays for keys of the set found by their compressed bytes: ok, R8's decompression status
+    // and the key index per lane (BJJ_KEY_NONE and ok = 0 for a key outside the set)
+    std::vector<uint8_t> verify_compressed_by_key(const std::vector<std::array<uint8_t, 32>>& pks,
+                                                  const std::vector<std::array<uint8_t, 64>>& sigs, const std::vector<U256>& msgs,
+                                                  std::vector<uint8_t>* status = nullptr,
+                                                  std::vector<uint32_t>* key_index = nullptr) const {
+        if (sigs.size() != msgs.size() || sigs.size() != pks.size()) throw std::invalid_argument("pks, sigs and msgs differ in length");
+        const size_t n = sigs.size();
+        std::vector<uint8_t> sg(64 * n), pk(32 * n), ok(n), st(n);
+        std::vector<uint32_t> ki(n);
+        for (size_t i = 0; i < n; i++) {
+            std::memcpy(&sg[64 * i], sigs[i].data(), 64);
+            std::memcpy(&pk[32 * i], pks[i].data(), 32);
+        }
+        auto m = pack(msgs);
+        Engine::check(bjj_verify_keyset_lookup_compressed_batch(e_.ctx(), ks_, n, sg.data(), pk.data(), m.data(), ok.data(), st.data(),
+                                                                ki.data()),
+                      "bjj_verify_keyset_lookup_compressed_batch");
+        if (status) *status = st;
+        if (key_index) *key_index = ki;
+        return ok;
     }
     // [keys[key_index[i]].mul_scalar(k[i])]; scalars are raw 256-bit values (reduce wider ones mod ORDER)
     std::vector<Point> mul_batch(const std::vector<uint32_t>& key_index, const std::vector<U256>& scalars) const {

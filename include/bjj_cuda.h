@@ -216,6 +216,32 @@ int bjj_keyset_mul_batch(bjj_ctx* ctx, const bjj_keyset* ks, size_t n, const uin
                          uint8_t* rx, uint8_t* ry);
 int bjj_keyset_mul_batch_dev(bjj_ctx* ctx, const bjj_keyset* ks, size_t n, const uint32_t* key_index, const uint8_t* scalar32,
                              uint8_t* rx, uint8_t* ry, void* stream);
+/* Keys by their compressed bytes.  bjj_keyset_create also indexes the set by compress(P_j) (src/lib.rs:166-178), on the
+ * host: 32 B plus at most 16 B of device memory per key, freed by bjj_keyset_destroy.  The index's hash is keyed with a
+ * seed drawn per set, so chosen keys cannot crowd one probe chain; results do not depend on it.
+ *   - bjj_keyset_lookup_batch: key_index[i] = the index j of the key with compress(P_j) == pk32[i], the smallest such j
+ *     if the set holds a point twice, else BJJ_KEY_NONE.  A miss is data, not an error.  P and -P (same y, bit 255
+ *     apart) are each found under their own index.  The keys with x = 0, (0, 1) and (0, Q-1), are not indexed and come
+ *     back BJJ_KEY_NONE: decompress_point rejects their compressed forms (src/utils.rs:118), so no lane of
+ *     bjj_verify_compressed_batch verifies against them.  One kernel launch per sub-batch of 2^21 lanes.
+ *   - bjj_verify_keyset_lookup_compressed_batch: decompress_signature + decompress_point(pk) + verify (src/lib.rs:260-268,
+ *     192-224, 395-412) for keys of ks found by their compressed bytes; the same arrays as bjj_verify_compressed_batch,
+ *     and key_index receives the lookup above.  A found lane's ok[i] and status[i] are byte for byte those of
+ *     bjj_verify_compressed_batch on the same (sig64, pk32, msg32).  Any other lane gets ok[i] = 0, status[i] = R8's
+ *     decompression status and key_index[i] = BJJ_KEY_NONE, with no error code from the call or from the next
+ *     bjj_sync.  Six kernel launches per sub-batch: R8's decompression (3), the lookup, then the two kernels of
+ *     bjj_verify_keyset_compressed_batch.
+ * A NULL pointer, a NULL handle or a handle of another context returns BJJ_ERR_ARG; n == 0 is a no-op. */
+#define BJJ_KEY_NONE 0xFFFFFFFFu   /* key_index output of the lookup calls: no key of the set has these bytes */
+int bjj_keyset_lookup_batch(bjj_ctx* ctx, const bjj_keyset* ks, size_t n, const uint8_t* pk32, uint32_t* key_index);
+int bjj_keyset_lookup_batch_dev(bjj_ctx* ctx, const bjj_keyset* ks, size_t n, const uint8_t* pk32, uint32_t* key_index,
+                                void* stream);
+int bjj_verify_keyset_lookup_compressed_batch(bjj_ctx* ctx, const bjj_keyset* ks, size_t n, const uint8_t* sig64,
+                                              const uint8_t* pk32, const uint8_t* msg32, uint8_t* ok, uint8_t* status,
+                                              uint32_t* key_index);
+int bjj_verify_keyset_lookup_compressed_batch_dev(bjj_ctx* ctx, const bjj_keyset* ks, size_t n, const uint8_t* sig64,
+                                                  const uint8_t* pk32, const uint8_t* msg32, uint8_t* ok, uint8_t* status,
+                                                  uint32_t* key_index, void* stream);
 
 /* ---- PrivateKey::public (src/lib.rs:304-306) = B8 * scalar_key(key);  scalar_key (:284-302) ------ */
 int bjj_public_batch(bjj_ctx* ctx, size_t n, const uint8_t* key32, uint8_t* rx, uint8_t* ry);

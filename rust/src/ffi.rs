@@ -25,6 +25,7 @@ pub const BJJ_ERR_CUDA: c_int = 1;
 pub const BJJ_ERR_ARG: c_int = 2;
 pub const BJJ_ERR_NONCANONICAL: c_int = 3;
 pub const BJJ_ERR_NOMEM: c_int = 4;
+pub const BJJ_KEY_NONE: u32 = 0xFFFF_FFFF;
 
 extern "C" {
     pub fn bjj_device_count() -> c_int;
@@ -86,6 +87,11 @@ extern "C" {
                                               sig64: *const u8, msg32: *const u8, ok: *mut u8, status: *mut u8) -> c_int;
     pub fn bjj_keyset_mul_batch(ctx: *mut bjj_ctx, ks: *const bjj_keyset, n: usize, key_index: *const u32, scalar32: *const u8,
                                 rx: *mut u8, ry: *mut u8) -> c_int;
+    // keys of a set by their compressed bytes: key_index[i] = the key's index or BJJ_KEY_NONE (a miss is not an error)
+    pub fn bjj_keyset_lookup_batch(ctx: *mut bjj_ctx, ks: *const bjj_keyset, n: usize, pk32: *const u8, key_index: *mut u32) -> c_int;
+    pub fn bjj_verify_keyset_lookup_compressed_batch(ctx: *mut bjj_ctx, ks: *const bjj_keyset, n: usize, sig64: *const u8,
+                                                     pk32: *const u8, msg32: *const u8, ok: *mut u8, status: *mut u8,
+                                                     key_index: *mut u32) -> c_int;
     // PrivateKey::public / scalar_key / sign (src/lib.rs:284-342)
     pub fn bjj_public_batch(ctx: *mut bjj_ctx, n: usize, key32: *const u8, rx: *mut u8, ry: *mut u8) -> c_int;
     pub fn bjj_scalar_key_batch(ctx: *mut bjj_ctx, n: usize, key32: *const u8, scalar32: *mut u8) -> c_int;

@@ -508,6 +508,30 @@ impl KeySet {
                                                             ok.as_mut_ptr(), st.as_mut_ptr()) }, "bjj_verify_schnorr_keyset_batch");
         schnorr_results(&ok, &st)
     }
+    /// the index of each 32-byte compressed key in the set (the smallest if the set holds the point twice), or `None`
+    pub fn lookup(&self, pks: &[[u8; 32]]) -> Vec<Option<u32>> {
+        let n = pks.len();
+        let pk: Vec<u8> = pks.iter().flat_map(|p| p.iter().copied()).collect();
+        let mut ki = vec![0u32; n];
+        check(unsafe { ffi::bjj_keyset_lookup_batch(engine().raw(), self.ks, n, pk.as_ptr(), ki.as_mut_ptr()) }, "bjj_keyset_lookup_batch");
+        ki.into_iter().map(|k| if k == ffi::BJJ_KEY_NONE { None } else { Some(k) }).collect()
+    }
+    /// `verify_compressed_batch` for keys of the set found by their compressed bytes: `Err` carries R8's decompression
+    /// error, `Ok(None)` a key that is not in the set
+    pub fn verify_compressed_by_key(&self, pks: &[[u8; 32]], sigs: &[[u8; 64]], msgs: &[BigInt]) -> Vec<Result<Option<bool>, String>> {
+        let n = sigs.len();
+        assert_eq!(n, msgs.len());
+        assert_eq!(n, pks.len());
+        let sg: Vec<u8> = sigs.iter().flat_map(|s| s.iter().copied()).collect();
+        let pk: Vec<u8> = pks.iter().flat_map(|p| p.iter().copied()).collect();
+        let m = col(n, |i| msg_le32(&msgs[i]));
+        let (mut ok, mut st, mut ki) = (vec![0u8; n], vec![0u8; n], vec![0u32; n]);
+        check(unsafe { ffi::bjj_verify_keyset_lookup_compressed_batch(engine().raw(), self.ks, n, sg.as_ptr(), pk.as_ptr(), m.as_ptr(),
+                                                                      ok.as_mut_ptr(), st.as_mut_ptr(), ki.as_mut_ptr()) },
+              "bjj_verify_keyset_lookup_compressed_batch");
+        (0..n).map(|i| if st[i] != 0 { Err(status_str(st[i])) } else if ki[i] == ffi::BJJ_KEY_NONE { Ok(None) } else { Ok(Some(ok[i] == 1)) })
+              .collect()
+    }
     /// `[keys[key_index[i]].mul_scalar(k[i])]`
     pub fn mul_batch(&self, key_index: &[u32], scalars: &[BigInt]) -> Vec<Point> {
         let n = scalars.len();
