@@ -469,6 +469,38 @@ class KeySet:
     def __len__(self):
         return len(self.points)
 
+    def _edit(self, fn, name, head, points):
+        pts = [(p.x, p.y) if isinstance(p, Point) else tuple(p) for p in points]
+        ax, ay = ints_to_le32([p[0] for p in pts]), ints_to_le32([p[1] for p in pts])
+        status = np.zeros(len(pts), dtype=np.uint8)
+        rc = fn(self.engine.ctx, _keyset_handle(self), *head, len(pts), _ptr(ax), _ptr(ay), _ptr(status))
+        if rc != 0:
+            try:
+                self.engine._check(rc, name)
+            except BjjError as e:
+                e.key_status = status
+                raise
+        return [Point(x, y) for x, y in pts], status
+
+    def append(self, points):
+        """adds keys under the indices len(self) ..; existing indices keep their keys, and `points` and `status` grow
+        with the new keys.  Raises BjjError with create's codes and `key_status` (one code per new key) on the
+        exception; the set, `points` and `status` then stay as they were."""
+        new, st = self._edit(self.engine.lib.bjj_keyset_append, "bjj_keyset_append", (), points)
+        self.points += new
+        self.status = np.concatenate([self.status, st])
+
+    def replace(self, first, points):
+        """gives keys first .. first + len(points) - 1 new coordinates (key rotation), in `points` and `status` too.
+        Raises BjjError with create's codes and `key_status` on the exception, or code 2 (BJJ_ERR_ARG) when the range
+        runs past the set; the set, `points` and `status` then stay as they were."""
+        first = int(first)
+        if first < 0:
+            raise ValueError("first must be >= 0")
+        new, st = self._edit(self.engine.lib.bjj_keyset_replace, "bjj_keyset_replace", (first,), points)
+        self.points[first:first + len(new)] = new
+        self.status[first:first + len(new)] = st
+
     def close(self):
         if getattr(self, "handle", None):
             self.engine.lib.bjj_keyset_destroy(self.engine.ctx, self.handle)

@@ -55,6 +55,8 @@ SIGNATURES = {
     "bjj_verify_base_compressed_batch": (_int, [_ctx, _base, _sz] + [_u8p] * 4),
     "bjj_keyset_create": (_int, [_ctx, _sz, _u8p, _u8p, _u8p, ctypes.POINTER(_keyset)]),
     "bjj_keyset_destroy": (None, [_ctx, _keyset]),
+    "bjj_keyset_append": (_int, [_ctx, _keyset, _sz, _u8p, _u8p, _u8p]),
+    "bjj_keyset_replace": (_int, [_ctx, _keyset, _sz, _sz, _u8p, _u8p, _u8p]),
     "bjj_verify_keyset_batch": (_int, [_ctx, _keyset, _sz] + [_u8p] * 6),
     "bjj_verify_keyset_compressed_batch": (_int, [_ctx, _keyset, _sz] + [_u8p] * 5),
     "bjj_keyset_mul_batch": (_int, [_ctx, _keyset, _sz] + [_u8p] * 4),

@@ -5,11 +5,14 @@
 // bound by the integer-multiply (fma) pipe, not by HBM: a lane reads <= 192 B and executes ~10^5-10^6
 // instructions.  Loads are two 16-byte vector loads per 32-byte element (1 KiB contiguous per warp).
 #include <cuda_runtime.h>
+#include <cudaTypedefs.h>   // PFN_cuMem*: the key-set tables' virtual memory calls, looked up at run time (libcuda is not linked)
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
 
+#include <new>
 #include <random>
+#include <utility>
 #include <vector>
 
 #include "../../include/bjj_cuda.h"
@@ -253,19 +256,28 @@ struct bjj_base {
 // x plane then the y plane (Montgomery form, 32 B per key each), `tables` the N Comb8 tables.  `index` is the lookup by
 // compressed bytes (lanes.cuh: keyset_index_build): compress(P_j) (32 B per key), then `slot_mask` + 1 uint32 slots,
 // then one flags word that the lookup verify passes to its kernels instead of the context's (nobody reads it).
+// The tables grow in place (bjj_keyset_append): `tables` is the start of a reserved virtual range of `va_bytes`, room
+// for the most keys the device's memory could hold, of which the first `mapped` bytes (a multiple of `gran`) are backed
+// by the physical allocations `maps` (offset, bytes), one per call that grew the set.  `comp` is a host copy of the
+// compressed keys, from which an edit rebuilds the slots.
 struct bjj_keyset {
-    bjj_ctx* ctx;
-    size_t n_keys;
-    uint8_t* keys;
-    CombEntry* tables;
-    uint8_t* index;
-    uint64_t slot_mask;
-    uint64_t seed;
+    bjj_ctx* ctx = nullptr;
+    size_t n_keys = 0;
+    uint8_t* keys = nullptr;
+    CombEntry* tables = nullptr;
+    uint8_t* index = nullptr;
+    uint64_t slot_mask = 0;
+    uint64_t seed = 0;
+    size_t va_bytes = 0, mapped = 0, gran = 0;
+    std::vector<std::pair<size_t, size_t>> maps;
+    std::vector<uint8_t> comp;
 };
 
 static const uint8_t* keyset_comp(const bjj_keyset* ks) { return ks->index; }
 static const uint32_t* keyset_slots(const bjj_keyset* ks) { return (const uint32_t*)(ks->index + 32 * ks->n_keys); }
 static uint32_t* keyset_quiet_flags(const bjj_keyset* ks) { return (uint32_t*)(ks->index + 32 * ks->n_keys) + ks->slot_mask + 1; }
+// a key-set call names its set: NULL or a handle of another context is an argument error
+static bool keyset_of(bjj_ctx* ctx, const bjj_keyset* ks) { return ks && ks->ctx == ctx; }
 
 #define CU(ctx, call)                      \
     do {                                   \
@@ -625,8 +637,9 @@ void bjj_base_destroy(bjj_ctx* ctx, bjj_base* base) {
     free(base);
 }
 
-// keys per build sub-batch of bjj_keyset_create: their build lanes fit the point kernels' sub-batch of scratch
+// keys per build sub-batch of the key-set build: their build lanes fit the point kernels' sub-batch of scratch
 #define BJJ_KEYSET_SUBBATCH (BJJ_POINT_SUBBATCH / BJJ_KEY_BUILD_POINTS)
+#define BJJ_KEY_TABLE_BYTES ((size_t)BJJ_KEY_COMB_TOTAL * sizeof(CombEntry))
 
 // cudaMalloc that reports a failure as BJJ_ERR_NOMEM with the CUDA error cleared: the tables of a large key set may
 // simply not fit
@@ -637,11 +650,235 @@ static int dev_alloc(void** p, size_t bytes) {
     return BJJ_ERR_NOMEM;
 }
 
+// The driver's virtual memory management, resolved once through the runtime so that libbjj_cuda.so loads where there
+// is no driver.  `ok` is false when an entry point is missing.
+struct VmmApi {
+    PFN_cuMemGetAllocationGranularity granularity;
+    PFN_cuMemAddressReserve reserve;
+    PFN_cuMemAddressFree address_free;
+    PFN_cuMemCreate create;
+    PFN_cuMemRelease release;
+    PFN_cuMemMap map;
+    PFN_cuMemUnmap unmap;
+    PFN_cuMemSetAccess set_access;
+    bool ok;
+};
+static const VmmApi& vmm() {
+    static const VmmApi api = [] {
+        VmmApi a{};
+        auto get = [](const char* name, auto* fn) {
+            cudaDriverEntryPointQueryResult q = cudaDriverEntryPointSymbolNotFound;
+            return cudaGetDriverEntryPoint(name, (void**)fn, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess;
+        };
+        a.ok = get("cuMemGetAllocationGranularity", &a.granularity) && get("cuMemAddressReserve", &a.reserve) &&
+               get("cuMemAddressFree", &a.address_free) && get("cuMemCreate", &a.create) && get("cuMemRelease", &a.release) &&
+               get("cuMemMap", &a.map) && get("cuMemUnmap", &a.unmap) && get("cuMemSetAccess", &a.set_access);
+        cudaGetLastError();
+        return a;
+    }();
+    return api;
+}
+
+static CUmemAllocationProp device_alloc_prop(int device) {
+    CUmemAllocationProp prop = {};
+    prop.type = CU_MEM_ALLOCATION_TYPE_PINNED;
+    prop.location.type = CU_MEM_LOCATION_TYPE_DEVICE;
+    prop.location.id = device;
+    return prop;
+}
+
+// reserves ks's table range: (total device memory / 396,480 B) tables, rounded up to the allocation granularity.  No
+// set can hold more keys, so the range never has to move.
+static int tables_reserve(bjj_ctx* ctx, bjj_keyset* ks) {
+    const VmmApi& v = vmm();
+    if (!v.ok) {
+        ctx->last = cudaErrorNotSupported;
+        return BJJ_ERR_CUDA;
+    }
+    size_t free_b = 0, total_b = 0;
+    CU(ctx, cudaMemGetInfo(&free_b, &total_b));
+    const CUmemAllocationProp prop = device_alloc_prop(ctx->device);
+    if (v.granularity(&ks->gran, &prop, CU_MEM_ALLOC_GRANULARITY_MINIMUM) != CUDA_SUCCESS || !ks->gran) return BJJ_ERR_NOMEM;
+    const size_t bytes = total_b / BJJ_KEY_TABLE_BYTES * BJJ_KEY_TABLE_BYTES;
+    ks->va_bytes = (bytes + ks->gran - 1) / ks->gran * ks->gran;
+    CUdeviceptr va = 0;
+    if (v.reserve(&va, ks->va_bytes, 0, 0, 0) != CUDA_SUCCESS) {
+        ks->va_bytes = 0;
+        return BJJ_ERR_NOMEM;
+    }
+    ks->tables = (CombEntry*)va;
+    return BJJ_OK;
+}
+
+// unmaps the physical allocations maps[from..] (their memory is freed with the mapping: each handle was released once
+// mapped)
+static void tables_unmap_from(bjj_keyset* ks, size_t from) {
+    while (ks->maps.size() > from) {
+        const std::pair<size_t, size_t> m = ks->maps.back();
+        vmm().unmap((CUdeviceptr)ks->tables + m.first, m.second);
+        ks->mapped = m.first;
+        ks->maps.pop_back();
+    }
+}
+
+// backs the tables of n keys with physical memory: one more allocation after the mapped part (whose last granule the
+// previous keys may fill only partly).  Anything but success leaves the mapping as it was and returns BJJ_ERR_NOMEM.
+static int tables_grow(bjj_ctx* ctx, bjj_keyset* ks, size_t n) {
+    const VmmApi& v = vmm();
+    if (n > ks->va_bytes / BJJ_KEY_TABLE_BYTES) return BJJ_ERR_NOMEM;
+    const size_t need = (n * BJJ_KEY_TABLE_BYTES + ks->gran - 1) / ks->gran * ks->gran;
+    if (need <= ks->mapped) return BJJ_OK;
+    const size_t off = ks->mapped, bytes = need - off;
+    const CUdeviceptr at = (CUdeviceptr)ks->tables + off;
+    const CUmemAllocationProp prop = device_alloc_prop(ctx->device);
+    CUmemGenericAllocationHandle h;
+    if (v.create(&h, bytes, &prop, 0) != CUDA_SUCCESS) return BJJ_ERR_NOMEM;
+    const bool mapped = v.map(at, bytes, 0, h, 0) == CUDA_SUCCESS;
+    v.release(h);
+    if (!mapped) return BJJ_ERR_NOMEM;
+    CUmemAccessDesc acc = {};
+    acc.location = prop.location;
+    acc.flags = CU_MEM_ACCESS_FLAGS_PROT_READWRITE;
+    ks->maps.push_back({off, bytes});
+    ks->mapped = need;
+    if (v.set_access(at, bytes, &acc, 1) != CUDA_SUCCESS) {
+        tables_unmap_from(ks, ks->maps.size() - 1);
+        return BJJ_ERR_NOMEM;
+    }
+    return BJJ_OK;
+}
+
 static void keyset_free(bjj_keyset* ks) {
     if (ks->keys) cudaFree(ks->keys);
-    if (ks->tables) cudaFree(ks->tables);
     if (ks->index) cudaFree(ks->index);
-    free(ks);
+    if (ks->tables) {
+        tables_unmap_from(ks, 0);
+        vmm().address_free((CUdeviceptr)ks->tables, ks->va_bytes);
+    }
+    delete ks;
+}
+
+// uploads n keys (canonical SoA ax, ay) into `stage` (x plane, y plane, one status byte per key: 65 B per key), checks
+// them and rewrites them in Montgomery form (k_keyset_check, one launch).  key_status (may be NULL) receives one
+// BJJ_KEY_* code per key.  A coordinate >= Q outranks a key off the curve; the reference's product with an off-curve
+// key depends on its double-and-add order, which a comb does not follow, so such keys are refused as by bjj_base_create.
+static int keyset_check(bjj_ctx* ctx, size_t n, const uint8_t* ax, const uint8_t* ay, uint8_t* stage, uint8_t* key_status) {
+    uint8_t *kx = stage, *ky = kx + 32 * n, *st_dev = ky + 32 * n;
+    cudaStream_t st = ctx->stream;
+    uint8_t* status = (uint8_t*)malloc(n);
+    if (!status) return BJJ_ERR_NOMEM;
+    auto body = [&]() -> int {
+        CU(ctx, cudaMemcpyAsync(kx, ax, 32 * n, cudaMemcpyHostToDevice, st));
+        CU(ctx, cudaMemcpyAsync(ky, ay, 32 * n, cudaMemcpyHostToDevice, st));
+        k_keyset_check<<<grid_for(ctx, k_keyset_check, n), BJJ_BLOCK, 0, st>>>(n, kx, ky, st_dev);
+        TRY(launched(ctx));
+        CU(ctx, cudaMemcpyAsync(status, st_dev, n, cudaMemcpyDeviceToHost, st));
+        CU(ctx, cudaStreamSynchronize(st));
+        if (key_status) memcpy(key_status, status, n);
+        bool off = false;
+        for (size_t j = 0; j < n; j++) {
+            if (status[j] == BJJ_BASE_NONCANONICAL) return BJJ_ERR_NONCANONICAL;
+            off = off || status[j] != BJJ_BASE_OK;
+        }
+        return off ? BJJ_ERR_ARG : BJJ_OK;
+    };
+    const int rc = body();
+    free(status);
+    return rc;
+}
+
+// the comb tables of n keys (Montgomery planes kx, ky, 32 B per key) into tables, key after key: per sub-batch of
+// BJJ_KEYSET_SUBBATCH keys the window chains, then the batched affine pass (2 launches).  The build borrows the
+// context's projective scratch, so the caller has synchronised the device (and grown the scratch: keyset_edit).
+static int keyset_build_tables(bjj_ctx* ctx, size_t n, const uint8_t* kx, const uint8_t* ky, CombEntry* tables) {
+    cudaStream_t st = ctx->stream;
+    for (size_t k0 = 0; k0 < n; k0 += BJJ_KEYSET_SUBBATCH) {
+        const size_t keys = n - k0 < BJJ_KEYSET_SUBBATCH ? n - k0 : BJJ_KEYSET_SUBBATCH;
+        const size_t lanes = keys * BJJ_KEY_BUILD_POINTS;
+        ProjScratch scr;
+        TRY(ensure_proj(ctx, &ctx->ws, lanes, &scr));
+        CombEntry* tbl = tables + k0 * BJJ_KEY_COMB_TOTAL;
+        k_keyset_build<<<grid_for(ctx, k_keyset_build, keys * Comb8::WINDOWS), BJJ_BLOCK, 0, st>>>(keys, kx + 32 * k0, ky + 32 * k0,
+                                                                                                 scr, tbl);
+        k_keyset_affine<<<affine_grid(ctx, lanes), BJJ_BLOCK, 0, st>>>(lanes, scr, tbl);
+        TRY(launched(ctx, 2));
+    }
+    return BJJ_OK;
+}
+
+// keys first .. first + n - 1 of ks get the coordinates ax, ay (first == ks->n_keys appends them): create, append and
+// replace all come here.  Everything the edit allocates comes first and every check passes before the set changes; on
+// an error before that point the allocations are undone and the set is as it was.
+static int keyset_edit(bjj_ctx* ctx, bjj_keyset* ks, size_t first, size_t n, const uint8_t* ax, const uint8_t* ay,
+                       uint8_t* key_status) {
+    CU(ctx, cudaSetDevice(ctx->device));
+    // _dev calls on other streams may still read the planes, tables and index that this call changes or frees
+    CU(ctx, cudaDeviceSynchronize());
+    const size_t n0 = ks->n_keys, n1 = first + n > n0 ? first + n : n0;
+    const size_t maps0 = ks->maps.size();
+    cudaStream_t st = ctx->stream;
+    uint8_t *stage = nullptr, *keys = ks->keys, *index = nullptr;
+    std::vector<uint8_t> comp;
+    uint64_t slot_mask = 0;
+    auto body = [&]() -> int {
+        TRY(dev_alloc((void**)&stage, 65 * n));
+        TRY(keyset_check(ctx, n, ax, ay, stage, key_status));
+        // the index of the edited key list, rebuilt on the host from the compressed keys
+        comp.resize(32 * n1);
+        if (n0) memcpy(comp.data(), ks->comp.data(), 32 * n0);
+        for (size_t j = 0; j < n; j++) keyset_compress(ax, ay, j, comp.data() + 32 * (first + j));
+        const size_t slots = keyset_index_slots(n1), index_bytes = 32 * n1 + 4 * slots + 4;
+        std::vector<uint8_t> host_index(index_bytes, 0);
+        memcpy(host_index.data(), comp.data(), 32 * n1);
+        keyset_index_fill(n1, comp.data(), ks->seed, (uint32_t*)(host_index.data() + 32 * n1));
+        slot_mask = slots - 1;
+        TRY(dev_alloc((void**)&index, index_bytes));
+        if (n1 > n0) {
+            TRY(dev_alloc((void**)&keys, 64 * n1));
+            TRY(tables_grow(ctx, ks, n1));
+        }
+        // the build's projective scratch, grown here so that nothing after this point allocates
+        ProjScratch scr;
+        const int rc_scr = ensure_proj(ctx, &ctx->ws, (n < BJJ_KEYSET_SUBBATCH ? n : BJJ_KEYSET_SUBBATCH) * BJJ_KEY_BUILD_POINTS, &scr);
+        if (rc_scr != BJJ_OK) {
+            if (ctx->last != cudaErrorMemoryAllocation) return rc_scr;
+            cudaGetLastError();
+            return BJJ_ERR_NOMEM;
+        }
+        // from here on the set changes
+        uint8_t *kx = keys, *ky = keys + 32 * n1;
+        if (keys != ks->keys && n0) {
+            CU(ctx, cudaMemcpyAsync(kx, ks->keys, 32 * n0, cudaMemcpyDeviceToDevice, st));
+            CU(ctx, cudaMemcpyAsync(ky, ks->keys + 32 * n0, 32 * n0, cudaMemcpyDeviceToDevice, st));
+        }
+        CU(ctx, cudaMemcpyAsync(kx + 32 * first, stage, 32 * n, cudaMemcpyDeviceToDevice, st));
+        CU(ctx, cudaMemcpyAsync(ky + 32 * first, stage + 32 * n, 32 * n, cudaMemcpyDeviceToDevice, st));
+        CU(ctx, cudaMemcpyAsync(index, host_index.data(), index_bytes, cudaMemcpyHostToDevice, st));
+        TRY(keyset_build_tables(ctx, n, kx + 32 * first, ky + 32 * first, ks->tables + first * BJJ_KEY_COMB_TOTAL));
+        CU(ctx, cudaStreamSynchronize(st));
+        return BJJ_OK;
+    };
+    int rc;
+    try {
+        rc = body();
+    } catch (const std::bad_alloc&) {
+        rc = BJJ_ERR_NOMEM;
+    }
+    if (stage) cudaFree(stage);
+    if (rc != BJJ_OK) {
+        if (index) cudaFree(index);
+        if (keys != ks->keys) cudaFree(keys);
+        tables_unmap_from(ks, maps0);
+        return rc;
+    }
+    if (keys != ks->keys && ks->keys) cudaFree(ks->keys);
+    if (ks->index) cudaFree(ks->index);
+    ks->keys = keys;
+    ks->index = index;
+    ks->slot_mask = slot_mask;
+    ks->comp.swap(comp);
+    ks->n_keys = n1;
+    return BJJ_OK;
 }
 
 int bjj_keyset_create(bjj_ctx* ctx, size_t n_keys, const uint8_t* ax, const uint8_t* ay, uint8_t* key_status, bjj_keyset** out) {
@@ -649,65 +886,33 @@ int bjj_keyset_create(bjj_ctx* ctx, size_t n_keys, const uint8_t* ax, const uint
     *out = nullptr;
     if (!ctx || !ax || !ay || n_keys == 0 || n_keys > 0xFFFFFFFFull) return BJJ_ERR_ARG;
     CU(ctx, cudaSetDevice(ctx->device));
-    bjj_keyset* ks = (bjj_keyset*)calloc(1, sizeof(bjj_keyset));
-    uint8_t* status = (uint8_t*)malloc(n_keys);
-    int rc = ks && status ? BJJ_OK : BJJ_ERR_NOMEM;
-    // the key planes, then one status byte per key
-    if (rc == BJJ_OK) rc = dev_alloc((void**)&ks->keys, 65 * n_keys);
-    auto body = [&]() -> int {
-        uint8_t *kx = ks->keys, *ky = kx + 32 * n_keys, *st_dev = ky + 32 * n_keys;
-        cudaStream_t st = ctx->stream;
-        CU(ctx, cudaMemcpyAsync(kx, ax, 32 * n_keys, cudaMemcpyHostToDevice, st));
-        CU(ctx, cudaMemcpyAsync(ky, ay, 32 * n_keys, cudaMemcpyHostToDevice, st));
-        k_keyset_check<<<grid_for(ctx, k_keyset_check, n_keys), BJJ_BLOCK, 0, st>>>(n_keys, kx, ky, st_dev);
-        TRY(launched(ctx));
-        CU(ctx, cudaMemcpyAsync(status, st_dev, n_keys, cudaMemcpyDeviceToHost, st));
-        CU(ctx, cudaStreamSynchronize(st));
-        if (key_status) memcpy(key_status, status, n_keys);
-        // a coordinate >= Q outranks a key off the curve; the reference's product with an off-curve key depends on its
-        // double-and-add order, which a comb does not follow, so such keys are refused as by bjj_base_create
-        bool off = false;
-        for (size_t j = 0; j < n_keys; j++) {
-            if (status[j] == BJJ_BASE_NONCANONICAL) return BJJ_ERR_NONCANONICAL;
-            off = off || status[j] != BJJ_BASE_OK;
-        }
-        if (off) return BJJ_ERR_ARG;
-        TRY(dev_alloc((void**)&ks->tables, n_keys * BJJ_KEY_COMB_TOTAL * sizeof(CombEntry)));
-        // the index by compressed bytes, built here from the caller's coordinates and uploaded before the final
-        // synchronise; its flags word starts at 0
-        const size_t slots = keyset_index_slots(n_keys), index_bytes = 32 * n_keys + 4 * slots + 4;
-        std::vector<uint8_t> index(index_bytes, 0);
-        ks->slot_mask = slots - 1;
-        ks->seed = (uint64_t)std::random_device{}() << 32 ^ std::random_device{}();
-        keyset_index_build(n_keys, ax, ay, ks->seed, index.data(), (uint32_t*)(index.data() + 32 * n_keys));
-        TRY(dev_alloc((void**)&ks->index, index_bytes));
-        CU(ctx, cudaMemcpyAsync(ks->index, index.data(), index_bytes, cudaMemcpyHostToDevice, st));
-        // the build borrows the context's projective scratch, which a _dev call on another stream may still use
-        CU(ctx, cudaDeviceSynchronize());
-        for (size_t k0 = 0; k0 < n_keys; k0 += BJJ_KEYSET_SUBBATCH) {
-            const size_t keys = n_keys - k0 < BJJ_KEYSET_SUBBATCH ? n_keys - k0 : BJJ_KEYSET_SUBBATCH;
-            const size_t lanes = keys * BJJ_KEY_BUILD_POINTS;
-            ProjScratch scr;
-            TRY(ensure_proj(ctx, &ctx->ws, lanes, &scr));
-            CombEntry* tbl = ks->tables + k0 * BJJ_KEY_COMB_TOTAL;
-            k_keyset_build<<<grid_for(ctx, k_keyset_build, keys * Comb8::WINDOWS), BJJ_BLOCK, 0, st>>>(keys, kx + 32 * k0, ky + 32 * k0,
-                                                                                                     scr, tbl);
-            k_keyset_affine<<<affine_grid(ctx, lanes), BJJ_BLOCK, 0, st>>>(lanes, scr, tbl);
-            TRY(launched(ctx, 2));
-        }
-        CU(ctx, cudaStreamSynchronize(st));
-        return BJJ_OK;
-    };
-    if (rc == BJJ_OK) rc = body();
-    free(status);
+    bjj_keyset* ks = new (std::nothrow) bjj_keyset();
+    if (!ks) return BJJ_ERR_NOMEM;
+    ks->ctx = ctx;
+    ks->seed = (uint64_t)std::random_device{}() << 32 ^ std::random_device{}();
+    int rc = tables_reserve(ctx, ks);
+    if (rc == BJJ_OK) rc = keyset_edit(ctx, ks, 0, n_keys, ax, ay, key_status);
     if (rc != BJJ_OK) {
-        if (ks) keyset_free(ks);
+        keyset_free(ks);
         return rc;
     }
-    ks->ctx = ctx;
-    ks->n_keys = n_keys;
     *out = ks;
     return BJJ_OK;
+}
+
+int bjj_keyset_append(bjj_ctx* ctx, bjj_keyset* ks, size_t n_new, const uint8_t* ax, const uint8_t* ay, uint8_t* key_status) {
+    if (!keyset_of(ctx, ks) || n_new > 0xFFFFFFFFull - ks->n_keys) return BJJ_ERR_ARG;
+    if (n_new == 0) return BJJ_OK;
+    if (!ax || !ay) return BJJ_ERR_ARG;
+    return keyset_edit(ctx, ks, ks->n_keys, n_new, ax, ay, key_status);
+}
+
+int bjj_keyset_replace(bjj_ctx* ctx, bjj_keyset* ks, size_t first, size_t count, const uint8_t* ax, const uint8_t* ay,
+                       uint8_t* key_status) {
+    if (!keyset_of(ctx, ks) || first > ks->n_keys || count > ks->n_keys - first) return BJJ_ERR_ARG;
+    if (count == 0) return BJJ_OK;
+    if (!ax || !ay) return BJJ_ERR_ARG;
+    return keyset_edit(ctx, ks, first, count, ax, ay, key_status);
 }
 
 void bjj_keyset_destroy(bjj_ctx* ctx, bjj_keyset* ks) {
@@ -1132,8 +1337,6 @@ static bool s_words_ok(int w) { return w >= 8 && w <= BJJ_MAX_SCALAR_WORDS + 8 &
 
 // a verify_base call names its key: NULL or a handle of another context is an argument error
 static bool base_of(bjj_ctx* ctx, const bjj_base* base) { return base && base->ctx == ctx; }
-// the same for a key set
-static bool keyset_of(bjj_ctx* ctx, const bjj_keyset* ks) { return ks && ks->ctx == ctx; }
 
 static int launch_poseidon(bjj_ctx* ctx, int n_inputs, size_t n, const uint8_t* const* in, uint8_t* out,
                            cudaStream_t st) {

@@ -1866,29 +1866,53 @@ inline size_t keyset_index_slots(size_t n) {
     return c;
 }
 
-// The index of n keys with canonical affine coordinates ax, ay (32 B per key, on the host): comp receives compress(P_j)
-// (32 B per key), slots the keyset_index_slots(n) table.
-inline void keyset_index_build(size_t n, const uint8_t* ax, const uint8_t* ay, uint64_t seed, uint8_t* comp, uint32_t* slots) {
+// compress(P_j) of key j with canonical affine coordinates ax, ay (32 B per key, on the host) into out (32 B)
+inline void keyset_compress(const uint8_t* ax, const uint8_t* ay, size_t j, uint8_t* out) {
+    const uint32_t q[8] = BJJ_LIMBS8(BJJ_Q);
+    uint32_t x[8], y[8], x2[8];
+    memcpy(x, ax + 32 * j, 32);
+    memcpy(y, ay + 32 * j, 32);
+    // x > (Q-1)/2 <=> 2x >= Q (x < Q < 2^254, so 2x fits)
+    for (int k = 0; k < 8; k++) x2[k] = x[k] << 1 | (k ? x[k - 1] >> 31 : 0);
+    if (!u256_lt(x2, q)) y[7] |= 0x80000000u;
+    memcpy(out, y, 32);
+}
+
+// whether the compressed bytes c of an on-curve key go into the index: not those of (0, 1) and (0, Q-1), which are 1 and
+// Q-1 (bit 255 clear).  On the curve y = +-1 forces x = 0 (a x^2 + 1 = 1 + d x^2 with a != d), so no other key has them.
+inline bool keyset_indexed(const uint8_t* c) {
+    uint32_t y[8], one = 0, qm1 = 0;
+    const uint32_t q[8] = BJJ_LIMBS8(BJJ_Q);
+    memcpy(y, c, 32);
+    for (int k = 0; k < 8; k++) {
+        one |= y[k] ^ (k ? 0u : 1u);
+        qm1 |= y[k] ^ (k ? q[k] : q[0] - 1);
+    }
+    return one && qm1;
+}
+
+// the slots (the keyset_index_slots(n) table) of the index of n keys with compressed bytes comp (32 B per key), inserted
+// in index order so that a point held twice is found under its smallest index
+inline void keyset_index_fill(size_t n, const uint8_t* comp, uint64_t seed, uint32_t* slots) {
     const size_t mask = keyset_index_slots(n) - 1;
     for (size_t s = 0; s <= mask; s++) slots[s] = BJJ_KEY_NONE;
-    const uint32_t q[8] = BJJ_LIMBS8(BJJ_Q);
     for (size_t j = 0; j < n; j++) {
-        uint32_t x[8], y[8], x2[8];
-        memcpy(x, ax + 32 * j, 32);
-        memcpy(y, ay + 32 * j, 32);
-        // x > (Q-1)/2 <=> 2x >= Q (x < Q < 2^254, so 2x fits)
-        uint32_t any = 0;
-        for (int k = 0; k < 8; k++) {
-            x2[k] = x[k] << 1 | (k ? x[k - 1] >> 31 : 0);
-            any |= x[k];
-        }
-        if (!u256_lt(x2, q)) y[7] |= 0x80000000u;
-        memcpy(comp + 32 * j, y, 32);
-        if (!any) continue;
+        const uint8_t* c = comp + 32 * j;
+        if (!keyset_indexed(c)) continue;
+        uint32_t y[8];
+        memcpy(y, c, 32);
         size_t s = keyset_hash(y, seed) & mask;
-        while (slots[s] != BJJ_KEY_NONE && memcmp(comp + 32 * (size_t)slots[s], y, 32) != 0) s = (s + 1) & mask;
+        while (slots[s] != BJJ_KEY_NONE && memcmp(comp + 32 * (size_t)slots[s], c, 32) != 0) s = (s + 1) & mask;
         if (slots[s] == BJJ_KEY_NONE) slots[s] = (uint32_t)j;
     }
+}
+
+// The index of n on-curve keys with canonical affine coordinates ax, ay (32 B per key, on the host): comp receives
+// compress(P_j) (32 B per key), slots the keyset_index_slots(n) table.  bjj_keyset_append / _replace rebuild the slots
+// from the set's host copy of comp with keyset_index_fill.
+inline void keyset_index_build(size_t n, const uint8_t* ax, const uint8_t* ay, uint64_t seed, uint8_t* comp, uint32_t* slots) {
+    for (size_t j = 0; j < n; j++) keyset_compress(ax, ay, j, comp + 32 * j);
+    keyset_index_fill(n, comp, seed, slots);
 }
 
 // key_index[i] = the key whose compressed bytes equal pk32[i], or BJJ_KEY_NONE: hash, then probe linearly to an empty

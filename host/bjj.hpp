@@ -445,6 +445,22 @@ class KeySet {
         n_ = n;
     }
     ~KeySet() { bjj_keyset_destroy(e_.ctx(), ks_); }
+
+    // adds keys under the indices size() ..; existing indices keep their keys.  Throws Error with the constructor's
+    // codes, and the set is then unchanged (key_status, when given, receives one BJJ_KEY_* code per new key).
+    void append(const std::vector<Point>& keys, std::vector<uint8_t>* key_status = nullptr) {
+        edit(keys, key_status, [&](const uint8_t* ax, const uint8_t* ay, uint8_t* st) {
+            return bjj_keyset_append(e_.ctx(), ks_, keys.size(), ax, ay, st);
+        }, "bjj_keyset_append");
+        n_ += keys.size();
+    }
+    // gives keys first .. first + keys.size() - 1 new coordinates (key rotation); BJJ_ERR_ARG when the range runs past
+    // the set.  On an error the set is unchanged.
+    void replace(size_t first, const std::vector<Point>& keys, std::vector<uint8_t>* key_status = nullptr) {
+        edit(keys, key_status, [&](const uint8_t* ax, const uint8_t* ay, uint8_t* st) {
+            return bjj_keyset_replace(e_.ctx(), ks_, first, keys.size(), ax, ay, st);
+        }, "bjj_keyset_replace");
+    }
     KeySet(const KeySet&) = delete;
     KeySet& operator=(const KeySet&) = delete;
     const bjj_keyset* raw() const { return ks_; }
@@ -540,6 +556,18 @@ class KeySet {
 
   private:
     Engine& e_;
+    template <class F>
+    static void edit(const std::vector<Point>& keys, std::vector<uint8_t>* key_status, F call, const char* what) {
+        const size_t n = keys.size();
+        std::vector<uint8_t> ax(32 * n), ay(32 * n), st(n);
+        for (size_t i = 0; i < n; i++) {
+            std::memcpy(&ax[32 * i], keys[i].x.data(), 32);
+            std::memcpy(&ay[32 * i], keys[i].y.data(), 32);
+        }
+        const int rc = call(ax.data(), ay.data(), st.data());
+        if (key_status) *key_status = st;
+        Engine::check(rc, what);
+    }
     bjj_keyset* ks_ = nullptr;
     size_t n_ = 0;
 };

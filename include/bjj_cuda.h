@@ -198,6 +198,32 @@ typedef struct bjj_keyset bjj_keyset;
 int bjj_keyset_create(bjj_ctx* ctx, size_t n_keys, const uint8_t* ax, const uint8_t* ay, uint8_t* key_status,
                       bjj_keyset** out);
 void bjj_keyset_destroy(bjj_ctx* ctx, bjj_keyset* ks);   /* waits for the device, then frees; NULL is a no-op */
+/* Editing a set in place.  bjj_keyset_append adds n_new keys (SoA, 32 B per coordinate) under the indices n_keys ..
+ * n_keys + n_new - 1; bjj_keyset_replace gives keys first .. first + count - 1 new coordinates (key rotation).
+ *   - Each new key is checked as by bjj_keyset_create: key_status (may be NULL) receives one BJJ_KEY_* code per new key,
+ *     a coordinate >= Q returns BJJ_ERR_NONCANONICAL, which outranks an off-curve key's BJJ_ERR_ARG.
+ *   - All or nothing: on any error the set is unchanged (size, tables, lookups), BJJ_ERR_NOMEM included, which also
+ *     clears the CUDA error.  (A CUDA fault while replace rebuilds tables in place is the exception: the device is
+ *     then unusable anyway.)
+ *   - BJJ_ERR_ARG, with nothing allocated: a NULL handle or one of another context, n_keys + n_new > 2^32 - 1
+ *     (BJJ_KEY_NONE stays reserved), first + count > n_keys (or an overflow in that sum), then a NULL ax or ay.  After
+ *     the first three checks, n_new == 0 or count == 0 returns BJJ_OK and does nothing.
+ *   - Synchronous, like create and destroy: both synchronise the device before they touch the set (_dev calls on
+ *     other streams may still read it) and return when it is ready.  The handle does not change.
+ *   - Existing indices keep their keys under append; replace changes only the replaced ones.  Afterwards every call
+ *     on the set returns byte for byte what it returns on a set created from the current key list: a point held twice
+ *     is found at its smallest index, x = 0 keys are not indexed, a replaced key's old bytes are no longer found unless
+ *     another key holds them.
+ *   - Address space: every set reserves GPU virtual address space for total device memory / 396,480 B tables
+ *     (191.5 GB on a 180 GB B200), so a process holds a few hundred sets at most (733 one-key sets were measured);
+ *     past that, bjj_keyset_create returns BJJ_ERR_NOMEM.
+ *   - Cost: the new or replaced keys only (1 + 2 * ceil(n / 511) kernel launches, as create of n keys), plus a host
+ *     rebuild of the lookup index.  The tables grow inside an address range reserved by create, so an append never
+ *     copies them: device memory peaks at the final set plus the build's scratch. */
+int bjj_keyset_append(bjj_ctx* ctx, bjj_keyset* ks, size_t n_new, const uint8_t* ax, const uint8_t* ay,
+                      uint8_t* key_status);
+int bjj_keyset_replace(bjj_ctx* ctx, bjj_keyset* ks, size_t first, size_t count, const uint8_t* ax, const uint8_t* ay,
+                       uint8_t* key_status);
 /* verify (src/lib.rs:395-412) with A = key key_index[i] of ks: byte for byte bjj_verify_batch with those keys in ax, ay
  * (msg > Q -> 0, msg == Q hashes as 0, S raw and unreduced, torsion components accepted, R8 off the curve replayed
  * literally, an R8 coordinate >= Q -> BJJ_ERR_NONCANONICAL), from two comb walks per lane like bjj_verify_base_batch */

@@ -81,6 +81,11 @@ extern "C" {
     pub fn bjj_keyset_create(ctx: *mut bjj_ctx, n_keys: usize, ax: *const u8, ay: *const u8, key_status: *mut u8,
                              out: *mut *mut bjj_keyset) -> c_int;
     pub fn bjj_keyset_destroy(ctx: *mut bjj_ctx, ks: *mut bjj_keyset);
+    // editing a set in place: all or nothing, synchronous; existing indices keep their keys under append
+    pub fn bjj_keyset_append(ctx: *mut bjj_ctx, ks: *mut bjj_keyset, n_new: usize, ax: *const u8, ay: *const u8,
+                             key_status: *mut u8) -> c_int;
+    pub fn bjj_keyset_replace(ctx: *mut bjj_ctx, ks: *mut bjj_keyset, first: usize, count: usize, ax: *const u8, ay: *const u8,
+                              key_status: *mut u8) -> c_int;
     pub fn bjj_verify_keyset_batch(ctx: *mut bjj_ctx, ks: *const bjj_keyset, n: usize, key_index: *const u32, r8x: *const u8,
                                    r8y: *const u8, s32: *const u8, msg32: *const u8, ok: *mut u8) -> c_int;
     pub fn bjj_verify_keyset_compressed_batch(ctx: *mut bjj_ctx, ks: *const bjj_keyset, n: usize, key_index: *const u32,

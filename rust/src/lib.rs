@@ -471,6 +471,30 @@ impl KeySet {
         }
         Ok(KeySet { ks })
     }
+    /// adds keys under the indices after the last; existing indices keep their keys.  `Err` as for `new`, and the set
+    /// is then unchanged
+    pub fn append(&mut self, keys: &[Point]) -> Result<(), (String, Vec<u8>)> {
+        let n = keys.len();
+        let (ax, ay) = (col(n, |i| keys[i].x), col(n, |i| keys[i].y));
+        let mut st = vec![0u8; n];
+        let rc = unsafe { ffi::bjj_keyset_append(engine().raw(), self.ks, n, ax.as_ptr(), ay.as_ptr(), st.as_mut_ptr()) };
+        if rc != ffi::BJJ_OK {
+            return Err((format!("bjj_keyset_append failed: {}", err_str(rc)), st));
+        }
+        Ok(())
+    }
+    /// gives keys `first ..` new coordinates (key rotation).  `Err` as for `new` or for a range past the set, and the
+    /// set is then unchanged
+    pub fn replace(&mut self, first: usize, keys: &[Point]) -> Result<(), (String, Vec<u8>)> {
+        let n = keys.len();
+        let (ax, ay) = (col(n, |i| keys[i].x), col(n, |i| keys[i].y));
+        let mut st = vec![0u8; n];
+        let rc = unsafe { ffi::bjj_keyset_replace(engine().raw(), self.ks, first, n, ax.as_ptr(), ay.as_ptr(), st.as_mut_ptr()) };
+        if rc != ffi::BJJ_OK {
+            return Err((format!("bjj_keyset_replace failed: {}", err_str(rc)), st));
+        }
+        Ok(())
+    }
     /// `verify(keys[key_index[i]], sigs[i], msgs[i])` (src/lib.rs:395-412) lane by lane: the results of `verify_batch`
     /// with those keys
     pub fn verify_batch(&self, key_index: &[u32], sigs: &[Signature], msgs: &[BigInt]) -> Vec<bool> {
