@@ -204,6 +204,23 @@ class Engine:
                                                  _ptr(ry)), "bjj_base_mul2_batch")
         return rx, ry
 
+    def msm_batch(self, px, py, scalars):
+        """R = sum_i k_i * P_i (include/bjj_cuda.h, bjj_msm_batch): 256-bit scalars, raw.  Returns (rx, ry, status): R's
+        coordinates as (1, 32) arrays and one BJJ_KEY_* code per point.  Raises BjjError with code 2 (BJJ_ERR_ARG) when a
+        point is off the curve or code 3 (BJJ_ERR_NONCANONICAL) for a coordinate >= Q, the status on the exception."""
+        px, py, k = _as_u8(px, 32), _as_u8(py, 32), _as_u8(scalars, 32)
+        if not len(px) == len(py) == len(k):
+            raise ValueError("px, py and scalars differ in length")
+        rx, ry = np.zeros((1, 32), np.uint8), np.zeros((1, 32), np.uint8)
+        st = np.zeros(len(px), np.uint8)
+        rc = self.lib.bjj_msm_batch(self.ctx, len(px), _ptr(px), _ptr(py), _ptr(k), _ptr(rx), _ptr(ry), _ptr(st))
+        try:
+            self._check(rc, "bjj_msm_batch")
+        except BjjError as e:
+            e.point_status = st
+            raise
+        return rx, ry, st
+
     def public_batch(self, keys):
         k = _as_u8(keys, 32)
         outs = [np.empty_like(k) for _ in range(2)]
@@ -801,6 +818,19 @@ def mul2_fixed_base_batch(p, ks, q, ls, engine=None):
     return [Point(x, y) for x, y in zip(le32_to_ints(rx), le32_to_ints(ry))]
 
 
+def msm(points, scalars, engine=None):
+    """sum_i points[i].mul_scalar(scalars[i]) as the reference's fold computes it, acc.add(P_i.mul_scalar(k_i).projective())
+    from (0 : 1 : 1), then affine() (src/lib.rs:70-131, 149-164), for on-curve points and BigInts of any size and sign:
+    the sign is dropped and wider values are reduced mod ORDER, as _base_scalar maps them.  Raises BjjError with code 2
+    (BJJ_ERR_ARG) when a point is off the curve, `point_status` on the exception naming it."""
+    eng = engine or default_engine()
+    if len(points) != len(scalars):
+        raise ValueError("points and scalars differ in length")
+    rx, ry, _ = eng.msm_batch(ints_to_le32([p.x for p in points]), ints_to_le32([p.y for p in points]),
+                              ints_to_le32([_base_scalar(k) for k in scalars]))
+    return Point(le32_to_ints(rx)[0], le32_to_ints(ry)[0])
+
+
 def public_batch(keys, engine=None):
     eng = engine or default_engine()
     rx, ry = eng.public_batch(np.frombuffer(b"".join(bytes(k.key if isinstance(k, PrivateKey) else k) for k in keys),
@@ -1060,6 +1090,21 @@ class MultiEngine:
         self._check(self.lib.bjj_multi_mul_scalar_batch(self.handle, len(px), _ptr(px), _ptr(py), _ptr(k), _ptr(rx), _ptr(ry)),
                     "bjj_multi_mul_scalar_batch")
         return rx, ry
+
+    def msm_batch(self, px, py, scalars):
+        """Engine.msm_batch over the devices: each sums its shard, device slot 0 sums the partial sums"""
+        px, py, k = _as_u8(px, 32), _as_u8(py, 32), _as_u8(scalars, 32)
+        if not len(px) == len(py) == len(k):
+            raise ValueError("px, py and scalars differ in length")
+        rx, ry = np.zeros((1, 32), np.uint8), np.zeros((1, 32), np.uint8)
+        st = np.zeros(len(px), np.uint8)
+        rc = self.lib.bjj_multi_msm_batch(self.handle, len(px), _ptr(px), _ptr(py), _ptr(k), _ptr(rx), _ptr(ry), _ptr(st))
+        try:
+            self._check(rc, "bjj_multi_msm_batch")
+        except BjjError as e:
+            e.point_status = st
+            raise
+        return rx, ry, st
 
     def public_batch(self, keys, out=None):
         keys = _as_u8(keys, 32)

@@ -51,6 +51,7 @@ SIGNATURES = {
     "bjj_base_destroy": (None, [_ctx, _base]),
     "bjj_base_mul_batch": (_int, [_ctx, _base, _sz] + [_u8p] * 3),
     "bjj_base_mul2_batch": (_int, [_ctx, _base, _base, _sz] + [_u8p] * 4),
+    "bjj_msm_batch": (_int, [_ctx, _sz] + [_u8p] * 6),
     "bjj_verify_base_batch": (_int, [_ctx, _base, _sz] + [_u8p] * 5),
     "bjj_verify_base_compressed_batch": (_int, [_ctx, _base, _sz] + [_u8p] * 4),
     "bjj_keyset_create": (_int, [_ctx, _sz, _u8p, _u8p, _u8p, ctypes.POINTER(_keyset)]),
@@ -91,6 +92,7 @@ SIGNATURES.update({
     "bjj_multi_verify_batch": (_int, [_multi, _sz] + [_u8p] * 7),
     "bjj_multi_verify_compressed_batch": (_int, [_multi, _sz] + [_u8p] * 5),
     "bjj_multi_mul_scalar_batch": (_int, [_multi, _sz] + [_u8p] * 5),
+    "bjj_multi_msm_batch": (_int, [_multi, _sz] + [_u8p] * 6),
     "bjj_multi_public_batch": (_int, [_multi, _sz] + [_u8p] * 3),
     "bjj_multi_public_compressed_batch": (_int, [_multi, _sz] + [_u8p] * 2),
     "bjj_multi_sign_compressed_batch": (_int, [_multi, _sz] + [_u8p] * 4),

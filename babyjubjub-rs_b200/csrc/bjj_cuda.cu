@@ -17,6 +17,7 @@
 
 #include "../../include/bjj_cuda.h"
 #include "kernels.h"
+#include "msm.cuh"
 
 using namespace bjj;
 
@@ -225,6 +226,26 @@ struct PipeSlot {
     size_t drain_off, drain_lanes;
 };
 
+// scratch of bjj_msm_batch, grown on demand: per sub-batch of points the Niels entries and the pairs (two key and two
+// value arrays of WINDOWS x points entries, the sort's double buffers) with the sort's temporary storage, the boundary
+// lists of the accumulate levels (a uint32 key and a 128-byte point per slot, two ping-pong buffers); per call the
+// buckets (WINDOWS x 2^(c-1) points of 128 B: 71 MB at c = 16), the segment and window sums, the flags word of the call
+// and the 64-byte result of the host flavour
+struct MsmWork {
+    CombEntry* niels;
+    size_t niels_cap;
+    uint32_t* pairs;
+    size_t pairs_cap;
+    uint8_t* sort_temp;
+    size_t sort_temp_cap;
+    uint8_t* bound[2];
+    size_t bound_cap[2];
+    uint8_t* status;         // the point_status of a call that passes NULL
+    size_t status_cap;
+    uint8_t* sums;           // buckets, then segment results, then window sums, then the flags word and the result
+    size_t sums_cap;
+};
+
 struct bjj_ctx {
     int device;
     int sms;
@@ -242,6 +263,7 @@ struct bjj_ctx {
     bool public_fused;          // BJJ_PUBLIC_FUSED=1: PrivateKey::public as ONE kernel (k_public) instead of k_scalar_key + k_fixed_base
     size_t lane_hint;           // host flavour: the largest chunk of the running call, so that lane-sized scratch is
                                 // allocated ONCE up front (a cudaFree in mid-pipeline is a device-wide synchronisation)
+    MsmWork msm;
 };
 
 // the comb table of a caller point, on the device of the context that built it, and the point's canonical affine
@@ -504,6 +526,9 @@ void bjj_destroy(bjj_ctx* ctx) {
     }
     free_workspace(&ctx->ws);
     free_workspace(&ctx->ws2);
+    for (void* p : {(void*)ctx->msm.niels, (void*)ctx->msm.pairs, (void*)ctx->msm.sort_temp, (void*)ctx->msm.bound[0],
+                    (void*)ctx->msm.bound[1], (void*)ctx->msm.status, (void*)ctx->msm.sums})
+        if (p) cudaFree(p);
     if (ctx->comb) cudaFree(ctx->comb);
     if (ctx->flags_dev) cudaFree(ctx->flags_dev);
     if (ctx->flags_host) cudaFreeHost(ctx->flags_host);
@@ -573,7 +598,7 @@ int bjj_sync(bjj_ctx* ctx) {
     CU(ctx, cudaMemsetAsync(ctx->flags_dev, 0, sizeof(uint32_t), ctx->stream));
     CU(ctx, cudaStreamSynchronize(ctx->stream));
     uint32_t f = *ctx->flags_host;
-    if (f & BJJ_FLAG_KEY_INDEX) return BJJ_ERR_ARG;
+    if (f & (BJJ_FLAG_KEY_INDEX | BJJ_FLAG_OFF_CURVE)) return BJJ_ERR_ARG;
     if (f & BJJ_FLAG_NONCANONICAL) return BJJ_ERR_NONCANONICAL;
     return BJJ_OK;
 }
@@ -1062,6 +1087,129 @@ static int launch_keyset_mul(bjj_ctx* ctx, const bjj_keyset* ks, size_t n, const
         k_batch_affine<<<affine_grid(ctx, m), BJJ_BLOCK, 0, st>>>(m, scr, rx + o, ry + o);
         return launched(ctx);
     });
+}
+// ---- bjj_msm_batch (msm.cuh): begin (clear the buckets), the points in sub-batches, end (reduce, finish) ----------------
+// Window width c from n.  c = 16 has 16 + 1 windows against 32 + 1 (half the additions per point) but 2^15 buckets per
+// window against 2^7, whose reduction costs the same at any n.  BJJ_MSM_C16_POINTS is the measured crossover (B200,
+// 1000 W, profiles/r10_msm.json): c = 8 against c = 16 took 2.26 / 2.30 ms at 2^14 points, 4.74 / 4.80 ms at 2^19,
+// 7.60 / 5.86 ms at 2^20 and 13.19 / 10.25 ms at 2^21.  BJJ_MSM_BITS=8 / 16 forces a width (A/B runs of tools/bench_msm.py).
+#define BJJ_MSM_C16_POINTS ((size_t)1 << 20)
+#define BJJ_MSM_SUBBATCH ((size_t)1 << 20)      // points per prepare / sort / accumulate pass
+#define BJJ_MSM_MAX_LEVELS 16
+static int msm_window_bits(size_t n) {
+    static const int forced = env_int("BJJ_MSM_BITS", 0);
+    if (forced == 8 || forced == 16) return forced;
+    return n < BJJ_MSM_C16_POINTS ? 8 : 16;
+}
+
+// grow() for bjj_msm_batch's scratch: a failed allocation is BJJ_ERR_NOMEM, with the CUDA error cleared
+template <class T>
+static int msm_grow(bjj_ctx* ctx, T** buf, size_t* cap, size_t want, size_t unit) {
+    const int rc = grow(ctx, buf, cap, want, unit);
+    if (rc == BJJ_ERR_CUDA && ctx->last == cudaErrorMemoryAllocation) {
+        cudaGetLastError();
+        ctx->last = cudaSuccess;
+        return BJJ_ERR_NOMEM;
+    }
+    return rc;
+}
+
+// the per-call part of the scratch: buckets, segment results, window sums, flags word, result (host flavour)
+struct MsmSums {
+    uint8_t *buckets, *seg, *wsum, *result;
+    uint32_t* flags;
+};
+static int msm_sums(bjj_ctx* ctx, int bits, MsmSums* out) {
+    const MsmGeom g = msm_geom(bits);
+    const size_t nb = g.buckets(), segs = (size_t)g.windows * (g.half / BJJ_MSM_SEG);
+    TRY(msm_grow(ctx, &ctx->msm.sums, &ctx->msm.sums_cap, 128 * (nb + segs + g.windows) + 128, 1));
+    out->buckets = ctx->msm.sums;
+    out->seg = out->buckets + 128 * nb;
+    out->wsum = out->seg + 128 * segs;
+    out->flags = (uint32_t*)(out->wsum + 128 * g.windows);
+    out->result = out->wsum + 128 * g.windows + 64;
+    return BJJ_OK;
+}
+
+// a boundary buffer of `slots` slots: the keys, then (256-byte aligned) the points
+static size_t msm_keys_bytes(size_t slots) { return (4 * slots + 255) & ~(size_t)255; }
+
+static int msm_begin(bjj_ctx* ctx, int bits, cudaStream_t st) {
+    MsmSums s;
+    TRY(msm_sums(ctx, bits, &s));
+    CU(ctx, cudaMemsetAsync(s.flags, 0, sizeof(uint32_t), st));
+    const size_t nb = msm_geom(bits).buckets();
+    bjjk::msm_clear(grid_cap(ctx, 8, nb), st, nb, s.buckets);
+    return launched(ctx);
+}
+
+// n points into the buckets: per sub-batch prepare, sort, then the accumulate levels (1 + 1 + levels launches; the radix
+// sort counts as one)
+static int launch_msm_points(bjj_ctx* ctx, size_t n, const uint8_t* px, const uint8_t* py, const uint8_t* k, uint8_t* status, int bits,
+                             cudaStream_t st) {
+    const MsmGeom g = msm_geom(bits);
+    const uint32_t nb = g.buckets();
+    int key_bits = 1;
+    while (((uint32_t)1 << key_bits) <= nb) key_bits++;
+    MsmSums s;
+    TRY(msm_sums(ctx, bits, &s));
+    MsmWork& w = ctx->msm;
+    for (size_t off = 0; off < n; off += BJJ_MSM_SUBBATCH) {
+        const size_t m = n - off < BJJ_MSM_SUBBATCH ? n - off : BJJ_MSM_SUBBATCH, pairs = m * g.windows;
+        size_t counts[BJJ_MSM_MAX_LEVELS];
+        const int levels = msm_levels(pairs, counts, BJJ_MSM_MAX_LEVELS);
+        const size_t slots0 = 2 * ((pairs + BJJ_MSM_RUN - 1) / BJJ_MSM_RUN), slots1 = levels > 1 ? 2 * ((counts[1] + BJJ_MSM_RUN - 1) / BJJ_MSM_RUN) : 2;
+        const size_t temp = bjjk::msm_sort_temp_bytes(pairs, key_bits);
+        TRY(msm_grow(ctx, &w.niels, &w.niels_cap, m, sizeof(CombEntry)));
+        TRY(msm_grow(ctx, &w.pairs, &w.pairs_cap, 4 * pairs, sizeof(uint32_t)));
+        TRY(msm_grow(ctx, &w.sort_temp, &w.sort_temp_cap, temp, 1));
+        const size_t slots[2] = {slots0, slots1};
+        for (int b = 0; b < 2; b++) TRY(msm_grow(ctx, &w.bound[b], &w.bound_cap[b], msm_keys_bytes(slots[b]) + 128 * slots[b], 1));
+        uint8_t* st_out = status ? status + off : nullptr;
+        if (!st_out) {
+            TRY(msm_grow(ctx, &w.status, &w.status_cap, m, 1));
+            st_out = w.status;
+        }
+        uint32_t* keys[2] = {w.pairs, w.pairs + pairs};
+        uint32_t* vals[2] = {w.pairs + 2 * pairs, w.pairs + 3 * pairs};
+        bjjk::msm_prepare(grid_cap(ctx, bjjk::msm_prepare_blocks_per_sm(), m), st, m, px + 32 * off, py + 32 * off, k + 32 * off, bits,
+                          w.niels, keys[0], vals[0], st_out, s.flags);
+        TRY(launched(ctx));
+        CU(ctx, bjjk::msm_sort(st, w.sort_temp, temp, keys, vals, pairs, key_bits));
+        TRY(launched(ctx));
+        // the boundary list that level l writes: bound[l & 1]
+        uint32_t* bkeys[2];
+        uint8_t* bpts[2];
+        for (int b = 0; b < 2; b++) {
+            bkeys[b] = (uint32_t*)w.bound[b];
+            bpts[b] = w.bound[b] + msm_keys_bytes(slots[b]);
+        }
+        for (int l = 0; l < levels; l++) {
+            const size_t runs = (counts[l] + BJJ_MSM_RUN - 1) / BJJ_MSM_RUN;
+            unsigned long long* work = nullptr;
+            TRY(claim_counter(ctx, &ctx->ws, st, &work));
+            if (l == 0)
+                bjjk::msm_accumulate(grid_cap(ctx, bjjk::msm_accumulate_blocks_per_sm(), runs), st, counts[0], keys[0], vals[0], w.niels, nb,
+                                     s.buckets, bkeys[0], bpts[0], work);
+            else
+                bjjk::msm_merge(grid_cap(ctx, bjjk::msm_merge_blocks_per_sm(), runs), st, counts[l], bkeys[(l - 1) & 1], bpts[(l - 1) & 1], nb,
+                                s.buckets, bkeys[l & 1], bpts[l & 1], work);
+            TRY(launched(ctx));
+        }
+    }
+    return BJJ_OK;
+}
+
+// R into (rx, ry), and the call's flags into the context's word (3 launches)
+static int msm_end(bjj_ctx* ctx, int bits, uint8_t* rx, uint8_t* ry, cudaStream_t st) {
+    const MsmGeom g = msm_geom(bits);
+    MsmSums s;
+    TRY(msm_sums(ctx, bits, &s));
+    const size_t segs = (size_t)g.windows * (g.half / BJJ_MSM_SEG);
+    bjjk::msm_bucket_reduce(grid_cap(ctx, bjjk::msm_bucket_reduce_blocks_per_sm(), segs), st, bits, s.buckets, s.seg);
+    bjjk::msm_window_sum(st, bits, s.seg, s.wsum);
+    bjjk::msm_finish(st, bits, s.wsum, s.flags, rx, ry, ctx->flags_dev);
+    return launched(ctx, 3);
 }
 static int launch_decompress(bjj_ctx* ctx, size_t n, const uint8_t* in32, uint8_t* rx, uint8_t* ry, uint8_t* status,
                              cudaStream_t st, Workspace* ws) {
@@ -1623,6 +1771,17 @@ int bjj_verify_keyset_lookup_compressed_batch_dev(bjj_ctx* ctx, const bjj_keyset
                               &ctx->ws, 0, pk32, key_index);
 }
 
+int bjj_msm_batch_dev(bjj_ctx* ctx, size_t n, const uint8_t* px, const uint8_t* py, const uint8_t* scalar32, uint8_t* rx32, uint8_t* ry32,
+                      uint8_t* point_status, void* stream) {
+    if (!ctx || !px || !py || !scalar32 || !rx32 || !ry32) return BJJ_ERR_ARG;
+    CU(ctx, cudaSetDevice(ctx->device));
+    cudaStream_t st = stream ? (cudaStream_t)stream : ctx->stream;
+    const int bits = msm_window_bits(n);
+    TRY(msm_begin(ctx, bits, st));
+    TRY(launch_msm_points(ctx, n, px, py, scalar32, point_status, bits, st));
+    return msm_end(ctx, bits, rx32, ry32, st);
+}
+
 int bjj_verify_schnorr_base_batch_dev(bjj_ctx* ctx, const bjj_base* pk, size_t n, const uint8_t* msg32, const uint8_t* rx,
                                       const uint8_t* ry, const uint8_t* s, int s_words, uint8_t* ok, uint8_t* status, void* stream) {
     if (!base_of(ctx, pk) || !s_words_ok(s_words)) return BJJ_ERR_ARG;
@@ -2092,6 +2251,30 @@ int bjj_verify_keyset_lookup_compressed_batch(bjj_ctx* ctx, const bjj_keyset* ks
         return launch_verify_base(ctx, nullptr, ks, d[5], m, nullptr, nullptr, nullptr, d[0], d[2], d[3], d[4], st, ws, 0, d[1],
                                   (uint32_t*)d[5]);
     }, /*heavy=*/true);
+}
+
+int bjj_msm_batch(bjj_ctx* ctx, size_t n, const uint8_t* px, const uint8_t* py, const uint8_t* scalar32, uint8_t* rx32, uint8_t* ry32,
+                  uint8_t* point_status) {
+    if (!ctx || !px || !py || !scalar32 || !rx32 || !ry32) return BJJ_ERR_ARG;
+    CU(ctx, cudaSetDevice(ctx->device));
+    std::vector<uint8_t> own_status;
+    if (!point_status) {
+        own_status.resize(n ? n : 1);
+        point_status = own_status.data();
+    }
+    const int bits = msm_window_bits(n);
+    TRY(msm_begin(ctx, bits, ctx->stream));
+    // every chunk adds into the same buckets; the reduction and the one inversion follow the last chunk
+    HostArg args[] = {H_IN(px, 32), H_IN(py, 32), H_IN(scalar32, 32), H_OUT(point_status, 1)};
+    TRY(run_host(ctx, n, args, 4, [&](size_t m, uint8_t** d, cudaStream_t st, Workspace*) -> int {
+        return launch_msm_points(ctx, m, d[0], d[1], d[2], d[3], bits, st);
+    }, /*heavy=*/true));
+    MsmSums s;
+    TRY(msm_sums(ctx, bits, &s));
+    TRY(msm_end(ctx, bits, s.result, s.result + 32, ctx->stream));
+    CU(ctx, cudaMemcpyAsync(rx32, s.result, 32, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(ctx, cudaMemcpyAsync(ry32, s.result + 32, 32, cudaMemcpyDeviceToHost, ctx->stream));
+    return bjj_sync(ctx);
 }
 
 int bjj_verify_schnorr_base_batch(bjj_ctx* ctx, const bjj_base* pk, size_t n, const uint8_t* msg32, const uint8_t* rx, const uint8_t* ry,

@@ -13,6 +13,8 @@
 // with caller nonces (:344-362).
 #include <cuda_runtime.h>
 
+#include <string.h>
+
 #include <condition_variable>
 #include <functional>
 #include <mutex>
@@ -225,6 +227,38 @@ int bjj_multi_decompress_batch(bjj_multi* m, size_t n, const uint8_t* in32, uint
         const size_t o = 32 * off;
         return bjj_decompress_batch(m->ctx[d], k, in32 + o, rx + o, ry + o, status + off);
     });
+}
+
+int bjj_multi_msm_batch(bjj_multi* m, size_t n, const uint8_t* px, const uint8_t* py, const uint8_t* scalar32, uint8_t* rx32,
+                        uint8_t* ry32, uint8_t* point_status) {
+    if (!m || !px || !py || !scalar32 || !rx32 || !ry32) return BJJ_ERR_ARG;
+    const size_t g = m->ctx.size();
+    std::vector<uint8_t> part(64 * g, 0);      // partial d: x at 32 d, y at 32 (g + d); an empty shard is the identity
+    for (size_t d = 0; d < g; d++) part[32 * (g + d)] = 1;
+    std::vector<int> rc(g, BJJ_OK);
+    const int rs = run_sharded(m, n, {{px, 32 * n}, {py, 32 * n}, {scalar32, 32 * n}, {point_status, point_status ? n : 0}},
+                               [&](int d, size_t off, size_t k) {
+                                   const size_t o = 32 * off;
+                                   rc[d] = bjj_msm_batch(m->ctx[d], k, px + o, py + o, scalar32 + o, &part[32 * d], &part[32 * (g + d)],
+                                                         point_status ? point_status + off : nullptr);
+                                   return BJJ_OK;
+                               });
+    if (rs != BJJ_OK) return rs;
+    // the worst outcome of the shards, ranked as bjj_sync ranks them
+    int worst = BJJ_OK;
+    for (int r : rc) {
+        if (r == BJJ_OK) continue;
+        if (r != BJJ_ERR_NONCANONICAL) {
+            memset(rx32, 0, 32);
+            memset(ry32, 0, 32);
+            return r;
+        }
+        worst = r;
+    }
+    std::vector<uint8_t> one(32 * g, 0);
+    for (size_t d = 0; d < g; d++) one[32 * d] = 1;
+    const int r0 = bjj_msm_batch(m->ctx[0], g, part.data(), part.data() + 32 * g, one.data(), rx32, ry32, nullptr);
+    return r0 != BJJ_OK ? r0 : worst;
 }
 
 }  // extern "C"

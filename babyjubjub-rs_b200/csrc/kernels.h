@@ -131,5 +131,24 @@ void verify_schnorr_keyset_ec(int grid, cudaStream_t st, size_t n, const uint8_t
                               const uint8_t* hm, uint8_t* ok, const bjj::CombEntry* comb, const uint8_t* key_index, uint32_t n_keys,
                               const bjj::CombEntry* tables, unsigned long long* work);
 int verify_schnorr_keyset_ec_blocks_per_sm();
+// the multi-scalar product sum_i k_i * P_i (k_msm.cu, pipeline in msm.cuh); `bits` is the window width c (8 or 16),
+// buckets / seg / wsum hold extended points of 128 B
+void msm_clear(int grid, cudaStream_t st, size_t nb, uint8_t* buckets);
+int msm_prepare_blocks_per_sm();
+void msm_prepare(int grid, cudaStream_t st, size_t m, const uint8_t* px, const uint8_t* py, const uint8_t* k, int bits,
+                 bjj::CombEntry* niels, uint32_t* keys, uint32_t* vals, uint8_t* status, uint32_t* mflags);
+// cub::DeviceRadixSort over the low key_bits of the keys; keys[0], vals[0] name the sorted arrays afterwards
+size_t msm_sort_temp_bytes(size_t items, int key_bits);
+cudaError_t msm_sort(cudaStream_t st, void* temp, size_t temp_bytes, uint32_t** keys, uint32_t** vals, size_t items, int key_bits);
+int msm_accumulate_blocks_per_sm();
+void msm_accumulate(int grid, cudaStream_t st, size_t count, const uint32_t* keys, const uint32_t* vals, const bjj::CombEntry* niels,
+                    uint32_t nb, uint8_t* buckets, uint32_t* out_keys, uint8_t* out_pts, unsigned long long* work);
+int msm_merge_blocks_per_sm();
+void msm_merge(int grid, cudaStream_t st, size_t count, const uint32_t* keys, const uint8_t* pts, uint32_t nb, uint8_t* buckets,
+               uint32_t* out_keys, uint8_t* out_pts, unsigned long long* work);
+int msm_bucket_reduce_blocks_per_sm();
+void msm_bucket_reduce(int grid, cudaStream_t st, int bits, const uint8_t* buckets, uint8_t* seg);
+void msm_window_sum(cudaStream_t st, int bits, const uint8_t* seg, uint8_t* wsum);
+void msm_finish(cudaStream_t st, int bits, const uint8_t* wsum, const uint32_t* mflags, uint8_t* rx, uint8_t* ry, uint32_t* gflags);
 
 }  // namespace bjjk

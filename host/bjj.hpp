@@ -218,6 +218,24 @@ inline std::vector<Point> mul_scalar_batch(const std::vector<Point>& pts, const 
     return out;
 }
 
+// sum_i pts[i].mul_scalar(scalars[i]) as ONE point: the reference's fold acc.add(P_i.mul_scalar(k_i).projective()) from
+// (0 : 1 : 1), then affine() (src/lib.rs:70-131, 149-164), by bucket accumulation on the device.  Points must be on the
+// curve: an off-curve point throws Error with BJJ_ERR_ARG.
+inline Point msm(const std::vector<Point>& pts, const std::vector<U256>& scalars, Engine& e = default_engine()) {
+    const size_t n = pts.size();
+    if (scalars.size() != n) throw Error(BJJ_ERR_ARG, "msm: points and scalars differ in length");
+    std::vector<uint8_t> px(32 * n + 32), py(32 * n + 32);     // never empty: the call takes non-NULL arrays at n == 0 too
+    for (size_t i = 0; i < n; i++) {
+        std::memcpy(&px[32 * i], pts[i].x.data(), 32);
+        std::memcpy(&py[32 * i], pts[i].y.data(), 32);
+    }
+    auto k = pack(scalars);
+    k.resize(32 * n + 32);
+    Point r;
+    Engine::check(bjj_msm_batch(e.ctx(), n, px.data(), py.data(), k.data(), r.x.data(), r.y.data(), nullptr), "bjj_msm_batch");
+    return r;
+}
+
 inline std::vector<Point> public_batch(const std::vector<PrivateKey>& keys, Engine& e = default_engine()) {
     const size_t n = keys.size();
     std::vector<uint8_t> k(32 * n), rx(32 * n), ry(32 * n);

@@ -269,6 +269,33 @@ int bjj_verify_keyset_lookup_compressed_batch_dev(bjj_ctx* ctx, const bjj_keyset
                                                   const uint8_t* pk32, const uint8_t* msg32, uint8_t* ok, uint8_t* status,
                                                   uint32_t* key_index, void* stream);
 
+/* ---- multi-scalar product: R = sum_i P_i.mul_scalar(k_i), one point for the whole batch ----------------------------
+ * The reference has no such call; its composition is the fold, in index order,
+ *     acc = (0 : 1 : 1);  for i: acc = acc.add(P_i.mul_scalar(k_i).projective());  R = acc.affine()
+ * (src/lib.rs:70-131, :149-164).  For points on the curve every P_i.mul_scalar(k_i) is the group element k_i * P_i (the
+ * order of an on-curve point divides ORDER, so the raw 256-bit k_i serves as is: 0, values >= ORDER and points with a
+ * torsion component included) and PointProjective::add is the complete group law (a is a square, d is not), so R does
+ * not depend on how the sum is computed and these calls return the fold's bytes.  Uses: Pedersen vector commitments
+ * sum m_i * G_i, weighted sums of ElGamal ciphertexts, batch checks built from random linear combinations.
+ *   - Inputs: SoA arrays of n 32-byte little-endian values; scalars raw 256-bit and unreduced (as bjj_base_mul_batch).
+ *     Output: ONE canonical affine point, 32 bytes in rx32 and 32 in ry32 (device pointers in _dev).  n == 0 and every
+ *     cancelling sum give the identity (0, 1).
+ *   - point_status (may be NULL) gets one BJJ_KEY_* code per point.  A point off the curve (the reference's fold past
+ *     it is no group law, and no bucket method reproduces its operation sequence) makes the result (0, 0), which is no
+ *     curve point, and the call returns BJJ_ERR_ARG; _dev returns it from the next bjj_sync (BJJ_ERR_ARG outranks
+ *     BJJ_ERR_NONCANONICAL there).  A coordinate >= Q: the sum is computed mod Q and the call returns
+ *     BJJ_ERR_NONCANONICAL.  A NULL ctx, input or output pointer returns BJJ_ERR_ARG; a failed scratch allocation
+ *     BJJ_ERR_NOMEM with the CUDA error cleared.
+ *   - Device memory: a bucket array of (256/c + 1) x 2^(c-1) points of 128 B (c = 8 below 2^20 points, else 16: 71 MB)
+ *     and about 0.5 KB (c = 16) or 0.9 KB (c = 8) per point of a sub-batch of up to 2^20 points, grown on demand and
+ *     kept by the context.
+ *   - The launch count depends on n only.  The host flavour streams its chunks into the same buckets and synchronises;
+ *     _dev is asynchronous on `stream`. */
+int bjj_msm_batch(bjj_ctx* ctx, size_t n, const uint8_t* px, const uint8_t* py, const uint8_t* scalar32, uint8_t* rx32,
+                  uint8_t* ry32, uint8_t* point_status);
+int bjj_msm_batch_dev(bjj_ctx* ctx, size_t n, const uint8_t* px, const uint8_t* py, const uint8_t* scalar32, uint8_t* rx32,
+                      uint8_t* ry32, uint8_t* point_status, void* stream);
+
 /* ---- PrivateKey::public (src/lib.rs:304-306) = B8 * scalar_key(key);  scalar_key (:284-302) ------ */
 int bjj_public_batch(bjj_ctx* ctx, size_t n, const uint8_t* key32, uint8_t* rx, uint8_t* ry);
 int bjj_public_batch_dev(bjj_ctx* ctx, size_t n, const uint8_t* key32, uint8_t* rx, uint8_t* ry, void* stream);
@@ -410,6 +437,11 @@ int bjj_multi_sign_schnorr_batch(bjj_multi* m, size_t n, const uint8_t* key32, c
                                  int nonce_words, uint8_t* rx, uint8_t* ry, uint8_t* s, uint8_t* status);
 int bjj_multi_fixed_base_batch(bjj_multi* m, size_t n, const uint8_t* scalar32, uint8_t* rx, uint8_t* ry);
 int bjj_multi_decompress_batch(bjj_multi* m, size_t n, const uint8_t* in32, uint8_t* rx, uint8_t* ry, uint8_t* status);
+/* bjj_msm_batch over the devices: each sums its shard of the points, and the N partial sums are summed by bjj_msm_batch
+ * on device slot 0 with scalar 1 each (exact: the group sum).  Only those N points cross between devices, through the
+ * host.  Errors and point_status as bjj_msm_batch. */
+int bjj_multi_msm_batch(bjj_multi* m, size_t n, const uint8_t* px, const uint8_t* py, const uint8_t* scalar32, uint8_t* rx32,
+                        uint8_t* ry32, uint8_t* point_status);
 
 #ifdef __cplusplus
 }

@@ -72,6 +72,9 @@ extern "C" {
     // (k*P).projective().add((l*Q).projective()).affine() (src/lib.rs:70-131, 149-164)
     pub fn bjj_base_mul2_batch(ctx: *mut bjj_ctx, p: *const bjj_base, q: *const bjj_base, n: usize, k32: *const u8,
                                l32: *const u8, rx: *mut u8, ry: *mut u8) -> c_int;
+    // sum_i P_i.mul_scalar(k_i) (src/lib.rs:70-131, 149-164) as ONE point; point_status may be null
+    pub fn bjj_msm_batch(ctx: *mut bjj_ctx, n: usize, px: *const u8, py: *const u8, scalar32: *const u8, rx32: *mut u8,
+                         ry32: *mut u8, point_status: *mut u8) -> c_int;
     // verify (src/lib.rs:395-412) of signatures made by the one key of `pk` (NULL is an argument error here)
     pub fn bjj_verify_base_batch(ctx: *mut bjj_ctx, pk: *const bjj_base, n: usize, r8x: *const u8, r8y: *const u8,
                                  s32: *const u8, msg32: *const u8, ok: *mut u8) -> c_int;
@@ -148,6 +151,8 @@ extern "C" {
                                              ok: *mut u8, status: *mut u8) -> c_int;
     pub fn bjj_multi_mul_scalar_batch(m: *mut bjj_multi, n: usize, px: *const u8, py: *const u8, scalar32: *const u8,
                                       rx: *mut u8, ry: *mut u8) -> c_int;
+    pub fn bjj_multi_msm_batch(m: *mut bjj_multi, n: usize, px: *const u8, py: *const u8, scalar32: *const u8, rx32: *mut u8,
+                               ry32: *mut u8, point_status: *mut u8) -> c_int;
     pub fn bjj_multi_public_batch(m: *mut bjj_multi, n: usize, key32: *const u8, rx: *mut u8, ry: *mut u8) -> c_int;
     pub fn bjj_multi_public_compressed_batch(m: *mut bjj_multi, n: usize, key32: *const u8, out32: *mut u8) -> c_int;
     pub fn bjj_multi_sign_compressed_batch(m: *mut bjj_multi, n: usize, key32: *const u8, msg32: *const u8, sig64: *mut u8,

@@ -372,6 +372,21 @@ pub fn scalar_base_le32(v: &BigInt) -> [u8; 32] {
     }
 }
 
+/// `sum_i points[i].mul_scalar(scalars[i])` as the reference's fold gives it (`acc.add(P_i.mul_scalar(k_i).projective())`
+/// from (0 : 1 : 1), then `affine()`, src/lib.rs:70-131, 149-164), computed on the device by bucket accumulation.  The
+/// points must be on the curve (an off-curve point panics with BJJ_ERR_ARG); scalars are mapped as `scalar_base_le32`
+/// maps them (sign dropped, wider values reduced mod ORDER).
+pub fn msm(points: &[Point], scalars: &[BigInt]) -> Point {
+    let n = points.len();
+    assert_eq!(n, scalars.len());
+    let (px, py) = (col(n, |i| points[i].x), col(n, |i| points[i].y));
+    let k = col(n, |i| scalar_base_le32(&scalars[i]));
+    let (mut rx, mut ry) = ([0u8; 32], [0u8; 32]);
+    check(unsafe { ffi::bjj_msm_batch(engine().raw(), n, px.as_ptr(), py.as_ptr(), k.as_ptr(), rx.as_mut_ptr(), ry.as_mut_ptr(),
+                                      std::ptr::null_mut()) }, "bjj_msm_batch");
+    Point { x: rx, y: ry }
+}
+
 /// The comb table of one on-curve point P (50 MB of device memory on the process-wide engine's device, freed on drop):
 /// `P.mul_scalar(k)` for many `k` at the rate of B8's fixed-base path, and `k*P + l*Q` in one pass.  An off-curve P has
 /// no table (its reference result depends on mul_scalar's exact double-and-add order): `new` returns Err and the caller
